@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the MFCC + modulation-spectrum hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): per GPU a batch of 1024 x 10 s 16 kHz mono
 clips, 25 ms / 10 ms frames, 512-point FFT, 40 mel bands, 13 MFCC + delta +
@@ -375,6 +375,10 @@ def run_b200(args):
     ms_step = ms_total / args.steps
     value = world * CLIPS * SECONDS / (ms_step * 1e-3)
     clocks = sampler.stop()
+    # what a caller of the step receives, as the last timed step left it
+    dev_res = {"totChange": last[0]["totChange"], "mfcc": last[0]["mfcc"], "delta": last[0]["delta"], "modspec": last[1], "band_energy": last[2]}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dev_res)
     gather_ok = None
     if gather is not None:
         # the gathered block of this rank's last step must be the curve it computed
@@ -443,7 +447,6 @@ def run_b200(args):
     e2e_value = world * CLIPS * SECONDS * e2e_steps / e2e_s
     # outside the timed region: what the e2e call (14 chunks over two streams) left in host memory must be
     # bit-identical to the device-resident step
-    dev_res = {"totChange": last[0]["totChange"], "mfcc": last[0]["mfcc"], "delta": last[0]["delta"], "modspec": last[1], "band_energy": last[2]}
     e2e_verified = all(bool(torch.equal(torch.from_numpy(out[k]), dev_res[k].cpu())) for k in want)
     # raw H2D ceiling of this host for the same pinned buffer, all ranks copying at once
     h2d_buf = torch.empty_like(pcm)
@@ -673,6 +676,23 @@ def run_b200(args):
     return line
 
 
+DUMP_CLIPS = 256  # the whole step's outputs are about 180 MB; this many clips keep a dump near 45 MB
+
+
+def dump_outputs(out_dir: str, outputs: dict) -> None:
+    """Write each output of the step as ``out_dir/<name>.npy`` for the same fixed, seeded sample of clips
+    (sorted indices from ``numpy.random.default_rng(0)``), so that two builds can be compared array for array."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    rows = np.sort(np.random.default_rng(0).choice(CLIPS, DUMP_CLIPS, replace=False))
+    for name, t in outputs.items():
+        sample = t.index_select(0, torch.from_numpy(rows).to(t.device)).cpu().numpy()
+        assert sample.dtype in (np.float32, np.float64), (name, sample.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), sample)
+
+
 _GATHER_MODE = {"mode": "none"}
 
 
@@ -707,7 +727,13 @@ def main():
     ap.add_argument("--no-sustained", action="store_true", help="skip the >= 2 s sustained-clock leg")
     ap.add_argument("--no-cfg5", action="store_true", help="skip the 100k-clip corpus leg (BASELINE configs[4])")
     ap.add_argument("--corpus-clips", type=int, default=100_000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help=f"write the last timed step's outputs for {DUMP_CLIPS} fixed clips of rank 0's batch as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 path computed")
     with _StdoutToStderr():
         line = run_reference(args) if args.impl == "reference" else run_b200(args)
     if line is not None:

@@ -20,8 +20,9 @@ stub modules in ``sys.modules``:
 * ``parselmouth``, ``pyqtgraph``, ``xarray`` -> empty stubs (Praat / GUI / EMA code paths
   are outside the hot path and raise if touched).
 
-The modules are executed from where they lie under ``/root/reference`` (never copied).
-``/root/reference`` does not exist on the GPU box, so the outputs of these functions are
+The modules are executed from where they lie in the checkout of the original project at
+``reference_path`` of ``BASELINE.json``, or at ``$MMF_REFERENCE_ROOT`` when that is set (never
+copied).  That checkout is not part of this repository, so the outputs of these functions are
 committed as golden vectors (``tests/golden/ref_*.npz``, minted by
 ``tests/golden/make_ref_golden.py``); ``available()`` says whether the live reference can
 be used in the current process.
@@ -30,19 +31,30 @@ be used in the current process.
 from __future__ import annotations
 
 import importlib.util
+import json
 import os
 import sys
 import types
 
 import numpy as np
 
-REFERENCE_ROOT = os.environ.get("MMF_REFERENCE_ROOT", "/root/reference")
-_SCRIPT = os.path.join(REFERENCE_ROOT, "script")
+
+def _baseline_reference_path() -> str:
+    with open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "BASELINE.json")) as f:
+        return json.load(f)["reference_path"]
+
+
+REFERENCE_ROOT = os.environ.get("MMF_REFERENCE_ROOT") or _baseline_reference_path()
 _loaded: dict[str, types.ModuleType] = {}
 
 
+def script_dir() -> str:
+    """Where the original ``script/mfcc.py`` and ``script/calc.py`` are looked for."""
+    return os.path.join(REFERENCE_ROOT, "script")
+
+
 def available() -> bool:
-    return os.path.isfile(os.path.join(_SCRIPT, "mfcc.py")) and os.path.isfile(os.path.join(_SCRIPT, "calc.py"))
+    return os.path.isfile(os.path.join(script_dir(), "mfcc.py")) and os.path.isfile(os.path.join(script_dir(), "calc.py"))
 
 
 class _Untouchable(types.ModuleType):
@@ -144,17 +156,17 @@ def _stubs():
 
 
 def load(name: str) -> types.ModuleType:
-    """Import ``/root/reference/script/<name>.py`` (``'mfcc'`` or ``'calc'``) unmodified, with the
+    """Import ``<REFERENCE_ROOT>/script/<name>.py`` (``'mfcc'`` or ``'calc'``) unmodified, with the
     stubs visible only while its top-level imports run."""
     if name in _loaded:
         return _loaded[name]
     if not available():
-        raise FileNotFoundError(f"reference scripts not found under {_SCRIPT}")
+        raise FileNotFoundError(f"reference scripts not found under {script_dir()} (BASELINE.json reference_path; $MMF_REFERENCE_ROOT overrides it)")
     stubs = _stubs()
     saved = {k: sys.modules.get(k) for k in stubs}
     sys.modules.update(stubs)
     try:
-        spec = importlib.util.spec_from_file_location(f"_mmf_reference_{name}", os.path.join(_SCRIPT, name + ".py"))
+        spec = importlib.util.spec_from_file_location(f"_mmf_reference_{name}", os.path.join(script_dir(), name + ".py"))
         mod = importlib.util.module_from_spec(spec)
         spec.loader.exec_module(mod)
     finally:

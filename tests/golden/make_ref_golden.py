@@ -2,11 +2,12 @@
 
     python tests/golden/make_ref_golden.py
 
-Runs ``/root/reference/script/mfcc.py`` and ``/root/reference/script/calc.py`` unmodified (imported by
+Runs the original ``script/mfcc.py`` and ``script/calc.py`` unmodified, from the checkout at ``reference_path``
+of ``BASELINE.json`` (``$MMF_REFERENCE_ROOT`` overrides it; imported by
 ``oracle/ref_loader.py`` with stub modules for the five third-party packages this image lacks; the one
 arithmetic step served by a stub is ``librosa.feature.mfcc`` -> the restated chain of ``oracle.mfcc``) over
-every case of ``tests/ref_cases.py`` and stores each returned array.  ``/root/reference`` does not exist on
-the GPU box, which is why the outputs are committed.
+every case of ``tests/ref_cases.py`` and stores each returned array.  The original project is not part of
+this repository, which is why the outputs are committed.
 """
 
 import os

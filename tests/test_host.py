@@ -161,13 +161,15 @@ def test_shim_signatures(key):
 
 
 def test_reference_signatures_table_matches_reference_source():
-    """When the reference checkout is present (this container), parse it and make
+    """When the checkout of the original project is present, parse it and make
     sure the table above is what the reference really declares."""
     import ast
 
-    ref = "/root/reference/script"
-    if not os.path.isdir(ref):
-        pytest.skip("reference checkout not present on this machine")
+    from oracle import ref_loader
+
+    ref = ref_loader.script_dir()
+    if not ref_loader.available():
+        pytest.skip(f"the original project's scripts are not under {ref} (set $MMF_REFERENCE_ROOT)")
     for (modname, fn), expect in REFERENCE_SIGNATURES.items():
         tree = ast.parse(open(os.path.join(ref, modname + ".py")).read())
         node = next(n for n in ast.walk(tree) if isinstance(n, ast.FunctionDef) and n.name == fn)

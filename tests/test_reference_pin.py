@@ -1,11 +1,12 @@
 """Parity pin to the reference's OWN code.
 
-``tests/golden/ref_outputs.npz`` holds what ``/root/reference/script/mfcc.py`` and ``script/calc.py`` --
+``tests/golden/ref_outputs.npz`` holds what the original project's ``script/mfcc.py`` and ``script/calc.py`` --
 executed unmodified through ``oracle/ref_loader.py`` -- return for every case of ``tests/ref_cases.py``.
 
-* CPU (``-m "not gpu"``): the oracle restatement must reproduce those outputs bit for bit, and, when
-  ``/root/reference`` is present (this container, not the GPU box), the live reference must still produce the
-  committed vectors and raise the same exceptions as the oracle.
+* CPU (``-m "not gpu"``): the oracle restatement must reproduce those outputs bit for bit and raise the error
+  cases' exceptions, and, when the checkout of the original project is present (``reference_path`` of
+  ``BASELINE.json``, or ``$MMF_REFERENCE_ROOT``), the live reference must still produce the committed vectors and
+  raise the same exceptions as the oracle.
 * GPU (``-m gpu``): the CUDA path, through the reference-facing Python mirror and the C ABI, must match the
   reference outputs within north_star's tolerances (1e-3 absolute on curves derived from MFCCs, 1e-9 relative
   for the float64 filters and stencils, exact time axes).
@@ -39,6 +40,7 @@ def _expected(golden, name):
 
 
 ORACLE_MODS = {"mfcc": oracle, "calc": oracle}
+NO_REFERENCE = f"the original project's scripts are not under {ref_loader.script_dir()} (set $MMF_REFERENCE_ROOT)"
 
 
 def test_every_case_has_a_golden_vector(golden):
@@ -56,7 +58,7 @@ def test_oracle_reproduces_reference_outputs(name, golden):
         assert np.array_equal(g, e), (name, float(np.max(np.abs(g - e))))
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference is not present on this machine")
+@pytest.mark.skipif(not ref_loader.available(), reason=NO_REFERENCE)
 @pytest.mark.parametrize("name", list(ref_cases.CASES))
 def test_live_reference_still_produces_the_golden_vectors(name, golden):
     mods = {"mfcc": ref_loader.ref_mfcc(), "calc": ref_loader.ref_calc()}
@@ -65,8 +67,19 @@ def test_live_reference_still_produces_the_golden_vectors(name, golden):
         assert np.array_equal(g, e), name
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference is not present on this machine")
-def test_reference_modules_are_loaded_from_the_reference_tree():
+# the top-level imports of the original script/mfcc.py and script/calc.py that the loader stubs
+_REFERENCE_IMPORTS = "import librosa\nimport parselmouth\nimport pyqtgraph as pg\nimport xarray\nfrom findiff import FinDiff\n"
+
+
+def test_reference_modules_are_loaded_from_the_reference_tree(tmp_path, monkeypatch):
+    """The loader executes the scripts where they lie, with its stubs, on a stand-in tree of the reference
+    (the same imports at the top of each module) when the real checkout is not present."""
+    if not ref_loader.available():
+        (tmp_path / "script").mkdir()
+        for name in ("mfcc", "calc"):
+            (tmp_path / "script" / f"{name}.py").write_text(_REFERENCE_IMPORTS + "MFCC = librosa.feature.mfcc\n")
+        monkeypatch.setattr(ref_loader, "REFERENCE_ROOT", str(tmp_path))
+        monkeypatch.setattr(ref_loader, "_loaded", {})
     m = ref_loader.ref_mfcc()
     assert os.path.realpath(m.__file__).startswith(os.path.realpath(ref_loader.REFERENCE_ROOT))
     # the loader leaves no stub behind
@@ -77,7 +90,7 @@ def test_reference_modules_are_loaded_from_the_reference_tree():
         assert mod is None or getattr(mod, "__file__", None) is not None
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference is not present on this machine")
+@pytest.mark.skipif(not ref_loader.available(), reason=NO_REFERENCE)
 @pytest.mark.parametrize("case", ref_cases.ERROR_CASES, ids=lambda c: c[0])
 def test_oracle_raises_what_the_reference_raises(case):
     _, module, func, make_x, args, kwargs, etype, frag = case
@@ -89,6 +102,14 @@ def test_oracle_raises_what_the_reference_raises(case):
     assert type(ref_exc.value) is type(ora_exc.value)
     assert str(ref_exc.value) == str(ora_exc.value)
     assert frag in str(ref_exc.value)
+
+
+@pytest.mark.parametrize("case", ref_cases.ERROR_CASES, ids=lambda c: c[0])
+def test_oracle_raises_the_reference_error_cases(case):
+    _, module, func, make_x, args, kwargs, etype, frag = case
+    with pytest.raises(etype) as exc:
+        getattr(oracle, func)(make_x(), *args, **kwargs)
+    assert frag in str(exc.value)
 
 
 # ------------------------------------------------------------------------------------------------------------
