@@ -167,6 +167,20 @@ static int ensure_mod_tables(mmf_plan* p, int win, int nfft, const int* lo, cons
   return MMF_OK;
 }
 
+// the modulation-spectrum geometry that mmf_modspec and the host-buffer bundle accept; band edges are checked when
+// band energies are requested
+static int validate_modspec(int win, int hop, int nfft, int n_bands, const int* lo, const int* hi, bool bands) {
+  if (win < 1 || hop < 1 || nfft < win || nfft < 32 || nfft > 4096 || (nfft & (nfft - 1)))
+    return fail(MMF_ERR_UNSUPPORTED, "need 1 <= win <= nfft, nfft a power of two in [32, 4096], hop >= 1");
+  if (n_bands < 0 || n_bands > 16) return fail(MMF_ERR_UNSUPPORTED, "n_bands must be in [0, 16]");
+  if (!bands) return MMF_OK;
+  if (n_bands > 0 && (!lo || !hi)) return fail(MMF_ERR_INVALID, "band edges are NULL");
+  for (int b = 0; b < n_bands; ++b)
+    if (lo[b] < 0 || hi[b] > nfft / 2 + 1 || lo[b] > hi[b])
+      return fail(MMF_ERR_INVALID, "band bin range outside [0, nfft/2+1]");
+  return MMF_OK;
+}
+
 static int run_modspec(mmf_plan* p, const float* mfcc, int64_t n_clips, int n_coef, int64_t T, int win, int hop,
                        int nfft, float* mag, float* band, const int* lo, const int* hi, int n_bands, cudaStream_t st) {
   if (T < win) return MMF_OK;
@@ -997,16 +1011,10 @@ int mmf_modspec(mmf_plan* plan, const float* mfcc_dev, int64_t n_clips, int32_t 
                 int32_t hop, int32_t nfft, float* mag_dev, float* band_dev, const int32_t* band_lo_host,
                 const int32_t* band_hi_host, int32_t n_bands, void* stream) {
   if (!plan || !mfcc_dev) return fail(MMF_ERR_INVALID, "NULL argument");
-  if (win < 1 || hop < 1 || nfft < win || nfft < 32 || nfft > 4096 || (nfft & (nfft - 1)))
-    return fail(MMF_ERR_UNSUPPORTED, "need 1 <= win <= nfft, nfft a power of two in [32, 4096], hop >= 1");
-  if (n_bands < 0 || n_bands > 16) return fail(MMF_ERR_UNSUPPORTED, "n_bands must be in [0, 16]");
-  if (band_dev && n_bands > 0 && (!band_lo_host || !band_hi_host)) return fail(MMF_ERR_INVALID, "band edges are NULL");
+  int rc = validate_modspec(win, hop, nfft, n_bands, band_lo_host, band_hi_host, band_dev != nullptr);
+  if (rc) return rc;
   if (n_clips < 1 || n_coef < 1) return fail(MMF_ERR_INVALID, "n_clips and n_coef must be positive");
   MMF_CUDA(cudaSetDevice(plan->cfg.device));
-  if (band_dev)
-    for (int b = 0; b < n_bands; ++b)
-      if (band_lo_host[b] < 0 || band_hi_host[b] > nfft / 2 + 1 || band_lo_host[b] > band_hi_host[b])
-        return fail(MMF_ERR_INVALID, "band bin range outside [0, nfft/2+1]");
   return run_modspec(plan, mfcc_dev, n_clips, n_coef, T, win, hop, nfft, mag_dev, band_dev, band_lo_host, band_hi_host,
                      n_bands, (cudaStream_t)stream);
 }
@@ -1188,9 +1196,9 @@ static int features_host_impl(mmf_plan* plan, const void* pcm_host_v, int pcm16,
   int64_t n_win = 0;
   int nbins = 0;
   if (want_mod) {
-    if (mod->hop < 1 || mod->nfft < mod->win || mod->nfft > 4096 || (mod->nfft & (mod->nfft - 1)) || mod->n_bands < 0 ||
-        mod->n_bands > 16)
-      return fail(MMF_ERR_UNSUPPORTED, "bad modulation-spectrum parameters");
+    const int rc = validate_modspec(mod->win, mod->hop, mod->nfft, mod->n_bands, mod->band_lo, mod->band_hi,
+                                    band_host != nullptr);
+    if (rc) return rc;
     n_win = T >= mod->win ? 1 + (T - mod->win) / mod->hop : 0;
     nbins = mod->nfft / 2 + 1;
   }

@@ -6,8 +6,11 @@
 // (the MFCC tensor is small and L2 resident), mean removal with a shuffle
 // reduction over the slot, periodic Hann, zero padding to nfft, real FFT
 // (16 x R2 x R3 passes, shared-memory exchange), |X| out, and the per-band
-// energies reduced over the warp with shuffles (all slots of a warp belong to the
-// same (clip, window) pair) followed by one atomicAdd per warp and band.
+// energies reduced over the warp with shuffles.  A CTA owns one (clip, window)
+// pair at a time: slot s takes coefficients s, s + SLOTS, ... in order, each warp
+// accumulates its band sums in shared memory, and the warps' sums are added in
+// warp order -- a fixed order, so the energies depend neither on scheduling nor
+// on the batch a clip came in.
 #include <cfloat>
 #include <type_traits>
 
@@ -21,7 +24,7 @@ constexpr int kModThreads = 256;
 template <int NFFT>
 __global__ void __launch_bounds__(kModThreads)
     modspec_fast_kernel(const float* __restrict__ mfcc, int n_coef, long T, int win, int hop, long n_win, long n_pairs,
-                        int cpad, const float* __restrict__ hann, const float2* __restrict__ g_tw1,
+                        const float* __restrict__ hann, const float2* __restrict__ g_tw1,
                         const float2* __restrict__ g_tw2, float* __restrict__ mag, float* __restrict__ band,
                         const int* __restrict__ band_lo, const int* __restrict__ band_hi, int n_bands) {
   using C = FftCfg<NFFT>;
@@ -32,7 +35,8 @@ __global__ void __launch_bounds__(kModThreads)
   float2* s_tw1 = s_xb + SLOTS * C::XSTRIDE;              // [TW1]
   float2* s_tw2 = s_tw1 + C::TW1;                      // [TW2]
   __shared__ int s_blo[16], s_bhi[16];
-  const int tid = threadIdx.x, lane = tid & 31;
+  __shared__ float s_band[kModThreads / 32][16];  // per-warp band sums of the current pair
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int tau = tid % C::TPF, slot_in_block = tid / C::TPF;
   for (int i = tid; i < C::TW1; i += kModThreads) s_tw1[i] = g_tw1[i];
   for (int i = tid; i < C::TW2; i += kModThreads) s_tw2[i] = g_tw2[i];
@@ -53,16 +57,12 @@ __global__ void __launch_bounds__(kModThreads)
   float2* xb = s_xb + slot_in_block * C::XSTRIDE;
   const int nb = NFFT / 2 + 1;
   const float inv_win = 1.0f / (float)win;
-  const long n_slots = n_pairs * cpad;
-  // round the trip count up so every thread of the block runs the same number of
-  // iterations (the exchanges synchronise whole warps)
-  const long stride = (long)gridDim.x * SLOTS;
-  for (long base = (long)blockIdx.x * SLOTS; base < n_slots; base += stride) {
-    const long slot = base + slot_in_block;
-    const long pair = slot / cpad;
-    const int coef = (int)(slot - pair * cpad);
-    const bool valid = slot < n_slots && coef < n_coef;
-    const long clip = pair / n_win, j = pair - clip * n_win;
+  for (long pair = blockIdx.x; pair < n_pairs; pair += gridDim.x) {
+  const long clip = pair / n_win, j = pair - clip * n_win;
+  // every thread of the block runs the same number of iterations (the exchanges synchronise whole warps)
+  for (int c0 = 0; c0 < n_coef; c0 += SLOTS) {
+    const int coef = c0 + slot_in_block;
+    const bool valid = coef < n_coef;
     const float* src = mfcc + ((size_t)clip * n_coef + coef) * T + j * hop;
     float2 v[16];
     float sum = 0.0f;
@@ -128,18 +128,27 @@ __global__ void __launch_bounds__(kModThreads)
       for (int k = tau; k < nb; k += C::TPF) mdst[k] = sqrtf(pw[k]);
     }
     if (band != nullptr) {
-      // every slot of this warp belongs to the same (clip, window) pair (cpad is a
-      // multiple of the slots per warp); invalid slots hold zeros
+      // invalid slots hold zeros
       for (int b = 0; b < n_bands; ++b) {
         float s = 0.0f;
         for (int k = s_blo[b] + tau; k < s_bhi[b]; k += C::TPF) s += pw[k];
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-        if (lane == 0 && slot < n_slots) atomicAdd(band + pair * n_bands + b, s);
+        if (lane == 0) s_band[warp][b] = c0 == 0 ? s : s_band[warp][b] + s;
       }
     }
     __syncwarp();
   }
+  if (band != nullptr) {
+    __syncthreads();
+    if (tid < n_bands) {
+      float acc = 0.0f;
+      for (int w = 0; w < kModThreads / 32; ++w) acc += s_band[w][tid];
+      band[pair * n_bands + tid] = acc;
+    }
+    __syncthreads();  // s_band is rewritten by the next pair
+  }
+  }  // pairs
 }
 
 template <int NFFT>
@@ -149,21 +158,13 @@ static cudaError_t launch_t(const float* mfcc, long n_clips, int n_coef, long T,
   using C = FftCfg<NFFT>;
   const long n_win = 1 + (T - win) / hop;
   const long n_pairs = n_clips * n_win;
-  const int spw = 32 / C::TPF;
-  const int cpad = (n_coef + spw - 1) / spw * spw;
-  const long n_slots = n_pairs * cpad;
   const int slots = kModThreads / C::TPF;
-  long blocks = (n_slots + slots - 1) / slots;
   const long cap = (long)sm_count * 8;
-  if (blocks > cap) blocks = cap;
-  if (band != nullptr) {
-    cudaError_t e = cudaMemsetAsync(band, 0, (size_t)n_pairs * n_bands * sizeof(float), st);
-    if (e != cudaSuccess) return e;
-  }
+  const long blocks = n_pairs < cap ? n_pairs : cap;
   const size_t smem = (size_t)(slots * C::XSTRIDE + C::TW1 + C::TW2 + 1) * sizeof(float2);
   MMF_SMEM_ONCE(modspec_fast_kernel<NFFT>, 200 * 1024);
-  modspec_fast_kernel<NFFT><<<(unsigned)blocks, kModThreads, smem, st>>>(mfcc, n_coef, T, win, hop, n_win, n_pairs, cpad,
-                                                                     hann, tw1, tw2, mag, band, lo, hi, n_bands);
+  modspec_fast_kernel<NFFT><<<(unsigned)blocks, kModThreads, smem, st>>>(mfcc, n_coef, T, win, hop, n_win, n_pairs, hann,
+                                                                      tw1, tw2, mag, band, lo, hi, n_bands);
   count_launch();
   return cudaGetLastError();
 }

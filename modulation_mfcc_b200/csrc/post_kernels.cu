@@ -780,20 +780,23 @@ cudaError_t stencil_launch(const double* x, long rows, long T, const double* coe
 // time: mean removal (shuffle reduction), periodic Hann, zero padding, radix-2
 // FFT in shared memory (float64 arithmetic: magnitudes reach 1e3 and the parity
 // budget is 1e-3 absolute), |X| out, and per-band energies reduced with warp
-// shuffles into shared accumulators shared by the coefficients.
+// shuffles into per-warp shared accumulators, summed in warp order at the end so
+// that the result does not depend on which warp finishes first.
 // ---------------------------------------------------------------------------
-constexpr int kModWarps = 4;
+constexpr int kModWarps = 4;  // at most; fewer when the warps' FFT buffers would not fit (nfft 4096)
 constexpr int kMaxBands = 16;
+constexpr size_t kModSmem = 220 * 1024;
 
 __global__ void __launch_bounds__(kModWarps * 32)
     modspec_kernel(const float* __restrict__ mfcc, int n_coef, long T, int win, int hop, int nfft, int log2n,
                    long n_win, float* __restrict__ mag, float* __restrict__ band, const int* __restrict__ band_lo,
                    const int* __restrict__ band_hi, int n_bands) {
   extern __shared__ __align__(16) unsigned char sm_raw[];
+  const int n_warps = blockDim.x >> 5;
   double2* s_tw = reinterpret_cast<double2*>(sm_raw);           // [nfft/2]
-  double2* s_buf = s_tw + nfft / 2;                             // [kModWarps][nfft]
-  double* s_hann = reinterpret_cast<double*>(s_buf + kModWarps * nfft);  // [win]
-  __shared__ double s_band[kMaxBands];
+  double2* s_buf = s_tw + nfft / 2;                             // [n_warps][nfft]
+  double* s_hann = reinterpret_cast<double*>(s_buf + n_warps * nfft);  // [win]
+  __shared__ double s_band[kModWarps][kMaxBands];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const long j = blockIdx.x;   // window
   const long clip = blockIdx.y;
@@ -805,11 +808,11 @@ __global__ void __launch_bounds__(kModWarps * 32)
     s_tw[i] = make_double2(c, s);
   }
   for (int i = tid; i < win; i += blockDim.x) s_hann[i] = 0.5 - 0.5 * cospi(2.0 * (double)i / (double)win);
-  if (tid < kMaxBands) s_band[tid] = 0.0;
+  for (int i = tid; i < kModWarps * kMaxBands; i += blockDim.x) s_band[i / kMaxBands][i % kMaxBands] = 0.0;
   __syncthreads();
 
   double2* buf = s_buf + warp * nfft;
-  for (int c = warp; c < n_coef; c += kModWarps) {
+  for (int c = warp; c < n_coef; c += n_warps) {
     const float* src = mfcc + ((size_t)clip * n_coef + c) * T + j * hop;
     double sum = 0.0;
     for (int i = lane; i < win; i += 32) sum += (double)src[i];
@@ -850,13 +853,17 @@ __global__ void __launch_bounds__(kModWarps * 32)
         }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) e += __shfl_xor_sync(0xffffffffu, e, o);
-        if (lane == 0) atomicAdd(&s_band[b], e);
+        if (lane == 0) s_band[warp][b] += e;
       }
     }
     __syncwarp();
   }
   __syncthreads();
-  if (band != nullptr && tid < n_bands) band[((size_t)clip * n_win + j) * n_bands + tid] = (float)s_band[tid];
+  if (band != nullptr && tid < n_bands) {
+    double acc = 0.0;
+    for (int w = 0; w < n_warps; ++w) acc += s_band[w][tid];
+    band[((size_t)clip * n_win + j) * n_bands + tid] = (float)acc;
+  }
 }
 
 cudaError_t modspec_launch(const float* mfcc, long n_clips, int n_coef, long T, int win, int hop, int nfft, float* mag,
@@ -865,14 +872,19 @@ cudaError_t modspec_launch(const float* mfcc, long n_clips, int n_coef, long T, 
   while ((1 << log2n) < nfft) ++log2n;
   const long n_win = T >= win ? 1 + (T - win) / hop : 0;
   if (n_win <= 0) return cudaSuccess;
-  size_t smem = (size_t)(nfft / 2) * 16 + (size_t)kModWarps * nfft * 16 + (size_t)win * 8;
-  cudaError_t e = cudaFuncSetAttribute(modspec_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
+  // warps per CTA from the shared-memory budget: each holds one nfft-point complex fp64 buffer (nfft 4096: 2 warps,
+  // 192 KB)
+  const size_t fixed = (size_t)(nfft / 2) * 16 + (size_t)win * 8;
+  const size_t per_warp = (size_t)nfft * 16;
+  const int warps = fixed + kModWarps * per_warp <= kModSmem ? kModWarps : (int)((kModSmem - fixed) / per_warp);
+  const size_t smem = fixed + (size_t)warps * per_warp;
+  cudaError_t e = cudaFuncSetAttribute(modspec_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kModSmem);
   if (e != cudaSuccess) return e;
   // grid.y is limited to 65535: fold clips beyond that into several launches
   for (long c0 = 0; c0 < n_clips; c0 += 65535) {
     const long nc = n_clips - c0 < 65535 ? n_clips - c0 : 65535;
     dim3 grid((unsigned)n_win, (unsigned)nc);
-    modspec_kernel<<<grid, kModWarps * 32, smem, st>>>(
+    modspec_kernel<<<grid, warps * 32, smem, st>>>(
         mfcc + (size_t)c0 * n_coef * T, n_coef, T, win, hop, nfft, log2n, n_win,
         mag ? mag + (size_t)c0 * n_coef * n_win * (nfft / 2 + 1) : nullptr,
         band ? band + (size_t)c0 * n_win * n_bands : nullptr, band_lo_dev, band_hi_dev, n_bands);

@@ -349,7 +349,7 @@ class Plan:
         torch = _torch()
         mfcc = mfcc.contiguous()
         B, Cc, T = mfcc.shape
-        n_win = 1 + (T - win) // hop if T >= win else 0
+        n_win = 1 + (T - win) // hop if T >= win and hop >= 1 else 0
         nb = nfft // 2 + 1
         mag = torch.empty((B, Cc, n_win, nb), device=self.device, dtype=torch.float32) if want_mag else None
         band = None
@@ -360,25 +360,25 @@ class Plan:
             lo = np.ascontiguousarray([b[0] for b in band_bins], dtype=np.int32)
             hi = np.ascontiguousarray([b[1] for b in band_bins], dtype=np.int32)
             band = torch.empty((B, n_win, n_bands), device=self.device, dtype=torch.float32)
-        if n_win > 0:
-            check(
-                _lib.lib().mmf_modspec(
-                    self._h,
-                    mfcc.data_ptr(),
-                    B,
-                    Cc,
-                    T,
-                    win,
-                    hop,
-                    nfft,
-                    mag.data_ptr() if want_mag else None,
-                    band.data_ptr() if band is not None else None,
-                    lo.ctypes.data if lo is not None else None,
-                    hi.ctypes.data if hi is not None else None,
-                    n_bands,
-                    _stream_ptr(self.device),
-                )
+        # called for n_win == 0 too: the library validates the geometry (and launches nothing)
+        check(
+            _lib.lib().mmf_modspec(
+                self._h,
+                mfcc.data_ptr(),
+                B,
+                Cc,
+                T,
+                win,
+                hop,
+                nfft,
+                mag.data_ptr() if want_mag and n_win > 0 else None,
+                band.data_ptr() if band is not None and n_win > 0 else None,
+                lo.ctypes.data if lo is not None else None,
+                hi.ctypes.data if hi is not None else None,
+                n_bands,
+                _stream_ptr(self.device),
             )
+        )
         return mag, band
 
     def rms(self, pcm, frame_length: int, hop_length: int, center: bool = True):
