@@ -4,6 +4,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <cudaTypedefs.h>
 
 #include "mmf_internal.h"
@@ -23,6 +24,11 @@ static int fail(int code, const std::string& msg) {
 }
 static int cuda_fail(cudaError_t e, const char* where) {
   return fail(MMF_ERR_CUDA, std::string(where) + ": " + cudaGetErrorString(e));
+}
+static int too_short(int padlen) {
+  char buf[128];
+  std::snprintf(buf, sizeof(buf), "The length of the input vector x must be greater than padlen, which is %d.", padlen);
+  return fail(MMF_ERR_TOO_SHORT, buf);
 }
 #define MMF_CUDA(call)                                   \
   do {                                                   \
@@ -44,11 +50,15 @@ static int validate_cfg(const mmf_config* c) {
   return MMF_OK;
 }
 
-template <typename T>
-static cudaError_t upload(T** dst, const std::vector<T>& src) {
-  cudaError_t e = cudaMalloc((void**)dst, std::max<size_t>(1, src.size()) * sizeof(T));
-  if (e != cudaSuccess) return e;
-  return cudaMemcpy(*dst, src.data(), src.size() * sizeof(T), cudaMemcpyHostToDevice);
+// the only allocator of plan tables: copies `src` to new device memory that `owner` (a list of the plan) frees.  A
+// no-op once `e` holds an error, so that a run of uploads is checked once at its end.
+template <typename D, typename T>
+static void upload(cudaError_t& e, std::vector<void*>& owner, D** dst, const std::vector<T>& src) {
+  void* d = nullptr;
+  if (e != cudaSuccess || (e = cudaMalloc(&d, std::max<size_t>(1, src.size()) * sizeof(T))) != cudaSuccess) return;
+  owner.push_back(d);
+  *dst = static_cast<D*>(d);
+  e = cudaMemcpy(d, src.data(), src.size() * sizeof(T), cudaMemcpyHostToDevice);
 }
 
 static int ensure_ws(mmf_plan* p, size_t bytes) {
@@ -95,8 +105,6 @@ static int fill_sos(const double* sos, int n_sections, SosArgs* a) {
   if (n_sections < 1 || n_sections > 16) return fail(MMF_ERR_UNSUPPORTED, "n_sections must be in [1, 16]");
   std::memset(a, 0, sizeof(*a));  // (also the padding: the struct is used as a cache key)
   a->n_sections = n_sections;
-  std::memset(a->sos, 0, sizeof(a->sos));
-  std::memset(a->zi, 0, sizeof(a->zi));
   for (int s = 0; s < n_sections; ++s)
     for (int k = 0; k < 6; ++k) a->sos[s][k] = sos[6 * s + k] / (k == 3 ? 1.0 : sos[6 * s + 3]);
   double zi[32];
@@ -122,12 +130,8 @@ static int ensure_mod_tables(mmf_plan* p, int win, int nfft, const int* lo, cons
   for (int b = 0; same && b < n_bands; ++b) same = p->mod_lo[b] == lo[b] && p->mod_hi[b] == hi[b];
   if (same) return MMF_OK;
   MMF_CUDA(cudaDeviceSynchronize());
-  cudaFree(p->d_mod_hann);
-  cudaFree(p->d_mod_tw1);
-  cudaFree(p->d_mod_tw2);
-  cudaFree(p->d_mod_lo);
-  cudaFree(p->d_mod_hi);
-  cudaFree(p->d_mod_g);
+  for (void* d : p->mod_tables) cudaFree(d);
+  p->mod_tables.clear();
   p->d_mod_g = nullptr;
   p->mod_g_kp = 0;
   p->d_mod_hann = nullptr;
@@ -145,17 +149,18 @@ static int ensure_mod_tables(mmf_plan* p, int win, int nfft, const int* lo, cons
     vlo[b] = lo[b];
     vhi[b] = hi[b];
   }
-  cudaError_t e;
-  if ((e = upload(&p->d_mod_hann, hann)) != cudaSuccess || (e = upload(&p->d_mod_tw1, tw1)) != cudaSuccess ||
-      (e = upload(&p->d_mod_tw2, tw2)) != cudaSuccess || (e = upload(&p->d_mod_lo, vlo)) != cudaSuccess ||
-      (e = upload(&p->d_mod_hi, vhi)) != cudaSuccess)
-    return cuda_fail(e, "uploading modulation-spectrum tables");
+  cudaError_t e = cudaSuccess;
+  upload(e, p->mod_tables, &p->d_mod_hann, hann);
+  upload(e, p->mod_tables, &p->d_mod_tw1, tw1);
+  upload(e, p->mod_tables, &p->d_mod_tw2, tw2);
+  upload(e, p->mod_tables, &p->d_mod_lo, vlo);
+  upload(e, p->mod_tables, &p->d_mod_hi, vhi);
+  if (e != cudaSuccess) return cuda_fail(e, "uploading modulation-spectrum tables");
   if (modspec_tc_supported(win, nfft) && !(p->cfg.flags & MMF_FLAG_NO_TC_MODSPEC)) {
     std::vector<uint16_t> g;
-    uint16_t* d_g = nullptr;
     modspec_tc_table(win, nfft, g, &p->mod_g_kp);
-    if ((e = upload(&d_g, g)) != cudaSuccess) return cuda_fail(e, "uploading modulation-spectrum GEMM operand");
-    p->d_mod_g = d_g;
+    upload(e, p->mod_tables, &p->d_mod_g, g);
+    if (e != cudaSuccess) return cuda_fail(e, "uploading modulation-spectrum GEMM operand");
   }
   p->mod_win = win;
   p->mod_nfft = nfft;
@@ -207,6 +212,215 @@ static int run_modspec(mmf_plan* p, const float* mfcc, int64_t n_clips, int n_co
   return MMF_OK;
 }
 
+// ---- stages of mmf_plan_create for the register FFT (host computations only)
+
+// Tables of the mma.sync mel projection (MMF_FLAG_MMA_MEL).  An n-tile is a run of up to 8 consecutive bands (the N
+// of mma.m16n8k8); it is cut short when its bands span more than kTileBlocks k-tiles of 8 bins, so that the wide top
+// bands do not pile all their blocks on one warp.  Per tile: the k-tiles whose 8x8 block of the filterbank is not all
+// zero, and per block the B fragments (b0: k = lane%4, b1: k = lane%4 + 4; n = lane/4) as plain fp32 (split into
+// TF32 hi/lo on the fly).
+struct MmaMelTables {
+  std::vector<float2> bw;
+  std::vector<int> pk8, npair = {0}, tile;  // tile[j] = first band | bands << 16
+};
+static MmaMelTables mma_mel_tables(const std::vector<float>& mel, int n_mels, int F) {
+  MmaMelTables t;
+  const int kTileBlocks = 8;
+  auto wgt = [&](int k, int band) -> float { return (k < F && band < n_mels) ? mel[(size_t)band * F + k] : 0.0f; };
+  auto blocks_of = [&](int b0, int nb, std::vector<int>* out) {
+    int cnt = 0;
+    for (int k8 = 0; k8 < (F + 7) / 8; ++k8) {
+      bool any = false;
+      for (int k = 8 * k8; k < 8 * k8 + 8 && !any; ++k)
+        for (int b = b0; b < b0 + nb && !any; ++b) any = wgt(k, b) != 0.0f;
+      if (any) {
+        ++cnt;
+        if (out) out->push_back(k8);
+      }
+    }
+    return cnt;
+  };
+  for (int b0 = 0; b0 < n_mels;) {
+    int nb = 1;
+    while (nb < 8 && b0 + nb < n_mels && blocks_of(b0, nb + 1, nullptr) <= kTileBlocks) ++nb;
+    std::vector<int> ks;
+    blocks_of(b0, nb, &ks);
+    for (int k8 : ks) {
+      t.pk8.push_back(k8);
+      for (int lane = 0; lane < 32; ++lane) {
+        const int g = lane >> 2, t4 = lane & 3;
+        const bool own = g < nb;  // columns beyond the tile's bands belong to the next tile
+        t.bw.push_back(make_float2(own ? wgt(8 * k8 + t4, b0 + g) : 0.0f, own ? wgt(8 * k8 + t4 + 4, b0 + g) : 0.0f));
+      }
+    }
+    t.tile.push_back(b0 | (nb << 16));
+    t.npair.push_back((int)t.pk8.size());
+    b0 += nb;
+  }
+  return t;
+}
+
+struct TileGeo {
+  int tf = 0, span_bufs = 2, pt_bufs = 2, ctas = 2, threads = 256, mel_mma = 0, ppitch = 0;
+  size_t smem = 0;
+};
+
+// Tile geometry of the register-FFT kernel (tf = 0: no tile fits).  Preference: the widest tile first (32 frames =
+// one frame per lane / two MMA row tiles in the mel phase), then as much double buffering as two CTAs per SM allow
+// (<= 113 KB each: 227 KB per SM, 1 KB reserved per CTA); one CTA per SM as the last resort.  `tpf`: threads per
+// frame of the 256-thread transform; `n_pairs`, `n_tiles`: sizes of the tensor-core mel tables.
+static TileGeo choose_tile_geometry(const mmf_config& c, int tpf, int packed, int lead, int mel_groups, int mg_n,
+                                    int n_pairs, int n_tiles) {
+  const int fpw = tpf < 32 ? 32 / tpf : 1;  // frames per warp in the FFT phase
+  auto pitch_for = [&](int tf) {
+    // bin-pair layout: 8-byte words per bin-pair row; = 2 (mod 16) keeps the 32-bit stores of the two
+    // thread groups of a warp on disjoint banks (stft_core.cuh: TilePairs)
+    if (mel_groups) return std::max(tf, 2) + 2;
+    if (packed) {
+      // two-frame path: 64-bit stores of (frame, frame+1) pairs by consecutive bins:
+      // pitch == 2 (mod 4) keeps them 8-byte aligned and conflict-free per half-warp
+      int pp = std::max(tf, 2);
+      while (pp % 4 != 2) ++pp;
+      return pp;
+    }
+    int pp = std::max(tf, fpw);
+    if (fpw == 1) {
+      if ((pp & 1) == 0) ++pp;
+    } else {
+      pp = (pp + fpw - 1) / fpw * fpw;
+      if (((pp / fpw) & 1) == 0) pp += fpw;
+    }
+    return pp;
+  };
+  const size_t budget2 = 113 * 1024, budget1 = 226 * 1024;
+  static const int kBufChoices[4][2] = {{2, 2}, {1, 2}, {2, 1}, {1, 1}};  // {span_bufs, pt_bufs}
+  auto smem_for = [&](int tf, int span_bufs, int pt_bufs, int mel_mma, int threads) {
+    const int span = (tf - 1) * c.hop_length + c.n_fft + lead + 3;
+    const int alloc = (span + 255) / 256 * 256;
+    return stft_smem_bytes(c.n_fft, alloc, span_bufs, pitch_for(tf), pt_bufs, packed,
+                           stft_mel_table_bytes(c.n_fft, c.n_mels, mel_mma, n_pairs, n_tiles, mel_groups, mg_n),
+                           threads, mel_groups);
+  };
+  auto fpi_for = [&](int threads) { return (threads / tpf) * (packed ? 2 : 1); };
+  // widest tile (then most double buffering) that fits `budget` with CTAs of `threads`
+  auto fit = [&](int mel_mma, int threads, size_t budget, TileGeo* g) {
+    const int fpi = fpi_for(threads);
+    if (fpi < 1 || fpi > 32) return false;
+    for (int cand = 32; cand >= 1; cand >>= 1) {
+      if (cand < fpi || cand % fpi) continue;
+      for (const auto& ch : kBufChoices) {
+        const size_t b = smem_for(cand, ch[0], ch[1], mel_mma, threads);
+        if (b <= budget) {
+          g->tf = cand;
+          g->span_bufs = ch[0];
+          g->pt_bufs = ch[1];
+          g->smem = b;
+          g->threads = threads;
+          return true;
+        }
+      }
+    }
+    return false;
+  };
+  auto choose = [&](int mel_mma) {
+    TileGeo g;
+    g.ctas = 2;
+    if (fit(mel_mma, 256, budget2, &g)) return g;
+    g.ctas = 1;
+    // one CTA per SM: 512 threads (16 warps) when the transform groups are whole warps and the
+    // tiles still fit, else 256
+    TileGeo g512;
+    g512.ctas = 1;
+    const bool ok512 = c.n_fft >= 1024 && !mel_mma && fit(mel_mma, 512, budget1, &g512);
+    const bool ok256 = fit(mel_mma, 256, budget1, &g);
+    if (ok512 && (!ok256 || g512.tf >= g.tf) && !std::getenv("MMF_NO_512")) return g512;
+    if (!ok256) g.tf = 0;
+    return g;
+  };
+  // The tensor-core mel (MMF_FLAG_MMA_MEL) keeps its B fragments in shared memory: honoured unless
+  // that costs tile width or the second CTA per SM (very wide filterbanks).  Default is the sparse
+  // FP32 walk: the filterbank is 95-98 % zeros and the split-precision MMA path measured 3-7 %
+  // slower on every BASELINE shape (DESIGN.md section 4).
+  TileGeo gs = choose(0), gm = choose(1);
+  const bool units_fit = n_tiles * 2 <= 8 * 16 && n_tiles <= 255;
+  const int mel_mma =
+      ((c.flags & MMF_FLAG_MMA_MEL) && units_fit && gm.tf != 0 && gm.tf >= gs.tf && gm.ctas >= gs.ctas) ? 1 : 0;
+  TileGeo g = mel_mma ? gm : gs;
+  // debugging / tuning overrides
+  if (const char* e = std::getenv("MMF_TF")) {
+    const int v = std::atoi(e);
+    const int fpi = fpi_for(256);
+    g.threads = 256;
+    if (v >= fpi && v <= 32 && (v & (v - 1)) == 0 && v % fpi == 0) g.tf = v;
+    if (const char* e2 = std::getenv("MMF_SPAN_BUFS")) g.span_bufs = std::atoi(e2) == 1 ? 1 : 2;
+    if (const char* e3 = std::getenv("MMF_PT_BUFS")) g.pt_bufs = std::atoi(e3) == 1 ? 1 : 2;
+    g.smem = smem_for(g.tf, g.span_bufs, g.pt_bufs, mel_mma, 256);
+    g.ctas = g.smem <= budget2 ? 2 : 1;
+    if (g.smem > budget1) g.tf = 0;
+  }
+  g.mel_mma = mel_mma;
+  g.ppitch = pitch_for(g.tf);
+  return g;
+}
+
+// Tensor-core mel work list: unit = (n-tile, 16-frame m-tile), cost = blocks of the n-tile (npair[n + 1] -
+// npair[n]); longest-processing-time assignment to the 8 warps (each unit is produced by exactly one warp).  Fills
+// units[w * 16 + i] with (n | m << 8); false if a warp would get more than 16 units.
+static bool assign_mma_units(const std::vector<int>& npair, int tf, std::vector<int>& units_out) {
+  const int NT = (int)npair.size() - 1, MT = (tf + 15) / 16;
+  std::vector<std::pair<int, int>> units;  // (cost, n | m << 8)
+  for (int n = 0; n < NT; ++n)
+    for (int m = 0; m < MT; ++m) units.push_back({npair[n + 1] - npair[n], n | (m << 8)});
+  std::stable_sort(units.begin(), units.end(),
+                   [](const std::pair<int, int>& a, const std::pair<int, int>& b) { return a.first > b.first; });
+  long load[8] = {0};
+  int cnt[8] = {0};
+  for (const auto& u : units) {
+    int w = 0;
+    for (int i = 1; i < 8; ++i)
+      if (load[i] < load[w] || (load[i] == load[w] && cnt[i] < cnt[w])) w = i;
+    if (cnt[w] >= 16) return false;
+    units_out[w * 16 + cnt[w]++] = u.second;
+    load[w] += u.first + 2;  // + epilogue
+  }
+  return true;
+}
+
+// Mel band groups of the mel walk: `workers` contiguous runs of bands, balanced on cost = bins walked + bands
+// emitted (smallest achievable maximum, greedy fill under a binary-searched bound).  Returns the first band of each
+// worker, padded to 257 entries with n_mels.
+static std::vector<int> balance_band_split(const MelSparse& sp, const MelGroups& mg, int mel_groups, int n_mels,
+                                           int workers) {
+  std::vector<int> split(257, n_mels);
+  const int cbin = 7, cband = 48;  // measured: 7 instructions per bin, 29 per segment + 19 per band
+  const int cgroup = 14, cseg = 41;  // grouped walk (SASS count): per 4-bin weight group, per segment
+  auto group_cost = [&](int a, int b) -> long {  // bands [a, b): segments a..b
+    if (mel_groups) return (long)cgroup * (mg.segtab[2 * (b + 1) + 1] - mg.segtab[2 * a + 1]) + (long)cseg * (b - a + 1);
+    return cbin * (sp.seg_start[b + 1] - sp.seg_start[a]) + cband * (b - a);
+  };
+  auto fill = [&](long bound, std::vector<int>* out) {
+    int a = 0, used = 0;
+    while (a < n_mels) {
+      if (used == workers) return false;
+      int b = a + 1;
+      if (group_cost(a, b) > bound) return false;
+      while (b < n_mels && group_cost(a, b + 1) <= bound) ++b;
+      if (out) (*out)[used] = a;
+      a = b;
+      ++used;
+    }
+    if (out)
+      for (int w = used; w < 257; ++w) (*out)[w] = n_mels;
+    return true;
+  };
+  long lo = 0, hi = group_cost(0, n_mels);
+  while (lo < hi) {
+    const long mid = (lo + hi) / 2;
+    if (fill(mid, nullptr)) hi = mid; else lo = mid + 1;
+  }
+  fill(lo, &split);
+  return split;
+}
 }  // namespace mmf
 
 using namespace mmf;
@@ -298,7 +512,8 @@ int mmf_plan_create(mmf_plan** out, const mmf_config* cfg) {
       pool_set[cfg->device] = true;
     }
   }
-  mmf_plan* p = new mmf_plan();
+  // every return below releases the plan and all it has allocated, except the final one
+  std::unique_ptr<mmf_plan, decltype(&mmf_plan_destroy)> p(new mmf_plan(), mmf_plan_destroy);
   p->cfg = *cfg;
   p->F = cfg->n_fft / 2 + 1;
   p->sm_count = prop.multiProcessorCount;
@@ -306,281 +521,77 @@ int mmf_plan_create(mmf_plan** out, const mmf_config* cfg) {
   // FP32 matrix-product DFT (dft_generic.cu)
   p->generic = (cfg->n_fft < 256 || (cfg->n_fft & (cfg->n_fft - 1))) ? 1 : 0;
   p->packed = (!p->generic && stft_packed_supported(cfg->n_fft) && !(cfg->flags & MMF_FLAG_SCALAR_FFT)) ? 1 : 0;
-  p->geo = StftGeometry{};
-  if (!p->generic) stft_geometry(cfg->n_fft, p->packed, 256, &p->geo);
   p->lead = cfg->preemph != 0.0f ? 2 : 0;
 
-  // ---- constant tables
+  // ---- constant tables of both transforms
   std::vector<float> window, mel, dct;
   std::vector<double> mel_f;
   host_window(cfg->win_length, cfg->n_fft, window);
   host_mel_dense(cfg->sample_rate, cfg->n_fft, cfg->n_mels, cfg->fmin, cfg->fmax, mel, mel_f);
   MelSparse sp;
-  if (!host_mel_sparse(mel, mel_f, cfg->sample_rate, cfg->n_fft, cfg->n_mels, sp)) {
-    delete p;
+  if (!host_mel_sparse(mel, mel_f, cfg->sample_rate, cfg->n_fft, cfg->n_mels, sp))
     return fail(MMF_ERR_UNSUPPORTED, "mel filterbank is not a two-slope (triangular) bank");
-  }
   host_dct(cfg->n_mfcc, cfg->n_mels, dct);
-  if (p->generic) {
-    std::vector<float> tab;
-    dft_generic_table(cfg->n_fft, window, tab, &p->dft_ld);
-    p->nc_pad = cfg->n_mfcc <= 16 ? 16 : (cfg->n_mfcc <= 32 ? 32 : (cfg->n_mfcc <= 64 ? 64 : 128));
-    std::vector<float> dct_pad((size_t)cfg->n_mels * p->nc_pad, 0.0f);
-    for (int k = 0; k < cfg->n_mfcc; ++k)
-      for (int m = 0; m < cfg->n_mels; ++m) dct_pad[(size_t)m * p->nc_pad + k] = dct[(size_t)k * cfg->n_mels + m];
-    std::vector<float2> w2(p->F);
-    for (int k = 0; k < p->F; ++k) w2[k] = make_float2(sp.w2[2 * k], sp.w2[2 * k + 1]);
-    std::vector<float4> dct_bfrag;
-    mfcc_mma_bfrag(dct.data(), cfg->n_mfcc, cfg->n_mels, dct_bfrag);
-    cudaError_t e;
-    if ((e = upload(&p->d_dft_tab, tab)) != cudaSuccess || (e = upload(&p->d_window, window)) != cudaSuccess ||
-        (e = upload(&p->d_seg, sp.seg_start)) != cudaSuccess || (e = upload(&p->d_w2, w2)) != cudaSuccess ||
-        (e = upload(&p->d_dct, dct_pad)) != cudaSuccess || (e = upload(&p->d_dct_bfrag, dct_bfrag)) != cudaSuccess) {
-      mmf_plan_destroy(p);
-      return cuda_fail(e, "uploading plan constants (generic n_fft)");
-    }
-    for (int i = 0; i < 2; ++i) cudaStreamCreateWithFlags(&p->streams[i], cudaStreamNonBlocking);
-    for (int i = 0; i < 4; ++i) cudaEventCreateWithFlags(&p->events[i], cudaEventDisableTiming);
-    *out = p;
-    return MMF_OK;
-  }
-  // grouped mel walk on the bin-pair power tile: the default; MMF_FLAG_MEL_WALK / MMF_FLAG_MMA_MEL select
-  // the [bin][frame] tile with the sparse walk / the mma.sync projection
-  MelGroups mg;
-  host_mel_groups(sp, p->F, cfg->n_mels, mg);
-  p->mel_groups = (cfg->flags & (MMF_FLAG_MEL_WALK | MMF_FLAG_MMA_MEL)) ? 0 : 1;
-  p->mg_n = mg.n_groups;
-
-  // ---- tensor-core mel tables.  An n-tile is a run of up to 8 consecutive bands (the N of
-  // mma.m16n8k8); it is cut short when its bands span more than kTileBlocks k-tiles of 8 bins, so
-  // that the wide top bands do not pile all their blocks on one warp.  Per tile: the k-tiles whose
-  // 8x8 block of the filterbank is not all zero, and per block the B fragments
-  // (b0: k = lane%4, b1: k = lane%4 + 4; n = lane/4) as plain fp32 (split into TF32 hi/lo on the fly).
-  std::vector<float2> mma_bw;
-  std::vector<int> mma_pk8, mma_npair(1, 0), mma_tile;  // mma_tile[j] = first band | bands << 16
-  {
-    const int F = p->F, kTileBlocks = 8;
-    auto wgt = [&](int k, int band) -> float {
-      return (k < F && band < cfg->n_mels) ? mel[(size_t)band * F + k] : 0.0f;
-    };
-    auto blocks_of = [&](int b0, int nb, std::vector<int>* out) {
-      int cnt = 0;
-      for (int k8 = 0; k8 < (F + 7) / 8; ++k8) {
-        bool any = false;
-        for (int k = 8 * k8; k < 8 * k8 + 8 && !any; ++k)
-          for (int b = b0; b < b0 + nb && !any; ++b) any = wgt(k, b) != 0.0f;
-        if (any) {
-          ++cnt;
-          if (out) out->push_back(k8);
-        }
-      }
-      return cnt;
-    };
-    for (int b0 = 0; b0 < cfg->n_mels;) {
-      int nb = 1;
-      while (nb < 8 && b0 + nb < cfg->n_mels && blocks_of(b0, nb + 1, nullptr) <= kTileBlocks) ++nb;
-      std::vector<int> ks;
-      blocks_of(b0, nb, &ks);
-      for (int k8 : ks) {
-        mma_pk8.push_back(k8);
-        for (int lane = 0; lane < 32; ++lane) {
-          const int g = lane >> 2, t4 = lane & 3;
-          const bool own = g < nb;  // columns beyond the tile's bands belong to the next tile
-          mma_bw.push_back(make_float2(own ? wgt(8 * k8 + t4, b0 + g) : 0.0f, own ? wgt(8 * k8 + t4 + 4, b0 + g) : 0.0f));
-        }
-      }
-      mma_tile.push_back(b0 | (nb << 16));
-      mma_npair.push_back((int)mma_pk8.size());
-      b0 += nb;
-    }
-  }
-  const int NT = (int)mma_tile.size();
-  p->mma_n_pairs = (int)mma_pk8.size();
-
-  // ---- tile geometry.  Preference: the widest tile first (32 frames = one frame per lane /
-  // two MMA row tiles in the mel phase), then as much double buffering as two CTAs per SM allow
-  // (<= 113 KB each: 227 KB per SM, 1 KB reserved per CTA); one CTA per SM as the last resort.
-  const int fpw = p->geo.tpf < 32 ? 32 / p->geo.tpf : 1;  // frames per warp in the FFT phase
-  auto pitch_for = [&](int tf) {
-    // bin-pair layout: 8-byte words per bin-pair row; = 2 (mod 16) keeps the 32-bit stores of the two
-    // thread groups of a warp on disjoint banks (stft_core.cuh: TilePairs)
-    if (p->mel_groups) return std::max(tf, 2) + 2;
-    if (p->packed) {
-      // two-frame path: 64-bit stores of (frame, frame+1) pairs by consecutive bins:
-      // pitch == 2 (mod 4) keeps them 8-byte aligned and conflict-free per half-warp
-      int pp = std::max(tf, 2);
-      while (pp % 4 != 2) ++pp;
-      return pp;
-    }
-    int pp = std::max(tf, fpw);
-    if (fpw == 1) {
-      if ((pp & 1) == 0) ++pp;
-    } else {
-      pp = (pp + fpw - 1) / fpw * fpw;
-      if (((pp / fpw) & 1) == 0) pp += fpw;
-    }
-    return pp;
-  };
-  const size_t budget2 = 113 * 1024, budget1 = 226 * 1024;
-  static const int kBufChoices[4][2] = {{2, 2}, {1, 2}, {2, 1}, {1, 1}};  // {span_bufs, pt_bufs}
-  struct Geo {
-    int tf = 0, span_bufs = 2, pt_bufs = 2, ctas = 2, threads = 256;
-    size_t smem = 0;
-  };
-  auto smem_for = [&](int tf, int span_bufs, int pt_bufs, int mel_mma, int threads) {
-    const int span = (tf - 1) * cfg->hop_length + cfg->n_fft + p->lead + 3;
-    const int alloc = (span + 255) / 256 * 256;
-    return stft_smem_bytes(cfg->n_fft, alloc, span_bufs, pitch_for(tf), pt_bufs, p->packed,
-                           stft_mel_table_bytes(cfg->n_fft, cfg->n_mels, mel_mma, p->mma_n_pairs, NT, p->mel_groups, p->mg_n),
-                           threads, p->mel_groups);
-  };
-  auto fpi_for = [&](int threads) { return (threads / p->geo.tpf) * (p->packed ? 2 : 1); };
-  // widest tile (then most double buffering) that fits `budget` with CTAs of `threads`
-  auto fit = [&](int mel_mma, int threads, size_t budget, Geo* g) {
-    const int fpi = fpi_for(threads);
-    if (fpi < 1 || fpi > 32) return false;
-    for (int cand = 32; cand >= 1; cand >>= 1) {
-      if (cand < fpi || cand % fpi) continue;
-      for (const auto& ch : kBufChoices) {
-        const size_t b = smem_for(cand, ch[0], ch[1], mel_mma, threads);
-        if (b <= budget) {
-          g->tf = cand;
-          g->span_bufs = ch[0];
-          g->pt_bufs = ch[1];
-          g->smem = b;
-          g->threads = threads;
-          return true;
-        }
-      }
-    }
-    return false;
-  };
-  auto choose = [&](int mel_mma) {
-    Geo g;
-    g.ctas = 2;
-    if (fit(mel_mma, 256, budget2, &g)) return g;
-    g.ctas = 1;
-    // one CTA per SM: 512 threads (16 warps) when the transform groups are whole warps and the
-    // tiles still fit, else 256
-    Geo g512;
-    g512.ctas = 1;
-    const bool ok512 = cfg->n_fft >= 1024 && !mel_mma && fit(mel_mma, 512, budget1, &g512);
-    const bool ok256 = fit(mel_mma, 256, budget1, &g);
-    if (ok512 && (!ok256 || g512.tf >= g.tf) && !std::getenv("MMF_NO_512")) return g512;
-    if (!ok256) g.tf = 0;
-    return g;
-  };
-  // The tensor-core mel (MMF_FLAG_MMA_MEL) keeps its B fragments in shared memory: honoured unless
-  // that costs tile width or the second CTA per SM (very wide filterbanks).  Default is the sparse
-  // FP32 walk: the filterbank is 95-98 % zeros and the split-precision MMA path measured 3-7 %
-  // slower on every BASELINE shape (DESIGN.md section 4).
-  Geo gs = choose(0), gm = choose(1);
-  const bool units_fit = NT * 2 <= 8 * 16 && NT <= 255;
-  p->mel_mma = ((cfg->flags & MMF_FLAG_MMA_MEL) && units_fit && gm.tf != 0 && gm.tf >= gs.tf &&
-                gm.ctas >= gs.ctas)
-                   ? 1
-                   : 0;
-  Geo g = p->mel_mma ? gm : gs;
-  // debugging / tuning overrides
-  if (const char* e = std::getenv("MMF_TF")) {
-    const int v = std::atoi(e);
-    const int fpi = fpi_for(256);
-    g.threads = 256;
-    if (v >= fpi && v <= 32 && (v & (v - 1)) == 0 && v % fpi == 0) g.tf = v;
-    if (const char* e2 = std::getenv("MMF_SPAN_BUFS")) g.span_bufs = std::atoi(e2) == 1 ? 1 : 2;
-    if (const char* e3 = std::getenv("MMF_PT_BUFS")) g.pt_bufs = std::atoi(e3) == 1 ? 1 : 2;
-    g.smem = smem_for(g.tf, g.span_bufs, g.pt_bufs, p->mel_mma, 256);
-    g.ctas = g.smem <= budget2 ? 2 : 1;
-    if (g.smem > budget1) g.tf = 0;
-  }
-  if (g.tf == 0) {
-    delete p;
-    return fail(MMF_ERR_UNSUPPORTED, "hop_length/n_fft combination needs more shared memory than one SM has");
-  }
-  p->threads = g.threads;
-  stft_geometry(cfg->n_fft, p->packed, p->threads, &p->geo);
-  const int tf = g.tf;
-  p->TF = tf;
-  p->pt_bufs = g.pt_bufs;
-  p->span_bufs = g.span_bufs;
-  p->ctas_per_sm = g.ctas;
-  p->ppitch = pitch_for(tf);
-  p->smem = g.smem;
-  p->mel_tab_bytes = stft_mel_table_bytes(cfg->n_fft, cfg->n_mels, p->mel_mma, p->mma_n_pairs, NT, p->mel_groups, p->mg_n);
-  p->mma_n_tiles = NT;
-
-  // ---- tensor-core mel work list: unit = (n-tile, 16-frame m-tile), cost = blocks of the n-tile;
-  // longest-processing-time assignment to the 8 warps (each unit is produced by exactly one warp)
-  std::vector<int> mma_units(8 * 16, -1);
-  if (p->mel_mma) {
-    const int MT = (tf + 15) / 16;
-    std::vector<std::pair<int, int>> units;  // (cost, n | m << 8)
-    for (int n = 0; n < NT; ++n)
-      for (int m = 0; m < MT; ++m) units.push_back({mma_npair[n + 1] - mma_npair[n], n | (m << 8)});
-    std::stable_sort(units.begin(), units.end(),
-                     [](const std::pair<int, int>& a, const std::pair<int, int>& b) { return a.first > b.first; });
-    long load[8] = {0};
-    int cnt[8] = {0};
-    for (const auto& u : units) {
-      int w = 0;
-      for (int i = 1; i < 8; ++i)
-        if (load[i] < load[w] || (load[i] == load[w] && cnt[i] < cnt[w])) w = i;
-      if (cnt[w] >= 16) {  // cannot happen with units_fit, kept as a guard
-        delete p;
-        return fail(MMF_ERR_UNSUPPORTED, "too many mel tiles per warp");
-      }
-      mma_units[w * 16 + cnt[w]++] = u.second;
-      load[w] += u.first + 2;  // + epilogue
-    }
-  }
-
-  // ---- mel band groups of the sparse FP32 walk: 8 warps * (32 / TF) workers, contiguous bands
-  // each, balanced on cost = bins walked + bands emitted (smallest achievable maximum, greedy
-  // fill under a binary-searched bound)
-  std::vector<int> band_split(257, cfg->n_mels);
-  {
-    const int workers = std::min(256, (p->threads / 32) * (32 / tf));
-    const int cbin = 7, cband = 48;  // measured: 7 instructions per bin, 29 per segment + 19 per band
-    const int cgroup = 14, cseg = 41;  // grouped walk (SASS count): per 4-bin weight group, per segment
-    auto group_cost = [&](int a, int b) -> long {  // bands [a, b): segments a..b
-      if (p->mel_groups) return (long)cgroup * (mg.segtab[2 * (b + 1) + 1] - mg.segtab[2 * a + 1]) + (long)cseg * (b - a + 1);
-      return cbin * (sp.seg_start[b + 1] - sp.seg_start[a]) + cband * (b - a);
-    };
-    auto fill = [&](long bound, std::vector<int>* out) {
-      int a = 0, used = 0;
-      while (a < cfg->n_mels) {
-        if (used == workers) return false;
-        int b = a + 1;
-        if (group_cost(a, b) > bound) return false;
-        while (b < cfg->n_mels && group_cost(a, b + 1) <= bound) ++b;
-        if (out) (*out)[used] = a;
-        a = b;
-        ++used;
-      }
-      if (out)
-        for (int w = used; w < 257; ++w) (*out)[w] = cfg->n_mels;
-      return true;
-    };
-    long lo = 0, hi = group_cost(0, cfg->n_mels);
-    while (lo < hi) {
-      const long mid = (lo + hi) / 2;
-      if (fill(mid, nullptr)) hi = mid; else lo = mid + 1;
-    }
-    fill(lo, &band_split);
-  }
-  std::vector<float2> tw1, tw2;
-  host_twiddles(cfg->n_fft, p->geo, tw1, tw2);
   p->nc_pad = cfg->n_mfcc <= 16 ? 16 : (cfg->n_mfcc <= 32 ? 32 : (cfg->n_mfcc <= 64 ? 64 : 128));
   std::vector<float> dct_pad((size_t)cfg->n_mels * p->nc_pad, 0.0f);
   for (int k = 0; k < cfg->n_mfcc; ++k)
     for (int m = 0; m < cfg->n_mels; ++m) dct_pad[(size_t)m * p->nc_pad + k] = dct[(size_t)k * cfg->n_mels + m];
   std::vector<float2> w2(p->F);
   for (int k = 0; k < p->F; ++k) w2[k] = make_float2(sp.w2[2 * k], sp.w2[2 * k + 1]);
-
   std::vector<float4> dct_bfrag;
   mfcc_mma_bfrag(dct.data(), cfg->n_mfcc, cfg->n_mels, dct_bfrag);
-  cudaError_t e;
-  {
+  const char* consts_msg = p->generic ? "uploading plan constants (generic n_fft)" : "uploading plan constants";
+  cudaError_t e = cudaSuccess;
+  upload(e, p->tables, &p->d_window, window);
+  upload(e, p->tables, &p->d_seg, sp.seg_start);
+  upload(e, p->tables, &p->d_w2, w2);
+  upload(e, p->tables, &p->d_dct, dct_pad);
+  upload(e, p->tables, &p->d_dct_bfrag, dct_bfrag);
+  if (e != cudaSuccess) return cuda_fail(e, consts_msg);
+
+  if (p->generic) {
+    std::vector<float> tab;
+    dft_generic_table(cfg->n_fft, window, tab, &p->dft_ld);
+    upload(e, p->tables, &p->d_dft_tab, tab);
+    if (e != cudaSuccess) return cuda_fail(e, consts_msg);
+  } else {
+    // grouped mel walk on the bin-pair power tile: the default; MMF_FLAG_MEL_WALK / MMF_FLAG_MMA_MEL select
+    // the [bin][frame] tile with the sparse walk / the mma.sync projection
+    MelGroups mg;
+    host_mel_groups(sp, p->F, cfg->n_mels, mg);
+    p->mel_groups = (cfg->flags & (MMF_FLAG_MEL_WALK | MMF_FLAG_MMA_MEL)) ? 0 : 1;
+    p->mg_n = mg.n_groups;
+    const MmaMelTables mma = mma_mel_tables(mel, cfg->n_mels, p->F);
+    const int NT = (int)mma.tile.size();
+    p->mma_n_pairs = (int)mma.pk8.size();
+    p->mma_n_tiles = NT;
+    StftGeometry geo{};
+    stft_geometry(cfg->n_fft, p->packed, 256, &geo);
+    const TileGeo g = choose_tile_geometry(*cfg, geo.tpf, p->packed, p->lead, p->mel_groups, p->mg_n,
+                                           p->mma_n_pairs, NT);
+    if (g.tf == 0)
+      return fail(MMF_ERR_UNSUPPORTED, "hop_length/n_fft combination needs more shared memory than one SM has");
+    p->mel_mma = g.mel_mma;
+    p->threads = g.threads;
+    p->TF = g.tf;
+    p->pt_bufs = g.pt_bufs;
+    p->span_bufs = g.span_bufs;
+    p->ctas_per_sm = g.ctas;
+    p->ppitch = g.ppitch;
+    p->smem = g.smem;
+    p->mel_tab_bytes =
+        stft_mel_table_bytes(cfg->n_fft, cfg->n_mels, p->mel_mma, p->mma_n_pairs, NT, p->mel_groups, p->mg_n);
+    stft_geometry(cfg->n_fft, p->packed, p->threads, &geo);
+
+    std::vector<int> mma_units(8 * 16, -1);  // [8 warps][16], -1 terminated
+    if (p->mel_mma && !assign_mma_units(mma.npair, p->TF, mma_units))
+      return fail(MMF_ERR_UNSUPPORTED, "too many mel tiles per warp");  // cannot happen with units_fit
+    // 8 warps * (32 / TF) workers of the mel walk
+    const std::vector<int> band_split =
+        balance_band_split(sp, mg, p->mel_groups, cfg->n_mels, std::min(256, (p->threads / 32) * (32 / p->TF)));
+    std::vector<float2> tw1, tw2;
+    host_twiddles(cfg->n_fft, geo, tw1, tw2);
+
     std::vector<int2> segtab(cfg->n_mels + 2);
     for (int j = 0; j < cfg->n_mels + 2; ++j) segtab[j] = make_int2(mg.segtab[2 * j], mg.segtab[2 * j + 1]);
     std::vector<float4> w4((size_t)2 * mg.n_groups);
@@ -588,22 +599,19 @@ int mmf_plan_create(mmf_plan** out, const mmf_config* cfg) {
     std::vector<int2> segstep(cfg->n_mels + 3);
     for (int j = 0; j < cfg->n_mels + 3; ++j)  // step in 8-byte tile words: two bin-pair rows per group
       segstep[j] = make_int2(mg.segstep[2 * j], mg.segstep[2 * j + 1] * 2 * p->ppitch);
-    if ((e = upload(&p->d_mg_seg, segtab)) != cudaSuccess || (e = upload(&p->d_mg_w, w4)) != cudaSuccess ||
-        (e = upload(&p->d_mg_step, segstep)) != cudaSuccess) {
-      mmf_plan_destroy(p);
-      return cuda_fail(e, "uploading the grouped mel tables");
-    }
-  }
-  if ((e = upload(&p->d_dct_bfrag, dct_bfrag)) != cudaSuccess || (e = upload(&p->d_window, window)) != cudaSuccess || (e = upload(&p->d_tw1, tw1)) != cudaSuccess ||
-      (e = upload(&p->d_tw2, tw2)) != cudaSuccess || (e = upload(&p->d_seg, sp.seg_start)) != cudaSuccess ||
-      (e = upload(&p->d_band_split, band_split)) != cudaSuccess ||
-      (e = upload(&p->d_mma_bw, mma_bw)) != cudaSuccess || (e = upload(&p->d_mma_pk8, mma_pk8)) != cudaSuccess ||
-      (e = upload(&p->d_mma_npair, mma_npair)) != cudaSuccess ||
-      (e = upload(&p->d_mma_tile, mma_tile)) != cudaSuccess ||
-      (e = upload(&p->d_mma_units, mma_units)) != cudaSuccess ||
-      (e = upload(&p->d_w2, w2)) != cudaSuccess || (e = upload(&p->d_dct, dct_pad)) != cudaSuccess) {
-    mmf_plan_destroy(p);
-    return cuda_fail(e, "uploading plan constants");
+    upload(e, p->tables, &p->d_mg_seg, segtab);
+    upload(e, p->tables, &p->d_mg_w, w4);
+    upload(e, p->tables, &p->d_mg_step, segstep);
+    if (e != cudaSuccess) return cuda_fail(e, "uploading the grouped mel tables");
+    upload(e, p->tables, &p->d_tw1, tw1);
+    upload(e, p->tables, &p->d_tw2, tw2);
+    upload(e, p->tables, &p->d_band_split, band_split);
+    upload(e, p->tables, &p->d_mma_bw, mma.bw);
+    upload(e, p->tables, &p->d_mma_pk8, mma.pk8);
+    upload(e, p->tables, &p->d_mma_npair, mma.npair);
+    upload(e, p->tables, &p->d_mma_tile, mma.tile);
+    upload(e, p->tables, &p->d_mma_units, mma_units);
+    if (e != cudaSuccess) return cuda_fail(e, consts_msg);
   }
 
   // mel projection as a tcgen05 GEMM (default where it applies; stft_mel_tc.cu)
@@ -611,13 +619,9 @@ int mmf_plan_create(mmf_plan** out, const mmf_config* cfg) {
       stft_mel_tc_supported(cfg->n_fft, stft_mel_tc_active_bands(mel, cfg->n_mels, p->F), cfg->hop_length, p->lead,
                             p->packed)) {
     std::vector<uint16_t> tab;
-    uint16_t* d_t = nullptr;
     stft_mel_tc_table(mel, cfg->n_mels, p->F, tab);
-    if ((e = upload(&d_t, tab)) != cudaSuccess) {
-      mmf_plan_destroy(p);
-      return cuda_fail(e, "uploading the tensor-core mel operand");
-    }
-    p->d_mel_tc = d_t;
+    upload(e, p->tables, &p->d_mel_tc, tab);
+    if (e != cudaSuccess) return cuda_fail(e, "uploading the tensor-core mel operand");
     p->mel_tc_act = stft_mel_tc_active_bands(mel, cfg->n_mels, p->F);
     // thread tau of a frame group holds samples 2 (tau + 16 n2), + 1: n2 selects a run of 32 samples
     p->win_lo = 16;
@@ -630,29 +634,21 @@ int mmf_plan_create(mmf_plan** out, const mmf_config* cfg) {
         }
     if (p->win_hi <= p->win_lo) p->win_lo = 0, p->win_hi = 16;
   }
-  if ((cfg->flags & MMF_FLAG_TC_DCT) && !(cfg->flags & MMF_FLAG_MMA_DCT) && mfcc_tc_supported(cfg->n_mfcc, cfg->n_mels)) {
+  // generic-n_fft plans keep the FP32 DCT kernel
+  if ((cfg->flags & MMF_FLAG_TC_DCT) && !(cfg->flags & MMF_FLAG_MMA_DCT) && !p->generic &&
+      mfcc_tc_supported(cfg->n_mfcc, cfg->n_mels)) {
     std::vector<uint16_t> tab;
-    uint16_t* d_t = nullptr;
     mfcc_tc_table(dct.data(), cfg->n_mfcc, cfg->n_mels, tab, &p->dct_tc_kp);
-    if ((e = upload(&d_t, tab)) != cudaSuccess) {
-      mmf_plan_destroy(p);
-      return cuda_fail(e, "uploading the tensor-core DCT operand");
-    }
-    p->d_dct_tc = d_t;
+    upload(e, p->tables, &p->d_dct_tc, tab);
+    if (e != cudaSuccess) return cuda_fail(e, "uploading the tensor-core DCT operand");
   }
   if ((cfg->flags & MMF_FLAG_TC_FFT) && tc_fft_supported(cfg->n_fft, cfg->hop_length, cfg->preemph)) {
     std::vector<uint16_t> btab;
     std::vector<float> twf;
     tc_fft_tables(btab, twf);
-    uint16_t* d_b = nullptr;
-    float* d_t = nullptr;
-    if ((e = upload(&d_b, btab)) != cudaSuccess || (e = upload(&d_t, twf)) != cudaSuccess) {
-      cudaFree(d_b);
-      mmf_plan_destroy(p);
-      return cuda_fail(e, "uploading tensor-core transform tables");
-    }
-    p->d_tc_btab = d_b;
-    p->d_tc_tw = reinterpret_cast<float2*>(d_t);
+    upload(e, p->tables, &p->d_tc_btab, btab);
+    upload(e, p->tables, &p->d_tc_tw, twf);
+    if (e != cudaSuccess) return cuda_fail(e, "uploading tensor-core transform tables");
   }
 
   // ---- driver entry point for tensor-map encoding (no link-time libcuda dependency)
@@ -661,8 +657,7 @@ int mmf_plan_create(mmf_plan** out, const mmf_config* cfg) {
   e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres);
   if (e == cudaSuccess && qres == cudaDriverEntryPointSuccess) p->encode = (PFN_cuTensorMapEncodeTiled_v12000)fn;
   for (int i = 0; i < 2; ++i) cudaStreamCreateWithFlags(&p->streams[i], cudaStreamNonBlocking);
-  for (int i = 0; i < 4; ++i) cudaEventCreateWithFlags(&p->events[i], cudaEventDisableTiming);
-  *out = p;
+  *out = p.release();
   return MMF_OK;
 }
 
@@ -670,40 +665,12 @@ int mmf_plan_destroy(mmf_plan* p) {
   if (!p) return MMF_OK;
   cudaSetDevice(p->cfg.device);
   cudaDeviceSynchronize();
-  cudaFree(p->d_window);
-  cudaFree(p->d_dft_tab);
-  cudaFree(p->d_dct_tc);
-  cudaFree(p->d_tc_btab);
-  cudaFree(p->d_tc_tw);
-  cudaFree(p->d_tw1);
-  cudaFree(p->d_tw2);
-  cudaFree(p->d_seg);
-  cudaFree(p->d_band_split);
-  cudaFree(p->d_mma_bw);
-  cudaFree(p->d_mma_pk8);
-  cudaFree(p->d_mma_npair);
-  cudaFree(p->d_mma_tile);
-  cudaFree(p->d_mma_units);
-  cudaFree(p->d_w2);
-  cudaFree(p->d_mg_seg);
-  cudaFree(p->d_mg_step);
-  cudaFree(p->d_mg_w);
-  cudaFree(p->d_dct);
-  cudaFree(p->d_mel_tc);
-  cudaFree(p->d_dct_bfrag);
+  for (void* d : p->tables) cudaFree(d);
+  for (void* d : p->mod_tables) cudaFree(d);
   cudaFree(p->ws);
   cudaFree(p->host_ws);
-  cudaFree(p->d_mod_hann);
-  cudaFree(p->d_mod_tw1);
-  cudaFree(p->d_mod_tw2);
-  cudaFree(p->d_mod_lo);
-  cudaFree(p->d_mod_hi);
-  cudaFree(p->d_mod_g);
-  if (p->pinned) cudaFreeHost(p->pinned);
-  for (int i = 0; i < 2; ++i)
-    if (p->streams[i]) cudaStreamDestroy(p->streams[i]);
-  for (int i = 0; i < 4; ++i)
-    if (p->events[i]) cudaEventDestroy(p->events[i]);
+  for (cudaStream_t s : p->streams)
+    if (s) cudaStreamDestroy(s);
   delete p;
   return MMF_OK;
 }
@@ -924,12 +891,7 @@ int mmf_sosfiltfilt(mmf_plan* plan, const void* x_dev, int32_t x_is_f32, int64_t
   SosArgs a;
   int rc = fill_sos(sos_host, n_sections, &a);
   if (rc) return rc;
-  if (T <= a.padlen) {
-    char buf[128];
-    std::snprintf(buf, sizeof(buf), "The length of the input vector x must be greater than padlen, which is %d.",
-                  a.padlen);
-    return fail(MMF_ERR_TOO_SHORT, buf);
-  }
+  if (T <= a.padlen) return too_short(a.padlen);
   MMF_CUDA(cudaSetDevice(plan->cfg.device));
   cudaError_t e = sosfiltfilt_any(x_dev, x_is_f32, rows, T, x_row_stride,
                                   (int)(rows > 0x7fffffffL ? 0x7fffffff : rows), 0, a, y_dev, y_row_stride,
@@ -967,12 +929,7 @@ int mmf_fir_filtfilt(mmf_plan* plan, const double* x_dev, int64_t rows, int64_t 
   if (!plan || !x_dev || !b_host || !y_dev || !work_dev) return fail(MMF_ERR_INVALID, "NULL argument");
   if (n_taps < 1 || n_taps > 4096) return fail(MMF_ERR_UNSUPPORTED, "n_taps must be in [1, 4096]");
   if (rows < 1 || rows > 65535) return fail(MMF_ERR_UNSUPPORTED, "rows must be in [1, 65535]");
-  if (T <= 3 * n_taps) {
-    char buf[128];
-    std::snprintf(buf, sizeof(buf), "The length of the input vector x must be greater than padlen, which is %d.",
-                  3 * n_taps);
-    return fail(MMF_ERR_TOO_SHORT, buf);
-  }
+  if (T <= 3 * n_taps) return too_short(3 * n_taps);
   MMF_CUDA(cudaSetDevice(plan->cfg.device));
   void* b_dev = nullptr;
   int rc = stage_consts(plan, b_host, (size_t)n_taps * 8, 0, &b_dev, (cudaStream_t)stream);
@@ -1050,12 +1007,6 @@ static size_t change_ws_bytes(const mmf_plan* p, int64_t n_clips, int64_t T, boo
   b += align_up((size_t)n_clips * rows * T * 8, 256);
   b += align_up((size_t)n_clips * T * 8, 256);
   return b;
-}
-
-static int too_short(int padlen) {
-  char buf[128];
-  std::snprintf(buf, sizeof(buf), "The length of the input vector x must be greater than padlen, which is %d.", padlen);
-  return fail(MMF_ERR_TOO_SHORT, buf);
 }
 
 // log-mel -> clamp -> MFCC (+delta) -> zero-phase Butterworth per coefficient ->

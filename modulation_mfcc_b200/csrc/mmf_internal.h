@@ -237,10 +237,12 @@ struct mmf_plan {
   mmf_config cfg;
   int F;
   int sm_count;
-  mmf::StftGeometry geo;
   // tile geometry
   int TF, ppitch, pt_bufs, span_bufs, ctas_per_sm, lead, packed, mel_mma, threads = 256;
   size_t smem;
+  // owners of every device table (d_*): upload() in c_api.cu allocates each one and records it here, the
+  // trajectory-FFT tables (d_mod_*) in `mod_tables` because they are rebuilt; mmf_plan_destroy frees both
+  std::vector<void*> tables, mod_tables;
   // generic n_fft: FP32 matrix-product DFT instead of the register FFT
   int generic = 0;
   float* d_dft_tab = nullptr;
@@ -290,8 +292,5 @@ struct mmf_plan {
   size_t ws_bytes = 0;
   void* host_ws = nullptr;  // workspace of the host-buffer entry points (they run on `streams`)
   size_t host_ws_bytes = 0;
-  void* pinned = nullptr;
-  size_t pinned_bytes = 0;
   cudaStream_t streams[2] = {nullptr, nullptr};
-  cudaEvent_t events[4] = {nullptr, nullptr, nullptr, nullptr};
 };

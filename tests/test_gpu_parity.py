@@ -201,6 +201,25 @@ def test_generic_n_fft_matrix_product_dft(name, cuda_device):
         assert np.array_equal(T, rT) and np.max(np.abs(tot - rtot)) < ABS_TOL
 
 
+def test_rejected_plan_leaves_the_next_plan_working(cuda_device):
+    """A hop so long that no tile of frames fits in shared memory is rejected when the plan is built. The failed
+    construction releases what it allocated, and a valid plan built next in the same process computes log-mel."""
+    cfg, secs = _cfg("cfg1_16k")
+    with pytest.raises(mm.MmfError) as ei:
+        mm.Plan(mm.plan.replace(cfg, hop_length=2000))
+    assert ei.value.code == _lib.MMF_ERR_UNSUPPORTED
+    assert ei.value.msg == "hop_length/n_fft combination needs more shared memory than one SM has"
+    y = synth_batch(12, 2, int(cfg.sample_rate * secs), cfg.sample_rate)
+    plan = mm.Plan(cfg)
+    try:
+        lm = plan.logmel(y)[0].cpu().numpy()
+    finally:
+        plan.close()
+    for i in range(y.shape[0]):
+        _, _, unclamped = _oracle_unclamped(y[i], cfg)
+        assert _mel_rel_err(lm[i], unclamped) < LOGMEL_REL
+
+
 def test_clamp_is_active_on_gui_default(cuda_device):
     """fmax above Nyquist leaves empty mel filters at -100 dB, so top_db=80 always clamps."""
     cfg, secs = _cfg("gui_default")
