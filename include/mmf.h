@@ -178,6 +178,20 @@ int mmf_mfcc_change(mmf_plan* plan, const float* pcm_dev, int64_t n_clips, int64
                     const mmf_change_params* prm, double* tot_dev, float* logmel_dev, float* mfcc_dev,
                     float* delta_dev, void* stream);
 
+/* mmf_mfcc_change for clips of different lengths in one call.  Clip i is the n_samples_host[i] samples at
+ * pcm_dev + i * clip_stride (1 <= n_samples_host[i] <= clip_stride); samples past a clip's length are never
+ * read as anything but zero, whatever the buffer holds there.  T_i = mmf_num_frames(n_samples_host[i], ...),
+ * T_max = max T_i; outputs are padded to T_max: tot_dev [n_clips, T_max], optional logmel_dev / mfcc_dev /
+ * delta_dev [n_clips, n_mels | n_mfcc, T_max].  Frames [0, T_i) of clip i are bit-identical to
+ * mmf_mfcc_change on that clip alone (n_clips = 1, n_samples = n_samples_host[i]); every element at a frame
+ * >= T_i is 0.  A clip with T_i <= padlen fails with MMF_ERR_TOO_SHORT, the message naming its index; all
+ * arguments are checked before anything is launched.  Clips on the default kernel routes run in one launch
+ * per stage for the whole batch; the others (generic n_fft, the non-default MFCC / change flags, rows longer
+ * than the fused kernel takes) run one by one. */
+int mmf_mfcc_change_varlen(mmf_plan* plan, const float* pcm_dev, int64_t n_clips, const int64_t* n_samples_host,
+                           int64_t clip_stride, const mmf_change_params* prm, double* tot_dev, float* logmel_dev,
+                           float* mfcc_dev, float* delta_dev, void* stream);
+
 /* Second half of mmf_mfcc_change, for callers that already hold the log-mel
  * (mmf_logmel): clamp -> MFCC (+delta) -> zero-phase Butterworth -> derivative +
  * norm -> output filter (script/mfcc.py:387 tail .. :425). */

@@ -27,6 +27,7 @@ from .api import (  # noqa: F401
     get_amplitude,
     get_MFCCS_change,
     get_MFCCS_change_batch,
+    get_MFCCS_change_many,
     get_velocity,
     load_channel,
     mfcc_features_batch,

@@ -179,6 +179,10 @@ _SIGNATURES = {
         C.c_int,
         [_vp, _vp, _i64, _i64, _i64, C.POINTER(mmf_change_params), _vp, _vp, _vp, _vp, _vp],
     ),
+    "mmf_mfcc_change_varlen": (
+        C.c_int,
+        [_vp, _vp, _i64, _vp, _i64, C.POINTER(mmf_change_params), _vp, _vp, _vp, _vp, _vp],
+    ),
     "mmf_mfcc_change_host": (C.c_int, [_vp, _vp, _i64, _i64, _i64, C.POINTER(mmf_change_params), _vp, _vp]),
     "mmf_change_from_logmel": (
         C.c_int,

@@ -393,25 +393,11 @@ def get_MFCCS_change_batch(
     if not isinstance(audio, torch.Tensor):
         audio = np.asarray(audio)
     _require_float_audio(audio)
-    plan = _change_setup(sigSr, tStep, winLen, n_mfcc, n_fft, minFreq, maxFreq, n_mels, preemph, device, flags)
-    cutOffNorm = filtCutoff / ((1 / tStep) / 2)  # script/mfcc.py:398
-    sos = _butter_sos(filtOrd, cutOffNorm, "low")  # script/mfcc.py:400
-    method = 0 if diffMethod == "grad" else 1
+    plan, prm, post = _change_request(
+        sigSr, tStep, winLen, n_mfcc, n_fft, minFreq, maxFreq, removeFirst, filtCutoff, filtOrd, diffMethod, outFilter,
+        outFiltType, outFiltCutOff, outFiltLen, outFiltPolyOrd, n_mels, preemph, device, flags,
+    )
     on_device = isinstance(audio, torch.Tensor) and audio.is_cuda
-
-    # output filter: None -> Goldstein's low-pass with the same sos (mfcc.py:417-421);
-    # 'iir' -> fused second sosfiltfilt; 'fir'/'sg' -> raw change, then the generic kernels
-    out_sos = None
-    post = None
-    if outFilter is None:
-        out_sos = sos
-    else:
-        # run the reference's validation up front (same exceptions, same order)
-        if outFilter == "iir":
-            out_sos = _design_iir(1 / tStep, outFiltCutOff, outFiltLen, outFiltType)
-        else:
-            post = dict(filt=outFilter, cutOff=outFiltCutOff, filtLen=outFiltLen, filtType=outFiltType, polyOrd=outFiltPolyOrd)
-    prm = make_change_params(sos, remove_first=removeFirst, diff_method=method, out_sos=out_sos)
     try:
         if not on_device and not return_features and post is None:
             a = np.asarray(audio)
@@ -437,6 +423,117 @@ def get_MFCCS_change_batch(
         res["totChange"] = tot
         return tot, T, res
     return tot, T
+
+
+def _change_request(sigSr, tStep, winLen, n_mfcc, n_fft, minFreq, maxFreq, removeFirst, filtCutoff, filtOrd, diffMethod,
+                    outFilter, outFiltType, outFiltCutOff, outFiltLen, outFiltPolyOrd, n_mels, preemph, device, flags):
+    """Plan, packed change parameters and the deferred 'fir'/'sg' output filter of one get_MFCCS_change request."""
+    plan = _change_setup(sigSr, tStep, winLen, n_mfcc, n_fft, minFreq, maxFreq, n_mels, preemph, device, flags)
+    cutOffNorm = filtCutoff / ((1 / tStep) / 2)  # script/mfcc.py:398
+    sos = _butter_sos(filtOrd, cutOffNorm, "low")  # script/mfcc.py:400
+    method = 0 if diffMethod == "grad" else 1
+
+    # output filter: None -> Goldstein's low-pass with the same sos (mfcc.py:417-421);
+    # 'iir' -> fused second sosfiltfilt; 'fir'/'sg' -> raw change, then the generic kernels
+    out_sos = None
+    post = None
+    if outFilter is None:
+        out_sos = sos
+    else:
+        # run the reference's validation up front (same exceptions, same order)
+        if outFilter == "iir":
+            out_sos = _design_iir(1 / tStep, outFiltCutOff, outFiltLen, outFiltType)
+        else:
+            post = dict(filt=outFilter, cutOff=outFiltCutOff, filtLen=outFiltLen, filtType=outFiltType, polyOrd=outFiltPolyOrd)
+    return plan, make_change_params(sos, remove_first=removeFirst, diff_method=method, out_sos=out_sos), post
+
+
+def get_MFCCS_change_many(
+    clips,
+    sigSr,
+    /,
+    *,
+    tStep=0.001,
+    winLen=0.025,
+    n_mfcc=13,
+    n_fft=512,
+    minFreq=100,
+    maxFreq=10000,
+    removeFirst=1,
+    filtCutoff=12,
+    filtOrd=6,
+    diffMethod="grad",
+    outFilter="iir",
+    outFiltType="low",
+    outFiltCutOff=[None],
+    outFiltLen=6,
+    outFiltPolyOrd=3,
+    n_mels=128,
+    preemph=0.0,
+    return_features=False,
+    device=None,
+    flags=0,
+):
+    """``get_MFCCS_change`` for a list of 1-D clips of any lengths, in one batched call.
+
+    ``clips`` holds numpy arrays and/or CUDA tensors.  Returns one ``(totChange, T)`` per clip -- or
+    ``(totChange, T, feats)`` with ``return_features`` -- equal to what ``get_MFCCS_change`` returns for that clip:
+    numpy for a numpy clip, CUDA tensors for a CUDA clip.  A clip too short for the filters raises the
+    single-clip call's exception, its message naming the clip's index."""
+    torch = _torch()
+    clips = [c if isinstance(c, torch.Tensor) else np.asarray(c) for c in clips]
+    for c in clips:
+        _require_float_audio(c)
+        if c.ndim != 1:
+            raise ValueError("get_MFCCS_change_many takes 1-D clips")
+    if not clips:
+        return []
+    plan, prm, post = _change_request(
+        sigSr, tStep, winLen, n_mfcc, n_fft, minFreq, maxFreq, removeFirst, filtCutoff, filtOrd, diffMethod, outFilter,
+        outFiltType, outFiltCutOff, outFiltLen, outFiltPolyOrd, n_mels, preemph, device, flags,
+    )
+    lengths = [int(c.shape[0]) for c in clips]
+    n_max = max(max(lengths), 1)
+    dev = plan.device
+    if all(not isinstance(c, torch.Tensor) for c in clips):  # one host->device copy of the padded batch
+        host = np.zeros((len(clips), n_max), np.float32)
+        for i, c in enumerate(clips):
+            host[i, : lengths[i]] = c
+        pcm = torch.as_tensor(host).to(dev)
+    else:
+        pcm = torch.zeros((len(clips), n_max), device=dev, dtype=torch.float32)
+        for i, c in enumerate(clips):
+            pcm[i, : lengths[i]] = c.to(dev) if isinstance(c, torch.Tensor) else torch.as_tensor(np.asarray(c, np.float32))
+    try:
+        res = plan.mfcc_change_varlen(
+            pcm, lengths, prm, want_logmel=return_features, want_mfcc=return_features, want_delta=return_features
+        )
+        frames = res.pop("frames")
+        tots = [res["totChange"][i, : frames[i]] for i in range(len(clips))]
+        if post is not None:
+            filtered = []
+            for i, t in enumerate(tots):
+                try:
+                    filtered.append(_apply_filter_dev(plan, t, 1 / tStep, **post))
+                except ValueError as e:  # a curve too short for the output filter: name the clip
+                    raise ValueError(f"clip {i}: {e}") from None
+            tots = filtered
+    except MmfError as e:
+        _raise_from(e)
+    out = []
+    for i, c in enumerate(clips):
+        on_device = isinstance(c, torch.Tensor) and c.is_cuda
+        conv = (lambda v: v) if on_device else (lambda v: v.cpu().numpy())
+        tot = tots[i]
+        T = _time_anchors(int(frames[i]), tStep, winLen)
+        tot = conv(tot) if tot is not None else None
+        if return_features:
+            feats = {k: (conv(v[i, ..., : frames[i]]) if v is not None else None) for k, v in res.items() if k != "totChange"}
+            feats["totChange"] = tot
+            out.append((tot, T, feats))
+        else:
+            out.append((tot, T))
+    return out
 
 
 def _design_iir(sr, cutOff, filtLen, filtType):

@@ -679,9 +679,10 @@ int mmf_plan_destroy(mmf_plan* p) {
 
 namespace mmf {
 
-// shared body of mmf_stft_power / mmf_logmel
+// shared body of mmf_stft_power / mmf_logmel.  vl: a variable-length batch (log-mel only, power-of-two n_fft) of
+// clips of at most n_samples samples, output rows vl->pitch frames apart
 static int run_stft(mmf_plan* p, const float* pcm, int64_t n_clips, int64_t n_samples, int64_t clip_stride,
-                    float* power, float* logmel, int* clipmax, cudaStream_t st) {
+                    float* power, float* logmel, int* clipmax, cudaStream_t st, const Varlen* vl = nullptr) {
   if (!p) return fail(MMF_ERR_INVALID, "plan is NULL");
   if (!pcm) return fail(MMF_ERR_INVALID, "pcm is NULL");
   if (n_clips < 1 || n_samples < 1) return fail(MMF_ERR_INVALID, "n_clips and n_samples must be positive");
@@ -771,6 +772,15 @@ static int run_stft(mmf_plan* p, const float* pcm, int64_t n_clips, int64_t n_sa
   a.logmel = logmel;
   a.clipmax = clipmax;
   a.power = power;
+  a.pitch = (int)T;
+  if (vl) {
+    a.n_tiles = vl->n_units;
+    a.pitch = vl->pitch;
+    a.vl_len = vl->len;
+    a.vl_T = vl->T;
+    a.vl_first = vl->first;
+    a.vl_clips = (int)n_clips;
+  }
 
   // TMA needs a 16-byte aligned base and row pitch; otherwise use the plain loader
   CUtensorMap tmap;
@@ -795,9 +805,9 @@ static int run_stft(mmf_plan* p, const float* pcm, int64_t n_clips, int64_t n_sa
   }
   // the mel projection on the tensor cores wherever the plan supports it -- a decision of the configuration alone, so
   // that a clip's features never depend on the size or the chunking of the batch it came in
-  if (p->d_mel_tc && logmel && !power && ((T + 127) / 128) * n_clips < 0x7fffffffLL) {
+  if (p->d_mel_tc && logmel && !power && (vl || ((T + 127) / 128) * n_clips < 0x7fffffffLL)) {
     cudaError_t e = stft_mel_tc_launch(tmap, tma ? 1 : 0, pcm, n_clips, n_samples, clip_stride, (int)T, c.hop_length, p->lead, c.n_mels, p->mel_tc_act, c.amin,
-                                       c.preemph, p->d_window, p->win_lo, p->win_hi, p->d_tw1, p->d_mel_tc, logmel, clipmax, p->sm_count, st);
+                                       c.preemph, p->d_window, p->win_lo, p->win_hi, p->d_tw1, p->d_mel_tc, logmel, clipmax, p->sm_count, st, vl);
     count_launch();
     if (e != cudaSuccess) return cuda_fail(e, "stft_mel_tc_kernel launch");
     return MMF_OK;
@@ -1124,6 +1134,223 @@ int mmf_change_from_logmel(mmf_plan* plan, float* logmel_dev, const int32_t* cli
   unsigned char* cur = (unsigned char*)plan->ws + (64 << 10);
   return run_post(plan, cur, logmel_dev, clipmax_dev, n_clips, T, prm, tot_dev, mfcc_dev, delta_dev, clamp_in_place,
                   (cudaStream_t)stream);
+}
+
+// Variable-length batch.  Each clip takes the route its own mmf_mfcc_change call would take -- which is what makes
+// its outputs bit-identical to that call: K1 is a decision of the configuration alone, the post-MFCC route depends on
+// the clip's T (the chunk-parallel IIR needs T + 2 padlen <= 6112, the fused kernel T <= 3456 and its shared memory).
+// Clips on the default routes -- clamp + DCT-II folded into the fused kernel, or the FP32 MFCC kernel followed by it
+// -- run in one launch per stage for the whole batch, each with the chunk tables (SosPar) of its own length; any other
+// clip runs the single-clip path in workspace and is copied into its padded rows.
+int mmf_mfcc_change_varlen(mmf_plan* plan, const float* pcm_dev, int64_t n_clips, const int64_t* n_samples_host,
+                           int64_t clip_stride, const mmf_change_params* prm, double* tot_dev, float* logmel_dev,
+                           float* mfcc_dev, float* delta_dev, void* stream) {
+  using namespace mmf;
+  // the lengths first: these checks need neither a plan nor a device
+  if (!n_samples_host) return fail(MMF_ERR_INVALID, "n_samples_host is NULL");
+  if (n_clips < 1) return fail(MMF_ERR_INVALID, "n_clips must be positive");
+  if (n_clips > 0x7fffffff) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 clips");
+  int64_t n_max = 0;
+  for (int64_t i = 0; i < n_clips; ++i) {
+    const int64_t n = n_samples_host[i];
+    if (n < 1 || n > clip_stride) {
+      char buf[160];
+      std::snprintf(buf, sizeof(buf), "clip %lld: n_samples %lld must be in [1, clip_stride = %lld]", (long long)i,
+                    (long long)n, (long long)clip_stride);
+      return fail(MMF_ERR_INVALID, buf);
+    }
+    n_max = std::max(n_max, n);
+  }
+  if (!plan || !pcm_dev || !prm || !tot_dev) return fail(MMF_ERR_INVALID, "NULL argument");
+  const mmf_config& c = plan->cfg;
+  if (n_max + c.n_fft > 0x7fffffffLL) return fail(MMF_ERR_UNSUPPORTED, "clip longer than 2^31 samples");
+  const int first = prm->remove_first ? 1 : 0;
+  const int rows = c.n_mfcc - first;
+  if (rows < 1) return fail(MMF_ERR_INVALID, "removeFirst leaves no MFCC rows");
+  SosArgs sa, so;
+  int rc = fill_sos(prm->sos, prm->n_sections, &sa);
+  if (rc) return rc;
+  const bool out_iir = prm->out_kind == 0;
+  if (out_iir && (rc = fill_sos(prm->out_sos, prm->out_n_sections, &so))) return rc;
+  const int pitch = (int)mmf_num_frames(n_max, c.n_fft, c.hop_length);
+  std::vector<int> T_all((size_t)n_clips);
+  for (int64_t i = 0; i < n_clips; ++i) {
+    T_all[i] = (int)mmf_num_frames(n_samples_host[i], c.n_fft, c.hop_length);
+    const int padlen = std::max(sa.padlen, out_iir ? so.padlen : 0);
+    if (T_all[i] <= padlen) {
+      char buf[192];
+      std::snprintf(buf, sizeof(buf),
+                    "clip %lld: The length of the input vector x must be greater than padlen, which is %d.",
+                    (long long)i, T_all[i] <= sa.padlen ? sa.padlen : so.padlen);
+      return fail(MMF_ERR_TOO_SHORT, buf);
+    }
+  }
+
+  // ---- routing (host only): route A = MFCC folded into the fused kernel, B = FP32 MFCC kernel + fused kernel
+  const bool fold = (c.flags & MMF_FLAG_FOLD_MFCC) || delta_dev == nullptr;
+  // (more than kFusedNC coefficients never fold: the solo call then takes route B, and so does the batch)
+  const bool route_a = fold && !(c.flags & (MMF_FLAG_SEPARATE_MFCC | MMF_FLAG_MMA_DCT)) && c.n_mfcc <= kFusedNC;
+  const bool mfcc_fp32 = !((c.flags & MMF_FLAG_MMA_DCT) && mfcc_mma_supported(c.n_mfcc, c.n_mels)) &&
+                         plan->d_dct_tc == nullptr;
+  const bool batched = !plan->generic && !(c.flags & MMF_FLAG_UNFUSED_CHANGE) && (route_a || mfcc_fp32) &&
+                       sa.n_sections <= kParMaxSections && (!out_iir || so.n_sections == sa.n_sections);
+  std::vector<SosPar> pars;  // distinct chunk tables of the call (they depend on the clip's length only)
+  std::vector<int> par_of_cl[2] = {std::vector<int>(kSosParMaxChunk + 1, -1), std::vector<int>(kSosParMaxChunk + 1, -1)};
+  auto par_index = [&](int which, const SosArgs& a, long T) -> int {
+    const long L = T + 2L * a.padlen;
+    if (L > 32L * kSosParMaxChunk) return -1;
+    const int cl = (int)((L + 31) / 32) | 1;  // sos_par_fill's chunk length
+    int& idx = par_of_cl[which][cl];
+    if (idx < 0) {
+      SosPar sp;
+      if (!sos_par_fill(a, T, &sp)) return -1;
+      idx = (int)pars.size();
+      pars.push_back(sp);
+    }
+    return idx;
+  };
+  const int unit = plan->d_mel_tc ? 128 : plan->TF;  // K1 work unit: a 128-frame block or a TF-frame tile
+  std::vector<int> T_k1((size_t)n_clips, 0), clips;
+  std::vector<int2> pidx((size_t)n_clips, int2{0, 0});
+  std::vector<unsigned> first_unit((size_t)n_clips + 1, 0);
+  std::vector<int64_t> fallback;
+  // the longest batched clip has the largest chunk of either cascade and needs the most shared memory: its tables
+  // and size go to the launches
+  int i1 = -1, i2 = -1, t_big = 0;
+  size_t fsmem = 0;
+  for (int64_t i = 0; i < n_clips; ++i) {
+    const int T = T_all[i];
+    bool ok = batched;
+    int a = -1, b = -1;
+    if (ok) {
+      a = par_index(0, sa, T);
+      b = out_iir ? par_index(1, so, T) : a;
+      ok = a >= 0 && b >= 0;
+    }
+    size_t sm = 0;
+    if (ok)
+      ok = route_a ? change_fused_lm_supported(pars[a], out_iir ? &pars[b] : nullptr, c.n_mfcc, c.n_mels, first, rows, T, &sm)
+                   : change_fused_supported(pars[a], out_iir ? &pars[b] : nullptr, rows, T, &sm);
+    const uint64_t units = first_unit[i] + (ok ? (uint64_t)(T + unit - 1) / unit : 0);
+    if (units > 0x7fffffffULL) return fail(MMF_ERR_UNSUPPORTED, "variable-length batch of more than 2^31 K1 blocks");
+    first_unit[i + 1] = (unsigned)units;
+    if (!ok) {
+      fallback.push_back(i);
+      continue;
+    }
+    T_k1[i] = T;
+    pidx[i] = int2{a, b};
+    clips.push_back((int)i);
+    if (T > t_big) {
+      t_big = T;
+      fsmem = sm;
+      i1 = a;
+      i2 = b;
+    }
+  }
+  const int64_t nv = (int64_t)clips.size();
+  const bool split_out = out_iir && nv >= 32;  // the batched output filter, as run_post does for a batch
+
+  // ---- workspace: descriptors, then the batched intermediates, then the single-clip region
+  MMF_CUDA(cudaSetDevice(c.device));
+  const size_t n = (size_t)n_clips;
+  size_t off = 0;
+  auto take = [&](size_t bytes) {
+    const size_t o = off;
+    off += align_up(bytes, 256);
+    return o;
+  };
+  const size_t o_len = take(n * 8), o_tall = take(n * 4), o_tk1 = take(n * 4), o_first = take((n + 1) * 4),
+               o_clips = take(std::max<size_t>(1, clips.size()) * 4), o_pidx = take(n * 8),
+               o_pars = take(std::max<size_t>(1, pars.size()) * sizeof(SosPar));
+  const size_t desc_bytes = off;
+  const size_t o_logmel = (nv && !logmel_dev) ? take(n * c.n_mels * pitch * 4) : 0;
+  const size_t o_clipmax = take(n * 4);
+  const size_t o_mfcc = (nv && !route_a && !mfcc_dev) ? take(n * c.n_mfcc * pitch * 4) : 0;
+  const size_t o_raw = split_out ? take(n * pitch * 8) : 0;
+  const size_t o_single = off;
+  size_t single_bytes = 0;
+  for (int64_t i : fallback) {
+    const size_t Ti = (size_t)T_all[i];
+    size_t b = change_ws_bytes(plan, 1, (int64_t)Ti, true, true, rows) + align_up(Ti * 8, 256);
+    if (logmel_dev) b += align_up((size_t)c.n_mels * Ti * 4, 256);
+    if (mfcc_dev) b += align_up((size_t)c.n_mfcc * Ti * 4, 256);
+    if (delta_dev) b += align_up((size_t)c.n_mfcc * Ti * 4, 256);
+    single_bytes = std::max(single_bytes, b);
+  }
+  if ((rc = ensure_ws(plan, (64 << 10) + o_single + single_bytes))) return rc;
+  unsigned char* base = (unsigned char*)plan->ws + (64 << 10);
+  std::vector<unsigned char> desc(desc_bytes);
+  std::memcpy(desc.data() + o_len, n_samples_host, n * 8);
+  std::memcpy(desc.data() + o_tall, T_all.data(), n * 4);
+  std::memcpy(desc.data() + o_tk1, T_k1.data(), n * 4);
+  std::memcpy(desc.data() + o_first, first_unit.data(), (n + 1) * 4);
+  if (nv) std::memcpy(desc.data() + o_clips, clips.data(), clips.size() * 4);
+  std::memcpy(desc.data() + o_pidx, pidx.data(), n * 8);
+  if (!pars.empty()) std::memcpy(desc.data() + o_pars, pars.data(), pars.size() * sizeof(SosPar));
+  cudaStream_t st = (cudaStream_t)stream;
+  MMF_CUDA(cudaMemcpyAsync(base, desc.data(), desc_bytes, cudaMemcpyHostToDevice, st));
+  const int* d_tall = (const int*)(base + o_tall);
+  const int* d_tk1 = (const int*)(base + o_tk1);
+
+  // ---- the batched clips: one launch per stage
+  if (nv) {
+    const Varlen vl{(const long*)(base + o_len), d_tk1, (const unsigned*)(base + o_first), (long)first_unit[n], pitch};
+    float* logmel = logmel_dev ? logmel_dev : (float*)(base + o_logmel);
+    int* clipmax = (int*)(base + o_clipmax);
+    if ((rc = run_stft(plan, pcm_dev, n_clips, n_max, clip_stride, nullptr, logmel, clipmax, st, &vl))) return rc;
+    const FusedVarlen fvl{(const int*)(base + o_clips), d_tall, (const SosPar*)(base + o_pars),
+                          (const int2*)(base + o_pidx)};
+    const int clamp = logmel_dev ? 1 : 0;
+    double* raw = split_out ? (double*)(base + o_raw) : nullptr;
+    const SosPar& pa = pars[i1];
+    const SosPar& po = pars[i2];
+    cudaError_t e;
+    if (route_a) {
+      const FusedMfccArgs lm{plan->d_dct, plan->nc_pad, logmel, clipmax, c.n_mels, c.top_db, mfcc_dev, delta_dev, clamp};
+      e = change_fused_launch(nullptr, nv, c.n_mfcc, first, rows, pitch, prm->diff_method, pa, po,
+                              split_out ? 1 : prm->out_kind, split_out ? raw : tot_dev, fsmem, &lm, st, &fvl);
+    } else {
+      float* mfcc = mfcc_dev ? mfcc_dev : (float*)(base + o_mfcc);
+      e = cudaSuccess;
+      for (int64_t c0 = 0; c0 < n_clips && e == cudaSuccess; c0 += 65535) {
+        const int64_t nc = std::min<int64_t>(65535, n_clips - c0);
+        e = mfcc_launch(plan->d_dct, plan->nc_pad, logmel + (size_t)c0 * c.n_mels * pitch, clipmax + c0, nc, pitch,
+                        c.n_mels, c.n_mfcc, c.top_db, mfcc + (size_t)c0 * c.n_mfcc * pitch,
+                        delta_dev ? delta_dev + (size_t)c0 * c.n_mfcc * pitch : nullptr, clamp, st, d_tk1 + c0);
+      }
+      if (e != cudaSuccess) return cuda_fail(e, "mfcc_kernel (variable-length) launch");
+      e = change_fused_launch(mfcc, nv, c.n_mfcc, first, rows, pitch, prm->diff_method, pa, po,
+                              split_out ? 1 : prm->out_kind, split_out ? raw : tot_dev, fsmem, nullptr, st, &fvl);
+    }
+    if (e == cudaSuccess && split_out) e = sosfiltfilt_par_varlen_launch(raw, nv, pitch, po, fvl, tot_dev, st);
+    if (e != cudaSuccess) return cuda_fail(e, "change_fused_kernel (variable-length) launch");
+  }
+
+  // ---- the other clips: the single-clip path, copied into their padded rows
+  for (int64_t i : fallback) {
+    const size_t Ti = (size_t)T_all[i];
+    unsigned char* cur = base + o_single + change_ws_bytes(plan, 1, (int64_t)Ti, true, true, rows);
+    double* tot1 = (double*)carve(cur, Ti * 8);
+    float* lm1 = logmel_dev ? (float*)carve(cur, (size_t)c.n_mels * Ti * 4) : nullptr;
+    float* mf1 = mfcc_dev ? (float*)carve(cur, (size_t)c.n_mfcc * Ti * 4) : nullptr;
+    float* dl1 = delta_dev ? (float*)carve(cur, (size_t)c.n_mfcc * Ti * 4) : nullptr;
+    if ((rc = run_change(plan, base + o_single, pcm_dev + (size_t)i * clip_stride, 1, n_samples_host[i],
+                         n_samples_host[i], prm, tot1, lm1, mf1, dl1, st)))
+      return rc;
+    MMF_CUDA(cudaMemcpyAsync(tot_dev + (size_t)i * pitch, tot1, Ti * 8, cudaMemcpyDeviceToDevice, st));
+    auto rows_to = [&](float* dst, const float* src, int r) {
+      return cudaMemcpy2DAsync(dst + (size_t)i * r * pitch, (size_t)pitch * 4, src, Ti * 4, Ti * 4, r,
+                               cudaMemcpyDeviceToDevice, st);
+    };
+    if (lm1) MMF_CUDA(rows_to(logmel_dev, lm1, c.n_mels));
+    if (mf1) MMF_CUDA(rows_to(mfcc_dev, mf1, c.n_mfcc));
+    if (dl1) MMF_CUDA(rows_to(delta_dev, dl1, c.n_mfcc));
+  }
+  cudaError_t e = varlen_tails_launch((long)n_clips, d_tall, pitch, tot_dev, logmel_dev, c.n_mels, mfcc_dev, delta_dev,
+                                      c.n_mfcc, st);
+  if (e != cudaSuccess) return cuda_fail(e, "varlen_tails_kernel launch");
+  return MMF_OK;
 }
 
 }  // extern "C"

@@ -63,7 +63,8 @@ static bool sos_par_fill_cl(const SosArgs& src, int cl, SosPar* out) {
   return true;
 }
 
-// the tables depend only on (cascade, chunk length): keep the last few per thread
+// the tables depend only on (cascade, chunk length): keep the last few per thread (a variable-length batch uses one
+// per odd chunk length of its clips, up to 96 per cascade)
 static bool sos_par_cached(const SosArgs& src, int cl, SosPar* out) {
   struct Entry {
     SosArgs key;
@@ -77,7 +78,7 @@ static bool sos_par_cached(const SosArgs& src, int cl, SosPar* out) {
       return true;
     }
   if (!sos_par_fill_cl(src, cl, out)) return false;
-  if (cache.size() >= 16) cache.erase(cache.begin());
+  if (cache.size() >= 256) cache.erase(cache.begin());
   Entry e;
   std::memcpy(&e.key, &src, sizeof(SosArgs));
   e.cl = cl;
@@ -101,17 +102,24 @@ constexpr int kParWarps = 4;
 constexpr int kFusedPerThread = 9;
 constexpr int kFusedMaxWarps = 12;  // 384 threads, <= 85 registers: two CTAs per SM
 
-template <typename TIn, int NS>
+// VL (variable-length batch): row r is clip vl.clips[r] at x + clip * x_row_stride with its own frame count and
+// cascade tables (vl.pidx[clip].y); a warp's buffer is `s_stride` doubles, the largest 32 * CL of the launch.
+template <typename TIn, int NS, bool VL>
 __global__ void __launch_bounds__(kParWarps * 32)
     sosfiltfilt_par_kernel(const TIn* __restrict__ x, long rows, int T, long x_row_stride, int group_rows,
-                           long group_stride, const __grid_constant__ SosPar a, double* __restrict__ y,
-                           long y_row_stride) {
+                           long group_stride, const __grid_constant__ SosPar a_, double* __restrict__ y,
+                           long y_row_stride, const __grid_constant__ FusedVarlen vl, int s_stride) {
   extern __shared__ __align__(16) double sm_par[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const long row = (long)blockIdx.x * kParWarps + warp;
+  long row = (long)blockIdx.x * kParWarps + warp;
   if (row >= rows) return;
+  if (VL) {
+    row = vl.clips[row];
+    T = vl.T[row];
+  }
+  const SosPar& a = VL ? vl.pars[vl.pidx[row].y] : a_;
   const int S = 32 * a.CL, p = a.padlen, L = T + 2 * p;
-  double* buf = sm_par + (size_t)warp * S;
+  double* buf = sm_par + (size_t)warp * s_stride;
   const long g = row / group_rows, gi = row - g * group_rows;
   warp_load_odd_ext<TIn>(x + g * group_stride + gi * x_row_stride, T, p, buf, S, lane);
   const SosRegs<NS> c(a);
@@ -125,11 +133,35 @@ static cudaError_t par_launch_ns(const TIn* x, long rows, long T, long xs, int g
                                  const SosPar& a, double* y, long ys, cudaStream_t st) {
   const unsigned grid = (unsigned)((rows + kParWarps - 1) / kParWarps);
   const size_t smem = (size_t)kParWarps * 32 * a.CL * sizeof(double);
-  auto kfn = sosfiltfilt_par_kernel<TIn, NS>;
+  auto kfn = sosfiltfilt_par_kernel<TIn, NS, false>;
   MMF_SMEM_ONCE(kfn, 200 * 1024);
-  kfn<<<grid, kParWarps * 32, smem, st>>>(x, rows, (int)T, xs, group_rows, group_stride, a, y, ys);
+  kfn<<<grid, kParWarps * 32, smem, st>>>(x, rows, (int)T, xs, group_rows, group_stride, a, y, ys, FusedVarlen{},
+                                          32 * a.CL);
   count_launch();
   return cudaGetLastError();
+}
+
+template <int NS>
+static cudaError_t par_varlen_ns(const double* x, long rows, long pitch, const SosPar& amax, const FusedVarlen& vl,
+                                 double* y, cudaStream_t st) {
+  const unsigned grid = (unsigned)((rows + kParWarps - 1) / kParWarps);
+  const size_t smem = (size_t)kParWarps * 32 * amax.CL * sizeof(double);
+  auto kfn = sosfiltfilt_par_kernel<double, NS, true>;
+  MMF_SMEM_ONCE(kfn, 200 * 1024);
+  kfn<<<grid, kParWarps * 32, smem, st>>>(x, rows, (int)pitch, pitch, 1, pitch, amax, y, pitch, vl, 32 * amax.CL);
+  count_launch();
+  return cudaGetLastError();
+}
+
+cudaError_t sosfiltfilt_par_varlen_launch(const double* x, long rows, long pitch, const SosPar& amax,
+                                          const FusedVarlen& vl, double* y, cudaStream_t st) {
+  switch (amax.ns) {
+    case 1: return par_varlen_ns<1>(x, rows, pitch, amax, vl, y, st);
+    case 2: return par_varlen_ns<2>(x, rows, pitch, amax, vl, y, st);
+    case 3: return par_varlen_ns<3>(x, rows, pitch, amax, vl, y, st);
+    case 4: return par_varlen_ns<4>(x, rows, pitch, amax, vl, y, st);
+    default: return cudaErrorInvalidValue;
+  }
 }
 
 template <typename TIn>
@@ -331,12 +363,11 @@ cudaError_t sosfiltfilt_long_launch(const void* x, int x_is_f32, long rows, long
 // K3 folded into the per-clip kernel: clamp + DCT-II of this clip's log-mel columns straight into the
 // float64 row buffers (and to HBM as float32 MFCC / delta when the caller wants them).  Same FMA order
 // per coefficient as mfcc_kernel (post_kernels.cu), so the MFCCs are bit-identical to the unfused path.
-constexpr int kFusedNC = 16;
 constexpr int kFusedDepth = 8;  // log-mel rows in flight per thread (16 measured slower)
 __device__ __forceinline__ float fused_key_to_float(int k) { return __int_as_float(k >= 0 ? k : k ^ 0x7FFFFFFF); }
 
 __device__ __forceinline__ void fused_mfcc_phase(const FusedMfccArgs& m, long clip, int n_mfcc, int first, int T,
-                                                 int S, int p, double* rowbuf, float* s_dct) {
+                                                 int pitch, int S, int p, double* rowbuf, float* s_dct) {
   const int tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31;
   const int n_mels = m.n_mels;
   for (int i = tid; i < n_mels * kFusedNC; i += nthr) {
@@ -358,20 +389,20 @@ __device__ __forceinline__ void fused_mfcc_phase(const FusedMfccArgs& m, long cl
 #pragma unroll
     for (int j = 0; j < kFusedNC; ++j) acc[j] = 0.0f;
     if (valid) {
-      float* col = m.logmel + (size_t)clip * n_mels * T + t;
+      float* col = m.logmel + (size_t)clip * n_mels * pitch + t;
       float cur[kFusedDepth], nxt[kFusedDepth];
 #pragma unroll
-      for (int u = 0; u < kFusedDepth; ++u) cur[u] = (u < n_mels) ? __ldcs(col + (size_t)u * T) : 0.0f;
+      for (int u = 0; u < kFusedDepth; ++u) cur[u] = (u < n_mels) ? __ldcs(col + (size_t)u * pitch) : 0.0f;
       for (int m0 = 0; m0 < n_mels; m0 += kFusedDepth) {
 #pragma unroll
         for (int u = 0; u < kFusedDepth; ++u)
-          nxt[u] = (m0 + kFusedDepth + u < n_mels) ? __ldcs(col + (size_t)(m0 + kFusedDepth + u) * T) : 0.0f;
+          nxt[u] = (m0 + kFusedDepth + u < n_mels) ? __ldcs(col + (size_t)(m0 + kFusedDepth + u) * pitch) : 0.0f;
 #pragma unroll
         for (int u = 0; u < kFusedDepth; ++u) {
           const int mm = m0 + u;
           if (mm < n_mels) {
             const float x = fmaxf(cur[u], thr);
-            if (m.clamp_in_place && own) col[(size_t)mm * T] = x;
+            if (m.clamp_in_place && own) col[(size_t)mm * pitch] = x;
             const float4* d4 = reinterpret_cast<const float4*>(s_dct + mm * kFusedNC);
 #pragma unroll
             for (int j4 = 0; j4 < kFusedNC / 4; ++j4) {
@@ -388,11 +419,11 @@ __device__ __forceinline__ void fused_mfcc_phase(const FusedMfccArgs& m, long cl
       }
     }
     if (own) {
-      float* dst = m.mfcc_out ? m.mfcc_out + (size_t)clip * n_mfcc * T + t : nullptr;
+      float* dst = m.mfcc_out ? m.mfcc_out + (size_t)clip * n_mfcc * pitch + t : nullptr;
 #pragma unroll
       for (int j = 0; j < kFusedNC; ++j) {
         if (j < n_mfcc) {
-          if (dst) dst[(size_t)j * T] = acc[j];
+          if (dst) dst[(size_t)j * pitch] = acc[j];
           if (j >= first) rowbuf[(size_t)(j - first) * S + p + t] = (double)acc[j];
         }
       }
@@ -400,7 +431,7 @@ __device__ __forceinline__ void fused_mfcc_phase(const FusedMfccArgs& m, long cl
     if (halo) {
       // delta = np.gradient along time in float32 (calc.py:642-645); shuffles stay outside any
       // lane-dependent branch
-      float* dst = m.delta_out + (size_t)clip * n_mfcc * T + t;
+      float* dst = m.delta_out + (size_t)clip * n_mfcc * pitch + t;
 #pragma unroll
       for (int j = 0; j < kFusedNC; ++j) {
         if (j < n_mfcc) {
@@ -411,7 +442,7 @@ __device__ __forceinline__ void fused_mfcc_phase(const FusedMfccArgs& m, long cl
           else if (t == 0) d = cp - acc[j];
           else if (t == T - 1) d = acc[j] - cm;
           else d = (cp - cm) / 2.0f;
-          if (own) dst[(size_t)j * T] = d;
+          if (own) dst[(size_t)j * pitch] = d;
         }
       }
     }
@@ -419,18 +450,25 @@ __device__ __forceinline__ void fused_mfcc_phase(const FusedMfccArgs& m, long cl
   __syncthreads();
 }
 
-template <int NS1, int NS2, bool FROM_LM>
+// VL (variable-length batch): CTA b takes clip vl.clips[b] with its own frame count and cascade tables; `T` is then
+// the row pitch of every input and output.
+template <int NS1, int NS2, bool FROM_LM, bool VL>
 __global__ void __launch_bounds__(kFusedMaxWarps * 32, 2)
     change_fused_kernel(const float* __restrict__ mfcc, int n_mfcc, int first, int rows, int T, int method,
-                        const __grid_constant__ SosPar a1, const __grid_constant__ SosPar a2, int out_kind,
-                        double* __restrict__ tot, const __grid_constant__ FusedMfccArgs lm, int sm_doubles) {
+                        const __grid_constant__ SosPar a1_, const __grid_constant__ SosPar a2_, int out_kind,
+                        double* __restrict__ tot, const __grid_constant__ FusedMfccArgs lm, int sm_doubles,
+                        const __grid_constant__ FusedVarlen vl) {
   extern __shared__ __align__(16) double sm_fused[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
-  const long clip = blockIdx.x;
+  const long clip = VL ? vl.clips[blockIdx.x] : blockIdx.x;
+  const int pitch = T;
+  if (VL) T = vl.T[clip];
+  const SosPar& a1 = VL ? vl.pars[vl.pidx[clip].x] : a1_;
+  const SosPar& a2 = VL ? vl.pars[vl.pidx[clip].y] : a2_;
   const int S = 32 * a1.CL, p = a1.padlen, L = T + 2 * p;
   if (FROM_LM) {
     float* s_dct = reinterpret_cast<float*>(sm_fused + sm_doubles);
-    fused_mfcc_phase(lm, clip, n_mfcc, first, T, S, p, sm_fused, s_dct);
+    fused_mfcc_phase(lm, clip, n_mfcc, first, T, pitch, S, p, sm_fused, s_dct);
   }
   // 1. zero-phase Butterworth of every kept coefficient row, in place in shared memory
   {
@@ -438,7 +476,7 @@ __global__ void __launch_bounds__(kFusedMaxWarps * 32, 2)
     for (int r = warp; r < rows; r += nwarps) {
       double* buf = sm_fused + (size_t)r * S;
       if (FROM_LM) warp_odd_ext_staged<float>(buf, T, p, S, lane);
-      else warp_load_odd_ext<float>(mfcc + ((size_t)clip * n_mfcc + first + r) * T, T, p, buf, S, lane);
+      else warp_load_odd_ext<float>(mfcc + ((size_t)clip * n_mfcc + first + r) * pitch, T, p, buf, S, lane);
       warp_sosfiltfilt<NS1>(buf, L, a1, c1, lane);
     }
   }
@@ -468,7 +506,7 @@ __global__ void __launch_bounds__(kFusedMaxWarps * 32, 2)
     }
     raw[q] = sqrt(s) / (double)rows;
   }
-  double* dst = tot + (size_t)clip * T;
+  double* dst = tot + (size_t)clip * pitch;
   if (out_kind != 0) {
 #pragma unroll
     for (int q = 0; q < kPerThread; ++q) {
@@ -528,25 +566,25 @@ bool change_fused_lm_supported(const SosPar& a1, const SosPar* a2, int n_mfcc, i
   return true;
 }
 
-template <int NS1, int NS2>
+template <int NS1, int NS2, bool VL>
 static cudaError_t fused_launch_cl(const float* mfcc, long n_clips, int n_mfcc, int first, int rows, long T,
                                    int method, const SosPar& a1, const SosPar& a2, int out_kind, double* tot,
-                                   size_t smem, const FusedMfccArgs* lm, cudaStream_t st) {
+                                   size_t smem, const FusedMfccArgs* lm, cudaStream_t st, const FusedVarlen& vl) {
   // >= ceil(T / (32*kFusedPerThread)) warps for the derivative phase, one per row if possible
   int warps = std::min(kFusedMaxWarps, std::max(rows, (int)((T + 32 * kFusedPerThread - 1) / (32 * kFusedPerThread))));
   const int sm_doubles = (int)fused_row_doubles(a1, out_kind == 0 ? &a2 : nullptr, rows);
   if (lm) {
     // the DCT phase streams the clip's log-mel columns: it wants every thread the CTA may have
     warps = kFusedMaxWarps;
-    auto kfn = change_fused_kernel<NS1, NS2, true>;
+    auto kfn = change_fused_kernel<NS1, NS2, true, VL>;
     MMF_SMEM_ONCE(kfn, 220 * 1024);
     kfn<<<(unsigned)n_clips, warps * 32, smem, st>>>(nullptr, n_mfcc, first, rows, (int)T, method, a1, a2, out_kind,
-                                                     tot, *lm, sm_doubles);
+                                                     tot, *lm, sm_doubles, vl);
   } else {
-    auto kfn = change_fused_kernel<NS1, NS2, false>;
+    auto kfn = change_fused_kernel<NS1, NS2, false, VL>;
     MMF_SMEM_ONCE(kfn, 220 * 1024);
     kfn<<<(unsigned)n_clips, warps * 32, smem, st>>>(mfcc, n_mfcc, first, rows, (int)T, method, a1, a2, out_kind,
-                                                     tot, FusedMfccArgs{}, sm_doubles);
+                                                     tot, FusedMfccArgs{}, sm_doubles, vl);
   }
   count_launch();
   return cudaGetLastError();
@@ -554,14 +592,17 @@ static cudaError_t fused_launch_cl(const float* mfcc, long n_clips, int n_mfcc, 
 
 cudaError_t change_fused_launch(const float* mfcc, long n_clips, int n_mfcc, int first, int rows, long T, int method,
                                 const SosPar& a1, const SosPar& a2, int out_kind, double* tot, size_t smem,
-                                const FusedMfccArgs* lm, cudaStream_t st) {
+                                const FusedMfccArgs* lm, cudaStream_t st, const FusedVarlen* vl) {
   // equal section counts (the reference's default: outFilter None reuses the row filter, 'iir' uses
   // the same order) get an instantiation; anything else goes through the unfused kernels
   const int k = a1.ns * 10 + (out_kind == 0 ? a2.ns : a1.ns);
   switch (k) {
-#define MMF_FUSED_CASE(A, B) \
-  case A * 10 + B:           \
-    return fused_launch_cl<A, B>(mfcc, n_clips, n_mfcc, first, rows, T, method, a1, a2, out_kind, tot, smem, lm, st);
+#define MMF_FUSED_CASE(A, B)                                                                                          \
+  case A * 10 + B:                                                                                                    \
+    return vl ? fused_launch_cl<A, B, true>(mfcc, n_clips, n_mfcc, first, rows, T, method, a1, a2, out_kind, tot, smem, \
+                                            lm, st, *vl)                                                              \
+              : fused_launch_cl<A, B, false>(mfcc, n_clips, n_mfcc, first, rows, T, method, a1, a2, out_kind, tot,    \
+                                             smem, lm, st, FusedVarlen{});
     MMF_FUSED_CASE(1, 1)
     MMF_FUSED_CASE(2, 2)
     MMF_FUSED_CASE(3, 3)

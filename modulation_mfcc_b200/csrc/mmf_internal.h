@@ -13,6 +13,18 @@
 
 namespace mmf {
 
+// ---- a variable-length batch (mmf_mfcc_change_varlen): device arrays built per call.  Clip i has len[i] samples
+// and T[i] frames; T[i] = 0 marks a clip the launch skips (it takes the single-clip path).  K1 walks a compacted list
+// of work units (128-frame blocks or TF-frame tiles): clip i owns units [first[i], first[i + 1]).  Output rows are
+// `pitch` (the longest clip's T) frames apart.
+struct Varlen {
+  const long* len;
+  const int* T;
+  const unsigned* first;
+  long n_units;
+  int pitch;
+};
+
 // ---- arguments of the fused STFT/mel kernel (passed by value)
 struct StftArgs {
   const float* pcm;
@@ -63,6 +75,11 @@ struct StftArgs {
   float* logmel;         // [n_clips, n_mels, T] or null
   int* clipmax;          // [n_clips] float keys or null
   float* power;          // [n_clips, F, T] or null
+  int pitch;             // frames per log-mel / power row (T, or the longest clip's T in a variable-length batch)
+  const long* vl_len;    // variable-length batch (else null): see Varlen
+  const int* vl_T;
+  const unsigned* vl_first;
+  int vl_clips;
 };
 
 struct StftGeometry {
@@ -86,7 +103,7 @@ cudaError_t stft_mel_tc_launch(const CUtensorMap& tmap, int use_tma, const float
                                long clip_stride, int T, int hop,
                                int lead, int n_mels, int n_act, float amin, float preemph, const float* window, int win_lo,
                                int win_hi, const float2* tw1, const void* wtab, float* logmel, int* clipmax,
-                               int sm_count, cudaStream_t st);
+                               int sm_count, cudaStream_t st, const Varlen* vl = nullptr);
 
 // ---- generic n_fft (anything but a power of two in [256, 4096]): FP32 matrix-product DFT (dft_generic.cu)
 void dft_generic_table(int n_fft, const std::vector<float>& window, std::vector<float>& tab, int* ld_out);
@@ -121,7 +138,7 @@ cudaError_t modspec_tc_launch(const float* mfcc, long n_clips, int n_coef, long 
 // ---- post-FFT kernels (post_kernels.cu)
 cudaError_t mfcc_launch(const float* dct_pad, int nc_pad, float* logmel, const int* clipmax, long n_clips, long T,
                         int n_mels, int n_mfcc, float top_db, float* mfcc, float* delta, int clamp_in_place,
-                        cudaStream_t st);
+                        cudaStream_t st, const int* vT = nullptr);
 
 void mfcc_mma_bfrag(const float* dct, int n_mfcc, int n_mels, std::vector<float4>& out);
 bool mfcc_mma_supported(int n_mfcc, int n_mels);
@@ -148,6 +165,8 @@ bool sos_long_supported(const SosArgs& a, long rows, long T);
 cudaError_t sosfiltfilt_long_launch(const void* x, int x_is_f32, long rows, long T, long xs, int group_rows,
                                     long group_stride, const SosArgs& a, double* y, long ys, cudaStream_t st);
 bool change_fused_supported(const SosPar& a1, const SosPar* a2, int rows, long T, size_t* smem_out);
+// K3 folded into the fused kernel (lm != nullptr) takes up to kFusedNC coefficients
+constexpr int kFusedNC = 16;
 // K3 folded into the fused kernel (lm != nullptr): the clip's MFCC rows go from the DCT straight into
 // the float64 row buffers; mfcc_out / delta_out are optional HBM copies for the caller
 struct FusedMfccArgs {
@@ -163,9 +182,22 @@ struct FusedMfccArgs {
 };
 bool change_fused_lm_supported(const SosPar& a1, const SosPar* a2, int n_mfcc, int n_mels, int first, int rows,
                                long T, size_t* smem_out);
+// variable-length batch of the fused kernel and the batched output filter: launch item b is clip clips[b] with T[clip]
+// frames and the cascade tables pars[pidx[clip].x] (row filter) / pars[pidx[clip].y] (output filter); the launch's
+// T is the row pitch and its SosPar arguments are the ones with the largest chunk (they size shared memory)
+struct FusedVarlen {
+  const int* clips;
+  const int* T;
+  const SosPar* pars;
+  const int2* pidx;
+};
 cudaError_t change_fused_launch(const float* mfcc, long n_clips, int n_mfcc, int first, int rows, long T, int method,
                                 const SosPar& a1, const SosPar& a2, int out_kind, double* tot, size_t smem,
-                                const FusedMfccArgs* lm, cudaStream_t st);
+                                const FusedMfccArgs* lm, cudaStream_t st, const FusedVarlen* vl = nullptr);
+cudaError_t sosfiltfilt_par_varlen_launch(const double* x, long rows, long pitch, const SosPar& amax,
+                                          const FusedVarlen& vl, double* y, cudaStream_t st);
+cudaError_t varlen_tails_launch(long n_clips, const int* T, int pitch, double* tot, float* logmel, int n_mels,
+                                float* mfcc, float* delta, int n_mfcc, cudaStream_t st);
 cudaError_t delta_norm_launch(const double* x, long n_clips, int rows, long T, int method, double* tot,
                               cudaStream_t st);
 cudaError_t fir_filtfilt_launch(const double* x, long rows, long T, const double* b_dev, int n_taps, double* y,

@@ -22,30 +22,33 @@ __device__ __forceinline__ float key_to_float(int k) { return __int_as_float(k >
 // K3: top_db clamp + DCT-II (+ delta).  One thread per frame; the DCT rows sit in
 // shared memory as [n_mels][NC] so each mel value feeds NC FMAs from broadcast
 // 128-bit shared loads.  Block = 128 frames with a one-frame halo on each side
-// when the delta (np.gradient) is requested.
+// when the delta (np.gradient) is requested.  T is the row pitch in frames; vT (a variable-length
+// batch, else null) gives each clip's own frame count, 0 for a clip the launch skips.
 // ---------------------------------------------------------------------------
 constexpr int kMfccThreads = 128;
 
-template <int NC>
+template <int NC, bool VL>
 __global__ void __launch_bounds__(kMfccThreads)
     mfcc_kernel(const float* __restrict__ dct_pad, int dct_pitch, float* logmel, const int* __restrict__ clipmax, long T,
                 int n_mels, int n_mfcc, float top_db, float* __restrict__ mfcc, float* __restrict__ delta,
-                int clamp_in_place) {
+                int clamp_in_place, const int* __restrict__ vT) {
   extern __shared__ __align__(16) float sm[];
   float* s_dct = sm;                 // [n_mels][NC]
   float* s_col = sm + n_mels * NC;   // [NC][kMfccThreads + 1]
   const int tid = threadIdx.x;
+  const long clip = blockIdx.y;
+  const int halo = delta != nullptr ? 1 : 0;
+  const int per_block = kMfccThreads - 2 * halo;
+  const long Tn = VL ? vT[clip] : T;  // frames of this clip
+  if (VL && (long)blockIdx.x * per_block >= Tn) return;
   for (int i = tid; i < n_mels * NC; i += kMfccThreads) {
     const int m = i / NC, j = i - m * NC;
     s_dct[i] = dct_pad[m * dct_pitch + j];
   }
   __syncthreads();
 
-  const long clip = blockIdx.y;
-  const int halo = delta != nullptr ? 1 : 0;
-  const int per_block = kMfccThreads - 2 * halo;
   const long t = (long)blockIdx.x * per_block - halo + tid;
-  const bool valid = t >= 0 && t < T;
+  const bool valid = t >= 0 && t < Tn;
   const bool own = valid && tid >= halo && tid < kMfccThreads - halo;
   const float thr = top_db >= 0.0f ? key_to_float(clipmax[clip]) - top_db : -FLT_MAX;
 
@@ -100,11 +103,11 @@ __global__ void __launch_bounds__(kMfccThreads)
         if (j < n_mfcc) {
           const float* c = s_col + j * (kMfccThreads + 1) + tid;
           float d;
-          if (T == 1) {
+          if (Tn == 1) {
             d = 0.0f;
           } else if (t == 0) {
             d = c[1] - c[0];
-          } else if (t == T - 1) {
+          } else if (t == Tn - 1) {
             d = c[0] - c[-1];
           } else {
             d = (c[1] - c[-1]) / 2.0f;
@@ -122,25 +125,28 @@ __global__ void __launch_bounds__(kMfccThreads)
 // packed FFMA2 (half the issue slots of the contraction), the mel rows are walked with pointer steps instead of
 // 64-bit index products, and the loop body carries no predicates.  ncu of mfcc_kernel<16> on the bench shape:
 // 83.4 M warp instructions of which 21 M are the FFMAs -- issue-bound at 95 us for a 271 MB stream.
-template <int NP, int PITCH>
+template <int NP, int PITCH, bool VL>
 __global__ void __launch_bounds__(kMfccThreads)
     mfcc_pk_kernel(const float* __restrict__ dct_pad, float* logmel, const int* __restrict__ clipmax, long T, int n_mels,
-                   int n_mfcc, float top_db, float* __restrict__ mfcc, float* __restrict__ delta, int clamp_in_place) {
+                   int n_mfcc, float top_db, float* __restrict__ mfcc, float* __restrict__ delta, int clamp_in_place,
+                   const int* __restrict__ vT) {
   extern __shared__ __align__(16) float sm[];
   static_assert(2 * NP <= PITCH, "coefficient pairs must fit the padded table row");
   float* s_dct = sm;                    // [n_mels][PITCH]
   float* s_col = sm + n_mels * PITCH;   // [2 NP][kMfccThreads + 1]
   const int tid = threadIdx.x;
+  const long clip = blockIdx.y;
+  const int halo = delta != nullptr ? 1 : 0;
+  const int per_block = kMfccThreads - 2 * halo;
+  const long Tn = VL ? vT[clip] : T;  // frames of this clip
+  if (VL && (long)blockIdx.x * per_block >= Tn) return;
   for (int i = tid; i < n_mels * (PITCH / 4); i += kMfccThreads)
     reinterpret_cast<float4*>(s_dct)[i] = reinterpret_cast<const float4*>(dct_pad)[i];
   __syncthreads();
 
-  const long clip = blockIdx.y;
   const int Ti = (int)T;  // row pitch as a 32-bit value: u * Ti is one IMAD.WIDE per address instead of a 64-bit product
-  const int halo = delta != nullptr ? 1 : 0;
-  const int per_block = kMfccThreads - 2 * halo;
   const long t = (long)blockIdx.x * per_block - halo + tid;
-  const bool valid = t >= 0 && t < T;
+  const bool valid = t >= 0 && t < Tn;
   const bool own = valid && tid >= halo && tid < kMfccThreads - halo;
   const float thr = top_db >= 0.0f ? key_to_float(clipmax[clip]) - top_db : -FLT_MAX;
 
@@ -148,7 +154,7 @@ __global__ void __launch_bounds__(kMfccThreads)
 #pragma unroll
   for (int j = 0; j < NP; ++j) acc[j] = pmake(0.0f, 0.0f);
   // frames outside the clip (halo of the first / last block) read frame 0 / T - 1: finite, never stored
-  const long tc = t < 0 ? 0 : (t >= T ? T - 1 : t);
+  const long tc = t < 0 ? 0 : (t >= Tn ? Tn - 1 : t);
   float* col = logmel + (size_t)clip * n_mels * T + tc;
   const bool store_clamped = clamp_in_place && own;
   {
@@ -203,14 +209,14 @@ __global__ void __launch_bounds__(kMfccThreads)
     if (own) {
       float* dst = delta + (size_t)clip * n_mfcc * T + t;
       // np.gradient: one-sided at the clip's ends, central inside
-      const int lo = t == 0 ? 0 : -1, hi = t == T - 1 ? 0 : 1;
+      const int lo = t == 0 ? 0 : -1, hi = t == Tn - 1 ? 0 : 1;
       const float scale = (lo != 0 && hi != 0) ? 0.5f : 1.0f;
 #pragma unroll
       for (int j = 0; j < 2 * NP; ++j) {
         if (j < n_mfcc) {
           const float* c = s_col + j * (kMfccThreads + 1) + tid;
           // (c[1] - c[-1]) / 2 and (c[1] - c[0]) / 1 exactly as mfcc_kernel: division by 2 = multiplication by 0.5
-          *dst = T == 1 ? 0.0f : (c[hi] - c[lo]) * scale;
+          *dst = Tn == 1 ? 0.0f : (c[hi] - c[lo]) * scale;
         }
         dst += Ti;
       }
@@ -220,7 +226,7 @@ __global__ void __launch_bounds__(kMfccThreads)
 
 cudaError_t mfcc_launch(const float* dct_pad, int nc_pad, float* logmel, const int* clipmax, long n_clips, long T,
                         int n_mels, int n_mfcc, float top_db, float* mfcc, float* delta, int clamp_in_place,
-                        cudaStream_t st) {
+                        cudaStream_t st, const int* vT) {
   const int halo = delta != nullptr ? 1 : 0;
   const int per_block = kMfccThreads - 2 * halo;
   dim3 grid((unsigned)((T + per_block - 1) / per_block), (unsigned)n_clips);
@@ -228,12 +234,17 @@ cudaError_t mfcc_launch(const float* dct_pad, int nc_pad, float* logmel, const i
   size_t smem = ((size_t)n_mels * nc + (size_t)nc * (kMfccThreads + 1)) * sizeof(float);
   if ((nc == 16 || nc == 32) && nc_pad == nc && n_mels % 8 == 0 && n_mels >= 8 && T < (1L << 27)) {
     const int np = n_mfcc <= 8 ? 4 : (n_mfcc + 1) / 2;
-#define MMF_MFCC_PK_CASE(N, P)                                                                                     \
-  case N: {                                                                                                        \
-    auto kfn = mfcc_pk_kernel<N, P>;                                                                               \
+#define MMF_MFCC_PK_LAUNCH(N, P, V)                                                                                \
+  {                                                                                                                \
+    auto kfn = mfcc_pk_kernel<N, P, V>;                                                                            \
     MMF_SMEM_ONCE(kfn, 200 * 1024);                                                                                \
     kfn<<<grid, kMfccThreads, smem, st>>>(dct_pad, logmel, clipmax, T, n_mels, n_mfcc, top_db, mfcc, delta,        \
-                                          clamp_in_place);                                                         \
+                                          clamp_in_place, vT);                                                     \
+  }
+#define MMF_MFCC_PK_CASE(N, P)                                                                                     \
+  case N: {                                                                                                        \
+    if (vT) MMF_MFCC_PK_LAUNCH(N, P, true)                                                                         \
+    else MMF_MFCC_PK_LAUNCH(N, P, false)                                                                           \
     break;                                                                                                         \
   }
     switch (np) {
@@ -252,14 +263,21 @@ cudaError_t mfcc_launch(const float* dct_pad, int nc_pad, float* logmel, const i
       MMF_MFCC_PK_CASE(16, 32)
     }
 #undef MMF_MFCC_PK_CASE
+#undef MMF_MFCC_PK_LAUNCH
     count_launch();
     return cudaGetLastError();
   }
+#define MMF_MFCC_LAUNCH(N, V)                                                                                    \
+  {                                                                                                              \
+    auto kfn = mfcc_kernel<N, V>;                                                                                \
+    MMF_SMEM_ONCE(kfn, 200 * 1024);                                                                              \
+    kfn<<<grid, kMfccThreads, smem, st>>>(dct_pad, nc_pad, logmel, clipmax, T, n_mels, n_mfcc, top_db, mfcc,     \
+                                          delta, clamp_in_place, vT);                                            \
+  }
 #define MMF_MFCC_CASE(N)                                                                                         \
   case N: {                                                                                                      \
-    MMF_SMEM_ONCE(mfcc_kernel<N>, 200 * 1024);                                                                   \
-    mfcc_kernel<N><<<grid, kMfccThreads, smem, st>>>(dct_pad, nc_pad, logmel, clipmax, T, n_mels, n_mfcc, top_db, \
-                                                     mfcc, delta, clamp_in_place);                               \
+    if (vT) MMF_MFCC_LAUNCH(N, true)                                                                             \
+    else MMF_MFCC_LAUNCH(N, false)                                                                               \
     break;                                                                                                       \
   }
   switch (nc) {
@@ -269,6 +287,35 @@ cudaError_t mfcc_launch(const float* dct_pad, int nc_pad, float* logmel, const i
     MMF_MFCC_CASE(128)
   }
 #undef MMF_MFCC_CASE
+#undef MMF_MFCC_LAUNCH
+  count_launch();
+  return cudaGetLastError();
+}
+
+// Variable-length batch: every output element at or past its clip's frame count is 0.  One CTA per clip; the
+// kernels before it write frames [0, T[clip]) only.
+__global__ void varlen_tails_kernel(const int* __restrict__ T, int pitch, double* __restrict__ tot,
+                                    float* __restrict__ logmel, int n_mels, float* __restrict__ mfcc,
+                                    float* __restrict__ delta, int n_mfcc) {
+  const long clip = blockIdx.x;
+  const int t0 = T[clip], w = pitch - t0;
+  if (w <= 0) return;
+  for (int i = threadIdx.x; i < w; i += blockDim.x) tot[(size_t)clip * pitch + t0 + i] = 0.0;
+  auto zero = [&](float* buf, int rows) {  // rows x w can pass 2^31 (long clips at small hops): 64-bit indices
+    if (!buf) return;
+    for (long e = threadIdx.x; e < (long)rows * w; e += blockDim.x) {
+      const long r = e / w;
+      buf[((size_t)clip * rows + r) * pitch + t0 + (e - r * w)] = 0.0f;
+    }
+  };
+  zero(logmel, n_mels);
+  zero(mfcc, n_mfcc);
+  zero(delta, n_mfcc);
+}
+
+cudaError_t varlen_tails_launch(long n_clips, const int* T, int pitch, double* tot, float* logmel, int n_mels,
+                                float* mfcc, float* delta, int n_mfcc, cudaStream_t st) {
+  varlen_tails_kernel<<<(unsigned)n_clips, 256, 0, st>>>(T, pitch, tot, logmel, n_mels, mfcc, delta, n_mfcc);
   count_launch();
   return cudaGetLastError();
 }

@@ -237,8 +237,24 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 2 : 1)
   long tile = blockIdx.x;
   const int tpc = p.tiles_per_clip;
   const int step_q = (int)(gridDim.x / (unsigned)tpc), step_r = (int)(gridDim.x % (unsigned)tpc);
+  // variable-length batch: the last clip whose first tile is <= tl (clips without tiles are skipped over)
+  auto locate = [&](long tl, int& c, int& t) {
+    int lo = 0, hi = p.vl_clips - 1;
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if ((long)p.vl_first[mid] <= tl) lo = mid;
+      else hi = mid - 1;
+    }
+    c = lo;
+    t = (int)(tl - (long)p.vl_first[lo]);
+  };
   int clip = (int)(tile / tpc), tin = (int)(tile % tpc);
+  if (p.vl_first) locate(tile, clip, tin);
   auto next_tile = [&](int& c, int& t) {
+    if (p.vl_first) {
+      locate(tile + gridDim.x, c, t);
+      return;
+    }
     c += step_q;
     t += step_r;
     if (t >= tpc) {
@@ -251,11 +267,15 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 2 : 1)
   while ((1 << tf_shift) < p.TF) ++tf_shift;
   if (p.use_tma && tid == 0 && tile < n_tiles) issue_span<NFFT>(&tmap, p, clip, tin << tf_shift, s_span, &s_bar[0]);
 
-  for (int it = 0; tile < n_tiles; tile += gridDim.x, ++it, next_tile(clip, tin)) {
+  int nclip = clip, ntin = tin;  // the tile after this one (prefetch target)
+  for (int it = 0; tile < n_tiles; tile += gridDim.x, ++it, clip = nclip, tin = ntin) {
     const int b = p.span_bufs == 2 ? (it & 1) : 0;
     const int t0 = tin << tf_shift;
-    int nclip = clip, ntin = tin;  // the tile after this one (prefetch target)
+    nclip = clip;
+    ntin = tin;
     next_tile(nclip, ntin);
+    const long len = p.vl_len ? p.vl_len[clip] : p.n_samples;  // this clip's samples and frames
+    const int Tc = p.vl_T ? p.vl_T[clip] : p.T;
     float* span = s_span + (size_t)b * p.span_alloc;
     // the span starts at the 16-byte aligned sample at or below the first needed one
     const int g_first = t0 * p.hop - NFFT / 2 - lead;
@@ -271,13 +291,20 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 2 : 1)
       if (p.span_bufs == 2 && tid == 0 && tile + gridDim.x < n_tiles)
         issue_span<NFFT>(&tmap, p, nclip, ntin << tf_shift, s_span + (size_t)(b ^ 1) * p.span_alloc, &s_bar[b ^ 1]);
       mbar_wait(&s_bar[b], (uint32_t)(p.span_bufs == 2 ? (it >> 1) : it) & 1u);
+      // variable-length batch: the TMA read the padded buffer, whose samples at and past the clip's end must read as
+      // zero -- overwrite them before the frames load
+      const long from = len - (long)(g_first & ~3);
+      if (p.vl_len && from < p.span_alloc) {
+        for (long i = max(0L, from) + tid; i < p.span_alloc; i += kThreads) span[i] = 0.0f;
+        __syncthreads();
+      }
     } else {
       // plain coalesced loader (clip stride or base not 16-byte aligned)
       const long g0 = (long)(g_first & ~3);
       const float* src = p.pcm + (size_t)clip * p.clip_stride;
       for (int i = tid; i < p.span_floats; i += kThreads) {
         const long n = g0 + i;
-        span[i] = (n >= 0 && n < p.n_samples) ? __ldg(src + n) : 0.0f;
+        span[i] = (n >= 0 && n < len) ? __ldg(src + n) : 0.0f;
       }
       __syncthreads();
     }
@@ -295,7 +322,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 2 : 1)
       }
       if (p.preemph != 0.0f) {
         // samples from this frame's start to the end of the clip (frame start = f*hop - n_fft/2)
-        const long n_valid = p.n_samples - ((long)(t0 + f) * p.hop - NFFT / 2);
+        const long n_valid = len - ((long)(t0 + f) * p.hop - NFFT / 2);
         ph_load_pre<NFFT>(v, span, off, p.hop, tau, wreg, p.preemph, n_valid);
       } else if (p.vec_ok && !(shift & 1)) {
         ph_load<NFFT, true>(v, span, off, p.hop, tau, wreg);
@@ -388,7 +415,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 2 : 1)
     if (p.use_tma && p.span_bufs == 1 && (!p.early_tma || (p.debug_skip & 1)) && tid == 0 && tile + gridDim.x < n_tiles)
       issue_span<NFFT>(&tmap, p, nclip, ntin << tf_shift, s_span, &s_bar[0]);  // (profiling mode without FFT phase)
 
-    const int t_valid = min(p.TF, p.T - t0);
+    const int t_valid = min(p.TF, Tc - t0);
     if (p.power != nullptr) {
       float* dst = p.power + (size_t)clip * C::F * p.T + t0;
       for (int e = tid; e < C::F * p.TF; e += kThreads) {
@@ -406,9 +433,9 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 2 : 1)
         const int m0 = s_mb[worker], m1 = s_mb[worker + 1];
         float mx = -FLT_MAX;
         if (m0 < m1 && t < t_valid) {
-          float* dst = p.logmel + ((size_t)clip * p.n_mels + m0) * p.T + t0 + t;
+          float* dst = p.logmel + ((size_t)clip * p.n_mels + m0) * p.pitch + t0 + t;
           const float amin = p.amin;
-          const int T = p.T;
+          const int T = p.pitch;
           auto emit = [&](int, float val) {
             // 10*log10(x) = 10*log10(2) * log2(x); MUFU.LG2 is within 1e-6 dB here (x >= amin, never denormal)
             const float db = 3.01029995663981195f * fast_log2(fmaxf(amin, val));
@@ -463,7 +490,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 2 : 1)
         // acc: (frame g, band 2*t4), (g, 2*t4+1), (g+8, 2*t4), (g+8, 2*t4+1) of this unit
         const int tile = s_tile[n];
         const int band0 = (tile & 0xffff) + 2 * t4, nb = tile >> 16;
-        float* orow = p.logmel + ((size_t)clip * p.n_mels + band0) * p.T + t0 + 16 * m + g;
+        float* orow = p.logmel + ((size_t)clip * p.n_mels + band0) * p.pitch + t0 + 16 * m + g;
 #pragma unroll
         for (int e = 0; e < 4; ++e) {
           const int f = 16 * m + g + ((e & 2) ? 8 : 0);
@@ -471,7 +498,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 2 : 1)
             // 10*log10(x) = 10*log10(2) * log2(x); lg2.approx is within 1e-6 dB here (x >= amin, never denormal)
             const float val = acc[e] + (acc_hl[e] + acc_lh[e]);
             const float db = 3.01029995663981195f * fast_log2(fmaxf(p.amin, val));
-            orow[((e & 1) ? p.T : 0) + ((e & 2) ? 8 : 0)] = db;
+            orow[((e & 1) ? p.pitch : 0) + ((e & 2) ? 8 : 0)] = db;
             mx = fmaxf(mx, db);
           }
         }
@@ -487,9 +514,9 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 2 : 1)
       const int m0 = s_mb[worker], m1 = s_mb[worker + 1];
       float mx = -FLT_MAX;
       if (m0 < m1 && t < t_valid) {
-        float* dst = p.logmel + ((size_t)clip * p.n_mels + m0) * p.T + t0 + t;
+        float* dst = p.logmel + ((size_t)clip * p.n_mels + m0) * p.pitch + t0 + t;
         const float amin = p.amin;
-        const int T = p.T;
+        const int T = p.pitch;
         auto emit = [&](int, float val) {
           // 10*log10(x) = 10*log10(2) * log2(x); MUFU.LG2 is within 1e-6 dB here (x >= amin, never denormal)
           const float db = 3.01029995663981195f * fast_log2(fmaxf(amin, val));

@@ -174,6 +174,13 @@ struct StftTcArgs {
   const uint16_t* wtab;     // bf16 [2 nb rows (w1 bands, then w2 bands) x 272] canonical K-major
   float* logmel;
   int* clipmax;
+  int pitch;                // frames per log-mel row (T; the longest clip's T in a variable-length batch)
+  // variable-length batch (null: every clip has n_samples samples and T frames): samples and frames of each clip,
+  // and the first block of each clip over the blocks of all clips (vl_first[n_clips] = n_blocks)
+  const long* vl_len;
+  const int* vl_T;
+  const unsigned* vl_first;
+  int vl_clips;
 };
 
 // NBQ = bands per epilogue warp = nb / 4 (nb = the non-empty bands n_act rounded up to 16)
@@ -189,7 +196,8 @@ struct StftTcArgs {
 // issues it (nobody waits), and every warp picks the result up one transform later.
 // FAST160 = the bench / speech configuration (hop 160, TMA loader, no pre-emphasis) with the other load variants
 // compiled out: the tile loop loses four code paths and their run-time predicates.
-template <int NBQ, bool FAST160>
+// VL = a variable-length batch (StftTcArgs::vl_*); compiled out of the equal-length instantiations.
+template <int NBQ, bool FAST160, bool VL>
 __global__ void __launch_bounds__(kTcThreads, 1)
     stft_mel_tc_kernel(const __grid_constant__ CUtensorMap tmap, const StftTcArgs p) {
   using C = FftCfg<kNfft>;
@@ -266,13 +274,36 @@ __global__ void __launch_bounds__(kTcThreads, 1)
   const uint32_t idesc1 = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(NB >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
   const uint64_t wdesc = tc_desc(tc_smem_u32(s_w), 128, (uint32_t)(kTcKP / 8) * 128);
 
-  const int T = p.T, hop = FAST160 ? 160 : p.hop, lead = FAST160 ? 0 : p.lead;
+  const int hop = FAST160 ? 160 : p.hop, lead = FAST160 ? 0 : p.lead;
   const uint32_t n_boxes = (uint32_t)span_alloc / kBox;
+  auto clip_len = [&](int clip) -> long { return VL ? p.vl_len[clip] : p.n_samples; };
+  auto clip_T = [&](int clip) -> int { return VL ? p.vl_T[clip] : p.T; };
 
   // block sequence of this CTA: blocks blockIdx.x, + gridDim.x, ...; 1 or 2 tiles of 64 frames per block
   auto block_pos = [&](unsigned blk, int& clip, int& t0) {
+    if (VL) {  // the last clip whose first block is <= blk (clips without blocks are skipped over)
+      int lo = 0, hi = p.vl_clips - 1;
+      while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (p.vl_first[mid] <= blk) lo = mid;
+        else hi = mid - 1;
+      }
+      clip = lo;
+      t0 = (int)(blk - p.vl_first[lo]) * kTcBlock;
+      return;
+    }
     clip = (int)(blk / p.blocks_per_clip);
     t0 = (int)(blk - (unsigned)clip * p.blocks_per_clip) * kTcBlock;
+  };
+  // variable-length batch: the TMA fills the span from the padded buffer, whose samples at and past the clip's end
+  // must read as zero -- overwrite them before the group's frames load (the group syncs only when it wrote)
+  auto zero_tail = [&](int clip, int t0) {
+    if (!VL) return;
+    const long g0 = (long)(((t0 + 16 * q) * hop - kNfft / 2 - lead) & ~3);
+    const long from = clip_len(clip) - g0;
+    if (from >= span_alloc) return;
+    for (long i = max(0L, from) + 32 * cg + lane; i < span_alloc; i += 128) span[i] = 0.0f;
+    group_sync();
   };
   // warp cg == 0 of the group: the PCM span of the group's 16 frames of tile t0, one 1 KB box per TMA
   auto issue_span = [&](int clip, int t0) {
@@ -288,9 +319,10 @@ __global__ void __launch_bounds__(kTcThreads, 1)
   auto fill_span = [&](int clip, int t0) {
     const long g0 = (long)(((t0 + 16 * q) * hop - kNfft / 2 - lead) & ~3);
     const float* src = p.pcm + (size_t)clip * p.clip_stride;
+    const long len = clip_len(clip);
     for (int i = 32 * cg + lane; i < p.span_floats; i += 128) {
       const long n = g0 + i;
-      span[i] = (n >= 0 && n < p.n_samples) ? __ldg(src + n) : 0.0f;
+      span[i] = (n >= 0 && n < len) ? __ldg(src + n) : 0.0f;
     }
     group_sync();
   };
@@ -314,9 +346,10 @@ __global__ void __launch_bounds__(kTcThreads, 1)
     }
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
     const int t = t0 + kTcTF * hw + 16 * q + (lane & 15);
+    const int pitch = p.pitch;
     float mx = -FLT_MAX;
-    if (t < T) {
-      float* dst = p.logmel + ((size_t)clip * p.n_mels + NBQ * cg) * T + t;
+    if (t < clip_T(clip)) {
+      float* dst = p.logmel + ((size_t)clip * p.n_mels + NBQ * cg) * pitch + t;
       const int n_here = min(NBQ, p.n_act - NBQ * cg);  // bands of this warp that exist
       const float amin = p.amin;
 #pragma unroll
@@ -325,7 +358,7 @@ __global__ void __launch_bounds__(kTcThreads, 1)
           // 10*log10(x) = 10*log10(2) * log2(x); MUFU.LG2 is within 1e-6 dB here (x >= amin, never denormal)
           const float db = 3.01029995663981195f * tc_log2(fmaxf(amin, d1[i] + d2[i]));
           *dst = db;
-          dst += T;
+          dst += pitch;
           mx = fmaxf(mx, db);
         }
       }
@@ -350,7 +383,7 @@ __global__ void __launch_bounds__(kTcThreads, 1)
   int pclip = 0, pt0 = 0;
 
   while (blk < p.n_blocks) {
-    const int n_tiles = (t0b + kTcTF < T) ? 2 : 1;
+    const int n_tiles = (t0b + kTcTF < clip_T(clip)) ? 2 : 1;
     const unsigned nblk = blk + gridDim.x;
     int nclip = clip + (int)step_q;
     unsigned nbin = bin + step_r;
@@ -358,7 +391,8 @@ __global__ void __launch_bounds__(kTcThreads, 1)
       nbin -= p.blocks_per_clip;
       ++nclip;
     }
-    const int nt0b = (int)nbin * kTcBlock;
+    int nt0b = (int)nbin * kTcBlock;
+    if (VL && nblk < p.n_blocks) block_pos(nblk, nclip, nt0b);
     for (int j = 0; j < n_tiles; ++j) {
       const int t0 = t0b + kTcTF * j;
       const int g_first = (t0 + 16 * q) * hop - kNfft / 2 - lead;
@@ -373,6 +407,7 @@ __global__ void __launch_bounds__(kTcThreads, 1)
         if constexpr (FAST160) {
           tc_mbar_wait(bar_tma, tma_par);
           tma_par ^= 1u;
+          zero_tail(clip, t0);
           // (shift == 0: the spans start 16-byte aligned.)  The 25 ms window of speech front ends (400 of 512) as
           // compile-time bounds: the 21 load predicates of the generic form disappear
           if (p.win_lo == 1 && p.win_hi == 15)
@@ -383,11 +418,12 @@ __global__ void __launch_bounds__(kTcThreads, 1)
           if (p.use_tma) {
             tc_mbar_wait(bar_tma, tma_par);
             tma_par ^= 1u;
+            zero_tail(clip, t0);
           } else {
             fill_span(clip, t0);  // (the previous tile's frames left the buffer before its first barrier)
           }
           if (p.preemph != 0.0f) {
-            const long n_valid = p.n_samples - ((long)(t0 + 16 * q + f_own) * hop - kNfft / 2);
+            const long n_valid = clip_len(clip) - ((long)(t0 + 16 * q + f_own) * hop - kNfft / 2);
             ph_load_pre<kNfft>(v, span, off, hop, tau, wreg, p.preemph, n_valid);
           } else if (hop == 160 && !(shift & 1)) {
             ph_load_shared<kNfft, 5, true>(v, span, off, tau, wreg, p.win_lo, p.win_hi);
@@ -520,13 +556,18 @@ __global__ void __launch_bounds__(kTcThreads, 1)
 
 // Bands without a single FFT bin (fmax above the Nyquist frequency: the reference's GUI default asks for 10 kHz at a
 // 10 kHz sampling rate, script/main.py:739) are not part of the GEMM: mel power 0 -> the amin floor, as librosa gives.
-__global__ void mel_empty_bands_kernel(float* __restrict__ logmel, int* __restrict__ clipmax, int T, int n_mels,
-                                       int n_act, float amin) {
+// vT (variable-length batch, else null): frames of each clip, 0 for a clip this launch does not cover.
+__global__ void mel_empty_bands_kernel(float* __restrict__ logmel, int* __restrict__ clipmax, int T, int pitch,
+                                       const int* __restrict__ vT, int n_mels, int n_act, float amin) {
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   const int clip = blockIdx.y;
+  if (vT) {
+    T = vT[clip];
+    if (T == 0) return;
+  }
   const float db0 = 3.01029995663981195f * tc_log2(fmaxf(amin, 0.0f));
   if (t < T)
-    for (int b = n_act; b < n_mels; ++b) logmel[((size_t)clip * n_mels + b) * T + t] = db0;
+    for (int b = n_act; b < n_mels; ++b) logmel[((size_t)clip * n_mels + b) * pitch + t] = db0;
   if (blockIdx.x == 0 && threadIdx.x == 0) atomicMax(clipmax + clip, tc_float_key(db0));
 }
 
@@ -595,19 +636,27 @@ cudaError_t stft_mel_tc_launch(const CUtensorMap& tmap, int use_tma, const float
                                long clip_stride, int T, int hop,
                                int lead, int n_mels, int n_act, float amin, float preemph, const float* window, int win_lo,
                                int win_hi, const float2* tw1, const void* wtab, float* logmel, int* clipmax,
-                               int sm_count, cudaStream_t st) {
+                               int sm_count, cudaStream_t st, const Varlen* vl) {
   StftTcArgs a{};
   a.win_lo = win_lo;
   a.win_hi = win_hi;
   const long bpc = (T + kTcBlock - 1) / kTcBlock;
   if (bpc * n_clips > 0x7fffffffL) return cudaErrorInvalidValue;
+  a.pitch = T;
+  if (vl) {
+    a.vl_len = vl->len;
+    a.vl_T = vl->T;
+    a.vl_first = vl->first;
+    a.vl_clips = (int)n_clips;
+    a.pitch = vl->pitch;
+  }
   a.pcm = pcm;
   a.n_samples = n_samples;
   a.clip_stride = clip_stride;
   a.use_tma = use_tma;
   a.span_floats = 15 * hop + kNfft + lead + 3;
   a.blocks_per_clip = (unsigned)bpc;
-  a.n_blocks = (unsigned)(bpc * n_clips);
+  a.n_blocks = vl ? (unsigned)vl->n_units : (unsigned)(bpc * n_clips);
   a.T = T;
   a.hop = hop;
   a.span_alloc = stft_mel_tc_span_alloc(hop, lead);
@@ -626,16 +675,20 @@ cudaError_t stft_mel_tc_launch(const CUtensorMap& tmap, int use_tma, const float
   const size_t smem = tc_smem_bytes(a.span_alloc, nb);
   const unsigned grid = (unsigned)std::min<long>((long)a.n_blocks, (long)sm_count);
   const bool fast160 = hop == 160 && use_tma && preemph == 0.0f && lead == 0 && a.span_alloc == 3072;
+#define MMF_TCMEL_LAUNCH(NBQ, F, V)                                \
+  {                                                                \
+    auto kfn = stft_mel_tc_kernel<NBQ, F, V>;                      \
+    MMF_SMEM_ONCE(kfn, 227 * 1024);                                \
+    kfn<<<grid, kTcThreads, smem, st>>>(tmap, a);                  \
+  }
 #define MMF_TCMEL_CASE(NBQ)                                        \
   case NBQ: {                                                      \
     if (fast160) {                                                 \
-      auto kfn = stft_mel_tc_kernel<NBQ, true>;                    \
-      MMF_SMEM_ONCE(kfn, 227 * 1024);                              \
-      kfn<<<grid, kTcThreads, smem, st>>>(tmap, a);                \
+      if (vl) MMF_TCMEL_LAUNCH(NBQ, true, true)                    \
+      else MMF_TCMEL_LAUNCH(NBQ, true, false)                      \
     } else {                                                       \
-      auto kfn = stft_mel_tc_kernel<NBQ, false>;                   \
-      MMF_SMEM_ONCE(kfn, 227 * 1024);                              \
-      kfn<<<grid, kTcThreads, smem, st>>>(tmap, a);                \
+      if (vl) MMF_TCMEL_LAUNCH(NBQ, false, true)                   \
+      else MMF_TCMEL_LAUNCH(NBQ, false, false)                     \
     }                                                              \
     break;                                                         \
   }
@@ -650,12 +703,14 @@ cudaError_t stft_mel_tc_launch(const CUtensorMap& tmap, int use_tma, const float
     default: return cudaErrorInvalidValue;
   }
 #undef MMF_TCMEL_CASE
+#undef MMF_TCMEL_LAUNCH
   cudaError_t e = cudaGetLastError();
   if (e == cudaSuccess && n_act < n_mels) {
     for (long c0 = 0; c0 < n_clips && e == cudaSuccess; c0 += 65535) {
       const unsigned nc = (unsigned)std::min<long>(65535, n_clips - c0);
-      mel_empty_bands_kernel<<<dim3((unsigned)((T + 255) / 256), nc), 256, 0, st>>>(
-          logmel + (size_t)c0 * n_mels * T, clipmax + c0, T, n_mels, n_act, amin);
+      mel_empty_bands_kernel<<<dim3((unsigned)((a.pitch + 255) / 256), nc), 256, 0, st>>>(
+          logmel + (size_t)c0 * n_mels * a.pitch, clipmax + c0, T, a.pitch, vl ? vl->T + c0 : nullptr, n_mels, n_act,
+          amin);
       count_launch();
       e = cudaGetLastError();
     }

@@ -521,6 +521,47 @@ class Plan:
         )
         return {"totChange": tot, "logmel": logmel, "mfcc": mfcc, "delta": delta}
 
+    def mfcc_change_varlen(self, pcm, lengths, prm: mmf_change_params, *, want_logmel=False, want_mfcc=False,
+                           want_delta=False):
+        """:meth:`mfcc_change` for clips of different lengths: row ``i`` of ``pcm`` ``[B, N_max]`` holds clip ``i`` in
+        its first ``lengths[i]`` samples (whatever follows is ignored).  Outputs are padded to the longest clip's
+        frame count; frames ``[0, frames[i])`` of clip ``i`` equal :meth:`mfcc_change` on that clip alone, bit for
+        bit, and the rest is 0.  Returns the dict of :meth:`mfcc_change` plus ``frames`` (numpy int64 ``[B]``)."""
+        torch = _torch()
+        pcm = self._pcm(pcm)
+        B, N = pcm.shape
+        lens = np.ascontiguousarray(np.asarray(lengths, dtype=np.int64).reshape(-1))
+        if lens.shape[0] != B:
+            raise ValueError(f"lengths has {lens.shape[0]} entries for {B} clips")
+        # mmf_num_frames for every clip at once (a ctypes call per clip costs ~1 us each)
+        padded = lens + 2 * (self.cfg.n_fft // 2)
+        frames = np.where(padded < self.cfg.n_fft, 0, 1 + np.maximum(padded - self.cfg.n_fft, 0) // self.cfg.hop_length)
+        T = int(frames.max()) if B else 0
+        tot = torch.empty((B, T), device=self.device, dtype=torch.float64)
+        logmel = torch.empty((B, self.cfg.n_mels, T), device=self.device, dtype=torch.float32) if want_logmel else None
+        mfcc = (
+            torch.empty((B, self.cfg.n_mfcc, T), device=self.device, dtype=torch.float32)
+            if (want_mfcc or want_delta)
+            else None
+        )
+        delta = torch.empty((B, self.cfg.n_mfcc, T), device=self.device, dtype=torch.float32) if want_delta else None
+        check(
+            _lib.lib().mmf_mfcc_change_varlen(
+                self._h,
+                pcm.data_ptr(),
+                B,
+                lens.ctypes.data,
+                pcm.stride(0) if B > 1 else N,
+                C.byref(prm),
+                tot.data_ptr(),
+                logmel.data_ptr() if logmel is not None else None,
+                mfcc.data_ptr() if mfcc is not None else None,
+                delta.data_ptr() if delta is not None else None,
+                _stream_ptr(self.device),
+            )
+        )
+        return {"totChange": tot, "logmel": logmel, "mfcc": mfcc, "delta": delta, "frames": frames}
+
     def change_from_logmel(self, logmel, clipmax, prm: mmf_change_params, *, want_delta=True, clamp_in_place=True):
         """Second half of :meth:`mfcc_change` for a log-mel already on the device."""
         torch = _torch()
