@@ -154,6 +154,20 @@ int mmf_modspec(mmf_plan* plan, const float* mfcc_dev, int64_t n_clips, int32_t 
                 int32_t hop, int32_t nfft, float* mag_dev, float* band_dev, const int32_t* band_lo_host,
                 const int32_t* band_hi_host, int32_t n_bands, void* stream);
 
+/* mmf_modspec for clips of different lengths in one call.  Clip i is n_coef rows of T_host[i] valid frames at
+ * mfcc_dev + i * n_coef * pitch, rows pitch frames apart (0 <= T_host[i] <= pitch); frames >= T_host[i] are never
+ * read into any output.  n_win_i = 1 + (T_host[i] - win) / hop (0 when T_host[i] < win), W = max n_win_i; outputs
+ * are padded to W: optional mag_dev [n_clips, n_coef, W, nfft/2+1] and band_dev [n_clips, W, n_bands].  Windows
+ * [0, n_win_i) of clip i are bit-identical to mmf_modspec on that clip alone (n_clips = 1, T = T_host[i], rows
+ * contiguous); every element at a window >= n_win_i is 0.  W = 0 launches nothing.  All arguments are checked
+ * before anything is launched (the lengths and the geometry without a plan or a device: a bad T_host[i] fails
+ * with MMF_ERR_INVALID, the message naming its index).  Each clip takes the kernel its own call takes; clips on
+ * the tcgen05 and the clip-resident kernels run in one launch per kernel for the whole batch (more than 2^31 - 1
+ * work items: MMF_ERR_UNSUPPORTED), the others one by one. */
+int mmf_modspec_varlen(mmf_plan* plan, const float* mfcc_dev, int64_t n_clips, int32_t n_coef, const int64_t* T_host,
+                       int64_t pitch, int32_t win, int32_t hop, int32_t nfft, float* mag_dev, float* band_dev,
+                       const int32_t* band_lo_host, const int32_t* band_hi_host, int32_t n_bands, void* stream);
+
 /* RMS envelope: librosa.feature.rms(frame_length, hop_length, center,
  * pad_mode='constant') (script/calc.py:326-331, script/mfcc.py:247) ->
  * rms_dev [n_clips, T_rms] float32, T_rms = 1 + (n + 2*pad - frame_length)/hop. */

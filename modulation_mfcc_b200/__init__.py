@@ -31,6 +31,7 @@ from .api import (  # noqa: F401
     get_velocity,
     load_channel,
     mfcc_features_batch,
+    mfcc_features_many,
     modspec_sizes,
 )
 from .shard import PeerGather, gather_features, shard_range, shard_sizes  # noqa: F401

@@ -174,6 +174,7 @@ _SIGNATURES = {
     "mmf_fir_filtfilt": (C.c_int, [_vp, _vp, _i64, _i64, _vp, _i32, _vp, _vp, _vp]),
     "mmf_stencil": (C.c_int, [_vp, _vp, _i64, _i64, _vp, _i32, _vp, _vp, _i32, _i32, _vp, _vp]),
     "mmf_modspec": (C.c_int, [_vp, _vp, _i64, _i32, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _i32, _vp]),
+    "mmf_modspec_varlen": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _i32, _vp]),
     "mmf_rms": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _i32, _i32, _i32, _vp, _vp]),
     "mmf_mfcc_change": (
         C.c_int,

@@ -830,6 +830,26 @@ class FeatureExtractor:
             res["modspec"], res["band_energy"] = mag, band
         return res
 
+    def varlen(self, pcm, lengths, *, want_logmel: bool = True, want_modspec: bool = True):
+        """:meth:`__call__` for clips of different lengths: row ``i`` of ``pcm [B, N_max]`` holds clip ``i`` in its
+        first ``lengths[i]`` samples (whatever follows is ignored).  Returns the dict of :meth:`__call__`, padded
+        to the longest clip (frames) and to the most modulation windows of any clip, plus ``frames`` and
+        ``windows`` (numpy int64 ``[B]``); clip ``i``'s first ``frames[i]`` frames and ``windows[i]`` windows equal
+        :meth:`__call__` on that clip alone, bit for bit, and the padding is 0."""
+        res = self.plan.mfcc_change_varlen(pcm, lengths, self.prm, want_logmel=want_logmel, want_mfcc=True,
+                                           want_delta=True)
+        frames = res["frames"]
+        # the modulation geometry does not depend on T, only each clip's window count does
+        Lw, Hw, nfft, _ = modspec_sizes(0, self.frame_rate, self.mod_win_s, self.mod_hop_s)
+        if want_modspec:
+            mag, band, windows = self.plan.modspec_varlen(res["mfcc"], frames, Lw, Hw, nfft,
+                                                          band_bins(nfft, self.frame_rate, self.bands_hz))
+            res["modspec"], res["band_energy"] = mag, band
+        else:
+            windows = np.where(frames >= Lw, 1 + (frames - Lw) // Hw, 0)
+        res["windows"] = windows
+        return res
+
 
 def mfcc_features_batch(audio, sr, *, device=None, **kw):
     """One-shot :class:`FeatureExtractor` call; numpy in -> numpy out, CUDA in -> CUDA out."""
@@ -845,3 +865,58 @@ def mfcc_features_batch(audio, sr, *, device=None, **kw):
     if not on_device:
         res = {k: (v.cpu().numpy() if hasattr(v, "cpu") else v) for k, v in res.items()}
     return res
+
+
+def mfcc_features_many(clips, sr, *, device=None, **kw):
+    """:func:`mfcc_features_batch` for a list of 1-D clips of any lengths, in one batched call
+    (:meth:`FeatureExtractor.varlen`).
+
+    ``clips`` holds numpy arrays and/or CUDA tensors.  Returns one dict per clip, equal bit for bit to
+    ``mfcc_features_batch(clip[None], sr, **kw)`` with the batch axis dropped: numpy for a numpy clip, CUDA tensors
+    for a CUDA clip.  A clip too short for the filters raises the single-clip call's ``ValueError``, its message
+    naming the clip's index."""
+    torch = _torch()
+    clips = [c if isinstance(c, torch.Tensor) else np.asarray(c) for c in clips]
+    for c in clips:
+        _require_float_audio(c)
+        if c.ndim != 1:
+            raise ValueError("mfcc_features_many takes 1-D clips")
+    if not clips:
+        return []
+    fx = FeatureExtractor(sr, device=device, **kw)
+    lengths = [int(c.shape[0]) for c in clips]
+    n_max = max(max(lengths), 1)
+    dev = fx.plan.device
+    if all(not isinstance(c, torch.Tensor) for c in clips):  # one host->device copy of the padded batch
+        host = np.zeros((len(clips), n_max), np.float32)
+        for i, c in enumerate(clips):
+            host[i, : lengths[i]] = c
+        pcm = torch.as_tensor(host).to(dev)
+    else:
+        pcm = torch.zeros((len(clips), n_max), device=dev, dtype=torch.float32)
+        for i, c in enumerate(clips):
+            pcm[i, : lengths[i]] = c.to(dev) if isinstance(c, torch.Tensor) else torch.as_tensor(np.asarray(c, np.float32))
+    try:
+        res = fx.varlen(pcm, lengths)
+    except MmfError as e:
+        _raise_from(e)
+    frames, windows = res.pop("frames"), res.pop("windows")
+    on_dev = [isinstance(c, torch.Tensor) and c.is_cuda for c in clips]
+    host = {k: v.cpu().numpy() for k, v in res.items() if v is not None} if not all(on_dev) else {}
+    out = []
+    for i in range(len(clips)):
+        src = res if on_dev[i] else host
+        T, W = int(frames[i]), int(windows[i])
+        d = {
+            "totChange": src["totChange"][i, :T],
+            "logmel": src["logmel"][i, :, :T],
+            "mfcc": src["mfcc"][i, :, :T],
+            "delta": src["delta"][i, :, :T],
+            "modspec": src["modspec"][i, :, :W],
+            "band_energy": src["band_energy"][i, :W],
+        }
+        if not on_dev[i]:
+            d = {k: np.ascontiguousarray(v) for k, v in d.items()}
+        d["T"] = _time_anchors(T, fx.tStep, fx.winLen)
+        out.append(d)
+    return out

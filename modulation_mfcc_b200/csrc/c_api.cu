@@ -186,30 +186,61 @@ static int validate_modspec(int win, int hop, int nfft, int n_bands, const int* 
   return MMF_OK;
 }
 
+ModRoute modspec_route(int win, int hop, int nfft, int n_coef, int n_bands, long T, unsigned flags, long n_clips) {
+  if (T < win || hop < 1) return ModRoute{kModNone, 0, 0};
+  const long n_win = 1 + (T - win) / hop;
+  // a kernel that would need more than 2^31 - 1 work items for the batch leaves it to the next one
+  auto chunked = [&](ModPath path, long wc) {
+    const long n_chunks = (n_win + wc - 1) / wc;
+    return wc > 0 && n_clips * n_chunks <= 0x7fffffffL ? ModRoute{path, wc, n_chunks} : ModRoute{kModNone, 0, 0};
+  };
+  if (!(flags & MMF_FLAG_NO_TC_MODSPEC)) {
+    // windowed DFT of 128 trajectory windows at a time as one tcgen05 GEMM (modspec_tc.cu)
+    const ModRoute r = chunked(kModTc, modspec_tc_chunk(win, hop, nfft, n_coef, n_bands, T));
+    if (r.path != kModNone) return r;
+  }
+  if (!modspec_fast_supported(nfft)) return ModRoute{kModGeneric, 0, 0};
+  const ModRoute r = chunked(kModClip, modspec_clip_chunk(win, hop, nfft, n_coef, n_bands, T));
+  return r.path != kModNone ? r : ModRoute{kModFast, 0, 0};
+}
+
+// launch route r (modspec_route) for n_clips clips of T frames; vl: a ragged batch of tc / clip work items instead
+static int launch_modspec(mmf_plan* p, const ModRoute& r, const float* mfcc, int64_t n_clips, int n_coef, int64_t T,
+                          int win, int hop, int nfft, float* mag, float* band, int n_bands, cudaStream_t st,
+                          const ModVarlen* vl = nullptr) {
+  float* b = n_bands > 0 ? band : nullptr;
+  cudaError_t e = cudaSuccess;
+  switch (r.path) {
+    case kModNone: return MMF_OK;
+    case kModTc:
+      e = modspec_tc_launch(mfcc, n_clips, n_coef, T, win, hop, nfft, p->d_mod_g, p->mod_g_kp, r.wc, mag, b,
+                            p->d_mod_lo, p->d_mod_hi, n_bands, p->sm_count, st, vl);
+      if (e != cudaSuccess) return cuda_fail(e, "modspec_tc_kernel launch");
+      return MMF_OK;
+    case kModClip:
+      e = modspec_clip_launch(mfcc, n_clips, n_coef, T, win, hop, nfft, r.wc, p->d_mod_hann, p->d_mod_tw1,
+                              p->d_mod_tw2, mag, b, p->d_mod_lo, p->d_mod_hi, n_bands, st, vl);
+      break;
+    case kModFast:
+      e = modspec_fast_launch(mfcc, n_clips, n_coef, T, win, hop, nfft, p->d_mod_hann, p->d_mod_tw1, p->d_mod_tw2, mag,
+                              b, p->d_mod_lo, p->d_mod_hi, n_bands, p->sm_count, st);
+      break;
+    case kModGeneric:
+      e = modspec_launch(mfcc, n_clips, n_coef, T, win, hop, nfft, mag, b, p->d_mod_lo, p->d_mod_hi, n_bands, st);
+      break;
+  }
+  if (e != cudaSuccess) return cuda_fail(e, "modspec kernel launch");
+  return MMF_OK;
+}
+
 static int run_modspec(mmf_plan* p, const float* mfcc, int64_t n_clips, int n_coef, int64_t T, int win, int hop,
                        int nfft, float* mag, float* band, const int* lo, const int* hi, int n_bands, cudaStream_t st) {
   if (T < win) return MMF_OK;
   if (!band) n_bands = 0;
   int rc = ensure_mod_tables(p, win, nfft, lo, hi, n_bands);
   if (rc) return rc;
-  cudaError_t e;
-  if (p->d_mod_g != nullptr) {
-    // windowed DFT of 128 trajectory windows at a time as one tcgen05 GEMM (modspec_tc.cu)
-    bool handled = false;
-    e = modspec_tc_launch(mfcc, n_clips, n_coef, T, win, hop, nfft, p->d_mod_g, p->mod_g_kp, mag,
-                          n_bands > 0 ? band : nullptr, p->d_mod_lo, p->d_mod_hi, n_bands, p->sm_count, st, &handled);
-    if (e != cudaSuccess) return cuda_fail(e, "modspec_tc_kernel launch");
-    if (handled) return MMF_OK;
-  }
-  if (modspec_fast_supported(nfft)) {
-    e = modspec_fast_launch(mfcc, n_clips, n_coef, T, win, hop, nfft, p->d_mod_hann, p->d_mod_tw1, p->d_mod_tw2, mag,
-                            n_bands > 0 ? band : nullptr, p->d_mod_lo, p->d_mod_hi, n_bands, p->sm_count, st);
-  } else {
-    e = modspec_launch(mfcc, n_clips, n_coef, T, win, hop, nfft, mag, n_bands > 0 ? band : nullptr, p->d_mod_lo,
-                       p->d_mod_hi, n_bands, st);
-  }
-  if (e != cudaSuccess) return cuda_fail(e, "modspec kernel launch");
-  return MMF_OK;
+  const ModRoute r = modspec_route(win, hop, nfft, n_coef, n_bands, T, p->cfg.flags, n_clips);
+  return launch_modspec(p, r, mfcc, n_clips, n_coef, T, win, hop, nfft, mag, band, n_bands, st);
 }
 
 // ---- stages of mmf_plan_create for the register FFT (host computations only)
@@ -984,6 +1015,125 @@ int mmf_modspec(mmf_plan* plan, const float* mfcc_dev, int64_t n_clips, int32_t 
   MMF_CUDA(cudaSetDevice(plan->cfg.device));
   return run_modspec(plan, mfcc_dev, n_clips, n_coef, T, win, hop, nfft, mag_dev, band_dev, band_lo_host, band_hi_host,
                      n_bands, (cudaStream_t)stream);
+}
+
+// Variable-length batch.  Each clip takes the route and the chunking its own mmf_modspec call would take
+// (modspec_route) -- which is what makes its outputs bit-identical to that call.  Clips on the tcgen05 and the
+// clip-resident kernel run in one launch per kernel for the whole batch, as a compacted list of (clip, chunk) work
+// items; clips on the fast or the generic kernel run one by one through workspace and are copied into their padded
+// rows.  One launch then zeroes every window past a clip's own.
+int mmf_modspec_varlen(mmf_plan* plan, const float* mfcc_dev, int64_t n_clips, int32_t n_coef, const int64_t* T_host,
+                       int64_t pitch, int32_t win, int32_t hop, int32_t nfft, float* mag_dev, float* band_dev,
+                       const int32_t* band_lo_host, const int32_t* band_hi_host, int32_t n_bands, void* stream) {
+  using namespace mmf;
+  // the geometry and the lengths first: these checks need neither a plan nor a device
+  int rc = validate_modspec(win, hop, nfft, n_bands, band_lo_host, band_hi_host, band_dev != nullptr);
+  if (rc) return rc;
+  if (!T_host) return fail(MMF_ERR_INVALID, "T_host is NULL");
+  if (n_clips < 1 || n_coef < 1) return fail(MMF_ERR_INVALID, "n_clips and n_coef must be positive");
+  if (n_clips > 0x7fffffff) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 clips");
+  int64_t W = 0;  // windows per output row: the most of any clip
+  for (int64_t i = 0; i < n_clips; ++i) {
+    const int64_t T = T_host[i];
+    if (T < 0 || T > pitch) {
+      char buf[160];
+      std::snprintf(buf, sizeof(buf), "clip %lld: T %lld must be in [0, pitch = %lld]", (long long)i, (long long)T,
+                    (long long)pitch);
+      return fail(MMF_ERR_INVALID, buf);
+    }
+    if (T >= win) W = std::max<int64_t>(W, 1 + (T - win) / hop);
+  }
+  if (!plan || !mfcc_dev) return fail(MMF_ERR_INVALID, "NULL argument");
+  if (W > 0x7fffffff) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 windows per clip");
+  if (W == 0) return MMF_OK;  // no clip reaches a window: nothing to compute or zero
+
+  // ---- routing (host only): each clip as its own call, the tc / clip kernels' chunks as work items
+  const int nbe = band_dev ? n_bands : 0;  // band outputs actually written
+  const int nb = nfft / 2 + 1;
+  std::vector<ModRoute> route((size_t)n_clips);
+  std::vector<int> n_win((size_t)n_clips, 0);
+  long n_items[2] = {0, 0}, wc_max[2] = {0, 0};  // [0] tc, [1] clip
+  std::vector<int64_t> single;                   // clips on the fast / generic kernel
+  bool tails = false;
+  for (int64_t i = 0; i < n_clips; ++i) {
+    const ModRoute r = modspec_route(win, hop, nfft, n_coef, nbe, T_host[i], (unsigned)plan->cfg.flags);
+    route[i] = r;
+    n_win[i] = T_host[i] >= win ? (int)(1 + (T_host[i] - win) / hop) : 0;
+    tails |= n_win[i] < W;
+    if (r.path == kModTc || r.path == kModClip) {
+      const int k = r.path == kModTc ? 0 : 1;
+      n_items[k] += r.n_chunks;
+      wc_max[k] = std::max(wc_max[k], r.wc);
+    } else if (r.path != kModNone) {
+      single.push_back(i);
+    }
+  }
+  if (n_items[0] > 0x7fffffffL || n_items[1] > 0x7fffffffL)
+    return fail(MMF_ERR_UNSUPPORTED, "variable-length batch of more than 2^31 - 1 modulation-spectrum work items");
+  std::vector<ModItem> items((size_t)(n_items[0] + n_items[1]));
+  {
+    size_t at[2] = {0, (size_t)n_items[0]};
+    for (int64_t i = 0; i < n_clips; ++i) {
+      const ModRoute& r = route[i];
+      if (r.path != kModTc && r.path != kModClip) continue;
+      size_t& k = at[r.path == kModTc ? 0 : 1];
+      for (long c = 0; c < r.n_chunks; ++c) {
+        const long w0 = c * r.wc;
+        items[k++] = ModItem{(int)i, (int)w0, (int)std::min<long>(r.wc, n_win[i] - w0), n_win[i]};
+      }
+    }
+  }
+
+  // ---- workspace: work items and window counts, then the single-clip region (input rows, magnitudes)
+  MMF_CUDA(cudaSetDevice(plan->cfg.device));
+  if ((rc = ensure_mod_tables(plan, win, nfft, band_lo_host, band_hi_host, nbe))) return rc;
+  const size_t n = (size_t)n_clips;
+  const size_t o_items = 0, o_nwin = align_up(items.size() * sizeof(ModItem), 256);
+  const size_t desc_bytes = o_nwin + n * 4;
+  const size_t o_single = align_up(desc_bytes, 256);
+  size_t single_bytes = 0;
+  for (int64_t i : single)
+    single_bytes = std::max(single_bytes, align_up((size_t)n_coef * T_host[i] * 4, 256) +
+                                              (mag_dev ? (size_t)n_coef * n_win[i] * nb * 4 : 0));
+  if ((rc = ensure_ws(plan, (64 << 10) + o_single + single_bytes))) return rc;
+  unsigned char* base = (unsigned char*)plan->ws + (64 << 10);
+  std::vector<unsigned char> desc(desc_bytes);
+  if (!items.empty()) std::memcpy(desc.data() + o_items, items.data(), items.size() * sizeof(ModItem));
+  std::memcpy(desc.data() + o_nwin, n_win.data(), n * 4);
+  cudaStream_t st = (cudaStream_t)stream;
+  MMF_CUDA(cudaMemcpyAsync(base, desc.data(), desc_bytes, cudaMemcpyHostToDevice, st));
+
+  // ---- the batched clips: one launch per kernel
+  for (int k = 0; k < 2; ++k) {
+    if (!n_items[k]) continue;
+    const ModVarlen vl{(const ModItem*)(base + o_items) + (k ? n_items[0] : 0), n_items[k], (long)W, (int)wc_max[k]};
+    const ModRoute r{k ? kModClip : kModTc, wc_max[k], 0};
+    if ((rc = launch_modspec(plan, r, mfcc_dev, n_clips, n_coef, pitch, win, hop, nfft, mag_dev, band_dev, nbe, st,
+                             &vl)))
+      return rc;
+  }
+
+  // ---- the other clips: the single-clip call on contiguous rows, copied into the padded rows
+  for (int64_t i : single) {
+    const size_t Ti = (size_t)T_host[i], wi = (size_t)n_win[i];
+    float* x1 = (float*)(base + o_single);
+    float* mag1 = mag_dev ? (float*)(base + o_single + align_up((size_t)n_coef * Ti * 4, 256)) : nullptr;
+    MMF_CUDA(cudaMemcpy2DAsync(x1, Ti * 4, mfcc_dev + (size_t)i * n_coef * pitch, (size_t)pitch * 4, Ti * 4,
+                               (size_t)n_coef, cudaMemcpyDeviceToDevice, st));
+    // a clip's band rows [n_win_i, n_bands] are the start of its padded rows [W, n_bands]: written in place
+    float* band1 = nbe > 0 ? band_dev + (size_t)i * W * nbe : nullptr;
+    if ((rc = launch_modspec(plan, route[i], x1, 1, n_coef, (int64_t)Ti, win, hop, nfft, mag1, band1, nbe, st)))
+      return rc;
+    if (mag1)
+      MMF_CUDA(cudaMemcpy2DAsync(mag_dev + (size_t)i * n_coef * W * nb, (size_t)W * nb * 4, mag1, wi * nb * 4,
+                                 wi * nb * 4, (size_t)n_coef, cudaMemcpyDeviceToDevice, st));
+  }
+  if (tails && (mag_dev || nbe > 0)) {
+    cudaError_t e = modspec_tails_launch((long)n_clips, (const int*)(base + o_nwin), (long)W, mag_dev, n_coef, nb,
+                                         nbe > 0 ? band_dev : nullptr, nbe, st);
+    if (e != cudaSuccess) return cuda_fail(e, "modspec_tails_kernel launch");
+  }
+  return MMF_OK;
 }
 
 int mmf_rms(mmf_plan* plan, const float* pcm_dev, int64_t n_clips, int64_t n_samples, int64_t clip_stride,

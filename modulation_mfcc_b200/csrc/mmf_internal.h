@@ -128,12 +128,42 @@ cudaError_t mfcc_tc_launch(const void* btab, int kp, float* logmel, const int* c
                            int n_mfcc, float top_db, float* mfcc, float* delta, int clamp_in_place, int sm_count,
                            cudaStream_t st);
 
+// ---- K6 routing: the kernel mmf_modspec runs for n_clips clips of T frames and the windows per CTA (wc) it cuts
+// each clip's windows into.  One function owns the decision (c_api.cu): mmf_modspec and mmf_modspec_varlen, which
+// routes every clip of a ragged batch as its own call would, both take it from here.  n_bands counts band outputs
+// actually written (0 without a band output); n_clips only matters through the grid limits.
+enum ModPath { kModNone = 0, kModTc, kModClip, kModFast, kModGeneric };
+struct ModRoute {
+  ModPath path;
+  long wc;        // tc / clip: windows per chunk
+  long n_chunks;  // tc / clip: chunks per clip
+};
+ModRoute modspec_route(int win, int hop, int nfft, int n_coef, int n_bands, long T, unsigned flags, long n_clips = 1);
+// the chunk sizes behind it: 0 when the kernel does not take the geometry
+long modspec_tc_chunk(int win, int hop, int nfft, int n_coef, int n_bands, long T);
+long modspec_clip_chunk(int win, int hop, int nfft, int n_coef, int n_bands, long T);
+
+// ---- a variable-length batch of K6 (mmf_modspec_varlen): the launch walks a compacted list of work items, one per
+// (clip, chunk of windows) exactly as the clip's own mmf_modspec call cuts it.  Input rows are the launch's T (the row
+// pitch) frames apart, output rows its n_win (the most windows of any clip) windows apart.
+struct alignas(16) ModItem {
+  int clip, w0, wca;  // clip, first window, windows of the chunk
+  int n_win;          // windows of the clip
+};
+struct ModVarlen {
+  const ModItem* items;
+  long n_items;
+  long n_win;  // windows per output row: the most windows of any clip
+  int wc_max;  // the most windows of any item: sizes shared memory
+};
+
 // ---- modulation spectrum as a tcgen05 GEMM (modspec_tc.cu)
 bool modspec_tc_supported(int win, int nfft);
 void modspec_tc_table(int win, int nfft, std::vector<uint16_t>& g, int* kp_out);
+// wc: modspec_route's chunk size (vl: the batch's items instead)
 cudaError_t modspec_tc_launch(const float* mfcc, long n_clips, int n_coef, long T, int win, int hop, int nfft,
-                              const void* g, int kp, float* mag, float* band, const int* lo, const int* hi,
-                              int n_bands, int sm_count, cudaStream_t st, bool* handled);
+                              const void* g, int kp, long wc, float* mag, float* band, const int* lo, const int* hi,
+                              int n_bands, int sm_count, cudaStream_t st, const ModVarlen* vl = nullptr);
 
 // ---- post-FFT kernels (post_kernels.cu)
 cudaError_t mfcc_launch(const float* dct_pad, int nc_pad, float* logmel, const int* clipmax, long n_clips, long T,
@@ -206,11 +236,18 @@ cudaError_t stencil_launch(const double* x, long rows, long T, const double* coe
                            const double* er_dev, int n_edge, int n_edge_in, double* y, cudaStream_t st);
 cudaError_t modspec_launch(const float* mfcc, long n_clips, int n_coef, long T, int win, int hop, int nfft, float* mag,
                            float* band, const int* band_lo_dev, const int* band_hi_dev, int n_bands, cudaStream_t st);
+cudaError_t modspec_tails_launch(long n_clips, const int* n_win, long W, float* mag, int n_coef, int nb, float* band,
+                                 int n_bands, cudaStream_t st);
 bool modspec_fast_supported(int nfft);
 void modspec_geometry(int nfft, StftGeometry* g);
 cudaError_t modspec_fast_launch(const float* mfcc, long n_clips, int n_coef, long T, int win, int hop, int nfft,
                                 const float* hann, const float2* tw1, const float2* tw2, float* mag, float* band,
                                 const int* lo, const int* hi, int n_bands, int sm_count, cudaStream_t st);
+// wc: modspec_route's chunk size (vl: the batch's items instead)
+cudaError_t modspec_clip_launch(const float* mfcc, long n_clips, int n_coef, long T, int win, int hop, int nfft,
+                                long wc, const float* hann, const float2* tw1, const float2* tw2, float* mag,
+                                float* band, const int* lo, const int* hi, int n_bands, cudaStream_t st,
+                                const ModVarlen* vl = nullptr);
 cudaError_t rms_launch(const float* pcm, long n_clips, long n, long stride, int frame_length, int hop, int pad,
                        long T, float* out, cudaStream_t st);
 cudaError_t fill_i32_launch(int* p, long n, int v, cudaStream_t st);

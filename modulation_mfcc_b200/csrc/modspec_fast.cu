@@ -177,13 +177,15 @@ static cudaError_t launch_t(const float* mfcc, long n_clips, int n_coef, long T,
 // over coefficients in shared memory -- no scattered global accesses, no atomics.
 // ---------------------------------------------------------------------------
 // V = float2: one (window, coefficient) item per thread group; V = c2: two items per thread
-// group on packed FP32 instructions (fft_regs.cuh), which halves the passes.
-template <int NFFT, typename V>
+// group on packed FP32 instructions (fft_regs.cuh), which halves the passes.  VARLEN: a ragged batch, the CTA's
+// (clip, chunk) is items[blockIdx.x], T the input row pitch and n_win the output window pitch.
+template <int NFFT, typename V, bool VARLEN>
 __global__ void __launch_bounds__(kModThreads, 2)
     modspec_clip_kernel(const float* __restrict__ mfcc, int n_coef, long T, int win, int hop, long n_win, int wc,
                         int n_chunks, int pitch, const float* __restrict__ hann, const float2* __restrict__ g_tw1,
                         const float2* __restrict__ g_tw2, float* __restrict__ mag, float* __restrict__ band,
-                        const int* __restrict__ band_lo, const int* __restrict__ band_hi, int n_bands) {
+                        const int* __restrict__ band_lo, const int* __restrict__ band_hi, int n_bands,
+                        const ModItem* __restrict__ items) {
   using C = FftCfg<NFFT>;
   using TR = CxTraits<V>;
   using Tw = typename TR::Tw;
@@ -205,10 +207,19 @@ __global__ void __launch_bounds__(kModThreads, 2)
   __shared__ int s_blo[16], s_bhi[16];
   const int tid = threadIdx.x;
   const int tau = tid % C::TPF, slot = tid / C::TPF;
-  const long clip = blockIdx.x / n_chunks;
-  const int chunk = (int)(blockIdx.x - clip * n_chunks);
-  const long w0 = (long)chunk * wc;
-  const int wca = (int)min((long)wc, n_win - w0);  // windows of this chunk
+  long clip, w0;
+  int wca;  // windows of this chunk
+  if constexpr (VARLEN) {
+    const ModItem it = items[blockIdx.x];
+    clip = it.clip;
+    w0 = it.w0;
+    wca = it.wca;
+  } else {
+    clip = blockIdx.x / n_chunks;
+    const int chunk = (int)(blockIdx.x - clip * n_chunks);
+    w0 = (long)chunk * wc;
+    wca = (int)min((long)wc, n_win - w0);
+  }
   const int span = (wca - 1) * hop + win;
 
   for (int i = tid; i < C::TW1; i += kModThreads) s_tw1[i] = make_tw<V>(g_tw1[i]);
@@ -415,65 +426,107 @@ __global__ void __launch_bounds__(kModThreads, 2)
   }
 }
 
+// the clip kernel's budget: its rows + per-item band sums within ~110 KB, so that two CTAs share an SM
 template <int NFFT>
-static cudaError_t launch_clip_t(const float* mfcc, long n_clips, int n_coef, long T, int win, int hop, const float* hann,
-                                 const float2* tw1, const float2* tw2, float* mag, float* band, const int* lo,
-                                 const int* hi, int n_bands, cudaStream_t st, bool* handled) {
+struct ClipSmem {
   using C = FftCfg<NFFT>;
-  *handled = false;
-  if constexpr (C::TPF > 32) {
-    return cudaSuccess;
-  } else {
-    constexpr int SLOTS = kModThreads / C::TPF;
-    constexpr int nb = NFFT / 2 + 1;
-    // two items per thread group (packed FP32) when both power rows fit in the slot's exchange buffer
-    constexpr bool kPacked = 2 * ((nb + 1) & ~1) * 4 <= C::XBUF * 8;
-    using V = typename std::conditional<kPacked, c2, float2>::type;
-    constexpr int NI = kPacked ? 2 : 1;
-    const long n_win = 1 + (T - win) / hop;
-    const int nbands = band != nullptr ? n_bands : 0;
-    // windows per chunk: rows + per-item band sums within ~110 KB so that two CTAs share an SM
+  static constexpr int SLOTS = kModThreads / C::TPF;
+  static constexpr int nb = NFFT / 2 + 1;
+  // two items per thread group (packed FP32) when both power rows fit in the slot's exchange buffer
+  static constexpr bool kPacked = 2 * ((nb + 1) & ~1) * 4 <= C::XBUF * 8;
+  using V = typename std::conditional<kPacked, c2, float2>::type;
+  static constexpr int NI = kPacked ? 2 : 1;
+  static constexpr size_t kBudget = 110 * 1024;
+  static size_t need(int n_coef, int win, int hop, int nbands, long w) {
     const size_t fixed = (size_t)SLOTS * C::XSTRIDE * 8 + (size_t)(C::TW1 + C::TW2 + 1) * sizeof(typename CxTraits<V>::Tw) +
                          (size_t)C::M * 8 + (size_t)SLOTS * NI * sizeof(float*) + 64;
-    const size_t budget = 110 * 1024;
-    long wc = n_win;
-    auto need = [&](long w) {
-      const long span = (w - 1) * hop + win;
-      const long pitch = (span + 1) & ~1L;
-      return fixed + (size_t)n_coef * pitch * 4 + ((((size_t)w * n_coef * nbands) + 1) & ~(size_t)1) * 4;
-    };
-    if (need(1) > budget) return cudaSuccess;  // not handled: the generic kernel takes it
-    while (wc > 1 && need(wc) > budget) wc = (wc + 1) / 2;
-    while (wc < n_win && need(wc + 1) <= budget) ++wc;
-    const long n_chunks = (n_win + wc - 1) / wc;
-    if (n_clips * n_chunks > 0x7fffffffL) return cudaSuccess;
-    const long span = (wc - 1) * hop + win;
-    const int pitch = (int)((span + 1) & ~1L);
-    auto kfn = modspec_clip_kernel<NFFT, V>;
-    MMF_SMEM_ONCE(kfn, 200 * 1024);
-    kfn<<<(unsigned)(n_clips * n_chunks), kModThreads, need(wc), st>>>(mfcc, n_coef, T, win, hop, n_win, (int)wc,
-                                                                        (int)n_chunks, pitch, hann, tw1, tw2, mag, band,
-                                                                        lo, hi, n_bands);
-    count_launch();
-    *handled = true;
-    return cudaGetLastError();
+    const long span = (w - 1) * hop + win;
+    const long pitch = (span + 1) & ~1L;
+    return fixed + (size_t)n_coef * pitch * 4 + ((((size_t)w * n_coef * nbands) + 1) & ~(size_t)1) * 4;
   }
+};
+
+// windows per CTA for one clip of T frames: as many as fit the budget (0: not even one fits, the fast kernel takes it)
+template <int NFFT>
+static long clip_chunk_t(int n_coef, int win, int hop, int nbands, long T) {
+  using S = ClipSmem<NFFT>;
+  const long n_win = 1 + (T - win) / hop;
+  long wc = n_win;
+  if (S::need(n_coef, win, hop, nbands, 1) > S::kBudget) return 0;
+  while (wc > 1 && S::need(n_coef, win, hop, nbands, wc) > S::kBudget) wc = (wc + 1) / 2;
+  while (wc < n_win && S::need(n_coef, win, hop, nbands, wc + 1) <= S::kBudget) ++wc;
+  return wc;
+}
+
+template <int NFFT>
+static cudaError_t launch_clip_t(const float* mfcc, long n_clips, int n_coef, long T, int win, int hop, long wc,
+                                 const float* hann, const float2* tw1, const float2* tw2, float* mag, float* band,
+                                 const int* lo, const int* hi, int n_bands, cudaStream_t st, const ModVarlen* vl) {
+  using S = ClipSmem<NFFT>;
+  const long n_win = vl ? vl->n_win : 1 + (T - win) / hop;
+  const int nbands = band != nullptr ? n_bands : 0;
+  const long wcs = vl ? vl->wc_max : wc;  // the largest chunk lays out shared memory
+  const long n_chunks = (n_win + wc - 1) / wc;
+  const long span = (wcs - 1) * hop + win;
+  const int pitch = (int)((span + 1) & ~1L);
+  const size_t smem = S::need(n_coef, win, hop, nbands, wcs);
+  const unsigned grid = (unsigned)(vl ? vl->n_items : n_clips * n_chunks);
+#define MMF_CLIP_LAUNCH(VL)                                                                                          \
+  {                                                                                                                  \
+    auto kfn = modspec_clip_kernel<NFFT, typename S::V, VL>;                                                         \
+    MMF_SMEM_ONCE(kfn, 200 * 1024);                                                                                  \
+    kfn<<<grid, kModThreads, smem, st>>>(mfcc, n_coef, T, win, hop, n_win, (int)wcs, (int)n_chunks, pitch, hann, tw1, \
+                                         tw2, mag, band, lo, hi, n_bands, vl ? vl->items : nullptr);                 \
+  }
+  if (vl)
+    MMF_CLIP_LAUNCH(true)
+  else
+    MMF_CLIP_LAUNCH(false)
+#undef MMF_CLIP_LAUNCH
+  count_launch();
+  return cudaGetLastError();
 }
 
 bool modspec_fast_supported(int nfft) { return nfft >= 32 && nfft <= 1024; }
+
+long modspec_clip_chunk(int win, int hop, int nfft, int n_coef, int n_bands, long T) {
+  if (T < win || hop < 1) return 0;
+  switch (nfft) {
+    case 32: return clip_chunk_t<32>(n_coef, win, hop, n_bands, T);
+    case 64: return clip_chunk_t<64>(n_coef, win, hop, n_bands, T);
+    case 128: return clip_chunk_t<128>(n_coef, win, hop, n_bands, T);
+    case 256: return clip_chunk_t<256>(n_coef, win, hop, n_bands, T);
+    case 512: return clip_chunk_t<512>(n_coef, win, hop, n_bands, T);
+    case 1024: return clip_chunk_t<1024>(n_coef, win, hop, n_bands, T);
+    default: return 0;
+  }
+}
+
+cudaError_t modspec_clip_launch(const float* mfcc, long n_clips, int n_coef, long T, int win, int hop, int nfft,
+                                long wc, const float* hann, const float2* tw1, const float2* tw2, float* mag,
+                                float* band, const int* lo, const int* hi, int n_bands, cudaStream_t st,
+                                const ModVarlen* vl) {
+#define MMF_MOD_CASE(N)                                                                                              \
+  case N:                                                                                                            \
+    return launch_clip_t<N>(mfcc, n_clips, n_coef, T, win, hop, wc, hann, tw1, tw2, mag, band, lo, hi, n_bands, st, vl);
+  switch (nfft) {
+    MMF_MOD_CASE(32)
+    MMF_MOD_CASE(64)
+    MMF_MOD_CASE(128)
+    MMF_MOD_CASE(256)
+    MMF_MOD_CASE(512)
+    MMF_MOD_CASE(1024)
+    default: return cudaErrorInvalidValue;
+  }
+#undef MMF_MOD_CASE
+}
 
 cudaError_t modspec_fast_launch(const float* mfcc, long n_clips, int n_coef, long T, int win, int hop, int nfft,
                                 const float* hann, const float2* tw1, const float2* tw2, float* mag, float* band,
                                 const int* lo, const int* hi, int n_bands, int sm_count, cudaStream_t st) {
   if (T < win) return cudaSuccess;
-#define MMF_MOD_CASE(N)                                                                                              \
-  case N: {                                                                                                          \
-    bool handled = false;                                                                                            \
-    cudaError_t e = launch_clip_t<N>(mfcc, n_clips, n_coef, T, win, hop, hann, tw1, tw2, mag, band, lo, hi, n_bands, \
-                                     st, &handled);                                                                  \
-    if (e != cudaSuccess || handled) return e;                                                                       \
-    return launch_t<N>(mfcc, n_clips, n_coef, T, win, hop, hann, tw1, tw2, mag, band, lo, hi, n_bands, sm_count, st); \
-  }
+#define MMF_MOD_CASE(N) \
+  case N: return launch_t<N>(mfcc, n_clips, n_coef, T, win, hop, hann, tw1, tw2, mag, band, lo, hi, n_bands, sm_count, st);
   switch (nfft) {
     MMF_MOD_CASE(32)
     MMF_MOD_CASE(64)

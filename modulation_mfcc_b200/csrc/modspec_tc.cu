@@ -103,7 +103,7 @@ struct ModTcArgs {
   int win, hop;
   long n_win;
   int wc, n_chunks;
-  long n_work;       // n_clips * n_chunks
+  long n_work;       // n_clips * n_chunks (VARLEN: the batch's items)
   int kp;            // win rounded up to 16
   const __half* g;   // [Ghi | Glo], each canonical K-major [NFFT rows x kp]
   float* mag;
@@ -111,11 +111,13 @@ struct ModTcArgs {
   const int* band_lo;
   const int* band_hi;
   int n_bands;
+  const ModItem* items;  // VARLEN: the batch's work items; T is then the row pitch, n_win the output window pitch
 };
 
 // half h, slot j (0..63): j < 32 -> Re X[32 h + j]; j >= 32 -> Im X[32 h + j - 32], except (h = 0, j = 32),
-// whose Im X[0] = 0 slot carries Re X[nfft / 2]
-template <int NFFT, int KS>
+// whose Im X[0] = 0 slot carries Re X[nfft / 2].  VARLEN: a ragged batch, work item = p.items[item] (the default
+// instantiation derives it from the item index and carries none of the ragged addressing).
+template <int NFFT, int KS, bool VARLEN>
 __global__ void __launch_bounds__(kMtThreads, 2) modspec_tc_kernel(const ModTcArgs p) {
   static_assert(NFFT == 128, "two halves of 32 bins");
   constexpr int nb = NFFT / 2 + 1;  // odd: conflict-free row pitch of the staging buffer
@@ -173,10 +175,21 @@ __global__ void __launch_bounds__(kMtThreads, 2) modspec_tc_kernel(const ModTcAr
 
   // persistent: the 57 KB operand table is loaded once per CTA, then (clip, chunk) work items round-robin
   for (long item = blockIdx.x; item < p.n_work; item += gridDim.x) {
-  const long clip = item / p.n_chunks;
-  const int chunk = (int)(item - clip * p.n_chunks);
-  const long w0 = (long)chunk * p.wc;
-  const int wca = (int)min((long)p.wc, p.n_win - w0);
+  long clip, w0, n_win_clip;  // n_win_clip: the clip's windows (p.n_win is the output pitch)
+  int wca;
+  if constexpr (VARLEN) {
+    const ModItem it = p.items[item];
+    clip = it.clip;
+    w0 = it.w0;
+    wca = it.wca;
+    n_win_clip = it.n_win;
+  } else {
+    clip = item / p.n_chunks;
+    const int chunk = (int)(item - clip * p.n_chunks);
+    w0 = (long)chunk * p.wc;
+    wca = (int)min((long)p.wc, p.n_win - w0);
+    n_win_clip = p.n_win;
+  }
   const int n_items = wca * p.n_coef;
   const int span = (wca - 1) * p.hop + p.win;
   for (int r0 = 0; r0 < n_items; r0 += kMtRows) {
@@ -184,7 +197,7 @@ __global__ void __launch_bounds__(kMtThreads, 2) modspec_tc_kernel(const ModTcAr
     const int c_lo = r0 / wca, c_hi = min(r0 + kMtRows - 1, n_items - 1) / wca;
     // whole clip in one chunk and the touched trajectories fit with their own pitch T: one flat copy
     const int n_tr = c_hi - c_lo + 1;
-    const bool flat_in = wca == p.n_win && (long)n_tr * p.T <= (long)kMtRows * nb;
+    const bool flat_in = wca == n_win_clip && (long)n_tr * p.T <= (long)kMtRows * nb;
     const int pitch = flat_in ? (int)p.T : span;
     if (flat_in) {
       const float* src0 = p.mfcc + ((size_t)clip * p.n_coef + c_lo) * p.T;
@@ -465,15 +478,13 @@ void modspec_tc_table(int win, int nfft, std::vector<uint16_t>& g, int* kp_out) 
   *kp_out = kp;
 }
 
-cudaError_t modspec_tc_launch(const float* mfcc, long n_clips, int n_coef, long T, int win, int hop, int nfft,
-                              const void* g, int kp, float* mag, float* band, const int* lo, const int* hi,
-                              int n_bands, int sm_count, cudaStream_t st, bool* handled) {
-  *handled = false;
-  if (!modspec_tc_supported(win, nfft) || T < win || hop < 1) return cudaSuccess;
+// windows per CTA for one clip of T frames (0: the kernel does not take it): the whole clip if its band table fits,
+// else chunks; a row block's trajectories (at most 128 / wc + 2 of them) must fit in the 128 x nb staging buffer
+long modspec_tc_chunk(int win, int hop, int nfft, int n_coef, int n_bands, long T) {
+  if (!modspec_tc_supported(win, nfft) || T < win || hop < 1) return 0;
   const int nb = nfft / 2 + 1;
+  const int kp = (win + 15) / 16 * 16;
   const long n_win = 1 + (T - win) / hop;
-  // windows per CTA: the whole clip if its band table fits, else chunks; a row block's trajectories
-  // (at most 128 / wc + 2 of them) must fit in the 128 x nb staging buffer
   long wc = n_win;
   auto fits = [&](long w) {
     const long span = (w - 1) * hop + win;
@@ -484,10 +495,19 @@ cudaError_t modspec_tc_launch(const float* mfcc, long n_clips, int n_coef, long 
     return n_tr * span <= (long)kMtRows * nb && fixed + w * n_coef * std::max(n_bands, 1) * 4 <= kMtSmemLimit - 2048;
   };
   while (wc > 1 && !fits(wc)) wc = (wc + 1) / 2;
-  if (!fits(wc)) return cudaSuccess;
+  if (!fits(wc)) return 0;
   const long n_chunks = (n_win + wc - 1) / wc;
-  if (!fits(n_win - (n_chunks - 1) * wc)) return cudaSuccess;  // the last chunk has fewer windows per coefficient
-  if (n_clips * n_chunks > 0x7fffffffL) return cudaSuccess;
+  if (!fits(n_win - (n_chunks - 1) * wc)) return 0;  // the last chunk has fewer windows per coefficient
+  return wc;
+}
+
+cudaError_t modspec_tc_launch(const float* mfcc, long n_clips, int n_coef, long T, int win, int hop, int nfft,
+                              const void* g, int kp, long wc, float* mag, float* band, const int* lo, const int* hi,
+                              int n_bands, int sm_count, cudaStream_t st, const ModVarlen* vl) {
+  const int nb = nfft / 2 + 1;
+  // T: frames per input row; n_win: windows per output row (a ragged batch: the row pitch and the most windows)
+  const long n_win = vl ? vl->n_win : 1 + (T - win) / hop;
+  const long n_chunks = (n_win + wc - 1) / wc;
   ModTcArgs a{};
   a.mfcc = mfcc;
   a.n_coef = n_coef;
@@ -497,7 +517,8 @@ cudaError_t modspec_tc_launch(const float* mfcc, long n_clips, int n_coef, long 
   a.n_win = n_win;
   a.wc = (int)wc;
   a.n_chunks = (int)n_chunks;
-  a.n_work = n_clips * n_chunks;
+  a.n_work = vl ? vl->n_items : n_clips * n_chunks;
+  a.items = vl ? vl->items : nullptr;
   a.kp = kp;
   a.g = reinterpret_cast<const __half*>(g);
   a.mag = mag;
@@ -505,14 +526,21 @@ cudaError_t modspec_tc_launch(const float* mfcc, long n_clips, int n_coef, long 
   a.band_lo = lo;
   a.band_hi = hi;
   a.n_bands = n_bands;
+  const long wc_smem = vl ? vl->wc_max : wc;
   const size_t smem = (size_t)2 * nfft * kp * 2 + (size_t)kMtRows * nb * 4 + kMtRows * sizeof(float*) +
-                      (size_t)wc * n_coef * std::max(n_bands, 1) * 4;
-#define MMF_MT_CASE(KS)                                                            \
-  case KS: {                                                                       \
-    auto kfn = modspec_tc_kernel<128, KS>;                                         \
-    MMF_SMEM_ONCE(kfn, kMtSmemLimit);                                              \
-    kfn<<<(unsigned)std::min<long>(a.n_work, 2L * sm_count), kMtThreads, smem, st>>>(a); \
-    break;                                                                         \
+                      (size_t)wc_smem * n_coef * std::max(n_bands, 1) * 4;
+  const unsigned grid = (unsigned)std::min<long>(a.n_work, 2L * sm_count);
+#define MMF_MT_LAUNCH(KS, V)                          \
+  {                                                   \
+    auto kfn = modspec_tc_kernel<128, KS, V>;         \
+    MMF_SMEM_ONCE(kfn, kMtSmemLimit);                 \
+    kfn<<<grid, kMtThreads, smem, st>>>(a);           \
+  }
+#define MMF_MT_CASE(KS)                 \
+  case KS: {                            \
+    if (vl) MMF_MT_LAUNCH(KS, true)     \
+    else MMF_MT_LAUNCH(KS, false)       \
+    break;                              \
   }
   switch (kp / 16) {
     MMF_MT_CASE(1)
@@ -523,11 +551,11 @@ cudaError_t modspec_tc_launch(const float* mfcc, long n_clips, int n_coef, long 
     MMF_MT_CASE(6)
     MMF_MT_CASE(7)
     MMF_MT_CASE(8)
-    default: return cudaSuccess;
+    default: return cudaErrorInvalidValue;
   }
 #undef MMF_MT_CASE
+#undef MMF_MT_LAUNCH
   count_launch();
-  *handled = true;
   return cudaGetLastError();
 }
 

@@ -320,6 +320,31 @@ cudaError_t varlen_tails_launch(long n_clips, const int* T, int pitch, double* t
   return cudaGetLastError();
 }
 
+// Variable-length K6 batch: windows [n_win[clip], W) of every magnitude row [n_coef][W][nb] and of the band rows
+// [W][n_bands] are 0.  One CTA per clip; the kernels before it write windows [0, n_win[clip]) only.
+__global__ void modspec_tails_kernel(const int* __restrict__ n_win, long W, float* __restrict__ mag, int n_coef, int nb,
+                                     float* __restrict__ band, int n_bands) {
+  const long clip = blockIdx.x;
+  const long w0 = n_win[clip];
+  if (w0 >= W) return;
+  if (mag) {
+    const long row = (W - w0) * nb;  // tail floats of one coefficient's row
+    for (long e = threadIdx.x; e < (long)n_coef * row; e += blockDim.x) {
+      const long c = e / row;
+      mag[(((size_t)clip * n_coef + c) * W + w0) * nb + (e - c * row)] = 0.0f;
+    }
+  }
+  if (band)
+    for (long e = threadIdx.x; e < (W - w0) * n_bands; e += blockDim.x) band[((size_t)clip * W + w0) * n_bands + e] = 0.0f;
+}
+
+cudaError_t modspec_tails_launch(long n_clips, const int* n_win, long W, float* mag, int n_coef, int nb, float* band,
+                                 int n_bands, cudaStream_t st) {
+  modspec_tails_kernel<<<(unsigned)n_clips, 256, 0, st>>>(n_win, W, mag, n_coef, nb, band, n_bands);
+  count_launch();
+  return cudaGetLastError();
+}
+
 // ---------------------------------------------------------------------------
 // K3 on the tensor cores: [frames x n_mels] . [n_mels x n_mfcc] with mma.sync m16n8k8 TF32 and
 // the 3-term operand split (hi*hi + hi*lo + lo*hi into independent fp32 accumulators, ~2^-21

@@ -381,6 +381,52 @@ class Plan:
         )
         return mag, band
 
+    def modspec_varlen(self, mfcc, frames, win: int, hop: int, nfft: int, band_bins=None, *, want_mag: bool = True):
+        """:meth:`modspec` for clips of different lengths: ``mfcc [B, C, T_max]`` holds clip ``i`` in its first
+        ``frames[i]`` frames (as :meth:`mfcc_change_varlen` returns it; whatever follows is ignored).  Outputs are
+        padded to the most windows of any clip; windows ``[0, windows[i])`` of clip ``i`` equal :meth:`modspec` on
+        that clip alone, bit for bit, and the rest is 0.  Returns ``(mag [B, C, W, nfft/2+1] or None,
+        band [B, W, n_bands] or None, windows)``, ``windows`` a numpy int64 ``[B]``."""
+        torch = _torch()
+        mfcc = mfcc.contiguous()
+        B, Cc, P = mfcc.shape
+        T = np.ascontiguousarray(np.asarray(frames, dtype=np.int64).reshape(-1))
+        if T.shape[0] != B:
+            raise ValueError(f"frames has {T.shape[0]} entries for {B} clips")
+        windows = np.where(T >= win, 1 + (T - win) // max(hop, 1), 0) if hop >= 1 else np.zeros(B, np.int64)
+        W = int(windows.max()) if B else 0
+        nb = nfft // 2 + 1
+        mag = torch.empty((B, Cc, W, nb), device=self.device, dtype=torch.float32) if want_mag else None
+        band = None
+        lo = hi = None
+        n_bands = 0
+        if band_bins is not None and len(band_bins):
+            n_bands = len(band_bins)
+            lo = np.ascontiguousarray([b[0] for b in band_bins], dtype=np.int32)
+            hi = np.ascontiguousarray([b[1] for b in band_bins], dtype=np.int32)
+            band = torch.empty((B, W, n_bands), device=self.device, dtype=torch.float32)
+        # called for W == 0 too: the library validates the lengths and the geometry (and launches nothing)
+        check(
+            _lib.lib().mmf_modspec_varlen(
+                self._h,
+                mfcc.data_ptr(),
+                B,
+                Cc,
+                T.ctypes.data,
+                P,
+                win,
+                hop,
+                nfft,
+                mag.data_ptr() if want_mag and W > 0 else None,
+                band.data_ptr() if band is not None and W > 0 else None,
+                lo.ctypes.data if lo is not None else None,
+                hi.ctypes.data if hi is not None else None,
+                n_bands,
+                _stream_ptr(self.device),
+            )
+        )
+        return mag, band, windows
+
     def rms(self, pcm, frame_length: int, hop_length: int, center: bool = True):
         """librosa.feature.rms -> float32 [B, T_rms]."""
         torch = _torch()
