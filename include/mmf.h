@@ -239,6 +239,39 @@ int mmf_features_host_pcm16(mmf_plan* plan, const int16_t* pcm16_host, int64_t n
                             double* tot_host, float* mfcc_host, float* delta_host, float* mag_host,
                             float* band_host);
 
+/* Host-only: output offsets of a packed batch (no plan, no device).  Clip i is samples
+ * [offsets_host[i], offsets_host[i+1]) of the packed input.  frame_off[n_clips+1] = prefix sums of T_i =
+ * mmf_num_frames(len_i, ...); win_off[n_clips+1] = prefix sums of n_win_i (all 0 when mod is NULL or win = 0).
+ * The offsets are checked as mmf_features_host_varlen checks them. */
+int mmf_features_varlen_sizes(const mmf_config* cfg, const mmf_modspec_params* mod, int64_t n_clips,
+                              const int64_t* offsets_host, int64_t* frame_off_host, int64_t* win_off_host);
+
+/* mmf_features_host for clips of different lengths packed back to back in one host buffer.
+ *  - Input: clip i is pcm_host[offsets_host[i] .. offsets_host[i+1]).  Offsets are non-decreasing from
+ *    offsets_host[0] >= 0 and every clip has at least 1 sample.  Nothing before offsets_host[0] or after
+ *    offsets_host[n_clips] is read, and no sample of one clip reaches another clip's outputs.
+ *  - Outputs are packed in clip order, with no padding.  With F_i = frame_off[i], W_i = win_off[i]
+ *    (mmf_features_varlen_sizes): tot_host[F_i .. F_i + T_i); mfcc_host / delta_host: clip i's [n_mfcc, T_i] block
+ *    at n_mfcc * F_i; mag_host: its [n_mfcc, n_win_i, nfft/2+1] block at n_mfcc * (nfft/2+1) * W_i; band_host: its
+ *    [n_win_i, n_bands] block at n_bands * W_i.  Optional outputs and their NULL rules are those of
+ *    mmf_features_host.
+ *  - Each clip's blocks are bit-identical to mmf_features_host (or _pcm16) on that clip alone, whatever chunk the
+ *    clip lands in and whoever its neighbours are.  For clips of equal length the packed layout is the padded one,
+ *    and the results equal mmf_features_host on the [n_clips, N] array byte for byte.
+ *  - Everything is checked before anything is queued: the offsets first, without a plan or a device (NULL or
+ *    decreasing offsets and empty clips fail with MMF_ERR_INVALID, the message naming the clip); a clip too short
+ *    for the filters fails with MMF_ERR_TOO_SHORT, naming its index.
+ *  - The batch runs in chunks of consecutive clips over the plan's two streams (copy in, compute and copy out
+ *    overlap); the call returns after draining both, on every exit. */
+int mmf_features_host_varlen(mmf_plan* plan, const float* pcm_host, int64_t n_clips, const int64_t* offsets_host,
+                             const mmf_change_params* prm, const mmf_modspec_params* mod, double* tot_host,
+                             float* mfcc_host, float* delta_host, float* mag_host, float* band_host);
+/* The same for 16-bit PCM, scaled to float32 = x / 32768 on the device as mmf_features_host_pcm16 does. */
+int mmf_features_host_varlen_pcm16(mmf_plan* plan, const int16_t* pcm16_host, int64_t n_clips,
+                                   const int64_t* offsets_host, const mmf_change_params* prm,
+                                   const mmf_modspec_params* mod, double* tot_host, float* mfcc_host,
+                                   float* delta_host, float* mag_host, float* band_host);
+
 /* Hilbert amplitude envelope |scipy.signal.hilbert(x)| of each row (script/calc.py:284-286, method 'Hilb'),
  * any length n <= 2^26 (an hour at 16 kHz): O(n log n) -- the length-n transforms scipy runs are evaluated as
  * Bluestein chirp transforms over a power-of-two FFT in float64; signals of at most 4096 samples use the

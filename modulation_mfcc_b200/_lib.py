@@ -197,6 +197,18 @@ _SIGNATURES = {
         C.c_int,
         [_vp, _vp, _i64, _i64, _i64, C.POINTER(mmf_change_params), C.POINTER(mmf_modspec_params), _vp, _vp, _vp, _vp, _vp],
     ),
+    "mmf_features_varlen_sizes": (
+        C.c_int,
+        [C.POINTER(mmf_config), C.POINTER(mmf_modspec_params), _i64, _vp, _vp, _vp],
+    ),
+    "mmf_features_host_varlen": (
+        C.c_int,
+        [_vp, _vp, _i64, _vp, C.POINTER(mmf_change_params), C.POINTER(mmf_modspec_params), _vp, _vp, _vp, _vp, _vp],
+    ),
+    "mmf_features_host_varlen_pcm16": (
+        C.c_int,
+        [_vp, _vp, _i64, _vp, C.POINTER(mmf_change_params), C.POINTER(mmf_modspec_params), _vp, _vp, _vp, _vp, _vp],
+    ),
     "mmf_pcm16_to_f32": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
     "mmf_hilbert_envelope": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _vp, _i64, _vp]),
     "mmf_find_peaks": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _i32, _i32, _vp, _vp, _vp]),

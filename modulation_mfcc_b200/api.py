@@ -821,6 +821,54 @@ class FeatureExtractor:
         except MmfError as e:
             _raise_from(e)
 
+    def host_varlen(self, pcm_host, offsets, *, want=("totChange", "mfcc", "delta", "modspec", "band_energy"),
+                    out=None):
+        """:meth:`host_call` for clips of different lengths packed back to back in one 1-D host buffer (float32, or
+        int16 WAV samples): clip ``i`` is ``pcm_host[offsets[i]:offsets[i + 1]]``.  Returns the packed arrays of
+        :meth:`Plan.features_host_varlen` with this extractor's modulation geometry; each clip's blocks equal
+        :meth:`host_call` on that clip alone, bit for bit."""
+        mod = self.modspec_geometry(0) if ("modspec" in want or "band_energy" in want) else None
+        try:
+            return self.plan.features_host_varlen(pcm_host, offsets, self.prm, mod, want=want, out=out)
+        except MmfError as e:
+            _raise_from(e)
+
+    def host_many(self, clips, *, want=("totChange", "mfcc", "delta", "modspec", "band_energy")):
+        """:meth:`host_varlen` for a list of 1-D numpy clips of any lengths (all int16, or anything else as float32).
+        Concatenates them once and returns one dict per clip of zero-copy views into the packed arrays, shaped as
+        :func:`mfcc_features_batch` returns one clip without its batch axis (``totChange [T]``, ``mfcc`` /
+        ``delta [n_mfcc, T]``, ``modspec [n_mfcc, W, nfft/2+1]``, ``band_energy [W, n_bands]``), plus ``T``, the
+        frame times.  A corpus already held in one buffer should call :meth:`host_varlen` with its offsets instead,
+        which saves the concatenation."""
+        clips = [np.asarray(c) for c in clips]
+        if not clips:
+            return []
+        if any(c.ndim != 1 for c in clips):
+            raise ValueError("host_many takes 1-D clips")
+        dt = np.int16 if all(c.dtype == np.int16 for c in clips) else np.float32
+        offsets = np.zeros(len(clips) + 1, np.int64)
+        np.cumsum([c.shape[0] for c in clips], out=offsets[1:])
+        res = self.host_varlen(np.concatenate(clips).astype(dt, copy=False), offsets, want=want)
+        nm = self.plan.cfg.n_mfcc
+        _, _, nfft, bins = self.modspec_geometry(0)
+        nb, n_bands = nfft // 2 + 1, len(bins)
+        fo, wo = res["frame_offsets"], res["window_offsets"]
+        out = []
+        for i in range(len(clips)):
+            f0, f1, w0, w1 = int(fo[i]), int(fo[i + 1]), int(wo[i]), int(wo[i + 1])
+            T, W = f1 - f0, w1 - w0
+            d = {"totChange": res["totChange"][f0:f1]}
+            for k in ("mfcc", "delta"):
+                if k in res:
+                    d[k] = res[k][nm * f0 : nm * f1].reshape(nm, T)
+            if "modspec" in res:
+                d["modspec"] = res["modspec"][nm * nb * w0 : nm * nb * w1].reshape(nm, W, nb)
+            if "band_energy" in res:
+                d["band_energy"] = res["band_energy"][n_bands * w0 : n_bands * w1].reshape(W, n_bands)
+            d["T"] = _time_anchors(T, self.tStep, self.winLen)
+            out.append(d)
+        return out
+
     def __call__(self, pcm, *, want_logmel: bool = True, want_modspec: bool = True):
         res = self.plan.mfcc_change(pcm, self.prm, want_logmel=want_logmel, want_mfcc=True, want_delta=True)
         if want_modspec:

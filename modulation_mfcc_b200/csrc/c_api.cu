@@ -1017,6 +1017,146 @@ int mmf_modspec(mmf_plan* plan, const float* mfcc_dev, int64_t n_clips, int32_t 
                      n_bands, (cudaStream_t)stream);
 }
 
+}  // extern "C"
+
+namespace mmf {
+
+// Host half of a variable-length K6 batch (mmf_modspec_varlen): each clip's route and the compacted work items, and
+// the layout of the workspace the run step carves from.  Clip i has T[i] <= pitch frames.
+struct ModspecVarlen {
+  int64_t n_clips = 0, W = 0;  // W: windows per output row, the most of any clip
+  int nbe = 0, nb = 0;         // band outputs actually written; bins per window
+  std::vector<int64_t> T;  // frames of each clip
+  std::vector<ModRoute> route;
+  std::vector<int> n_win;
+  long n_items[2] = {0, 0}, wc_max[2] = {0, 0};  // [0] tc, [1] clip
+  std::vector<int64_t> single;                   // clips on the fast / generic kernel
+  std::vector<ModItem> items;
+  bool tails = false;
+  size_t o_items = 0, o_nwin = 0, desc_bytes = 0, o_single = 0, bytes = 0;  // workspace layout (bytes: all of it)
+  std::vector<unsigned char> desc;  // the descriptors (work items, window counts): desc_bytes at the workspace start
+};
+
+// W of a batch, checking every T[i] in [0, pitch] (no plan or device needed)
+static int modspec_varlen_windows(const int64_t* T_host, int64_t n_clips, int64_t pitch, int win, int hop, int64_t* W) {
+  *W = 0;
+  for (int64_t i = 0; i < n_clips; ++i) {
+    const int64_t T = T_host[i];
+    if (T < 0 || T > pitch) {
+      char buf[160];
+      std::snprintf(buf, sizeof(buf), "clip %lld: T %lld must be in [0, pitch = %lld]", (long long)i, (long long)T,
+                    (long long)pitch);
+      return fail(MMF_ERR_INVALID, buf);
+    }
+    if (T >= win) *W = std::max<int64_t>(*W, 1 + (T - win) / hop);
+  }
+  return MMF_OK;
+}
+
+// routing (host only): each clip as its own call, the tc / clip kernels' chunks as work items.  W > 0.
+static int modspec_varlen_route(unsigned flags, const int64_t* T_host, int64_t n_clips, int n_coef, int64_t W, int win,
+                                int hop, int nfft, int nbe, bool want_mag, ModspecVarlen& v) {
+  v.n_clips = n_clips;
+  v.W = W;
+  v.nbe = nbe;
+  v.nb = nfft / 2 + 1;
+  v.T.assign(T_host, T_host + n_clips);
+  v.route.assign((size_t)n_clips, ModRoute{});
+  v.n_win.assign((size_t)n_clips, 0);
+  for (int64_t i = 0; i < n_clips; ++i) {
+    const ModRoute r = modspec_route(win, hop, nfft, n_coef, nbe, T_host[i], flags);
+    v.route[i] = r;
+    v.n_win[i] = T_host[i] >= win ? (int)(1 + (T_host[i] - win) / hop) : 0;
+    v.tails |= v.n_win[i] < W;
+    if (r.path == kModTc || r.path == kModClip) {
+      const int k = r.path == kModTc ? 0 : 1;
+      v.n_items[k] += r.n_chunks;
+      v.wc_max[k] = std::max(v.wc_max[k], r.wc);
+    } else if (r.path != kModNone) {
+      v.single.push_back(i);
+    }
+  }
+  if (v.n_items[0] > 0x7fffffffL || v.n_items[1] > 0x7fffffffL)
+    return fail(MMF_ERR_UNSUPPORTED, "variable-length batch of more than 2^31 - 1 modulation-spectrum work items");
+  v.items.resize((size_t)(v.n_items[0] + v.n_items[1]));
+  size_t at[2] = {0, (size_t)v.n_items[0]};
+  for (int64_t i = 0; i < n_clips; ++i) {
+    const ModRoute& r = v.route[i];
+    if (r.path != kModTc && r.path != kModClip) continue;
+    size_t& k = at[r.path == kModTc ? 0 : 1];
+    for (long c = 0; c < r.n_chunks; ++c) {
+      const long w0 = c * r.wc;
+      v.items[k++] = ModItem{(int)i, (int)w0, (int)std::min<long>(r.wc, v.n_win[i] - w0), v.n_win[i]};
+    }
+  }
+  // workspace: work items and window counts, then the single-clip region (input rows, magnitudes)
+  v.o_items = 0;
+  v.o_nwin = align_up(v.items.size() * sizeof(ModItem), 256);
+  v.desc_bytes = v.o_nwin + (size_t)n_clips * 4;
+  v.o_single = align_up(v.desc_bytes, 256);
+  size_t single_bytes = 0;
+  for (int64_t i : v.single)
+    single_bytes = std::max(single_bytes, align_up((size_t)n_coef * T_host[i] * 4, 256) +
+                                              (want_mag ? (size_t)n_coef * v.n_win[i] * v.nb * 4 : 0));
+  v.bytes = v.o_single + single_bytes;
+  v.desc.assign(v.desc_bytes, 0);
+  if (!v.items.empty()) std::memcpy(v.desc.data() + v.o_items, v.items.data(), v.items.size() * sizeof(ModItem));
+  std::memcpy(v.desc.data() + v.o_nwin, v.n_win.data(), (size_t)n_clips * 4);
+  return MMF_OK;
+}
+
+// device half: launches the batch routed by v on `st`, carving from `base` (v.bytes).  `dd`: v.desc already on the
+// device (null: uploaded to `base` here, a copy that waits for the stream).  The modulation tables must be current
+// (ensure_mod_tables).
+static int modspec_varlen_run(mmf_plan* plan, const ModspecVarlen& v, unsigned char* base, const unsigned char* dd,
+                              const float* mfcc_dev, int n_coef, int64_t pitch, int win, int hop, int nfft,
+                              float* mag_dev, float* band_dev, cudaStream_t st) {
+  int rc;
+  const int64_t n_clips = v.n_clips, W = v.W;
+  const int nbe = v.nbe, nb = v.nb;
+  if (!dd) {
+    MMF_CUDA(cudaMemcpyAsync(base, v.desc.data(), v.desc_bytes, cudaMemcpyHostToDevice, st));
+    dd = base;
+  }
+
+  // ---- the batched clips: one launch per kernel
+  for (int k = 0; k < 2; ++k) {
+    if (!v.n_items[k]) continue;
+    const ModVarlen vl{(const ModItem*)(dd + v.o_items) + (k ? v.n_items[0] : 0), v.n_items[k], (long)W,
+                       (int)v.wc_max[k]};
+    const ModRoute r{k ? kModClip : kModTc, v.wc_max[k], 0};
+    if ((rc = launch_modspec(plan, r, mfcc_dev, n_clips, n_coef, pitch, win, hop, nfft, mag_dev, band_dev, nbe, st,
+                             &vl)))
+      return rc;
+  }
+
+  // ---- the other clips: the single-clip call on contiguous rows, copied into the padded rows
+  for (int64_t i : v.single) {
+    const size_t Ti = (size_t)v.T[i], wi = (size_t)v.n_win[i];
+    float* x1 = (float*)(base + v.o_single);
+    float* mag1 = mag_dev ? (float*)(base + v.o_single + align_up((size_t)n_coef * Ti * 4, 256)) : nullptr;
+    MMF_CUDA(cudaMemcpy2DAsync(x1, Ti * 4, mfcc_dev + (size_t)i * n_coef * pitch, (size_t)pitch * 4, Ti * 4,
+                               (size_t)n_coef, cudaMemcpyDeviceToDevice, st));
+    // a clip's band rows [n_win_i, n_bands] are the start of its padded rows [W, n_bands]: written in place
+    float* band1 = nbe > 0 ? band_dev + (size_t)i * W * nbe : nullptr;
+    if ((rc = launch_modspec(plan, v.route[i], x1, 1, n_coef, (int64_t)Ti, win, hop, nfft, mag1, band1, nbe, st)))
+      return rc;
+    if (mag1)
+      MMF_CUDA(cudaMemcpy2DAsync(mag_dev + (size_t)i * n_coef * W * nb, (size_t)W * nb * 4, mag1, wi * nb * 4,
+                                 wi * nb * 4, (size_t)n_coef, cudaMemcpyDeviceToDevice, st));
+  }
+  if (v.tails && (mag_dev || nbe > 0)) {
+    cudaError_t e = modspec_tails_launch((long)n_clips, (const int*)(dd + v.o_nwin), (long)W, mag_dev, n_coef, nb,
+                                         nbe > 0 ? band_dev : nullptr, nbe, st);
+    if (e != cudaSuccess) return cuda_fail(e, "modspec_tails_kernel launch");
+  }
+  return MMF_OK;
+}
+
+}  // namespace mmf
+
+extern "C" {
+
 // Variable-length batch.  Each clip takes the route and the chunking its own mmf_modspec call would take
 // (modspec_route) -- which is what makes its outputs bit-identical to that call.  Clips on the tcgen05 and the
 // clip-resident kernel run in one launch per kernel for the whole batch, as a compacted list of (clip, chunk) work
@@ -1033,107 +1173,21 @@ int mmf_modspec_varlen(mmf_plan* plan, const float* mfcc_dev, int64_t n_clips, i
   if (n_clips < 1 || n_coef < 1) return fail(MMF_ERR_INVALID, "n_clips and n_coef must be positive");
   if (n_clips > 0x7fffffff) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 clips");
   int64_t W = 0;  // windows per output row: the most of any clip
-  for (int64_t i = 0; i < n_clips; ++i) {
-    const int64_t T = T_host[i];
-    if (T < 0 || T > pitch) {
-      char buf[160];
-      std::snprintf(buf, sizeof(buf), "clip %lld: T %lld must be in [0, pitch = %lld]", (long long)i, (long long)T,
-                    (long long)pitch);
-      return fail(MMF_ERR_INVALID, buf);
-    }
-    if (T >= win) W = std::max<int64_t>(W, 1 + (T - win) / hop);
-  }
+  if ((rc = modspec_varlen_windows(T_host, n_clips, pitch, win, hop, &W))) return rc;
   if (!plan || !mfcc_dev) return fail(MMF_ERR_INVALID, "NULL argument");
   if (W > 0x7fffffff) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 windows per clip");
   if (W == 0) return MMF_OK;  // no clip reaches a window: nothing to compute or zero
 
-  // ---- routing (host only): each clip as its own call, the tc / clip kernels' chunks as work items
   const int nbe = band_dev ? n_bands : 0;  // band outputs actually written
-  const int nb = nfft / 2 + 1;
-  std::vector<ModRoute> route((size_t)n_clips);
-  std::vector<int> n_win((size_t)n_clips, 0);
-  long n_items[2] = {0, 0}, wc_max[2] = {0, 0};  // [0] tc, [1] clip
-  std::vector<int64_t> single;                   // clips on the fast / generic kernel
-  bool tails = false;
-  for (int64_t i = 0; i < n_clips; ++i) {
-    const ModRoute r = modspec_route(win, hop, nfft, n_coef, nbe, T_host[i], (unsigned)plan->cfg.flags);
-    route[i] = r;
-    n_win[i] = T_host[i] >= win ? (int)(1 + (T_host[i] - win) / hop) : 0;
-    tails |= n_win[i] < W;
-    if (r.path == kModTc || r.path == kModClip) {
-      const int k = r.path == kModTc ? 0 : 1;
-      n_items[k] += r.n_chunks;
-      wc_max[k] = std::max(wc_max[k], r.wc);
-    } else if (r.path != kModNone) {
-      single.push_back(i);
-    }
-  }
-  if (n_items[0] > 0x7fffffffL || n_items[1] > 0x7fffffffL)
-    return fail(MMF_ERR_UNSUPPORTED, "variable-length batch of more than 2^31 - 1 modulation-spectrum work items");
-  std::vector<ModItem> items((size_t)(n_items[0] + n_items[1]));
-  {
-    size_t at[2] = {0, (size_t)n_items[0]};
-    for (int64_t i = 0; i < n_clips; ++i) {
-      const ModRoute& r = route[i];
-      if (r.path != kModTc && r.path != kModClip) continue;
-      size_t& k = at[r.path == kModTc ? 0 : 1];
-      for (long c = 0; c < r.n_chunks; ++c) {
-        const long w0 = c * r.wc;
-        items[k++] = ModItem{(int)i, (int)w0, (int)std::min<long>(r.wc, n_win[i] - w0), n_win[i]};
-      }
-    }
-  }
-
-  // ---- workspace: work items and window counts, then the single-clip region (input rows, magnitudes)
+  ModspecVarlen v;
+  if ((rc = modspec_varlen_route((unsigned)plan->cfg.flags, T_host, n_clips, n_coef, W, win, hop, nfft, nbe,
+                                 mag_dev != nullptr, v)))
+    return rc;
   MMF_CUDA(cudaSetDevice(plan->cfg.device));
   if ((rc = ensure_mod_tables(plan, win, nfft, band_lo_host, band_hi_host, nbe))) return rc;
-  const size_t n = (size_t)n_clips;
-  const size_t o_items = 0, o_nwin = align_up(items.size() * sizeof(ModItem), 256);
-  const size_t desc_bytes = o_nwin + n * 4;
-  const size_t o_single = align_up(desc_bytes, 256);
-  size_t single_bytes = 0;
-  for (int64_t i : single)
-    single_bytes = std::max(single_bytes, align_up((size_t)n_coef * T_host[i] * 4, 256) +
-                                              (mag_dev ? (size_t)n_coef * n_win[i] * nb * 4 : 0));
-  if ((rc = ensure_ws(plan, (64 << 10) + o_single + single_bytes))) return rc;
-  unsigned char* base = (unsigned char*)plan->ws + (64 << 10);
-  std::vector<unsigned char> desc(desc_bytes);
-  if (!items.empty()) std::memcpy(desc.data() + o_items, items.data(), items.size() * sizeof(ModItem));
-  std::memcpy(desc.data() + o_nwin, n_win.data(), n * 4);
-  cudaStream_t st = (cudaStream_t)stream;
-  MMF_CUDA(cudaMemcpyAsync(base, desc.data(), desc_bytes, cudaMemcpyHostToDevice, st));
-
-  // ---- the batched clips: one launch per kernel
-  for (int k = 0; k < 2; ++k) {
-    if (!n_items[k]) continue;
-    const ModVarlen vl{(const ModItem*)(base + o_items) + (k ? n_items[0] : 0), n_items[k], (long)W, (int)wc_max[k]};
-    const ModRoute r{k ? kModClip : kModTc, wc_max[k], 0};
-    if ((rc = launch_modspec(plan, r, mfcc_dev, n_clips, n_coef, pitch, win, hop, nfft, mag_dev, band_dev, nbe, st,
-                             &vl)))
-      return rc;
-  }
-
-  // ---- the other clips: the single-clip call on contiguous rows, copied into the padded rows
-  for (int64_t i : single) {
-    const size_t Ti = (size_t)T_host[i], wi = (size_t)n_win[i];
-    float* x1 = (float*)(base + o_single);
-    float* mag1 = mag_dev ? (float*)(base + o_single + align_up((size_t)n_coef * Ti * 4, 256)) : nullptr;
-    MMF_CUDA(cudaMemcpy2DAsync(x1, Ti * 4, mfcc_dev + (size_t)i * n_coef * pitch, (size_t)pitch * 4, Ti * 4,
-                               (size_t)n_coef, cudaMemcpyDeviceToDevice, st));
-    // a clip's band rows [n_win_i, n_bands] are the start of its padded rows [W, n_bands]: written in place
-    float* band1 = nbe > 0 ? band_dev + (size_t)i * W * nbe : nullptr;
-    if ((rc = launch_modspec(plan, route[i], x1, 1, n_coef, (int64_t)Ti, win, hop, nfft, mag1, band1, nbe, st)))
-      return rc;
-    if (mag1)
-      MMF_CUDA(cudaMemcpy2DAsync(mag_dev + (size_t)i * n_coef * W * nb, (size_t)W * nb * 4, mag1, wi * nb * 4,
-                                 wi * nb * 4, (size_t)n_coef, cudaMemcpyDeviceToDevice, st));
-  }
-  if (tails && (mag_dev || nbe > 0)) {
-    cudaError_t e = modspec_tails_launch((long)n_clips, (const int*)(base + o_nwin), (long)W, mag_dev, n_coef, nb,
-                                         nbe > 0 ? band_dev : nullptr, nbe, st);
-    if (e != cudaSuccess) return cuda_fail(e, "modspec_tails_kernel launch");
-  }
-  return MMF_OK;
+  if ((rc = ensure_ws(plan, (64 << 10) + v.bytes))) return rc;
+  return modspec_varlen_run(plan, v, (unsigned char*)plan->ws + (64 << 10), nullptr, mfcc_dev, n_coef, pitch, win, hop,
+                            nfft, mag_dev, band_dev, (cudaStream_t)stream);
 }
 
 int mmf_rms(mmf_plan* plan, const float* pcm_dev, int64_t n_clips, int64_t n_samples, int64_t clip_stride,
@@ -1286,65 +1340,75 @@ int mmf_change_from_logmel(mmf_plan* plan, float* logmel_dev, const int32_t* cli
                   (cudaStream_t)stream);
 }
 
-// Variable-length batch.  Each clip takes the route its own mmf_mfcc_change call would take -- which is what makes
-// its outputs bit-identical to that call: K1 is a decision of the configuration alone, the post-MFCC route depends on
-// the clip's T (the chunk-parallel IIR needs T + 2 padlen <= 6112, the fused kernel T <= 3456 and its shared memory).
-// Clips on the default routes -- clamp + DCT-II folded into the fused kernel, or the FP32 MFCC kernel followed by it
-// -- run in one launch per stage for the whole batch, each with the chunk tables (SosPar) of its own length; any other
-// clip runs the single-clip path in workspace and is copied into its padded rows.
-int mmf_mfcc_change_varlen(mmf_plan* plan, const float* pcm_dev, int64_t n_clips, const int64_t* n_samples_host,
-                           int64_t clip_stride, const mmf_change_params* prm, double* tot_dev, float* logmel_dev,
-                           float* mfcc_dev, float* delta_dev, void* stream) {
-  using namespace mmf;
-  // the lengths first: these checks need neither a plan nor a device
-  if (!n_samples_host) return fail(MMF_ERR_INVALID, "n_samples_host is NULL");
-  if (n_clips < 1) return fail(MMF_ERR_INVALID, "n_clips must be positive");
-  if (n_clips > 0x7fffffff) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 clips");
-  int64_t n_max = 0;
-  for (int64_t i = 0; i < n_clips; ++i) {
-    const int64_t n = n_samples_host[i];
-    if (n < 1 || n > clip_stride) {
-      char buf[160];
-      std::snprintf(buf, sizeof(buf), "clip %lld: n_samples %lld must be in [1, clip_stride = %lld]", (long long)i,
-                    (long long)n, (long long)clip_stride);
-      return fail(MMF_ERR_INVALID, buf);
-    }
-    n_max = std::max(n_max, n);
-  }
-  if (!plan || !pcm_dev || !prm || !tot_dev) return fail(MMF_ERR_INVALID, "NULL argument");
+}  // extern "C"
+
+namespace mmf {
+
+// Host half of a variable-length MFCC-change batch (mmf_mfcc_change_varlen): every clip's route, the chunk tables of
+// the batched clips, and the layout of the workspace the run step carves from.  Which optional outputs the caller
+// wants is part of the routing (a delta output keeps clamp + DCT-II out of the fused kernel, as in the solo call).
+struct ChangeVarlen {
+  int64_t n_clips = 0;
+  int pitch = 0;  // frames per output row: the longest clip's T
+  int first = 0, rows = 0;
+  bool out_iir = false, route_a = false, split_out = false;
+  std::vector<int64_t> len;
+  std::vector<int> T_all, T_k1, clips;
+  std::vector<int2> pidx;
+  std::vector<unsigned> first_unit;
+  std::vector<int64_t> fallback;  // clips on the single-clip path
+  std::vector<SosPar> pars;       // distinct chunk tables of the call (they depend on the clip's length only)
+  int i1 = -1, i2 = -1;           // the longest batched clip's tables: they size the launches' shared memory
+  size_t fsmem = 0;
+  // workspace layout (bytes: all of it)
+  size_t o_len = 0, o_tall = 0, o_tk1 = 0, o_first = 0, o_clips = 0, o_pidx = 0, o_pars = 0, desc_bytes = 0;
+  size_t o_logmel = 0, o_clipmax = 0, o_mfcc = 0, o_raw = 0, o_single = 0, bytes = 0;
+  std::vector<unsigned char> desc;  // the descriptors: desc_bytes at the workspace start
+};
+
+// Routing (host only).  The lengths are in [1, 2^31 - n_fft); `index_base` is added to the clip index that a
+// too-short error names.
+static int change_varlen_route(const mmf_plan* plan, int64_t n_clips, const int64_t* n_samples_host,
+                               const mmf_change_params* prm, bool want_logmel, bool want_mfcc, bool want_delta,
+                               int64_t index_base, ChangeVarlen& v) {
   const mmf_config& c = plan->cfg;
+  int64_t n_max = 0;
+  for (int64_t i = 0; i < n_clips; ++i) n_max = std::max(n_max, n_samples_host[i]);
   if (n_max + c.n_fft > 0x7fffffffLL) return fail(MMF_ERR_UNSUPPORTED, "clip longer than 2^31 samples");
-  const int first = prm->remove_first ? 1 : 0;
-  const int rows = c.n_mfcc - first;
+  v.n_clips = n_clips;
+  v.len.assign(n_samples_host, n_samples_host + n_clips);
+  v.first = prm->remove_first ? 1 : 0;
+  const int first = v.first;
+  const int rows = v.rows = c.n_mfcc - first;
   if (rows < 1) return fail(MMF_ERR_INVALID, "removeFirst leaves no MFCC rows");
   SosArgs sa, so;
   int rc = fill_sos(prm->sos, prm->n_sections, &sa);
   if (rc) return rc;
-  const bool out_iir = prm->out_kind == 0;
+  const bool out_iir = v.out_iir = prm->out_kind == 0;
   if (out_iir && (rc = fill_sos(prm->out_sos, prm->out_n_sections, &so))) return rc;
-  const int pitch = (int)mmf_num_frames(n_max, c.n_fft, c.hop_length);
-  std::vector<int> T_all((size_t)n_clips);
+  v.pitch = (int)mmf_num_frames(n_max, c.n_fft, c.hop_length);
+  v.T_all.assign((size_t)n_clips, 0);
   for (int64_t i = 0; i < n_clips; ++i) {
-    T_all[i] = (int)mmf_num_frames(n_samples_host[i], c.n_fft, c.hop_length);
+    v.T_all[i] = (int)mmf_num_frames(n_samples_host[i], c.n_fft, c.hop_length);
     const int padlen = std::max(sa.padlen, out_iir ? so.padlen : 0);
-    if (T_all[i] <= padlen) {
+    if (v.T_all[i] <= padlen) {
       char buf[192];
       std::snprintf(buf, sizeof(buf),
                     "clip %lld: The length of the input vector x must be greater than padlen, which is %d.",
-                    (long long)i, T_all[i] <= sa.padlen ? sa.padlen : so.padlen);
+                    (long long)(index_base + i), v.T_all[i] <= sa.padlen ? sa.padlen : so.padlen);
       return fail(MMF_ERR_TOO_SHORT, buf);
     }
   }
 
-  // ---- routing (host only): route A = MFCC folded into the fused kernel, B = FP32 MFCC kernel + fused kernel
-  const bool fold = (c.flags & MMF_FLAG_FOLD_MFCC) || delta_dev == nullptr;
+  // route A = MFCC folded into the fused kernel, B = FP32 MFCC kernel + fused kernel
+  const bool fold = (c.flags & MMF_FLAG_FOLD_MFCC) || !want_delta;
   // (more than kFusedNC coefficients never fold: the solo call then takes route B, and so does the batch)
-  const bool route_a = fold && !(c.flags & (MMF_FLAG_SEPARATE_MFCC | MMF_FLAG_MMA_DCT)) && c.n_mfcc <= kFusedNC;
+  const bool route_a = v.route_a = fold && !(c.flags & (MMF_FLAG_SEPARATE_MFCC | MMF_FLAG_MMA_DCT)) && c.n_mfcc <= kFusedNC;
   const bool mfcc_fp32 = !((c.flags & MMF_FLAG_MMA_DCT) && mfcc_mma_supported(c.n_mfcc, c.n_mels)) &&
                          plan->d_dct_tc == nullptr;
   const bool batched = !plan->generic && !(c.flags & MMF_FLAG_UNFUSED_CHANGE) && (route_a || mfcc_fp32) &&
                        sa.n_sections <= kParMaxSections && (!out_iir || so.n_sections == sa.n_sections);
-  std::vector<SosPar> pars;  // distinct chunk tables of the call (they depend on the clip's length only)
+  std::vector<SosPar>& pars = v.pars;
   std::vector<int> par_of_cl[2] = {std::vector<int>(kSosParMaxChunk + 1, -1), std::vector<int>(kSosParMaxChunk + 1, -1)};
   auto par_index = [&](int which, const SosArgs& a, long T) -> int {
     const long L = T + 2L * a.padlen;
@@ -1360,16 +1424,14 @@ int mmf_mfcc_change_varlen(mmf_plan* plan, const float* pcm_dev, int64_t n_clips
     return idx;
   };
   const int unit = plan->d_mel_tc ? 128 : plan->TF;  // K1 work unit: a 128-frame block or a TF-frame tile
-  std::vector<int> T_k1((size_t)n_clips, 0), clips;
-  std::vector<int2> pidx((size_t)n_clips, int2{0, 0});
-  std::vector<unsigned> first_unit((size_t)n_clips + 1, 0);
-  std::vector<int64_t> fallback;
+  v.T_k1.assign((size_t)n_clips, 0);
+  v.pidx.assign((size_t)n_clips, int2{0, 0});
+  v.first_unit.assign((size_t)n_clips + 1, 0);
   // the longest batched clip has the largest chunk of either cascade and needs the most shared memory: its tables
   // and size go to the launches
-  int i1 = -1, i2 = -1, t_big = 0;
-  size_t fsmem = 0;
+  int t_big = 0;
   for (int64_t i = 0; i < n_clips; ++i) {
-    const int T = T_all[i];
+    const int T = v.T_all[i];
     bool ok = batched;
     int a = -1, b = -1;
     if (ok) {
@@ -1381,87 +1443,109 @@ int mmf_mfcc_change_varlen(mmf_plan* plan, const float* pcm_dev, int64_t n_clips
     if (ok)
       ok = route_a ? change_fused_lm_supported(pars[a], out_iir ? &pars[b] : nullptr, c.n_mfcc, c.n_mels, first, rows, T, &sm)
                    : change_fused_supported(pars[a], out_iir ? &pars[b] : nullptr, rows, T, &sm);
-    const uint64_t units = first_unit[i] + (ok ? (uint64_t)(T + unit - 1) / unit : 0);
+    const uint64_t units = v.first_unit[i] + (ok ? (uint64_t)(T + unit - 1) / unit : 0);
     if (units > 0x7fffffffULL) return fail(MMF_ERR_UNSUPPORTED, "variable-length batch of more than 2^31 K1 blocks");
-    first_unit[i + 1] = (unsigned)units;
+    v.first_unit[i + 1] = (unsigned)units;
     if (!ok) {
-      fallback.push_back(i);
+      v.fallback.push_back(i);
       continue;
     }
-    T_k1[i] = T;
-    pidx[i] = int2{a, b};
-    clips.push_back((int)i);
+    v.T_k1[i] = T;
+    v.pidx[i] = int2{a, b};
+    v.clips.push_back((int)i);
     if (T > t_big) {
       t_big = T;
-      fsmem = sm;
-      i1 = a;
-      i2 = b;
+      v.fsmem = sm;
+      v.i1 = a;
+      v.i2 = b;
     }
   }
-  const int64_t nv = (int64_t)clips.size();
-  const bool split_out = out_iir && nv >= 32;  // the batched output filter, as run_post does for a batch
+  const int64_t nv = (int64_t)v.clips.size();
+  v.split_out = out_iir && nv >= 32;  // the batched output filter, as run_post does for a batch
 
-  // ---- workspace: descriptors, then the batched intermediates, then the single-clip region
-  MMF_CUDA(cudaSetDevice(c.device));
+  // workspace: descriptors, then the batched intermediates, then the single-clip region
   const size_t n = (size_t)n_clips;
+  const int pitch = v.pitch;
   size_t off = 0;
   auto take = [&](size_t bytes) {
     const size_t o = off;
     off += align_up(bytes, 256);
     return o;
   };
-  const size_t o_len = take(n * 8), o_tall = take(n * 4), o_tk1 = take(n * 4), o_first = take((n + 1) * 4),
-               o_clips = take(std::max<size_t>(1, clips.size()) * 4), o_pidx = take(n * 8),
-               o_pars = take(std::max<size_t>(1, pars.size()) * sizeof(SosPar));
-  const size_t desc_bytes = off;
-  const size_t o_logmel = (nv && !logmel_dev) ? take(n * c.n_mels * pitch * 4) : 0;
-  const size_t o_clipmax = take(n * 4);
-  const size_t o_mfcc = (nv && !route_a && !mfcc_dev) ? take(n * c.n_mfcc * pitch * 4) : 0;
-  const size_t o_raw = split_out ? take(n * pitch * 8) : 0;
-  const size_t o_single = off;
+  v.o_len = take(n * 8);
+  v.o_tall = take(n * 4);
+  v.o_tk1 = take(n * 4);
+  v.o_first = take((n + 1) * 4);
+  v.o_clips = take(std::max<size_t>(1, v.clips.size()) * 4);
+  v.o_pidx = take(n * 8);
+  v.o_pars = take(std::max<size_t>(1, pars.size()) * sizeof(SosPar));
+  v.desc_bytes = off;
+  v.o_logmel = (nv && !want_logmel) ? take(n * c.n_mels * pitch * 4) : 0;
+  v.o_clipmax = take(n * 4);
+  v.o_mfcc = (nv && !route_a && !want_mfcc) ? take(n * c.n_mfcc * pitch * 4) : 0;
+  v.o_raw = v.split_out ? take(n * pitch * 8) : 0;
+  v.o_single = off;
   size_t single_bytes = 0;
-  for (int64_t i : fallback) {
-    const size_t Ti = (size_t)T_all[i];
+  for (int64_t i : v.fallback) {
+    const size_t Ti = (size_t)v.T_all[i];
     size_t b = change_ws_bytes(plan, 1, (int64_t)Ti, true, true, rows) + align_up(Ti * 8, 256);
-    if (logmel_dev) b += align_up((size_t)c.n_mels * Ti * 4, 256);
-    if (mfcc_dev) b += align_up((size_t)c.n_mfcc * Ti * 4, 256);
-    if (delta_dev) b += align_up((size_t)c.n_mfcc * Ti * 4, 256);
+    if (want_logmel) b += align_up((size_t)c.n_mels * Ti * 4, 256);
+    if (want_mfcc) b += align_up((size_t)c.n_mfcc * Ti * 4, 256);
+    if (want_delta) b += align_up((size_t)c.n_mfcc * Ti * 4, 256);
     single_bytes = std::max(single_bytes, b);
   }
-  if ((rc = ensure_ws(plan, (64 << 10) + o_single + single_bytes))) return rc;
-  unsigned char* base = (unsigned char*)plan->ws + (64 << 10);
-  std::vector<unsigned char> desc(desc_bytes);
-  std::memcpy(desc.data() + o_len, n_samples_host, n * 8);
-  std::memcpy(desc.data() + o_tall, T_all.data(), n * 4);
-  std::memcpy(desc.data() + o_tk1, T_k1.data(), n * 4);
-  std::memcpy(desc.data() + o_first, first_unit.data(), (n + 1) * 4);
-  if (nv) std::memcpy(desc.data() + o_clips, clips.data(), clips.size() * 4);
-  std::memcpy(desc.data() + o_pidx, pidx.data(), n * 8);
-  if (!pars.empty()) std::memcpy(desc.data() + o_pars, pars.data(), pars.size() * sizeof(SosPar));
-  cudaStream_t st = (cudaStream_t)stream;
-  MMF_CUDA(cudaMemcpyAsync(base, desc.data(), desc_bytes, cudaMemcpyHostToDevice, st));
-  const int* d_tall = (const int*)(base + o_tall);
-  const int* d_tk1 = (const int*)(base + o_tk1);
+  v.bytes = v.o_single + single_bytes;
+  v.desc.assign(v.desc_bytes, 0);
+  std::memcpy(v.desc.data() + v.o_len, v.len.data(), n * 8);
+  std::memcpy(v.desc.data() + v.o_tall, v.T_all.data(), n * 4);
+  std::memcpy(v.desc.data() + v.o_tk1, v.T_k1.data(), n * 4);
+  std::memcpy(v.desc.data() + v.o_first, v.first_unit.data(), (n + 1) * 4);
+  if (nv) std::memcpy(v.desc.data() + v.o_clips, v.clips.data(), v.clips.size() * 4);
+  std::memcpy(v.desc.data() + v.o_pidx, v.pidx.data(), n * 8);
+  if (!pars.empty()) std::memcpy(v.desc.data() + v.o_pars, pars.data(), pars.size() * sizeof(SosPar));
+  return MMF_OK;
+}
+
+// Device half: runs the batch routed by v on `st`, carving from `base` (v.bytes).  `dd`: v.desc already on the device
+// (null: uploaded to `base` here, a copy that waits for the stream).  Clip i is the v.len[i] samples at
+// pcm_dev + i * clip_stride; the outputs given must be the ones v was routed for.
+static int change_varlen_run(mmf_plan* plan, const ChangeVarlen& v, unsigned char* base, const unsigned char* dd,
+                             const float* pcm_dev, int64_t clip_stride, const mmf_change_params* prm, double* tot_dev,
+                             float* logmel_dev, float* mfcc_dev, float* delta_dev, cudaStream_t st) {
+  const mmf_config& c = plan->cfg;
+  const int64_t n_clips = v.n_clips;
+  const size_t n = (size_t)n_clips;
+  const int pitch = v.pitch, first = v.first, rows = v.rows;
+  const int64_t nv = (int64_t)v.clips.size();
+  int rc;
+  if (!dd) {
+    MMF_CUDA(cudaMemcpyAsync(base, v.desc.data(), v.desc_bytes, cudaMemcpyHostToDevice, st));
+    dd = base;
+  }
+  const int* d_tall = (const int*)(dd + v.o_tall);
+  const int* d_tk1 = (const int*)(dd + v.o_tk1);
 
   // ---- the batched clips: one launch per stage
   if (nv) {
-    const Varlen vl{(const long*)(base + o_len), d_tk1, (const unsigned*)(base + o_first), (long)first_unit[n], pitch};
-    float* logmel = logmel_dev ? logmel_dev : (float*)(base + o_logmel);
-    int* clipmax = (int*)(base + o_clipmax);
+    const int64_t n_max = *std::max_element(v.len.begin(), v.len.end());
+    const Varlen vl{(const long*)(dd + v.o_len), d_tk1, (const unsigned*)(dd + v.o_first), (long)v.first_unit[n],
+                    pitch};
+    float* logmel = logmel_dev ? logmel_dev : (float*)(base + v.o_logmel);
+    int* clipmax = (int*)(base + v.o_clipmax);
     if ((rc = run_stft(plan, pcm_dev, n_clips, n_max, clip_stride, nullptr, logmel, clipmax, st, &vl))) return rc;
-    const FusedVarlen fvl{(const int*)(base + o_clips), d_tall, (const SosPar*)(base + o_pars),
-                          (const int2*)(base + o_pidx)};
+    const FusedVarlen fvl{(const int*)(dd + v.o_clips), d_tall, (const SosPar*)(dd + v.o_pars),
+                          (const int2*)(dd + v.o_pidx)};
     const int clamp = logmel_dev ? 1 : 0;
-    double* raw = split_out ? (double*)(base + o_raw) : nullptr;
-    const SosPar& pa = pars[i1];
-    const SosPar& po = pars[i2];
+    double* raw = v.split_out ? (double*)(base + v.o_raw) : nullptr;
+    const SosPar& pa = v.pars[v.i1];
+    const SosPar& po = v.pars[v.i2];
     cudaError_t e;
-    if (route_a) {
+    if (v.route_a) {
       const FusedMfccArgs lm{plan->d_dct, plan->nc_pad, logmel, clipmax, c.n_mels, c.top_db, mfcc_dev, delta_dev, clamp};
       e = change_fused_launch(nullptr, nv, c.n_mfcc, first, rows, pitch, prm->diff_method, pa, po,
-                              split_out ? 1 : prm->out_kind, split_out ? raw : tot_dev, fsmem, &lm, st, &fvl);
+                              v.split_out ? 1 : prm->out_kind, v.split_out ? raw : tot_dev, v.fsmem, &lm, st, &fvl);
     } else {
-      float* mfcc = mfcc_dev ? mfcc_dev : (float*)(base + o_mfcc);
+      float* mfcc = mfcc_dev ? mfcc_dev : (float*)(base + v.o_mfcc);
       e = cudaSuccess;
       for (int64_t c0 = 0; c0 < n_clips && e == cudaSuccess; c0 += 65535) {
         const int64_t nc = std::min<int64_t>(65535, n_clips - c0);
@@ -1471,22 +1555,22 @@ int mmf_mfcc_change_varlen(mmf_plan* plan, const float* pcm_dev, int64_t n_clips
       }
       if (e != cudaSuccess) return cuda_fail(e, "mfcc_kernel (variable-length) launch");
       e = change_fused_launch(mfcc, nv, c.n_mfcc, first, rows, pitch, prm->diff_method, pa, po,
-                              split_out ? 1 : prm->out_kind, split_out ? raw : tot_dev, fsmem, nullptr, st, &fvl);
+                              v.split_out ? 1 : prm->out_kind, v.split_out ? raw : tot_dev, v.fsmem, nullptr, st, &fvl);
     }
-    if (e == cudaSuccess && split_out) e = sosfiltfilt_par_varlen_launch(raw, nv, pitch, po, fvl, tot_dev, st);
+    if (e == cudaSuccess && v.split_out) e = sosfiltfilt_par_varlen_launch(raw, nv, pitch, po, fvl, tot_dev, st);
     if (e != cudaSuccess) return cuda_fail(e, "change_fused_kernel (variable-length) launch");
   }
 
   // ---- the other clips: the single-clip path, copied into their padded rows
-  for (int64_t i : fallback) {
-    const size_t Ti = (size_t)T_all[i];
-    unsigned char* cur = base + o_single + change_ws_bytes(plan, 1, (int64_t)Ti, true, true, rows);
+  for (int64_t i : v.fallback) {
+    const size_t Ti = (size_t)v.T_all[i];
+    unsigned char* cur = base + v.o_single + change_ws_bytes(plan, 1, (int64_t)Ti, true, true, rows);
     double* tot1 = (double*)carve(cur, Ti * 8);
     float* lm1 = logmel_dev ? (float*)carve(cur, (size_t)c.n_mels * Ti * 4) : nullptr;
     float* mf1 = mfcc_dev ? (float*)carve(cur, (size_t)c.n_mfcc * Ti * 4) : nullptr;
     float* dl1 = delta_dev ? (float*)carve(cur, (size_t)c.n_mfcc * Ti * 4) : nullptr;
-    if ((rc = run_change(plan, base + o_single, pcm_dev + (size_t)i * clip_stride, 1, n_samples_host[i],
-                         n_samples_host[i], prm, tot1, lm1, mf1, dl1, st)))
+    if ((rc = run_change(plan, base + v.o_single, pcm_dev + (size_t)i * clip_stride, 1, v.len[i], v.len[i], prm, tot1,
+                         lm1, mf1, dl1, st)))
       return rc;
     MMF_CUDA(cudaMemcpyAsync(tot_dev + (size_t)i * pitch, tot1, Ti * 8, cudaMemcpyDeviceToDevice, st));
     auto rows_to = [&](float* dst, const float* src, int r) {
@@ -1501,6 +1585,44 @@ int mmf_mfcc_change_varlen(mmf_plan* plan, const float* pcm_dev, int64_t n_clips
                                       c.n_mfcc, st);
   if (e != cudaSuccess) return cuda_fail(e, "varlen_tails_kernel launch");
   return MMF_OK;
+}
+
+}  // namespace mmf
+
+extern "C" {
+
+// Variable-length batch.  Each clip takes the route its own mmf_mfcc_change call would take -- which is what makes
+// its outputs bit-identical to that call: K1 is a decision of the configuration alone, the post-MFCC route depends on
+// the clip's T (the chunk-parallel IIR needs T + 2 padlen <= 6112, the fused kernel T <= 3456 and its shared memory).
+// Clips on the default routes -- clamp + DCT-II folded into the fused kernel, or the FP32 MFCC kernel followed by it
+// -- run in one launch per stage for the whole batch, each with the chunk tables (SosPar) of its own length; any other
+// clip runs the single-clip path in workspace and is copied into its padded rows.
+int mmf_mfcc_change_varlen(mmf_plan* plan, const float* pcm_dev, int64_t n_clips, const int64_t* n_samples_host,
+                           int64_t clip_stride, const mmf_change_params* prm, double* tot_dev, float* logmel_dev,
+                           float* mfcc_dev, float* delta_dev, void* stream) {
+  using namespace mmf;
+  // the lengths first: these checks need neither a plan nor a device
+  if (!n_samples_host) return fail(MMF_ERR_INVALID, "n_samples_host is NULL");
+  if (n_clips < 1) return fail(MMF_ERR_INVALID, "n_clips must be positive");
+  if (n_clips > 0x7fffffff) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 clips");
+  for (int64_t i = 0; i < n_clips; ++i) {
+    const int64_t n = n_samples_host[i];
+    if (n < 1 || n > clip_stride) {
+      char buf[160];
+      std::snprintf(buf, sizeof(buf), "clip %lld: n_samples %lld must be in [1, clip_stride = %lld]", (long long)i,
+                    (long long)n, (long long)clip_stride);
+      return fail(MMF_ERR_INVALID, buf);
+    }
+  }
+  if (!plan || !pcm_dev || !prm || !tot_dev) return fail(MMF_ERR_INVALID, "NULL argument");
+  ChangeVarlen v;
+  int rc = change_varlen_route(plan, n_clips, n_samples_host, prm, logmel_dev != nullptr, mfcc_dev != nullptr,
+                               delta_dev != nullptr, 0, v);
+  if (rc) return rc;
+  MMF_CUDA(cudaSetDevice(plan->cfg.device));
+  if ((rc = ensure_ws(plan, (64 << 10) + v.bytes))) return rc;
+  return change_varlen_run(plan, v, (unsigned char*)plan->ws + (64 << 10), nullptr, pcm_dev, clip_stride, prm, tot_dev,
+                           logmel_dev, mfcc_dev, delta_dev, (cudaStream_t)stream);
 }
 
 }  // extern "C"
@@ -1629,6 +1751,288 @@ static int features_host_impl(mmf_plan* plan, const void* pcm_host_v, int pcm16,
   if (e1 != cudaSuccess) return cuda_fail(e1, "host path, stream 1");
   return MMF_OK;
 }
+
+namespace mmf {
+
+// offsets[n_clips + 1] of a packed batch: non-decreasing from offsets[0] >= 0, every clip at least one sample (no plan
+// or device needed)
+static int validate_offsets(int64_t n_clips, const int64_t* offsets) {
+  if (!offsets) return fail(MMF_ERR_INVALID, "offsets is NULL");
+  if (n_clips < 1) return fail(MMF_ERR_INVALID, "n_clips must be positive");
+  if (n_clips > 0x7fffffff) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 clips");
+  if (offsets[0] < 0) return fail(MMF_ERR_INVALID, "clip 0: offsets[0] must be >= 0");
+  for (int64_t i = 0; i < n_clips; ++i)
+    if (offsets[i + 1] <= offsets[i]) {
+      char buf[192];
+      std::snprintf(buf, sizeof(buf), "clip %lld: offsets[%lld] = %lld, offsets[%lld] = %lld: every clip needs at least "
+                    "one sample, in buffer order", (long long)i, (long long)i, (long long)offsets[i],
+                    (long long)(i + 1), (long long)offsets[i + 1]);
+      return fail(MMF_ERR_INVALID, buf);
+    }
+  return MMF_OK;
+}
+
+// frame_off / win_off of a packed batch (mmf_features_varlen_sizes); n_win_i = 0 without modulation windows
+static void packed_sizes(int n_fft, int hop, int win, int mod_hop, int64_t n_clips, const int64_t* offsets,
+                         int64_t* frame_off, int64_t* win_off) {
+  frame_off[0] = win_off[0] = 0;
+  for (int64_t i = 0; i < n_clips; ++i) {
+    const int64_t T = mmf_num_frames(offsets[i + 1] - offsets[i], n_fft, hop);
+    frame_off[i + 1] = frame_off[i] + T;
+    win_off[i + 1] = win_off[i] + (win > 0 && T >= win ? 1 + (T - win) / mod_hop : 0);
+  }
+}
+
+// One chunk of a packed host-buffer batch: a run of consecutive clips, its routing, and where its buffers sit in its
+// slot of the host-path workspace (byte offsets from the slot's start).
+struct HostChunk {
+  int64_t c0, c1;  // clips [c0, c1)
+  int64_t stride;  // samples per staged row: the chunk's longest clip, rounded up to 16 bytes for the TMA
+  ChangeVarlen cv;
+  ModspecVarlen mv;  // routed when the chunk has modulation windows (mv.W > 0)
+  std::vector<unsigned char> desc;  // staging offsets and compaction descriptors
+  size_t o_off, o_cnt_t, o_off_t, o_cnt_w, o_off_w;  // within desc
+  size_t o_desc, o_cv_desc, o_mv_desc;  // desc, cv.desc and mv.desc in the descriptor region of the call
+  size_t o_h2d, o_pcm, o_tot, o_mfcc, o_delta, o_mag, o_band, o_ptot, o_pmfcc, o_pdelta, o_pmag, o_pband,
+      o_scratch, end;
+};
+
+// pcm_host: float32 samples, or (pcm16 != 0) int16 samples converted on the device
+static int features_host_varlen_impl(mmf_plan* plan, const void* pcm_host_v, int pcm16, int64_t n_clips,
+                                     const int64_t* offsets, const mmf_change_params* prm,
+                                     const mmf_modspec_params* mod, double* tot_host, float* mfcc_host,
+                                     float* delta_host, float* mag_host, float* band_host) {
+  int rc = validate_offsets(n_clips, offsets);
+  if (rc) return rc;
+  if (!plan || !pcm_host_v || !prm || !tot_host) return fail(MMF_ERR_INVALID, "NULL argument");
+  if ((mag_host || band_host) && !mod) return fail(MMF_ERR_INVALID, "modulation outputs requested without parameters");
+  const mmf_config& c = plan->cfg;
+  const bool want_mod = mod && (mag_host || band_host) && mod->win > 0;
+  if (want_mod && (rc = validate_modspec(mod->win, mod->hop, mod->nfft, mod->n_bands, mod->band_lo, mod->band_hi,
+                                         band_host != nullptr)))
+    return rc;
+  const int nm = c.n_mfcc;
+  const int nb = want_mod ? mod->nfft / 2 + 1 : 0;
+  const int nbe = want_mod && band_host ? mod->n_bands : 0;  // band outputs actually written
+  const bool need_mfcc_dev = mfcc_host || want_mod;
+  const size_t n = (size_t)n_clips;
+  std::vector<int64_t> len(n), T(n), F(n + 1), Wo(n + 1);
+  for (size_t i = 0; i < n; ++i) len[i] = offsets[i + 1] - offsets[i];
+  packed_sizes(c.n_fft, c.hop_length, want_mod ? mod->win : 0, want_mod ? mod->hop : 1, n_clips, offsets, F.data(),
+               Wo.data());
+  for (size_t i = 0; i < n; ++i) T[i] = F[i + 1] - F[i];
+
+  // ---- chunks, planned and routed before anything is queued.  Budgets in bytes of float32 samples, those of
+  // features_host_impl (from its sweep): the real samples of a chunk, and its staged rows at twice that, so that one
+  // long clip among short ones cannot inflate the padded intermediates.  A clip over either budget is a chunk alone.
+  const int64_t budget = pcm16 ? (96 << 20) : (32 << 20);
+  const size_t isz = pcm16 ? 2 : 4;
+  std::vector<HostChunk> chunks;
+  size_t slot = 0, desc_bytes = 0;
+  for (int64_t c0 = 0; c0 < n_clips;) {
+    int64_t c1 = c0 + 1, real = len[c0], n_max = len[c0];
+    // (at most 65535 clips: the compaction's one CTA per row stays far inside the grid limit)
+    while (c1 < n_clips && c1 - c0 < 65535) {
+      const int64_t m = std::max(n_max, len[c1]);
+      if ((real + len[c1]) * 4 > budget || (c1 + 1 - c0) * ((m + 3) & ~3LL) * 4 > 2 * budget) break;
+      real += len[c1];
+      n_max = m;
+      ++c1;
+    }
+    chunks.emplace_back();
+    HostChunk& h = chunks.back();
+    h.c0 = c0;
+    h.c1 = c1;
+    h.stride = (n_max + 3) & ~3LL;
+    const int64_t nc = c1 - c0;
+    if ((rc = change_varlen_route(plan, nc, len.data() + c0, prm, false, need_mfcc_dev, delta_host != nullptr, c0,
+                                  h.cv)))
+      return rc;
+    int64_t W = 0;
+    for (int64_t i = c0; i < c1; ++i) W = std::max(W, Wo[i + 1] - Wo[i]);
+    if (W > 0x7fffffff) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 windows per clip");
+    if (want_mod && W > 0 &&
+        (rc = modspec_varlen_route((unsigned)c.flags, T.data() + c0, nc, nm, W, mod->win, mod->hop, mod->nfft, nbe,
+                                   mag_host != nullptr, h.mv)))
+      return rc;
+    // descriptors: staging offsets [nc + 1], then frames / windows and their packed offsets per clip
+    size_t d = 0;
+    auto dtake = [&](size_t bytes) {
+      const size_t o = d;
+      d += align_up(bytes, 16);
+      return o;
+    };
+    h.o_off = dtake((nc + 1) * 8);
+    h.o_cnt_t = dtake(nc * 4);
+    h.o_off_t = dtake(nc * 8);
+    h.o_cnt_w = dtake(nc * 4);
+    h.o_off_w = dtake(nc * 8);
+    h.desc.assign(d, 0);
+    for (int64_t i = 0; i <= nc; ++i) ((int64_t*)(h.desc.data() + h.o_off))[i] = offsets[c0 + i] - offsets[c0];
+    for (int64_t i = 0; i < nc; ++i) {
+      ((int*)(h.desc.data() + h.o_cnt_t))[i] = (int)T[c0 + i];
+      ((int64_t*)(h.desc.data() + h.o_off_t))[i] = F[c0 + i] - F[c0];
+      ((int*)(h.desc.data() + h.o_cnt_w))[i] = (int)(Wo[c0 + i + 1] - Wo[c0 + i]);
+      ((int64_t*)(h.desc.data() + h.o_off_w))[i] = Wo[c0 + i] - Wo[c0];
+    }
+    // descriptors of every chunk go up together before the first chunk runs (a copy from pageable memory waits for
+    // its stream: inside the loop it would hold back the next chunk's queueing)
+    const bool mod_c = h.mv.W > 0;
+    h.o_desc = desc_bytes;
+    desc_bytes += align_up(h.desc.size(), 256);
+    h.o_cv_desc = desc_bytes;
+    desc_bytes += align_up(h.cv.desc.size(), 256);
+    h.o_mv_desc = desc_bytes;
+    desc_bytes += mod_c ? align_up(h.mv.desc.size(), 256) : 0;
+    // the slot: PCM as it crossed PCIe, staged rows, padded outputs, packed outputs, ragged scratch
+    const size_t pitch = (size_t)h.cv.pitch, frames = (size_t)(F[c1] - F[c0]), wins = (size_t)(Wo[c1] - Wo[c0]);
+    size_t o = 0;
+    auto take = [&](size_t bytes) {
+      const size_t r = o;
+      o += align_up(bytes, 256);
+      return r;
+    };
+    h.o_h2d = take((size_t)real * isz);
+    h.o_pcm = take((size_t)nc * h.stride * 4);
+    h.o_tot = take((size_t)nc * pitch * 8);
+    h.o_mfcc = need_mfcc_dev ? take((size_t)nc * nm * pitch * 4) : 0;
+    h.o_delta = delta_host ? take((size_t)nc * nm * pitch * 4) : 0;
+    h.o_mag = mod_c && mag_host ? take((size_t)nc * nm * W * nb * 4) : 0;
+    h.o_band = mod_c && nbe > 0 ? take((size_t)nc * W * nbe * 4) : 0;
+    h.o_ptot = take(frames * 8);
+    h.o_pmfcc = mfcc_host ? take((size_t)nm * frames * 4) : 0;
+    h.o_pdelta = delta_host ? take((size_t)nm * frames * 4) : 0;
+    h.o_pmag = mod_c && mag_host ? take((size_t)nm * wins * nb * 4) : 0;
+    h.o_pband = mod_c && nbe > 0 ? take(wins * nbe * 4) : 0;
+    h.o_scratch = take(std::max(h.cv.bytes, mod_c ? h.mv.bytes : 0));
+    h.end = o;
+    slot = std::max(slot, o);
+    c0 = c1;
+  }
+
+  MMF_CUDA(cudaSetDevice(c.device));
+  slot = align_up(slot, 256);
+  if ((rc = ensure_host_ws(plan, desc_bytes + 2 * slot))) return rc;
+  // the modulation tables are (re)built with a device-wide synchronisation: do it before any copy is queued
+  bool any_mod = false;
+  for (const HostChunk& h : chunks) any_mod |= h.mv.W > 0;
+  if (any_mod && (rc = ensure_mod_tables(plan, mod->win, mod->nfft, mod->band_lo, mod->band_hi, nbe))) return rc;
+
+  // every exit below drains both streams: queued copies target caller-owned host buffers
+  auto body = [&]() -> int {
+    unsigned char* d_desc = (unsigned char*)plan->host_ws;
+    {
+      std::vector<unsigned char> all(desc_bytes);
+      for (const HostChunk& h : chunks) {
+        std::memcpy(all.data() + h.o_desc, h.desc.data(), h.desc.size());
+        std::memcpy(all.data() + h.o_cv_desc, h.cv.desc.data(), h.cv.desc.size());
+        if (h.mv.W > 0) std::memcpy(all.data() + h.o_mv_desc, h.mv.desc.data(), h.mv.desc.size());
+      }
+      // (complete before either stream reads it)
+      MMF_CUDA(cudaMemcpyAsync(d_desc, all.data(), desc_bytes, cudaMemcpyHostToDevice, plan->streams[0]));
+      MMF_CUDA(cudaStreamSynchronize(plan->streams[0]));
+    }
+    for (size_t k = 0; k < chunks.size(); ++k) {
+      const HostChunk& h = chunks[k];
+      const int s = (int)(k & 1);
+      cudaStream_t st = plan->streams[s];
+      // stream order serialises reuse of slot s (chunk k-2 ran on the same stream)
+      unsigned char* base = (unsigned char*)plan->host_ws + desc_bytes + (size_t)s * slot;
+      const int64_t nc = h.c1 - h.c0;
+      auto dev = [&](size_t o) { return (void*)(base + o); };
+      const unsigned char* dd = d_desc + h.o_desc;
+      MMF_CUDA(cudaMemcpyAsync(dev(h.o_h2d), (const unsigned char*)pcm_host_v + (size_t)offsets[h.c0] * isz,
+                               (size_t)(offsets[h.c1] - offsets[h.c0]) * isz, cudaMemcpyHostToDevice, st));
+      float* d_pcm = (float*)dev(h.o_pcm);
+      cudaError_t e = stage_rows_launch(dev(h.o_h2d), pcm16, (const long*)(dd + h.o_off), (long)nc, (long)h.stride,
+                                        d_pcm, st);
+      if (e != cudaSuccess) return cuda_fail(e, "stage_rows_kernel launch");
+      double* d_tot = (double*)dev(h.o_tot);
+      float* d_mfcc = need_mfcc_dev ? (float*)dev(h.o_mfcc) : nullptr;
+      float* d_delta = delta_host ? (float*)dev(h.o_delta) : nullptr;
+      int rc2 = change_varlen_run(plan, h.cv, base + h.o_scratch, d_desc + h.o_cv_desc, d_pcm, h.stride, prm, d_tot,
+                                  nullptr, d_mfcc, d_delta, st);
+      if (rc2) return rc2;
+      const bool mod_c = h.mv.W > 0;
+      float* d_mag = mod_c && mag_host ? (float*)dev(h.o_mag) : nullptr;
+      float* d_band = mod_c && nbe > 0 ? (float*)dev(h.o_band) : nullptr;
+      if (mod_c && (rc2 = modspec_varlen_run(plan, h.mv, base + h.o_scratch, d_desc + h.o_mv_desc, d_mfcc, nm,
+                                             h.cv.pitch, mod->win, mod->hop, mod->nfft, d_mag, d_band, st)))
+        return rc2;
+      // padded rows -> packed blocks -> one copy back per output
+      const int* cnt_t = (const int*)(dd + h.o_cnt_t);
+      const long* off_t = (const long*)(dd + h.o_off_t);
+      const int* cnt_w = (const int*)(dd + h.o_cnt_w);
+      const long* off_w = (const long*)(dd + h.o_off_w);
+      const size_t frames = (size_t)(F[h.c1] - F[h.c0]), wins = (size_t)(Wo[h.c1] - Wo[h.c0]);
+      const long pitch = h.cv.pitch, W = (long)h.mv.W;
+      auto out = [&](const void* src, size_t o_dst, int eb, int rows, int unit, long pitch_el, const int* cnt,
+                     const long* off, void* host, size_t bytes) -> int {
+        if (!bytes) return MMF_OK;
+        cudaError_t ce = compact_rows_launch(src, dev(o_dst), eb, (long)nc, rows, unit, pitch_el, cnt, off, st);
+        if (ce != cudaSuccess) return cuda_fail(ce, "compact_rows_kernel launch");
+        MMF_CUDA(cudaMemcpyAsync(host, dev(o_dst), bytes, cudaMemcpyDeviceToHost, st));
+        return MMF_OK;
+      };
+      if ((rc2 = out(d_tot, h.o_ptot, 8, 1, 1, pitch, cnt_t, off_t, tot_host + F[h.c0], frames * 8))) return rc2;
+      if (mfcc_host && (rc2 = out(d_mfcc, h.o_pmfcc, 4, nm, 1, pitch, cnt_t, off_t, mfcc_host + (size_t)nm * F[h.c0],
+                                  (size_t)nm * frames * 4)))
+        return rc2;
+      if (delta_host && (rc2 = out(d_delta, h.o_pdelta, 4, nm, 1, pitch, cnt_t, off_t,
+                                   delta_host + (size_t)nm * F[h.c0], (size_t)nm * frames * 4)))
+        return rc2;
+      if (d_mag && (rc2 = out(d_mag, h.o_pmag, 4, nm, nb, W * nb, cnt_w, off_w,
+                              mag_host + (size_t)nm * nb * Wo[h.c0], (size_t)nm * nb * wins * 4)))
+        return rc2;
+      if (d_band && (rc2 = out(d_band, h.o_pband, 4, 1, nbe, W * nbe, cnt_w, off_w, band_host + (size_t)nbe * Wo[h.c0],
+                               (size_t)nbe * wins * 4)))
+        return rc2;
+    }
+    return MMF_OK;
+  };
+  rc = body();
+  const cudaError_t e0 = cudaStreamSynchronize(plan->streams[0]);
+  const cudaError_t e1 = cudaStreamSynchronize(plan->streams[1]);
+  if (rc) return rc;
+  if (e0 != cudaSuccess) return cuda_fail(e0, "host path, stream 0");
+  if (e1 != cudaSuccess) return cuda_fail(e1, "host path, stream 1");
+  return MMF_OK;
+}
+
+}  // namespace mmf
+
+extern "C" {
+
+int mmf_features_varlen_sizes(const mmf_config* cfg, const mmf_modspec_params* mod, int64_t n_clips,
+                              const int64_t* offsets_host, int64_t* frame_off_host, int64_t* win_off_host) {
+  using namespace mmf;
+  int rc = validate_offsets(n_clips, offsets_host);
+  if (rc) return rc;
+  if (!cfg || !frame_off_host || !win_off_host) return fail(MMF_ERR_INVALID, "NULL argument");
+  if (cfg->n_fft < 1 || cfg->hop_length < 1) return fail(MMF_ERR_INVALID, "need n_fft >= 1 and hop_length >= 1");
+  const bool windows = mod && mod->win > 0;
+  if (windows && mod->hop < 1) return fail(MMF_ERR_INVALID, "modulation hop must be >= 1");
+  packed_sizes(cfg->n_fft, cfg->hop_length, windows ? mod->win : 0, windows ? mod->hop : 1, n_clips, offsets_host,
+               frame_off_host, win_off_host);
+  return MMF_OK;
+}
+
+int mmf_features_host_varlen(mmf_plan* plan, const float* pcm_host, int64_t n_clips, const int64_t* offsets_host,
+                             const mmf_change_params* prm, const mmf_modspec_params* mod, double* tot_host,
+                             float* mfcc_host, float* delta_host, float* mag_host, float* band_host) {
+  return mmf::features_host_varlen_impl(plan, pcm_host, 0, n_clips, offsets_host, prm, mod, tot_host, mfcc_host,
+                                        delta_host, mag_host, band_host);
+}
+
+int mmf_features_host_varlen_pcm16(mmf_plan* plan, const int16_t* pcm16_host, int64_t n_clips,
+                                   const int64_t* offsets_host, const mmf_change_params* prm,
+                                   const mmf_modspec_params* mod, double* tot_host, float* mfcc_host,
+                                   float* delta_host, float* mag_host, float* band_host) {
+  return mmf::features_host_varlen_impl(plan, pcm16_host, 1, n_clips, offsets_host, prm, mod, tot_host, mfcc_host,
+                                        delta_host, mag_host, band_host);
+}
+
+}  // extern "C"
 
 extern "C" {
 

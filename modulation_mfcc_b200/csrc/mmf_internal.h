@@ -259,6 +259,12 @@ cudaError_t hilbert_fft_launch(const float* x, long n_clips, long n, long stride
 cudaError_t find_peaks_launch(const double* x, long rows, long T, long stride, int minima, int max_peaks, int* idx,
                               int* count, cudaStream_t st);
 cudaError_t pcm16_to_f32_launch(const int16_t* x, long n, float* y, cudaStream_t st);
+// packed batch of the host-buffer bundle: clip i (samples [off[i], off[i + 1]) of x, float32 or int16) -> row i of
+// y [n_clips, stride]; and padded output rows -> packed blocks (see post_kernels.cu)
+cudaError_t stage_rows_launch(const void* x, int pcm16, const long* off, long n_clips, long stride, float* y,
+                              cudaStream_t st);
+cudaError_t compact_rows_launch(const void* src, void* dst, int elem_bytes, long n_clips, int rows, int unit,
+                                long pitch, const int* cnt, const long* off, cudaStream_t st);
 cudaError_t resample_poly_launch(const float* x, long n_clips, long n_in, long x_stride, const float* h_dev, int len_h,
                                  int up, int down, long n_pre_remove, long n_out, long y_stride, float* y,
                                  cudaStream_t st);

@@ -1027,6 +1027,58 @@ cudaError_t pcm16_to_f32_launch(const int16_t* x, long n, float* y, cudaStream_t
   return cudaGetLastError();
 }
 
+// Host-buffer bundle of a packed batch: clip i, samples [off[i], off[i + 1]) of the chunk as it crossed PCIe, goes to
+// row i of the [n_clips, stride] buffer the ragged K1 reads.  Samples of a row past its clip's length are not written
+// (the ragged path reads them as zero whatever they hold).  int16 input is scaled as pcm16_to_f32_kernel scales it.
+template <typename X>
+__global__ void stage_rows_kernel(const X* __restrict__ x, const long* __restrict__ off, long n_clips, long stride,
+                                  float* __restrict__ y) {
+  constexpr float k = 1.0f / 32768.0f;
+  for (long e = (long)blockIdx.x * blockDim.x + threadIdx.x; e < n_clips * stride; e += (long)gridDim.x * blockDim.x) {
+    const long clip = e / stride, s = e - clip * stride;
+    const long src = off[clip] + s;
+    if (src >= off[clip + 1]) continue;
+    if constexpr (sizeof(X) == 2) y[e] = (float)x[src] * k;
+    else y[e] = x[src];
+  }
+}
+
+cudaError_t stage_rows_launch(const void* x, int pcm16, const long* off, long n_clips, long stride, float* y,
+                              cudaStream_t st) {
+  const long blocks = std::min<long>((n_clips * stride + 255) / 256, 1L << 20);
+  if (pcm16)
+    stage_rows_kernel<<<(unsigned)blocks, 256, 0, st>>>((const int16_t*)x, off, n_clips, stride, y);
+  else
+    stage_rows_kernel<<<(unsigned)blocks, 256, 0, st>>>((const float*)x, off, n_clips, stride, y);
+  count_launch();
+  return cudaGetLastError();
+}
+
+// Padded rows -> packed blocks.  Clip i owns `rows` rows of cnt[i] * unit elements, the first at
+// src + i * rows * pitch, the next `pitch` elements on; they leave back to back at dst + off[i] * rows * unit.  One CTA
+// per (clip, row); a plain copy, so the bits are kept.
+template <typename E>
+__global__ void compact_rows_kernel(const E* __restrict__ src, E* __restrict__ dst, int rows, int unit, long pitch,
+                                    const int* __restrict__ cnt, const long* __restrict__ off) {
+  const long clip = blockIdx.x / rows;
+  const int r = (int)(blockIdx.x - clip * rows);
+  const long len = (long)cnt[clip] * unit;
+  const E* s = src + ((size_t)clip * rows + r) * pitch;
+  E* d = dst + ((size_t)off[clip] * rows + (size_t)r * cnt[clip]) * unit;
+  for (long e = threadIdx.x; e < len; e += blockDim.x) d[e] = s[e];
+}
+
+cudaError_t compact_rows_launch(const void* src, void* dst, int elem_bytes, long n_clips, int rows, int unit,
+                                long pitch, const int* cnt, const long* off, cudaStream_t st) {
+  const unsigned grid = (unsigned)(n_clips * rows);
+  if (elem_bytes == 8)
+    compact_rows_kernel<<<grid, 256, 0, st>>>((const double*)src, (double*)dst, rows, unit, pitch, cnt, off);
+  else
+    compact_rows_kernel<<<grid, 256, 0, st>>>((const float*)src, (float*)dst, rows, unit, pitch, cnt, off);
+  count_launch();
+  return cudaGetLastError();
+}
+
 // ---------------------------------------------------------------------------
 // Polyphase rational resampler: scipy.signal.resample_poly / upfirdn semantics,
 // y_full[m] = sum_i h[m*down - i*up] * x[i], then y = y_full[n_pre_remove : n_pre_remove + n_out]

@@ -651,14 +651,10 @@ class Plan:
         T = self.num_frames(N)
         nm = self.cfg.n_mfcc
         out = {} if out is None else out
-        mp = None
+        mp = _modspec_params(mod)
         n_win = nb = n_bands = 0
         if mod is not None:
             win, hop, nfft, bins = mod
-            mp = mmf_modspec_params()
-            mp.win, mp.hop, mp.nfft, mp.n_bands = int(win), int(hop), int(nfft), len(bins)
-            for i, (lo, hi) in enumerate(bins):
-                mp.band_lo[i], mp.band_hi[i] = int(lo), int(hi)
             n_win = 1 + (T - win) // hop if T >= win else 0
             nb, n_bands = nfft // 2 + 1, len(bins)
         shapes = {
@@ -697,6 +693,87 @@ class Plan:
         )
         return out
 
+    def features_host_varlen(self, pcm_host: np.ndarray, offsets, prm: mmf_change_params, mod=None, *,
+                             want=("totChange",), out=None):
+        """:meth:`features_host` for clips of different lengths packed back to back in one host buffer.
+
+        ``pcm_host`` is 1-D float32 or int16 (raw WAV samples, scaled by 1/32768 on the device); clip ``i`` is
+        ``pcm_host[offsets[i]:offsets[i + 1]]``, ``offsets`` int64 ``[B + 1]``.  Returns the keys of
+        :meth:`features_host` as flat packed arrays, clip after clip with no padding (clip ``i``'s ``[n_mfcc, T_i]``
+        MFCC block starts at ``n_mfcc * frame_offsets[i]``, its ``[n_mfcc, n_win_i, nfft/2+1]`` modulation block at
+        ``n_mfcc * (nfft/2+1) * window_offsets[i]``), plus ``frames``, ``windows`` (int64 ``[B]``), ``frame_offsets``
+        and ``window_offsets`` (int64 ``[B + 1]``).  Each clip's blocks equal :meth:`features_host` on that clip
+        alone, bit for bit.  Pinned buffers (``pcm_host`` and the arrays in ``out``) make the copies asynchronous."""
+        pcm_host = np.asarray(pcm_host)
+        pcm16 = pcm_host.dtype == np.int16
+        if not pcm16 and pcm_host.dtype != np.float32:
+            pcm_host = pcm_host.astype(np.float32)
+        if pcm_host.ndim != 1:
+            raise ValueError("features_host_varlen takes a 1-D packed buffer")
+        pcm_host = np.ascontiguousarray(pcm_host)
+        offs = np.ascontiguousarray(np.asarray(offsets, dtype=np.int64).reshape(-1))
+        B = offs.shape[0] - 1
+        if B < 1:
+            raise ValueError("offsets needs at least two entries")
+        if offs[-1] > pcm_host.shape[0]:
+            raise ValueError(f"offsets[{B}] = {offs[-1]} is past the end of the {pcm_host.shape[0]}-sample buffer")
+        mp = _modspec_params(mod)
+        frame_off = np.empty(B + 1, np.int64)
+        win_off = np.empty(B + 1, np.int64)
+        # the library owns the size formulas (and checks the offsets, naming a bad clip)
+        check(
+            _lib.lib().mmf_features_varlen_sizes(
+                C.byref(self.cfg.to_c()), C.byref(mp) if mp is not None else None, B, offs.ctypes.data,
+                frame_off.ctypes.data, win_off.ctypes.data,
+            )
+        )
+        nm = self.cfg.n_mfcc
+        F, Wt = int(frame_off[-1]), int(win_off[-1])
+        nb = n_bands = 0
+        if mod is not None:
+            nb, n_bands = int(mod[2]) // 2 + 1, len(mod[3])
+        shapes = {
+            "totChange": ((F,), np.float64),
+            "mfcc": ((nm * F,), np.float32),
+            "delta": ((nm * F,), np.float32),
+            "modspec": ((nm * Wt * nb,), np.float32),
+            "band_energy": ((Wt * n_bands,), np.float32),
+        }
+        out = {} if out is None else out
+        ptr = {}
+        for k, (shp, dt) in shapes.items():
+            if k in want or k == "totChange":
+                a = out.get(k)
+                if a is None or a.shape != shp or a.dtype != dt or not a.flags.c_contiguous:
+                    a = np.empty(shp, dt)
+                    out[k] = a
+                ptr[k] = a.ctypes.data if a.size else None  # (no modulation window in any clip: nothing to write)
+            else:
+                ptr[k] = None
+        if ("modspec" in want or "band_energy" in want) and mp is None:
+            raise ValueError("modspec / band_energy requested without modulation parameters")
+        fn = _lib.lib().mmf_features_host_varlen_pcm16 if pcm16 else _lib.lib().mmf_features_host_varlen
+        check(
+            fn(
+                self._h,
+                pcm_host.ctypes.data,
+                B,
+                offs.ctypes.data,
+                C.byref(prm),
+                C.byref(mp) if mp is not None else None,
+                ptr["totChange"],
+                ptr["mfcc"],
+                ptr["delta"],
+                ptr["modspec"],
+                ptr["band_energy"],
+            )
+        )
+        out["frames"] = np.diff(frame_off)
+        out["windows"] = np.diff(win_off)
+        out["frame_offsets"] = frame_off
+        out["window_offsets"] = win_off
+        return out
+
     def mfcc_change_host(self, pcm_host: np.ndarray, prm: mmf_change_params, *, want_mfcc: bool = False):
         """Host buffers in and out through the single C-ABI call (H2D/D2H inside).
 
@@ -731,6 +808,18 @@ class Plan:
                 )
             )
         return (tot, mf) if want_mfcc else tot
+
+
+def _modspec_params(mod):
+    """``mod`` = (win, hop, nfft, band_bins) or None -> mmf_modspec_params or None."""
+    if mod is None:
+        return None
+    win, hop, nfft, bins = mod
+    mp = mmf_modspec_params()
+    mp.win, mp.hop, mp.nfft, mp.n_bands = int(win), int(hop), int(nfft), len(bins)
+    for i, (lo, hi) in enumerate(bins):
+        mp.band_lo[i], mp.band_hi[i] = int(lo), int(hi)
+    return mp
 
 
 _PLANS: "OrderedDict[MfccConfig, Plan]" = OrderedDict()

@@ -11,17 +11,25 @@ The features leg runs FeatureExtractor with its defaults (log-mel, MFCC, delta, 
 spectrum at 1 s / 0.5 s windows: the tcgen05 kernel, the clip kernel for the few window counts it declines): FeatureExtractor.varlen, a loop of one FeatureExtractor call
 per clip, and one call over the zero-padded batch (whose windows past a clip's end are spectra of the padding).
 
+The host leg times the host-buffer bundle (every output of FeatureExtractor.host_call) once with float32 and once
+with int16 samples, three ways: FeatureExtractor.host_varlen on a pinned packed buffer, host_call on the pinned batch
+zero-padded to 20 s, and mfcc_features_many on the list of numpy clips (float32: it takes no int16).  Outputs of the
+first two land in pinned arrays.  One pinned host-to-device copy of the packed bytes is timed as the ceiling.  Host
+calls end in a synchronise, so a host clock times them.  Each way reports its median ms, audio-s/s and the bytes it
+moves each way over PCIe.
+
 Workload: 1024 clips at 16 kHz with the bench's frame geometry (win 400 / hop 160 / n_fft 512, 40 mel, 13 MFCC,
 gradient, Butterworth output filter), lengths uniform in [2 s, 20 s] from a fixed seed.  Prints, per leg, the median
 ms of each way and audio-seconds per second as one JSON line, with the GPU's name and power limit.
 
-    python tools/bench_varlen.py [--clips 1024] [--iters 10] [--loop-iters 3] [--legs change,features]
+    python tools/bench_varlen.py [--clips 1024] [--iters 10] [--loop-iters 3] [--legs change,features,host]
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import time
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -41,6 +49,80 @@ def _median_ms(fn, iters):
         torch.cuda.synchronize()
         times.append(e0.elapsed_time(e1))
     return float(np.median(times))
+
+
+def _median_host_ms(fn, iters):
+    times = []
+    for _ in range(iters):
+        t0 = time.perf_counter()
+        fn()
+        times.append((time.perf_counter() - t0) * 1e3)
+    return float(np.median(times))
+
+
+def _pinned(shape, dtype):
+    t = torch.empty(shape, dtype={np.float32: torch.float32, np.float64: torch.float64, np.int16: torch.int16}[dtype],
+                    pin_memory=True)
+    return t.numpy()
+
+
+def _host_leg(fx, pcm, lengths, sr, iters, power_limit, dev):
+    """One JSON line per input type; see the module docstring."""
+    want = ("totChange", "mfcc", "delta", "modspec", "band_energy")
+    B, n_max = pcm.shape
+    host = pcm.cpu().numpy()
+    clips = [host[i, : lengths[i]] for i in range(B)]
+    offsets = np.zeros(B + 1, np.int64)
+    np.cumsum(lengths, out=offsets[1:])
+    audio_s = sum(lengths) / sr
+    for dt in (np.float32, np.int16):
+        if dt == np.int16:
+            clips_t = [np.clip(np.round(c * 32768.0), -32768, 32767).astype(np.int16) for c in clips]
+            floats = [c.astype(np.float32) / 32768.0 for c in clips_t]
+        else:
+            clips_t = clips
+            floats = clips
+        packed = _pinned((int(offsets[-1]),), dt)
+        padded = _pinned((B, n_max), dt)
+        padded[:] = 0
+        for i, c in enumerate(clips_t):
+            packed[offsets[i] : offsets[i + 1]] = c
+            padded[i, : lengths[i]] = c
+        # pinned outputs shaped by a first (warm-up) call
+        out_v = {k: v for k, v in fx.host_varlen(packed, offsets, want=want).items() if k in want}
+        out_v = {k: _pinned(v.shape, v.dtype.type) for k, v in out_v.items()}
+        out_p = {k: _pinned(v.shape, v.dtype.type) for k, v in fx.host_call(padded, want=want).items()}
+        mm.mfcc_features_many(floats, sr)
+        ways = {
+            "host_varlen": lambda: fx.host_varlen(packed, offsets, want=want, out=out_v),
+            "host_padded": lambda: fx.host_call(padded, want=want, out=out_p),
+            "many": lambda: mm.mfcc_features_many(floats, sr),
+        }
+        dev_out = fx.varlen(torch.zeros((B, n_max), device=dev), lengths)  # what mfcc_features_many copies back
+        bytes_io = {
+            "host_varlen": (packed.nbytes, sum(v.nbytes for v in out_v.values())),
+            "host_padded": (padded.nbytes, sum(v.nbytes for v in out_p.values())),
+            "many": (B * n_max * 4, sum(v.numel() * v.element_size() for v in dev_out.values() if hasattr(v, "numel"))),
+        }
+        src = torch.from_numpy(packed)
+        ceiling = lambda: (src.to(dev, non_blocking=True), torch.cuda.synchronize())  # noqa: E731
+        ceiling()
+        res = {
+            "leg": "host",
+            "input": np.dtype(dt).name,
+            "gpu": torch.cuda.get_device_name(dev),
+            "power_limit": power_limit,
+            "clips": B,
+            "audio_s": audio_s,
+            "h2d_ceiling_ms": _median_host_ms(ceiling, iters),
+        }
+        for k, fn in ways.items():
+            fn()
+            res[f"{k}_ms"] = _median_host_ms(fn, iters)
+            res[f"{k}_audio_s_per_s"] = audio_s / (res[f"{k}_ms"] / 1e3)
+            res[f"{k}_h2d_bytes"], res[f"{k}_d2h_bytes"] = bytes_io[k]
+        res["h2d_ceiling_audio_s_per_s"] = audio_s / (res["h2d_ceiling_ms"] / 1e3)
+        print(json.dumps(res), flush=True)
 
 
 def main():
@@ -87,6 +169,9 @@ def main():
         power_limit = None
     frames = [plan.num_frames(n) for n in lengths]
     for leg in a.legs.split(","):
+        if leg == "host":
+            _host_leg(fx, pcm, lengths, sr, a.iters, power_limit, dev)
+            continue
         varlen, loop, pad = ways[leg]
         for fn in (varlen, pad, loop):  # warm-up: modules, workspace growth
             fn()
