@@ -20,32 +20,30 @@ __device__ __forceinline__ float key_to_float(int k) { return __int_as_float(k >
 
 // ---------------------------------------------------------------------------
 // K3: top_db clamp + DCT-II (+ delta).  One thread per frame; the DCT rows sit in
-// shared memory as [n_mels][NC] so each mel value feeds NC FMAs from broadcast
+// shared memory as [mel_chunk][NC] so each mel value feeds NC FMAs from broadcast
 // 128-bit shared loads.  Block = 128 frames with a one-frame halo on each side
 // when the delta (np.gradient) is requested.  T is the row pitch in frames; vT (a variable-length
 // batch, else null) gives each clip's own frame count, 0 for a clip the launch skips.
+// mel_chunk = n_mels unless the whole table does not fit shared memory (n_mfcc > 64 with n_mels >= 272):
+// then the rows are staged mel_chunk at a time, and each coefficient still accumulates m = 0, 1, ... in order.
 // ---------------------------------------------------------------------------
 constexpr int kMfccThreads = 128;
+constexpr size_t kMfccSmem = 200 * 1024;
 
 template <int NC, bool VL>
 __global__ void __launch_bounds__(kMfccThreads)
     mfcc_kernel(const float* __restrict__ dct_pad, int dct_pitch, float* logmel, const int* __restrict__ clipmax, long T,
                 int n_mels, int n_mfcc, float top_db, float* __restrict__ mfcc, float* __restrict__ delta,
-                int clamp_in_place, const int* __restrict__ vT) {
+                int clamp_in_place, const int* __restrict__ vT, int mel_chunk) {
   extern __shared__ __align__(16) float sm[];
-  float* s_dct = sm;                 // [n_mels][NC]
-  float* s_col = sm + n_mels * NC;   // [NC][kMfccThreads + 1]
+  float* s_dct = sm;                    // [mel_chunk][NC]
+  float* s_col = sm + mel_chunk * NC;   // [NC][kMfccThreads + 1]
   const int tid = threadIdx.x;
   const long clip = blockIdx.y;
   const int halo = delta != nullptr ? 1 : 0;
   const int per_block = kMfccThreads - 2 * halo;
   const long Tn = VL ? vT[clip] : T;  // frames of this clip
   if (VL && (long)blockIdx.x * per_block >= Tn) return;
-  for (int i = tid; i < n_mels * NC; i += kMfccThreads) {
-    const int m = i / NC, j = i - m * NC;
-    s_dct[i] = dct_pad[m * dct_pitch + j];
-  }
-  __syncthreads();
 
   const long t = (long)blockIdx.x * per_block - halo + tid;
   const bool valid = t >= 0 && t < Tn;
@@ -55,23 +53,32 @@ __global__ void __launch_bounds__(kMfccThreads)
   float acc[NC];
 #pragma unroll
   for (int j = 0; j < NC; ++j) acc[j] = 0.0f;
-  if (valid) {
-    float* col = logmel + (size_t)clip * n_mels * T + t;
+  float* col = logmel + (size_t)clip * n_mels * T + (valid ? t : 0);
+  // every thread of the block takes every chunk's barriers; only frames of the clip read and accumulate
+  for (int c0 = 0; c0 < n_mels; c0 += mel_chunk) {
+    const int c1 = min(n_mels, c0 + mel_chunk);
+    if (c0 > 0) __syncthreads();  // the previous chunk's rows have been read by every thread
+    for (int i = tid; i < (c1 - c0) * NC; i += kMfccThreads) {
+      const int m = i / NC, j = i - m * NC;
+      s_dct[i] = dct_pad[(c0 + m) * dct_pitch + j];
+    }
+    __syncthreads();
+    if (!valid) continue;
     // software pipeline: the next 8 mel rows are in flight while the current 8 feed their FMAs
     // (the kernel is a pure stream: 4*n_mels bytes in, 8*n_mfcc bytes out per frame)
     float cur[8], nxt[8];
 #pragma unroll
-    for (int u = 0; u < 8; ++u) cur[u] = (u < n_mels) ? __ldcs(col + (size_t)u * T) : 0.0f;
-    for (int m0 = 0; m0 < n_mels; m0 += 8) {
+    for (int u = 0; u < 8; ++u) cur[u] = (c0 + u < c1) ? __ldcs(col + (size_t)(c0 + u) * T) : 0.0f;
+    for (int m0 = c0; m0 < c1; m0 += 8) {
 #pragma unroll
-      for (int u = 0; u < 8; ++u) nxt[u] = (m0 + 8 + u < n_mels) ? __ldcs(col + (size_t)(m0 + 8 + u) * T) : 0.0f;
+      for (int u = 0; u < 8; ++u) nxt[u] = (m0 + 8 + u < c1) ? __ldcs(col + (size_t)(m0 + 8 + u) * T) : 0.0f;
 #pragma unroll
       for (int u = 0; u < 8; ++u) {
         const int m = m0 + u;
-        if (m < n_mels) {
+        if (m < c1) {
           const float x = fmaxf(cur[u], thr);
           if (clamp_in_place && own) col[(size_t)m * T] = x;
-          const float4* d4 = reinterpret_cast<const float4*>(s_dct + m * NC);
+          const float4* d4 = reinterpret_cast<const float4*>(s_dct + (m - c0) * NC);
 #pragma unroll
           for (int j4 = 0; j4 < NC / 4; ++j4) {
             const float4 d = d4[j4];
@@ -231,7 +238,9 @@ cudaError_t mfcc_launch(const float* dct_pad, int nc_pad, float* logmel, const i
   const int per_block = kMfccThreads - 2 * halo;
   dim3 grid((unsigned)((T + per_block - 1) / per_block), (unsigned)n_clips);
   int nc = n_mfcc <= 16 ? 16 : (n_mfcc <= 32 ? 32 : (n_mfcc <= 64 ? 64 : 128));
-  size_t smem = ((size_t)n_mels * nc + (size_t)nc * (kMfccThreads + 1)) * sizeof(float);
+  // DCT rows that fit beside the delta tile: every n_mels up to 512 for nc <= 64, 271 for nc = 128
+  const int mel_chunk = std::min<int>(n_mels, (int)(kMfccSmem / sizeof(float) / nc) - (kMfccThreads + 1));
+  size_t smem = ((size_t)mel_chunk * nc + (size_t)nc * (kMfccThreads + 1)) * sizeof(float);
   if ((nc == 16 || nc == 32) && nc_pad == nc && n_mels % 8 == 0 && n_mels >= 8 && T < (1L << 27)) {
     const int np = n_mfcc <= 8 ? 4 : (n_mfcc + 1) / 2;
 #define MMF_MFCC_PK_LAUNCH(N, P, V)                                                                                \
@@ -270,9 +279,9 @@ cudaError_t mfcc_launch(const float* dct_pad, int nc_pad, float* logmel, const i
 #define MMF_MFCC_LAUNCH(N, V)                                                                                    \
   {                                                                                                              \
     auto kfn = mfcc_kernel<N, V>;                                                                                \
-    MMF_SMEM_ONCE(kfn, 200 * 1024);                                                                              \
+    MMF_SMEM_ONCE(kfn, kMfccSmem);                                                                               \
     kfn<<<grid, kMfccThreads, smem, st>>>(dct_pad, nc_pad, logmel, clipmax, T, n_mels, n_mfcc, top_db, mfcc,     \
-                                          delta, clamp_in_place, vT);                                            \
+                                          delta, clamp_in_place, vT, mel_chunk);                                 \
   }
 #define MMF_MFCC_CASE(N)                                                                                         \
   case N: {                                                                                                      \
