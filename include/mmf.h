@@ -272,6 +272,47 @@ int mmf_features_host_varlen_pcm16(mmf_plan* plan, const int16_t* pcm16_host, in
                                    const mmf_modspec_params* mod, double* tot_host, float* mfcc_host,
                                    float* delta_host, float* mag_host, float* band_host);
 
+/* How one clip of a packed batch reaches the plan's rate.  up = down = 1: the clip is already at the plan's rate and is
+ * taken as it is (n_out = its length; tap0, len_h and n_pre_remove are not read).  Otherwise the clip is resampled
+ * exactly as mmf_resample_poly resamples a row with the filter h[tap0 .. tap0 + len_h) of the call's tap table
+ * (design: plan.design_resample_filter), n_pre_remove and n_out = ceil(len * up / down). */
+typedef struct {
+  int32_t up, down;
+  int64_t tap0;
+  int32_t len_h;
+  int64_t n_pre_remove, n_out;
+} mmf_resample_clip;
+
+/* mmf_features_host_varlen for packed clips that each arrive at their own sample rate.
+ *  - Input: clip i is pcm_host[offsets_host[i] .. offsets_host[i+1]), float32 or (pcm16 != 0) int16 scaled by
+ *    1/32768; rs_host[i] says how it reaches the plan's rate, with taps from h_host[n_h] (NULL when every clip is at
+ *    the plan's rate).  Each clip's native samples cross PCIe once and are resampled on the device straight into the
+ *    rows the ragged path reads, in one staging launch per chunk whatever its mix of rates.
+ *  - Outputs are packed as mmf_features_host_varlen packs them, with T_i = mmf_num_frames(n_out_i, ...): frame and
+ *    window offsets come from mmf_features_varlen_sizes given the prefix sums of n_out_i as offsets.
+ *  - Each clip's blocks are bit-identical to mmf_features_host on mmf_resample_poly's output for that clip alone
+ *    (after mmf_pcm16_to_f32 for int16), whatever chunk the clip lands in and whoever its neighbours are; a plan-rate
+ *    clip's blocks equal mmf_features_host_varlen's.
+ *  - Everything is checked before anything is queued, the offsets and descriptors without a plan or a device (the
+ *    message names the clip): the offsets as mmf_features_host_varlen checks them, up, down >= 1, n_out =
+ *    ceil(len * up / down) (= len at the plan's rate), and for a resampled clip 1 <= len_h <= 2^22, tap0 >= 0,
+ *    tap0 + len_h <= n_h and n_pre_remove >= 0 (MMF_ERR_INVALID).  A clip too short for the filters after resampling
+ *    fails with MMF_ERR_TOO_SHORT, naming its index. */
+int mmf_features_host_varlen_resampled(mmf_plan* plan, const void* pcm_host, int32_t pcm16, int64_t n_clips,
+                                       const int64_t* offsets_host, const mmf_resample_clip* rs_host,
+                                       const float* h_host, int64_t n_h, const mmf_change_params* prm,
+                                       const mmf_modspec_params* mod, double* tot_host, float* mfcc_host,
+                                       float* delta_host, float* mag_host, float* band_host);
+
+/* The resampling stage of mmf_features_host_varlen_resampled alone, on the device: clip i of the packed float32
+ * x_dev[offsets_host[i] .. offsets_host[i+1]) goes to y_dev + i * y_stride (rs_host[i].n_out samples; the rest of the
+ * row is not written; y_stride >= max n_out).  The checks are those of mmf_features_host_varlen_resampled.  One
+ * launch, asynchronous on `stream` (the call's descriptors and taps are copied from pageable memory before it
+ * returns). */
+int mmf_resample_varlen(mmf_plan* plan, const float* x_dev, int64_t n_clips, const int64_t* offsets_host,
+                        const mmf_resample_clip* rs_host, const float* h_host, int64_t n_h, float* y_dev,
+                        int64_t y_stride, void* stream);
+
 /* Hilbert amplitude envelope |scipy.signal.hilbert(x)| of each row (script/calc.py:284-286, method 'Hilb'),
  * any length n <= 2^26 (an hour at 16 kHz): O(n log n) -- the length-n transforms scipy runs are evaluated as
  * Bluestein chirp transforms over a power-of-two FFT in float64; signals of at most 4096 samples use the
@@ -290,7 +331,8 @@ int mmf_find_peaks(mmf_plan* plan, const double* x_dev, int64_t rows, int64_t T,
 /* Device-side PCM16 -> float32 in [-1, 1): y = x / 32768 (script/mfcc.py:373, :284 decode step). */
 int mmf_pcm16_to_f32(mmf_plan* plan, const int16_t* pcm16_dev, int64_t n, float* pcm_dev, void* stream);
 
-/* Rational-rate polyphase resampler with scipy.signal.resample_poly / upfirdn semantics:
+/* Rational-rate polyphase resampler with scipy.signal.resample_poly / upfirdn semantics, one launch for all rows
+ * (n_clips rows of n_in samples, x_stride apart):
  * y_full[m] = sum_i h[m*down - i*up] * x[i];  y = y_full[n_pre_remove : n_pre_remove + n_out].
  * h (already scaled by `up` and zero-padded as resample_poly does) is designed on the host.  The
  * step before the path: librosa.load(path, sr=sigSr) at script/mfcc.py:373, :284 (librosa uses
@@ -307,7 +349,7 @@ int mmf_mfcc_change_host(mmf_plan* plan, const float* pcm_host, int64_t n_clips,
                          int64_t clip_stride, const mmf_change_params* prm, double* tot_host, float* mfcc_host);
 
 /* sizeof() of the ABI structs as this library was compiled (0: mmf_config,
- * 1: mmf_change_params, 2: mmf_modspec_params) so bindings can verify their layout. */
+ * 1: mmf_change_params, 2: mmf_modspec_params, 3: mmf_resample_clip) so bindings can verify their layout. */
 int mmf_abi_sizeof(int32_t which);
 
 /* Number of kernels this library has launched on the calling thread since the

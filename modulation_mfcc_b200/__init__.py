@@ -15,6 +15,8 @@ from .plan import (  # noqa: F401
     host_tables,
     make_change_params,
     num_frames,
+    resample_descriptors,
+    resample_ratio,
     sos_zi,
 )
 from .api import (  # noqa: F401

@@ -102,6 +102,17 @@ class mmf_modspec_params(C.Structure):
     ]
 
 
+class mmf_resample_clip(C.Structure):
+    _fields_ = [
+        ("up", C.c_int32),
+        ("down", C.c_int32),
+        ("tap0", C.c_int64),
+        ("len_h", C.c_int32),
+        ("n_pre_remove", C.c_int64),
+        ("n_out", C.c_int64),
+    ]
+
+
 OBJ_DIR = PKG_DIR / "build"
 
 
@@ -209,6 +220,12 @@ _SIGNATURES = {
         C.c_int,
         [_vp, _vp, _i64, _vp, C.POINTER(mmf_change_params), C.POINTER(mmf_modspec_params), _vp, _vp, _vp, _vp, _vp],
     ),
+    "mmf_features_host_varlen_resampled": (
+        C.c_int,
+        [_vp, _vp, _i32, _i64, _vp, _vp, _vp, _i64, C.POINTER(mmf_change_params), C.POINTER(mmf_modspec_params),
+         _vp, _vp, _vp, _vp, _vp],
+    ),
+    "mmf_resample_varlen": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _i64, _vp]),
     "mmf_pcm16_to_f32": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
     "mmf_hilbert_envelope": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _vp, _i64, _vp]),
     "mmf_find_peaks": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _i32, _i32, _vp, _vp, _vp]),

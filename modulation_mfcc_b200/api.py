@@ -28,7 +28,7 @@ import scipy.signal
 
 from . import _lib
 from ._lib import MmfError
-from .plan import MfccConfig, Plan, frame_sizes, get_plan, make_change_params
+from .plan import MfccConfig, Plan, frame_sizes, get_plan, make_change_params, resample_ratio
 
 MODULATION_BANDS_HZ = ((0.5, 2.0), (2.0, 4.0), (4.0, 8.0), (8.0, 16.0), (16.0, 32.0))
 
@@ -281,19 +281,12 @@ def applyFilter(x, sr, /, *, filt="iir", cutOff=[None], filtLen=6, filtType="low
 # ---------------------------------------------------------------------------
 
 
-def _read_audio(path: str, sr: float, device=None, *, to_host: bool = True):
-    """Decode a WAV file to float32 in [-1, 1] shaped [channels, n] or [n] and bring
-    it to ``sr`` (librosa.load(path, sr=sr, mono=False) at script/mfcc.py:373).
-
-    Decode/resample sits *before* the measured path (SURVEY.md section 8f rank 2).
-    The file is parsed on the host (scipy's WAV reader); 16-bit PCM is scaled on the
-    device (``mmf_pcm16_to_f32``) and the rate conversion is a polyphase resampler on
-    the device (``mmf_resample_poly``: polyphase FIR with libsoxr HQ's band limits -- pass band to 0.913
-    of the lower Nyquist, 120 dB -- which is what librosa.load applies; within 1e-5 of the ideal band-limited
-    resampling below the band edge, not bit-identical to libsoxr: DESIGN.md section 6b)."""
+def _parse_wav(path: str):
+    """Host half of the WAV loader: ``(file_sr, samples)``, shaped [channels, n] or [n] (one channel).  16-bit PCM
+    stays int16 (scaled by 1/32768 on the device); 32-bit and 8-bit PCM and float files become float32 in [-1, 1]
+    here.  Anything but RIFF/WAVE raises ``ValueError`` naming the path."""
     from scipy.io import wavfile
 
-    torch = _torch()
     try:
         file_sr, data = wavfile.read(path)
     except ValueError as e:
@@ -305,23 +298,37 @@ def _read_audio(path: str, sr: float, device=None, *, to_host: bool = True):
         if data.shape[0] == 1:
             data = data[0]
     data = np.ascontiguousarray(data)
+    if data.dtype == np.int16:
+        return file_sr, data
+    if data.dtype == np.int32:
+        return file_sr, (data.astype(np.float64) / 2147483648.0).astype(np.float32)
+    if data.dtype == np.uint8:
+        return file_sr, (data.astype(np.float32) - 128.0) / 128.0
+    return file_sr, data.astype(np.float32)
+
+
+def _read_audio(path: str, sr: float, device=None, *, to_host: bool = True):
+    """Decode a WAV file to float32 in [-1, 1] shaped [channels, n] or [n] and bring
+    it to ``sr`` (librosa.load(path, sr=sr, mono=False) at script/mfcc.py:373).
+
+    Decode/resample sits *before* the measured path (SURVEY.md section 8f rank 2).
+    The file is parsed on the host (scipy's WAV reader); 16-bit PCM is scaled on the
+    device (``mmf_pcm16_to_f32``) and the rate conversion is a polyphase resampler on
+    the device (``mmf_resample_poly``: polyphase FIR with libsoxr HQ's band limits -- pass band to 0.913
+    of the lower Nyquist, 120 dB -- which is what librosa.load applies; within 1e-5 of the ideal band-limited
+    resampling below the band edge, not bit-identical to libsoxr: DESIGN.md section 6b).  A corpus of files goes
+    through :meth:`FeatureExtractor.host_files` instead, in one call."""
+    torch = _torch()
+    file_sr, data = _parse_wav(path)
     plan = _any_plan(_device_index(device))
     try:
         if data.dtype == np.int16:
             y = plan.pcm16_to_f32(data)
         else:
-            if data.dtype == np.int32:
-                host = (data.astype(np.float64) / 2147483648.0).astype(np.float32)
-            elif data.dtype == np.uint8:
-                host = (data.astype(np.float32) - 128.0) / 128.0
-            else:
-                host = data.astype(np.float32)
-            y = _to_dev(host, torch.float32, plan.cfg.device)
+            y = _to_dev(data, torch.float32, plan.cfg.device)
         if sr is not None and float(file_sr) != float(sr):
-            from fractions import Fraction
-
-            fr = Fraction(float(sr) / float(file_sr)).limit_denominator(1000)
-            y = plan.resample_poly(y, fr.numerator, fr.denominator, quality="hq")
+            up, down = resample_ratio(file_sr, sr)
+            y = plan.resample_poly(y, up, down, quality="hq")
     except MmfError as e:
         _raise_from(e)
     return np.ascontiguousarray(y.cpu().numpy()) if to_host else y
@@ -822,24 +829,26 @@ class FeatureExtractor:
             _raise_from(e)
 
     def host_varlen(self, pcm_host, offsets, *, want=("totChange", "mfcc", "delta", "modspec", "band_energy"),
-                    out=None):
+                    out=None, rates=None):
         """:meth:`host_call` for clips of different lengths packed back to back in one 1-D host buffer (float32, or
         int16 WAV samples): clip ``i`` is ``pcm_host[offsets[i]:offsets[i + 1]]``.  Returns the packed arrays of
         :meth:`Plan.features_host_varlen` with this extractor's modulation geometry; each clip's blocks equal
-        :meth:`host_call` on that clip alone, bit for bit."""
+        :meth:`host_call` on that clip alone, bit for bit.  ``rates``: each clip's sample rate; clips are then
+        resampled to the extractor's rate on the device as the WAV loader resamples them, and each clip's blocks
+        equal :meth:`host_call` on the loader's resampled clip."""
         mod = self.modspec_geometry(0) if ("modspec" in want or "band_energy" in want) else None
         try:
-            return self.plan.features_host_varlen(pcm_host, offsets, self.prm, mod, want=want, out=out)
+            return self.plan.features_host_varlen(pcm_host, offsets, self.prm, mod, want=want, out=out, rates=rates)
         except MmfError as e:
             _raise_from(e)
 
-    def host_many(self, clips, *, want=("totChange", "mfcc", "delta", "modspec", "band_energy")):
+    def host_many(self, clips, *, want=("totChange", "mfcc", "delta", "modspec", "band_energy"), rates=None):
         """:meth:`host_varlen` for a list of 1-D numpy clips of any lengths (all int16, or anything else as float32).
         Concatenates them once and returns one dict per clip of zero-copy views into the packed arrays, shaped as
         :func:`mfcc_features_batch` returns one clip without its batch axis (``totChange [T]``, ``mfcc`` /
         ``delta [n_mfcc, T]``, ``modspec [n_mfcc, W, nfft/2+1]``, ``band_energy [W, n_bands]``), plus ``T``, the
-        frame times.  A corpus already held in one buffer should call :meth:`host_varlen` with its offsets instead,
-        which saves the concatenation."""
+        frame times (at the extractor's rate when ``rates`` are given).  A corpus already held in one buffer should
+        call :meth:`host_varlen` with its offsets instead, which saves the concatenation."""
         clips = [np.asarray(c) for c in clips]
         if not clips:
             return []
@@ -848,7 +857,7 @@ class FeatureExtractor:
         dt = np.int16 if all(c.dtype == np.int16 for c in clips) else np.float32
         offsets = np.zeros(len(clips) + 1, np.int64)
         np.cumsum([c.shape[0] for c in clips], out=offsets[1:])
-        res = self.host_varlen(np.concatenate(clips).astype(dt, copy=False), offsets, want=want)
+        res = self.host_varlen(np.concatenate(clips).astype(dt, copy=False), offsets, want=want, rates=rates)
         nm = self.plan.cfg.n_mfcc
         _, _, nfft, bins = self.modspec_geometry(0)
         nb, n_bands = nfft // 2 + 1, len(bins)
@@ -868,6 +877,23 @@ class FeatureExtractor:
             d["T"] = _time_anchors(T, self.tStep, self.winLen)
             out.append(d)
         return out
+
+    def host_files(self, paths, *, channel: int = 0, want=("totChange", "mfcc", "delta", "modspec", "band_energy")):
+        """A corpus of WAV files at any sample rates through one :meth:`host_many` call.  Each file is parsed on the
+        host, channel ``channel`` of a multi-channel file is kept, and its native samples cross PCIe once (as int16
+        when every file is 16-bit PCM, else as float32) to be resampled on the device to the extractor's rate.
+        Returns one dict per file, as :meth:`host_many` does; each file's blocks equal :meth:`host_call` on
+        ``_read_audio(path, sr)[channel]``, bit for bit (rows are resampled independently, so selecting the channel
+        first changes nothing).  A file that is not RIFF/WAVE raises ``ValueError`` naming its path."""
+        rates, clips = [], []
+        for p in paths:
+            file_sr, data = _parse_wav(p)
+            rates.append(float(file_sr))
+            clips.append(data[channel] if data.ndim > 1 else data)
+        if clips and not all(c.dtype == np.int16 for c in clips):
+            # (float)x * 2^-15, as the device scales int16
+            clips = [c.astype(np.float32) / np.float32(32768.0) if c.dtype == np.int16 else c for c in clips]
+        return self.host_many(clips, want=want, rates=rates)
 
     def __call__(self, pcm, *, want_logmel: bool = True, want_modspec: bool = True):
         res = self.plan.mfcc_change(pcm, self.prm, want_logmel=want_logmel, want_mfcc=True, want_delta=True)

@@ -464,6 +464,7 @@ int mmf_abi_sizeof(int32_t which) {
     case 0: return (int)sizeof(mmf_config);
     case 1: return (int)sizeof(mmf_change_params);
     case 2: return (int)sizeof(mmf_modspec_params);
+    case 3: return (int)sizeof(mmf_resample_clip);
     default: return -1;
   }
 }
@@ -1772,6 +1773,70 @@ static int validate_offsets(int64_t n_clips, const int64_t* offsets) {
   return MMF_OK;
 }
 
+// Resampling descriptors of a packed batch (mmf_features_host_varlen_resampled, mmf_resample_varlen), after the
+// offsets passed validate_offsets; no plan or device needed.  Taps are checked only for the clips that read them.
+static int validate_resample(int64_t n_clips, const int64_t* offsets, const mmf_resample_clip* rs, const float* h,
+                             int64_t n_h) {
+  if (!rs) return fail(MMF_ERR_INVALID, "rs_host is NULL");
+  for (int64_t i = 0; i < n_clips; ++i) {
+    const mmf_resample_clip& r = rs[i];
+    const int64_t len = offsets[i + 1] - offsets[i];
+    char buf[256];
+    auto bad = [&](const char* what) {
+      std::snprintf(buf, sizeof(buf), "clip %lld: %s (up %d, down %d, tap0 %lld, len_h %d, n_pre_remove %lld, n_out "
+                    "%lld, %lld samples, %lld taps)", (long long)i, what, r.up, r.down, (long long)r.tap0, r.len_h,
+                    (long long)r.n_pre_remove, (long long)r.n_out, (long long)len, (long long)n_h);
+      return fail(MMF_ERR_INVALID, buf);
+    };
+    if (r.up < 1 || r.down < 1) return bad("up and down must be >= 1");
+    const bool copy = r.up == 1 && r.down == 1;
+    const __int128 num = (__int128)len * r.up;
+    if (r.n_out != (int64_t)((num + r.down - 1) / r.down))
+      return bad(copy ? "a clip at the plan's rate needs n_out = its length" : "n_out must be ceil(len * up / down)");
+    if (copy) continue;
+    if (r.len_h < 1 || r.len_h > (1 << 22)) return bad("len_h must be in [1, 2^22]");
+    if (!h || r.tap0 < 0 || r.tap0 > n_h - r.len_h) return bad("taps [tap0, tap0 + len_h) must lie in the tap table");
+    if (r.n_pre_remove < 0) return bad("n_pre_remove must be >= 0");
+  }
+  return MMF_OK;
+}
+
+// Device descriptors of clips [c0, c1) of a packed batch for resample_rows_launch: RsClip[nc], then first_item[nc + 1],
+// appended to `desc` (16-byte aligned parts).  Sources count from `base`; rs == NULL: every clip at the plan's rate.
+// Returns the number of work items, or -1 past 2^31 - 1.
+static int64_t resample_desc(int64_t c0, int64_t c1, const int64_t* offsets, int64_t base,
+                             const mmf_resample_clip* rs, std::vector<unsigned char>& desc, size_t& o_clips,
+                             size_t& o_first) {
+  const int64_t nc = c1 - c0;
+  o_clips = align_up(desc.size(), 16);
+  o_first = align_up(o_clips + (size_t)nc * sizeof(RsClip), 16);
+  desc.resize(align_up(o_first + (size_t)(nc + 1) * 4, 16), 0);
+  RsClip* cl = (RsClip*)(desc.data() + o_clips);
+  unsigned* first = (unsigned*)(desc.data() + o_first);
+  int64_t items = 0;
+  for (int64_t k = 0; k < nc; ++k) {
+    const int64_t i = c0 + k, len = offsets[i + 1] - offsets[i];
+    RsClip r{};
+    r.src = (long)(offsets[i] - base);
+    r.n_in = (long)len;
+    r.copy = !rs || (rs[i].up == 1 && rs[i].down == 1);
+    r.n_out = (long)(r.copy ? len : rs[i].n_out);
+    if (!r.copy) {
+      r.up = rs[i].up;
+      r.down = rs[i].down;
+      r.len_h = rs[i].len_h;
+      r.n_pre_remove = (long)rs[i].n_pre_remove;
+      r.tap0 = (long)rs[i].tap0;
+    }
+    cl[k] = r;
+    first[k] = (unsigned)items;
+    items += (r.n_out + kRsOut - 1) / kRsOut;
+    if (items > 0x7fffffffLL) return -1;
+  }
+  first[nc] = (unsigned)items;
+  return items;
+}
+
 // frame_off / win_off of a packed batch (mmf_features_varlen_sizes); n_win_i = 0 without modulation windows
 static void packed_sizes(int n_fft, int hop, int win, int mod_hop, int64_t n_clips, const int64_t* offsets,
                          int64_t* frame_off, int64_t* win_off) {
@@ -1790,20 +1855,24 @@ struct HostChunk {
   int64_t stride;  // samples per staged row: the chunk's longest clip, rounded up to 16 bytes for the TMA
   ChangeVarlen cv;
   ModspecVarlen mv;  // routed when the chunk has modulation windows (mv.W > 0)
-  std::vector<unsigned char> desc;  // staging offsets and compaction descriptors
-  size_t o_off, o_cnt_t, o_off_t, o_cnt_w, o_off_w;  // within desc
+  int64_t items;   // staging work items (resample_rows_launch)
+  std::vector<unsigned char> desc;  // staging and compaction descriptors
+  size_t o_rs, o_first, o_cnt_t, o_off_t, o_cnt_w, o_off_w;  // within desc
   size_t o_desc, o_cv_desc, o_mv_desc;  // desc, cv.desc and mv.desc in the descriptor region of the call
   size_t o_h2d, o_pcm, o_tot, o_mfcc, o_delta, o_mag, o_band, o_ptot, o_pmfcc, o_pdelta, o_pmag, o_pband,
       o_scratch, end;
 };
 
-// pcm_host: float32 samples, or (pcm16 != 0) int16 samples converted on the device
+// pcm_host: float32 samples, or (pcm16 != 0) int16 samples converted on the device.  resampled: clip i reaches the
+// plan's rate as rs[i] says, with taps from h[n_h]; otherwise every clip is at the plan's rate.
 static int features_host_varlen_impl(mmf_plan* plan, const void* pcm_host_v, int pcm16, int64_t n_clips,
-                                     const int64_t* offsets, const mmf_change_params* prm,
+                                     const int64_t* offsets, bool resampled, const mmf_resample_clip* rs,
+                                     const float* h_taps, int64_t n_h, const mmf_change_params* prm,
                                      const mmf_modspec_params* mod, double* tot_host, float* mfcc_host,
                                      float* delta_host, float* mag_host, float* band_host) {
   int rc = validate_offsets(n_clips, offsets);
   if (rc) return rc;
+  if (resampled && (rc = validate_resample(n_clips, offsets, rs, h_taps, n_h))) return rc;
   if (!plan || !pcm_host_v || !prm || !tot_host) return fail(MMF_ERR_INVALID, "NULL argument");
   if ((mag_host || band_host) && !mod) return fail(MMF_ERR_INVALID, "modulation outputs requested without parameters");
   const mmf_config& c = plan->cfg;
@@ -1816,26 +1885,36 @@ static int features_host_varlen_impl(mmf_plan* plan, const void* pcm_host_v, int
   const int nbe = want_mod && band_host ? mod->n_bands : 0;  // band outputs actually written
   const bool need_mfcc_dev = mfcc_host || want_mod;
   const size_t n = (size_t)n_clips;
-  std::vector<int64_t> len(n), T(n), F(n + 1), Wo(n + 1);
-  for (size_t i = 0; i < n; ++i) len[i] = offsets[i + 1] - offsets[i];
-  packed_sizes(c.n_fft, c.hop_length, want_mod ? mod->win : 0, want_mod ? mod->hop : 1, n_clips, offsets, F.data(),
-               Wo.data());
+  // len_in: samples as they cross PCIe; len: samples at the plan's rate (what the ragged path sees)
+  std::vector<int64_t> len_in(n), len(n), out_off(n + 1, 0), T(n), F(n + 1), Wo(n + 1);
+  for (size_t i = 0; i < n; ++i) {
+    len_in[i] = offsets[i + 1] - offsets[i];
+    len[i] = rs ? rs[i].n_out : len_in[i];
+    out_off[i + 1] = out_off[i] + len[i];
+  }
+  packed_sizes(c.n_fft, c.hop_length, want_mod ? mod->win : 0, want_mod ? mod->hop : 1, n_clips, out_off.data(),
+               F.data(), Wo.data());
   for (size_t i = 0; i < n; ++i) T[i] = F[i + 1] - F[i];
+  // the tap table goes up with the descriptors when some clip reads it
+  int64_t n_taps = 0;
+  for (size_t i = 0; rs && i < n; ++i) n_taps = (rs[i].up == 1 && rs[i].down == 1) ? n_taps : n_h;
 
   // ---- chunks, planned and routed before anything is queued.  Budgets in bytes of float32 samples, those of
-  // features_host_impl (from its sweep): the real samples of a chunk, and its staged rows at twice that, so that one
-  // long clip among short ones cannot inflate the padded intermediates.  A clip over either budget is a chunk alone.
+  // features_host_impl (from its sweep): the samples of a chunk as they cross PCIe, and its staged rows at the plan's
+  // rate at twice that, so that one long clip among short ones cannot inflate the padded intermediates.  A clip over
+  // either budget is a chunk alone.
   const int64_t budget = pcm16 ? (96 << 20) : (32 << 20);
   const size_t isz = pcm16 ? 2 : 4;
   std::vector<HostChunk> chunks;
-  size_t slot = 0, desc_bytes = 0;
+  // the descriptor region: the taps, then each chunk's descriptors
+  size_t slot = 0, desc_bytes = align_up((size_t)n_taps * 4, 256);
   for (int64_t c0 = 0; c0 < n_clips;) {
-    int64_t c1 = c0 + 1, real = len[c0], n_max = len[c0];
+    int64_t c1 = c0 + 1, real = len_in[c0], n_max = len[c0];
     // (at most 65535 clips: the compaction's one CTA per row stays far inside the grid limit)
     while (c1 < n_clips && c1 - c0 < 65535) {
       const int64_t m = std::max(n_max, len[c1]);
-      if ((real + len[c1]) * 4 > budget || (c1 + 1 - c0) * ((m + 3) & ~3LL) * 4 > 2 * budget) break;
-      real += len[c1];
+      if ((real + len_in[c1]) * 4 > budget || (c1 + 1 - c0) * ((m + 3) & ~3LL) * 4 > 2 * budget) break;
+      real += len_in[c1];
       n_max = m;
       ++c1;
     }
@@ -1855,20 +1934,20 @@ static int features_host_varlen_impl(mmf_plan* plan, const void* pcm_host_v, int
         (rc = modspec_varlen_route((unsigned)c.flags, T.data() + c0, nc, nm, W, mod->win, mod->hop, mod->nfft, nbe,
                                    mag_host != nullptr, h.mv)))
       return rc;
-    // descriptors: staging offsets [nc + 1], then frames / windows and their packed offsets per clip
-    size_t d = 0;
+    // descriptors: the staging launch's, then frames / windows and their packed offsets per clip
+    h.items = resample_desc(c0, c1, offsets, offsets[c0], rs, h.desc, h.o_rs, h.o_first);
+    if (h.items < 0) return fail(MMF_ERR_UNSUPPORTED, "a chunk of more than 2^31 - 1 staging work items");
+    size_t d = h.desc.size();
     auto dtake = [&](size_t bytes) {
       const size_t o = d;
       d += align_up(bytes, 16);
       return o;
     };
-    h.o_off = dtake((nc + 1) * 8);
     h.o_cnt_t = dtake(nc * 4);
     h.o_off_t = dtake(nc * 8);
     h.o_cnt_w = dtake(nc * 4);
     h.o_off_w = dtake(nc * 8);
-    h.desc.assign(d, 0);
-    for (int64_t i = 0; i <= nc; ++i) ((int64_t*)(h.desc.data() + h.o_off))[i] = offsets[c0 + i] - offsets[c0];
+    h.desc.resize(d, 0);
     for (int64_t i = 0; i < nc; ++i) {
       ((int*)(h.desc.data() + h.o_cnt_t))[i] = (int)T[c0 + i];
       ((int64_t*)(h.desc.data() + h.o_off_t))[i] = F[c0 + i] - F[c0];
@@ -1923,6 +2002,7 @@ static int features_host_varlen_impl(mmf_plan* plan, const void* pcm_host_v, int
     unsigned char* d_desc = (unsigned char*)plan->host_ws;
     {
       std::vector<unsigned char> all(desc_bytes);
+      if (n_taps) std::memcpy(all.data(), h_taps, (size_t)n_taps * 4);
       for (const HostChunk& h : chunks) {
         std::memcpy(all.data() + h.o_desc, h.desc.data(), h.desc.size());
         std::memcpy(all.data() + h.o_cv_desc, h.cv.desc.data(), h.cv.desc.size());
@@ -1944,9 +2024,10 @@ static int features_host_varlen_impl(mmf_plan* plan, const void* pcm_host_v, int
       MMF_CUDA(cudaMemcpyAsync(dev(h.o_h2d), (const unsigned char*)pcm_host_v + (size_t)offsets[h.c0] * isz,
                                (size_t)(offsets[h.c1] - offsets[h.c0]) * isz, cudaMemcpyHostToDevice, st));
       float* d_pcm = (float*)dev(h.o_pcm);
-      cudaError_t e = stage_rows_launch(dev(h.o_h2d), pcm16, (const long*)(dd + h.o_off), (long)nc, (long)h.stride,
-                                        d_pcm, st);
-      if (e != cudaSuccess) return cuda_fail(e, "stage_rows_kernel launch");
+      cudaError_t e = resample_rows_launch(dev(h.o_h2d), pcm16, (const RsClip*)(dd + h.o_rs),
+                                           (const unsigned*)(dd + h.o_first), (long)nc, (long)h.items,
+                                           (const float*)d_desc, d_pcm, (long)h.stride, st);
+      if (e != cudaSuccess) return cuda_fail(e, "resample_rows_kernel launch");
       double* d_tot = (double*)dev(h.o_tot);
       float* d_mfcc = need_mfcc_dev ? (float*)dev(h.o_mfcc) : nullptr;
       float* d_delta = delta_host ? (float*)dev(h.o_delta) : nullptr;
@@ -1999,6 +2080,30 @@ static int features_host_varlen_impl(mmf_plan* plan, const void* pcm_host_v, int
   return MMF_OK;
 }
 
+// One ragged resampling launch on `st` from host descriptors: descriptors, work-item offsets and taps h[n_h] go up in
+// one copy to stream-ordered scratch (pageable source: the copy is staged, so the host data may go when this returns).
+static int resample_dev(mmf_plan* plan, const float* x_dev, const std::vector<RsClip>& cl,
+                        const std::vector<unsigned>& first, const float* h, int64_t n_h, float* y_dev,
+                        int64_t y_stride, cudaStream_t st) {
+  const size_t o_first = align_up(cl.size() * sizeof(RsClip), 256);
+  const size_t o_h = align_up(o_first + first.size() * 4, 256);
+  const size_t bytes = o_h + (size_t)n_h * 4;
+  std::vector<unsigned char> up(bytes);
+  std::memcpy(up.data(), cl.data(), cl.size() * sizeof(RsClip));
+  std::memcpy(up.data() + o_first, first.data(), first.size() * 4);
+  if (n_h) std::memcpy(up.data() + o_h, h, (size_t)n_h * 4);
+  MMF_CUDA(cudaSetDevice(plan->cfg.device));
+  unsigned char* d = nullptr;
+  MMF_CUDA(cudaMallocAsync((void**)&d, bytes, st));
+  cudaError_t e = cudaMemcpyAsync(d, up.data(), bytes, cudaMemcpyHostToDevice, st);
+  if (e == cudaSuccess)
+    e = resample_rows_launch(x_dev, 0, (const RsClip*)d, (const unsigned*)(d + o_first), (long)cl.size(),
+                             (long)first.back(), (const float*)(d + o_h), y_dev, (long)y_stride, st);
+  cudaFreeAsync(d, st);
+  if (e != cudaSuccess) return cuda_fail(e, "resample_rows_kernel launch");
+  return MMF_OK;
+}
+
 }  // namespace mmf
 
 extern "C" {
@@ -2020,16 +2125,25 @@ int mmf_features_varlen_sizes(const mmf_config* cfg, const mmf_modspec_params* m
 int mmf_features_host_varlen(mmf_plan* plan, const float* pcm_host, int64_t n_clips, const int64_t* offsets_host,
                              const mmf_change_params* prm, const mmf_modspec_params* mod, double* tot_host,
                              float* mfcc_host, float* delta_host, float* mag_host, float* band_host) {
-  return mmf::features_host_varlen_impl(plan, pcm_host, 0, n_clips, offsets_host, prm, mod, tot_host, mfcc_host,
-                                        delta_host, mag_host, band_host);
+  return mmf::features_host_varlen_impl(plan, pcm_host, 0, n_clips, offsets_host, false, nullptr, nullptr, 0, prm, mod,
+                                        tot_host, mfcc_host, delta_host, mag_host, band_host);
+}
+
+int mmf_features_host_varlen_resampled(mmf_plan* plan, const void* pcm_host, int32_t pcm16, int64_t n_clips,
+                                       const int64_t* offsets_host, const mmf_resample_clip* rs_host,
+                                       const float* h_host, int64_t n_h, const mmf_change_params* prm,
+                                       const mmf_modspec_params* mod, double* tot_host, float* mfcc_host,
+                                       float* delta_host, float* mag_host, float* band_host) {
+  return mmf::features_host_varlen_impl(plan, pcm_host, pcm16 ? 1 : 0, n_clips, offsets_host, true, rs_host, h_host,
+                                        n_h, prm, mod, tot_host, mfcc_host, delta_host, mag_host, band_host);
 }
 
 int mmf_features_host_varlen_pcm16(mmf_plan* plan, const int16_t* pcm16_host, int64_t n_clips,
                                    const int64_t* offsets_host, const mmf_change_params* prm,
                                    const mmf_modspec_params* mod, double* tot_host, float* mfcc_host,
                                    float* delta_host, float* mag_host, float* band_host) {
-  return mmf::features_host_varlen_impl(plan, pcm16_host, 1, n_clips, offsets_host, prm, mod, tot_host, mfcc_host,
-                                        delta_host, mag_host, band_host);
+  return mmf::features_host_varlen_impl(plan, pcm16_host, 1, n_clips, offsets_host, false, nullptr, nullptr, 0, prm, mod,
+                                        tot_host, mfcc_host, delta_host, mag_host, band_host);
 }
 
 }  // extern "C"
@@ -2095,18 +2209,42 @@ int mmf_resample_poly(mmf_plan* plan, const float* x_dev, int64_t n_clips, int64
   if (n_clips < 1 || n_clips > 65535 || n_in < 1 || n_out < 1) return fail(MMF_ERR_INVALID, "bad sizes");
   if (up < 1 || down < 1 || len_h < 1 || len_h > (1 << 22))
     return fail(MMF_ERR_UNSUPPORTED, "need up, down >= 1 and a filter of at most 2^22 taps");
-  MMF_CUDA(cudaSetDevice(plan->cfg.device));
-  cudaStream_t st = (cudaStream_t)stream;
-  float* h_dev = nullptr;  // stream-ordered scratch for the taps (pageable source: the copy is staged, so
-                           // h_host may be reused as soon as this call returns)
-  MMF_CUDA(cudaMallocAsync((void**)&h_dev, (size_t)len_h * 4, st));
-  cudaError_t e = cudaMemcpyAsync(h_dev, h_host, (size_t)len_h * 4, cudaMemcpyHostToDevice, st);
-  if (e == cudaSuccess)
-    e = resample_poly_launch(x_dev, n_clips, n_in, x_stride, h_dev, len_h, up, down, n_pre_remove, n_out, y_stride,
-                             y_dev, st);
-  cudaFreeAsync(h_dev, st);
-  if (e != cudaSuccess) return cuda_fail(e, "resample_poly_kernel launch");
-  return MMF_OK;
+  if ((n_out + kRsOut - 1) / kRsOut * n_clips > 0x7fffffffLL) return fail(MMF_ERR_UNSUPPORTED, "too many outputs");
+  // one descriptor per row, all reading the one filter (up = down = 1 filters too: nothing here is a copy)
+  std::vector<RsClip> cl((size_t)n_clips);
+  std::vector<unsigned> first((size_t)n_clips + 1);
+  const int64_t per = (n_out + kRsOut - 1) / kRsOut;
+  for (int64_t r = 0; r < n_clips; ++r) {
+    cl[r] = RsClip{(long)(r * x_stride), (long)n_in, (long)n_pre_remove, (long)n_out, 0, up, down, len_h, 0};
+    first[r] = (unsigned)(r * per);
+  }
+  first[n_clips] = (unsigned)(n_clips * per);
+  return resample_dev(plan, x_dev, cl, first, h_host, len_h, y_dev, y_stride, (cudaStream_t)stream);
+}
+
+int mmf_resample_varlen(mmf_plan* plan, const float* x_dev, int64_t n_clips, const int64_t* offsets_host,
+                        const mmf_resample_clip* rs_host, const float* h_host, int64_t n_h, float* y_dev,
+                        int64_t y_stride, void* stream) {
+  int rc = validate_offsets(n_clips, offsets_host);
+  if (rc || (rc = validate_resample(n_clips, offsets_host, rs_host, h_host, n_h))) return rc;
+  if (!plan || !x_dev || !y_dev) return fail(MMF_ERR_INVALID, "NULL argument");
+  for (int64_t i = 0; i < n_clips; ++i)
+    if (rs_host[i].n_out > y_stride) {
+      char buf[128];
+      std::snprintf(buf, sizeof(buf), "clip %lld: n_out %lld exceeds y_stride %lld", (long long)i,
+                    (long long)rs_host[i].n_out, (long long)y_stride);
+      return fail(MMF_ERR_INVALID, buf);
+    }
+  int64_t n_taps = 0;
+  for (int64_t i = 0; i < n_clips; ++i) n_taps = (rs_host[i].up == 1 && rs_host[i].down == 1) ? n_taps : n_h;
+  std::vector<unsigned char> desc;
+  size_t o_rs, o_first;
+  const int64_t items = resample_desc(0, n_clips, offsets_host, 0, rs_host, desc, o_rs, o_first);
+  if (items < 0) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 work items");
+  const RsClip* c = (const RsClip*)(desc.data() + o_rs);
+  const unsigned* f = (const unsigned*)(desc.data() + o_first);
+  return resample_dev(plan, x_dev, std::vector<RsClip>(c, c + n_clips), std::vector<unsigned>(f, f + n_clips + 1),
+                      h_host, n_taps, y_dev, y_stride, (cudaStream_t)stream);
 }
 
 int mmf_mfcc_change_host(mmf_plan* plan, const float* pcm_host, int64_t n_clips, int64_t n_samples,

@@ -259,15 +259,22 @@ cudaError_t hilbert_fft_launch(const float* x, long n_clips, long n, long stride
 cudaError_t find_peaks_launch(const double* x, long rows, long T, long stride, int minima, int max_peaks, int* idx,
                               int* count, cudaStream_t st);
 cudaError_t pcm16_to_f32_launch(const int16_t* x, long n, float* y, cudaStream_t st);
-// packed batch of the host-buffer bundle: clip i (samples [off[i], off[i + 1]) of x, float32 or int16) -> row i of
-// y [n_clips, stride]; and padded output rows -> packed blocks (see post_kernels.cu)
-cudaError_t stage_rows_launch(const void* x, int pcm16, const long* off, long n_clips, long stride, float* y,
-                              cudaStream_t st);
+// One clip of a ragged resampling launch (device descriptor, built on the host).  Output sample m of the clip is
+// y_full[m + n_pre_remove] of upfirdn(h, x, up, down) over the clip's n_in samples at x + src; a plan-rate clip
+// (copy != 0) is copied instead.  The clip's filter is h[tap0 .. tap0 + len_h) of the launch's tap table.
+struct RsClip {
+  long src, n_in, n_pre_remove, n_out, tap0;
+  int up, down, len_h, copy;
+};
+constexpr int kRsOut = 256;  // outputs per work item of resample_rows_launch (one per thread)
+// Clip c owns work items [first_item[c], first_item[c + 1]) (ceil(n_out / kRsOut) each); item k of the clip writes
+// outputs [k * kRsOut, (k + 1) * kRsOut) of row c of y.  x is float32 or (pcm16) int16 scaled by 1/32768.
+cudaError_t resample_rows_launch(const void* x, int pcm16, const RsClip* clips, const unsigned* first_item,
+                                 long n_clips, long n_items, const float* h, float* y, long y_stride,
+                                 cudaStream_t st);
+// padded output rows -> packed blocks of the host-buffer bundle (see post_kernels.cu)
 cudaError_t compact_rows_launch(const void* src, void* dst, int elem_bytes, long n_clips, int rows, int unit,
                                 long pitch, const int* cnt, const long* off, cudaStream_t st);
-cudaError_t resample_poly_launch(const float* x, long n_clips, long n_in, long x_stride, const float* h_dev, int len_h,
-                                 int up, int down, long n_pre_remove, long n_out, long y_stride, float* y,
-                                 cudaStream_t st);
 
 // ---- host tables (host_tables.cpp)
 struct MelSparse {

@@ -1036,33 +1036,6 @@ cudaError_t pcm16_to_f32_launch(const int16_t* x, long n, float* y, cudaStream_t
   return cudaGetLastError();
 }
 
-// Host-buffer bundle of a packed batch: clip i, samples [off[i], off[i + 1]) of the chunk as it crossed PCIe, goes to
-// row i of the [n_clips, stride] buffer the ragged K1 reads.  Samples of a row past its clip's length are not written
-// (the ragged path reads them as zero whatever they hold).  int16 input is scaled as pcm16_to_f32_kernel scales it.
-template <typename X>
-__global__ void stage_rows_kernel(const X* __restrict__ x, const long* __restrict__ off, long n_clips, long stride,
-                                  float* __restrict__ y) {
-  constexpr float k = 1.0f / 32768.0f;
-  for (long e = (long)blockIdx.x * blockDim.x + threadIdx.x; e < n_clips * stride; e += (long)gridDim.x * blockDim.x) {
-    const long clip = e / stride, s = e - clip * stride;
-    const long src = off[clip] + s;
-    if (src >= off[clip + 1]) continue;
-    if constexpr (sizeof(X) == 2) y[e] = (float)x[src] * k;
-    else y[e] = x[src];
-  }
-}
-
-cudaError_t stage_rows_launch(const void* x, int pcm16, const long* off, long n_clips, long stride, float* y,
-                              cudaStream_t st) {
-  const long blocks = std::min<long>((n_clips * stride + 255) / 256, 1L << 20);
-  if (pcm16)
-    stage_rows_kernel<<<(unsigned)blocks, 256, 0, st>>>((const int16_t*)x, off, n_clips, stride, y);
-  else
-    stage_rows_kernel<<<(unsigned)blocks, 256, 0, st>>>((const float*)x, off, n_clips, stride, y);
-  count_launch();
-  return cudaGetLastError();
-}
-
 // Padded rows -> packed blocks.  Clip i owns `rows` rows of cnt[i] * unit elements, the first at
 // src + i * rows * pitch, the next `pitch` elements on; they leave back to back at dst + off[i] * rows * unit.  One CTA
 // per (clip, row); a plain copy, so the bits are kept.
@@ -1089,35 +1062,83 @@ cudaError_t compact_rows_launch(const void* src, void* dst, int elem_bytes, long
 }
 
 // ---------------------------------------------------------------------------
-// Polyphase rational resampler: scipy.signal.resample_poly / upfirdn semantics,
-// y_full[m] = sum_i h[m*down - i*up] * x[i], then y = y_full[n_pre_remove : n_pre_remove + n_out]
-// (the step before the path: librosa.load(sr=sigSr) at script/mfcc.py:373, :284).
-// One thread per output sample, ~len(h)/up taps each, float64 accumulation.
+// Ragged, multi-ratio polyphase resampler with scipy.signal.resample_poly / upfirdn semantics
+// (the step before the path: librosa.load(sr=sigSr) at script/mfcc.py:373, :284).  For each clip,
+//   y_full[m] = sum_i h[m*down - i*up] * x[i],  y = y_full[n_pre_remove : n_pre_remove + n_out],
+// each output one float64 fma chain over i ascending from i_lo to i_hi (the bounds below, from the clip's own len_h).
+// That order is the contract: every output's bits are fixed by it, whatever the layout of taps and samples.
+// A work item is kRsOut consecutive outputs of one clip, one per thread.  Its input span goes through shared memory in
+// coalesced tiles (int16 scaled on load, as pcm16_to_f32_kernel scales it); one tile holds the span of every ratio
+// whose 256 outputs need at most kRsTile inputs (all the usual audio rates), more tiles walk i in order.  The tap
+// table in its natural order is already polyphase (tap j of phase p at j * up + p): at each step of the chain, the
+// threads of a warp away from the clip's edges read taps within one window of about 2 * up floats, from L1.  Plan-rate
+// clips (copy) are staged as the packed host path always staged them: x, or (float)x / 32768 for int16, in the same
+// launch.
 // ---------------------------------------------------------------------------
-__global__ void resample_poly_kernel(const float* __restrict__ x, long n_in, long x_stride, const float* __restrict__ h,
-                                     int len_h, int up, int down, long n_pre_remove, long n_out, long y_stride,
-                                     float* __restrict__ y) {
-  const long mo = (long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (mo >= n_out) return;
-  const float* xr = x + (size_t)blockIdx.y * x_stride;
-  const long pos = (mo + n_pre_remove) * down;  // position in the zero-stuffed input
-  long i_hi = pos / up;                         // largest i with pos - i*up >= 0
-  if (i_hi > n_in - 1) i_hi = n_in - 1;
-  long i_lo = (pos - len_h + up) / up;          // smallest i with pos - i*up <= len_h - 1 (ceil for pos >= len_h - 1)
-  if (pos - len_h + 1 <= 0) i_lo = 0;
-  double acc = 0.0;
-  for (long i = i_lo; i <= i_hi; ++i) {
-    const long k = pos - i * up;
-    if (k >= 0 && k < len_h) acc = fma((double)h[k], (double)xr[i], acc);
+constexpr int kRsTile = 4096;
+
+template <typename X>
+__global__ void __launch_bounds__(kRsOut) resample_rows_kernel(const X* __restrict__ x, const RsClip* __restrict__ clips,
+                                                               const unsigned* __restrict__ first_item, long n_clips,
+                                                               const float* __restrict__ hp, float* __restrict__ y,
+                                                               long y_stride) {
+  __shared__ float xs[kRsTile];
+  constexpr float kq = 1.0f / 32768.0f;
+  const unsigned item = blockIdx.x;
+  long clip = 0, hi_c = n_clips - 1;  // the clip owning this item: the last with first_item[clip] <= item
+  while (clip < hi_c) {
+    const long mid = (clip + hi_c + 1) >> 1;
+    if (first_item[mid] <= item) clip = mid;
+    else hi_c = mid - 1;
   }
-  y[(size_t)blockIdx.y * y_stride + mo] = (float)acc;
+  const RsClip c = clips[clip];
+  const X* xr = x + c.src;
+  float* yr = y + clip * y_stride;
+  const long m0 = (long)(item - first_item[clip]) * kRsOut, mo = m0 + threadIdx.x;
+  const long m_last = min(m0 + kRsOut, c.n_out) - 1;
+  auto ld = [&](long i) -> float {
+    if constexpr (sizeof(X) == 2) return (float)xr[i] * kq;
+    else return xr[i];
+  };
+  if (c.copy) {
+    if (mo <= m_last) yr[mo] = ld(mo);
+    return;
+  }
+  // i_hi: largest i with pos - i*up >= 0; i_lo: smallest i with pos - i*up <= len_h - 1
+  auto lo_of = [&](long pos) { return pos - c.len_h + 1 <= 0 ? 0L : (pos - c.len_h + c.up) / c.up; };
+  auto hi_of = [&](long pos) { return min(pos / c.up, c.n_in - 1); };
+  const long pos = (min(mo, m_last) + c.n_pre_remove) * c.down;  // position in the zero-stuffed input
+  const long q = pos / c.up;
+  long i_lo = lo_of(pos), i_hi = hi_of(pos);
+  if (mo > m_last) i_lo = 1, i_hi = 0;
+  const long I0 = lo_of((m0 + c.n_pre_remove) * c.down), I1 = hi_of((m_last + c.n_pre_remove) * c.down);
+  const float* h = hp + c.tap0 + (pos - q * c.up);  // this output's phase: h[k] at h[(q - i) * up]
+  double acc = 0.0;
+  for (long t0 = I0; t0 <= I1; t0 += kRsTile) {
+    const long t1 = min(t0 + kRsTile, I1 + 1);
+    __syncthreads();
+    for (long i = t0 + threadIdx.x; i < t1; i += kRsOut) xs[i - t0] = ld(i);
+    __syncthreads();
+    const long a = max(i_lo, t0), b = min(i_hi, t1 - 1);
+    if (a > b) continue;
+    const float* hj = h + (q - a) * c.up;
+    const float* xi = xs + (a - t0);
+    const int n = (int)(b - a + 1);
+#pragma unroll 4
+    for (int s = 0; s < n; ++s) acc = fma((double)hj[-(long)s * c.up], (double)xi[s], acc);
+  }
+  if (mo <= m_last) yr[mo] = (float)acc;
 }
 
-cudaError_t resample_poly_launch(const float* x, long n_clips, long n_in, long x_stride, const float* h_dev, int len_h,
-                                 int up, int down, long n_pre_remove, long n_out, long y_stride, float* y,
+cudaError_t resample_rows_launch(const void* x, int pcm16, const RsClip* clips, const unsigned* first_item,
+                                 long n_clips, long n_items, const float* h_poly, float* y, long y_stride,
                                  cudaStream_t st) {
-  dim3 grid((unsigned)((n_out + 255) / 256), (unsigned)n_clips);
-  resample_poly_kernel<<<grid, 256, 0, st>>>(x, n_in, x_stride, h_dev, len_h, up, down, n_pre_remove, n_out, y_stride, y);
+  if (pcm16)
+    resample_rows_kernel<<<(unsigned)n_items, kRsOut, 0, st>>>((const int16_t*)x, clips, first_item, n_clips, h_poly,
+                                                               y, y_stride);
+  else
+    resample_rows_kernel<<<(unsigned)n_items, kRsOut, 0, st>>>((const float*)x, clips, first_item, n_clips, h_poly, y,
+                                                               y_stride);
   count_launch();
   return cudaGetLastError();
 }

@@ -9,6 +9,8 @@ memory and streams only; all arithmetic happens in ``libmmf_b200.so``).
 from __future__ import annotations
 
 import ctypes as C
+import functools
+import math
 from collections import OrderedDict
 from dataclasses import dataclass, replace
 
@@ -135,27 +137,91 @@ def design_resample_filter(n_in: int, up: int, down: int, quality: str = "scipy"
     (tests/test_host.py::test_hq_resampler_is_transparent_below_the_band_edge); libsoxr's own output cannot be
     compared here (not installed, no network)."""
     import scipy.signal
+
+    half_len, n_pre_pad, n_post_pad, n_pre_remove, n_out = _resample_geometry(n_in, up, down, quality)
+    max_rate = max(up, down)
+    if quality == "scipy":
+        h = scipy.signal.firwin(2 * half_len + 1, 1.0 / max_rate, window=("kaiser", 5.0))
+    else:
+        h = scipy.signal.firwin(2 * half_len + 1, 0.9565 / max_rate, window=("kaiser", 12.27))
+    h = h.astype(np.float32) * up
+    h = np.concatenate((np.zeros(n_pre_pad, dtype=h.dtype), h, np.zeros(n_post_pad, dtype=h.dtype)))
+    return np.ascontiguousarray(h, dtype=np.float32), n_pre_remove, n_out
+
+
+def _resample_geometry(n_in: int, up: int, down: int, quality: str):
+    """The edge bookkeeping of :func:`design_resample_filter` without the filter design: (half_len, n_pre_pad,
+    n_post_pad, n_pre_remove, n_out).  The taps are ``n_pre_pad`` zeros, the ``2 * half_len + 1`` designed taps and
+    ``n_post_pad`` zeros; only the padding depends on ``n_in``."""
     from scipy.signal._upfirdn import _output_len
 
     n_out = n_in * up
     n_out = n_out // down + bool(n_out % down)
-    max_rate = max(up, down)
-    if quality == "scipy":
-        half_len = 10 * max_rate
-        h = scipy.signal.firwin(2 * half_len + 1, 1.0 / max_rate, window=("kaiser", 5.0))
-    elif quality == "hq":
-        half_len = 90 * max_rate
-        h = scipy.signal.firwin(2 * half_len + 1, 0.9565 / max_rate, window=("kaiser", 12.27))
-    else:
+    if quality not in ("scipy", "hq"):
         raise ValueError("quality must be 'scipy' or 'hq'")
-    h = h.astype(np.float32) * up
+    half_len = (10 if quality == "scipy" else 90) * max(up, down)
     n_pre_pad = down - half_len % down
     n_post_pad = 0
     n_pre_remove = (half_len + n_pre_pad) // down
-    while _output_len(len(h) + n_pre_pad + n_post_pad, n_in, up, down) < n_out + n_pre_remove:
+    while _output_len(2 * half_len + 1 + n_pre_pad + n_post_pad, n_in, up, down) < n_out + n_pre_remove:
         n_post_pad += 1
-    h = np.concatenate((np.zeros(n_pre_pad, dtype=h.dtype), h, np.zeros(n_post_pad, dtype=h.dtype)))
-    return np.ascontiguousarray(h, dtype=np.float32), n_pre_remove, n_out
+    return half_len, n_pre_pad, n_post_pad, n_pre_remove, n_out
+
+
+def resample_ratio(sr_in: float, sr: float):
+    """``(up, down)`` that brings audio at ``sr_in`` to ``sr``: ``Fraction(sr / sr_in).limit_denominator(1000)``,
+    reduced by the gcd as :meth:`Plan.resample_poly` reduces it; ``(1, 1)`` when the rates are equal.  The WAV loader
+    and the packed resampling bundle share it, so a clip gets the same ratio on either route."""
+    from fractions import Fraction
+
+    if float(sr_in) == float(sr):
+        return 1, 1
+    fr = Fraction(float(sr) / float(sr_in)).limit_denominator(1000)
+    g = math.gcd(fr.numerator, fr.denominator)
+    return fr.numerator // g, fr.denominator // g
+
+
+# mmf_resample_clip as a numpy record (C layout; mmf_abi_sizeof(3) checks it)
+RESAMPLE_CLIP = np.dtype(
+    [("up", np.int32), ("down", np.int32), ("tap0", np.int64), ("len_h", np.int32), ("n_pre_remove", np.int64),
+     ("n_out", np.int64)],
+    align=True,
+)
+
+
+def resample_descriptors(lengths, rates, sr: float):
+    """The tap table and the ``mmf_resample_clip`` descriptors that bring clips of ``lengths`` samples at ``rates``
+    to ``sr`` with the ``"hq"`` filter (the loader's).  One table entry per distinct ratio, designed for the longest
+    clip of that ratio and zero-padded to the longest ``len_h`` of any of them (the designs of one ratio differ only in
+    trailing zeros); each clip's ``len_h``, ``n_pre_remove`` and ``n_out`` are ``design_resample_filter``'s for its own
+    length.  Plan-rate clips get ``up = down = 1``.  Returns ``(rs, h)``: a ``RESAMPLE_CLIP`` array and float32 taps."""
+    lengths = np.asarray(lengths, dtype=np.int64).reshape(-1)
+    rates = list(np.asarray(rates, dtype=np.float64).reshape(-1))
+    if len(rates) != len(lengths):
+        raise ValueError(f"rates has {len(rates)} entries for {len(lengths)} clips")
+    rs = np.zeros(len(lengths), RESAMPLE_CLIP)
+    ratio = [resample_ratio(r, sr) for r in rates]
+    groups = {}
+    for i, (up, down) in enumerate(ratio):
+        n = int(lengths[i])
+        rs[i]["up"], rs[i]["down"] = up, down
+        if (up, down) == (1, 1):
+            rs[i]["n_out"] = n
+            continue
+        half_len, n_pre_pad, n_post_pad, n_pre_remove, n_out = _resample_geometry(n, up, down, "hq")
+        rs[i]["len_h"] = n_pre_pad + 2 * half_len + 1 + n_post_pad
+        rs[i]["n_pre_remove"], rs[i]["n_out"] = n_pre_remove, n_out
+        groups.setdefault((up, down), []).append(i)
+    tables, tap0 = [], 0
+    for (up, down), idx in groups.items():
+        longest = max(idx, key=lambda i: int(lengths[i]))
+        h, _, _ = design_resample_filter(int(lengths[longest]), up, down, "hq")
+        h = np.concatenate([h, np.zeros(max(int(rs[i]["len_h"]) for i in idx) - len(h), np.float32)])
+        rs["tap0"][idx] = tap0
+        tables.append(h)
+        tap0 += len(h)
+    h = np.concatenate(tables) if tables else np.zeros(0, np.float32)
+    return rs, np.ascontiguousarray(h, dtype=np.float32)
 
 
 class Plan:
@@ -694,7 +760,7 @@ class Plan:
         return out
 
     def features_host_varlen(self, pcm_host: np.ndarray, offsets, prm: mmf_change_params, mod=None, *,
-                             want=("totChange",), out=None):
+                             want=("totChange",), out=None, rates=None):
         """:meth:`features_host` for clips of different lengths packed back to back in one host buffer.
 
         ``pcm_host`` is 1-D float32 or int16 (raw WAV samples, scaled by 1/32768 on the device); clip ``i`` is
@@ -703,7 +769,12 @@ class Plan:
         MFCC block starts at ``n_mfcc * frame_offsets[i]``, its ``[n_mfcc, n_win_i, nfft/2+1]`` modulation block at
         ``n_mfcc * (nfft/2+1) * window_offsets[i]``), plus ``frames``, ``windows`` (int64 ``[B]``), ``frame_offsets``
         and ``window_offsets`` (int64 ``[B + 1]``).  Each clip's blocks equal :meth:`features_host` on that clip
-        alone, bit for bit.  Pinned buffers (``pcm_host`` and the arrays in ``out``) make the copies asynchronous."""
+        alone, bit for bit.  Pinned buffers (``pcm_host`` and the arrays in ``out``) make the copies asynchronous.
+
+        ``rates``: one source sample rate per clip.  Each clip then crosses PCIe at its own rate and is resampled on
+        the device to the plan's rate with the loader's filter (:func:`resample_descriptors`), straight into the rows
+        the ragged path reads; its blocks equal :meth:`features_host` on ``resample_poly(x, up, down, "hq")`` of that
+        clip alone (after ``pcm16_to_f32`` for int16), bit for bit, and ``frames`` count frames at the plan's rate."""
         pcm_host = np.asarray(pcm_host)
         pcm16 = pcm_host.dtype == np.int16
         if not pcm16 and pcm_host.dtype != np.float32:
@@ -721,12 +792,19 @@ class Plan:
         frame_off = np.empty(B + 1, np.int64)
         win_off = np.empty(B + 1, np.int64)
         # the library owns the size formulas (and checks the offsets, naming a bad clip)
-        check(
+        sizes = lambda o: check(  # noqa: E731
             _lib.lib().mmf_features_varlen_sizes(
-                C.byref(self.cfg.to_c()), C.byref(mp) if mp is not None else None, B, offs.ctypes.data,
+                C.byref(self.cfg.to_c()), C.byref(mp) if mp is not None else None, B, o.ctypes.data,
                 frame_off.ctypes.data, win_off.ctypes.data,
             )
         )
+        sizes(offs)
+        if rates is not None:
+            # the blocks follow the lengths at the plan's rate: sizes of the prefix sums of n_out
+            rs, h = resample_descriptors(np.diff(offs), rates, self.cfg.sample_rate)
+            out_offs = np.zeros(B + 1, np.int64)
+            np.cumsum(rs["n_out"], out=out_offs[1:])
+            sizes(out_offs)
         nm = self.cfg.n_mfcc
         F, Wt = int(frame_off[-1]), int(win_off[-1])
         nb = n_bands = 0
@@ -752,13 +830,16 @@ class Plan:
                 ptr[k] = None
         if ("modspec" in want or "band_energy" in want) and mp is None:
             raise ValueError("modspec / band_energy requested without modulation parameters")
-        fn = _lib.lib().mmf_features_host_varlen_pcm16 if pcm16 else _lib.lib().mmf_features_host_varlen
+        if rates is not None:
+            fn = functools.partial(_lib.lib().mmf_features_host_varlen_resampled, self._h, pcm_host.ctypes.data,
+                                   1 if pcm16 else 0, B, offs.ctypes.data, rs.ctypes.data,
+                                   h.ctypes.data if len(h) else None, len(h))
+        else:
+            fn = functools.partial(_lib.lib().mmf_features_host_varlen_pcm16 if pcm16 else
+                                   _lib.lib().mmf_features_host_varlen, self._h, pcm_host.ctypes.data, B,
+                                   offs.ctypes.data)
         check(
             fn(
-                self._h,
-                pcm_host.ctypes.data,
-                B,
-                offs.ctypes.data,
                 C.byref(prm),
                 C.byref(mp) if mp is not None else None,
                 ptr["totChange"],
@@ -850,6 +931,8 @@ def clear_plans() -> None:
 
 __all__ = [
     "design_resample_filter",
+    "resample_descriptors",
+    "resample_ratio",
     "MfccConfig",
     "Plan",
     "get_plan",

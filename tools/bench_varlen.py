@@ -18,11 +18,19 @@ first two land in pinned arrays.  One pinned host-to-device copy of the packed b
 calls end in a synchronise, so a host clock times them.  Each way reports its median ms, audio-s/s and the bytes it
 moves each way over PCIe.
 
+The resample leg feeds 1024 int16 clips of 2-20 s at 44.1 kHz (pinned) to FeatureExtractor's defaults at 16 kHz:
+one host_varlen(rates=) call, which resamples on the device inside the bundle, against the route before it (each
+clip scaled and resampled on the device as the WAV loader does, copied back, then one host_many call).  It also
+times the resampler kernels over the same clips with torch.profiler: Plan.resample_poly per clip (whatever kernel
+the tree's mmf_resample_poly launches, so the leg can time an older tree too) and, where the tree has it, one
+mmf_resample_varlen launch over all of them; and one pinned copy of the packed int16 bytes, against which the
+call's own time shows whether resampling and features stay under the copy.
+
 Workload: 1024 clips at 16 kHz with the bench's frame geometry (win 400 / hop 160 / n_fft 512, 40 mel, 13 MFCC,
 gradient, Butterworth output filter), lengths uniform in [2 s, 20 s] from a fixed seed.  Prints, per leg, the median
 ms of each way and audio-seconds per second as one JSON line, with the GPU's name and power limit.
 
-    python tools/bench_varlen.py [--clips 1024] [--iters 10] [--loop-iters 3] [--legs change,features,host]
+    python tools/bench_varlen.py [--clips 1024] [--iters 10] [--loop-iters 3] [--legs change,features,host,resample]
 """
 import argparse
 import json
@@ -125,6 +133,74 @@ def _host_leg(fx, pcm, lengths, sr, iters, power_limit, dev):
         print(json.dumps(res), flush=True)
 
 
+def _profiled_kernel_ms(fn, match):
+    """Device time of the kernels whose name contains `match`, summed over one call of fn (torch.profiler)."""
+    from torch.profiler import ProfilerActivity, profile
+
+    fn()
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    return sum(e.device_time_total for e in prof.key_averages() if match in e.key) / 1e3
+
+
+def _resample_leg(n_clips, iters, seed, power_limit, dev):
+    from modulation_mfcc_b200 import _lib
+
+    sr_in, sr = 44100, 16000
+    rng = np.random.default_rng(seed)
+    lengths = [int(n) for n in rng.integers(2 * sr_in, 20 * sr_in + 1, n_clips)]
+    offsets = np.zeros(n_clips + 1, np.int64)
+    np.cumsum(lengths, out=offsets[1:])
+    packed = _pinned((int(offsets[-1]),), np.int16)
+    for i in range(n_clips):
+        x = mm.synth_clip(seed + i, lengths[i], sr_in)
+        packed[offsets[i] : offsets[i + 1]] = np.clip(np.round(x * 32768.0), -32768, 32767).astype(np.int16)
+    clips = [packed[offsets[i] : offsets[i + 1]] for i in range(n_clips)]
+    audio_s = sum(lengths) / sr_in
+    fx = mm.FeatureExtractor(sr, device=0)
+    plan = fx.plan
+    res = {"leg": "resample", "gpu": torch.cuda.get_device_name(dev), "power_limit": power_limit, "clips": n_clips,
+           "sr_in": sr_in, "sr": sr, "audio_s": audio_s, "h2d_bytes": packed.nbytes}
+    src = torch.from_numpy(packed)
+    copy = lambda: (src.to(dev, non_blocking=True), torch.cuda.synchronize())  # noqa: E731
+    copy()
+    res["h2d_ms"] = _median_host_ms(copy, iters)
+    x_dev = plan.pcm16_to_f32(torch.from_numpy(packed).to(dev))
+    rows = [x_dev[offsets[i] : offsets[i + 1]] for i in range(n_clips)]
+    # per-clip calls: the filter is designed on the host per call, so only the kernels' device time is counted
+    res["resample_poly_per_clip_kernel_ms"] = _profiled_kernel_ms(
+        lambda: [plan.resample_poly(r, 160, 441, "hq") for r in rows], "resample")
+    if hasattr(_lib.lib(), "mmf_resample_varlen"):
+        rs, h = mm.resample_descriptors(lengths, [sr_in] * n_clips, sr)
+        y = torch.empty((n_clips, int(rs["n_out"].max())), device=dev)
+        st = int(torch.cuda.current_stream(dev).cuda_stream)
+        varlen = lambda: _lib.check(_lib.lib().mmf_resample_varlen(  # noqa: E731
+            plan._h, x_dev.data_ptr(), n_clips, offsets.ctypes.data, rs.ctypes.data, h.ctypes.data, len(h),
+            y.data_ptr(), y.shape[1], st))
+        res["resample_varlen_kernel_ms"] = _profiled_kernel_ms(varlen, "resample")
+        res["resample_varlen_outputs_per_s"] = float(rs["n_out"].sum()) / (res["resample_varlen_kernel_ms"] / 1e3)
+
+        def before():  # the route without rates=: per clip, the loader's device resample and a copy back
+            ys = []
+            for c in clips:
+                up, down = mm.resample_ratio(sr_in, sr)
+                ys.append(plan.resample_poly(plan.pcm16_to_f32(c), up, down, "hq").cpu().numpy())
+            return fx.host_many(ys)
+
+        out = {k: v for k, v in fx.host_varlen(packed, offsets, rates=[sr_in] * n_clips).items() if k in
+               ("totChange", "mfcc", "delta", "modspec", "band_energy")}
+        out = {k: _pinned(v.shape, v.dtype.type) for k, v in out.items()}
+        call = lambda: fx.host_varlen(packed, offsets, out=out, rates=[sr_in] * n_clips)  # noqa: E731
+        res["host_varlen_rates_ms"] = _median_host_ms(call, iters)
+        res["host_varlen_rates_audio_s_per_s"] = audio_s / (res["host_varlen_rates_ms"] / 1e3)
+        before()
+        res["resample_then_host_many_ms"] = _median_host_ms(before, max(1, iters // 5))
+        res["resample_then_host_many_audio_s_per_s"] = audio_s / (res["resample_then_host_many_ms"] / 1e3)
+    print(json.dumps(res), flush=True)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--clips", type=int, default=1024)
@@ -171,6 +247,9 @@ def main():
     for leg in a.legs.split(","):
         if leg == "host":
             _host_leg(fx, pcm, lengths, sr, a.iters, power_limit, dev)
+            continue
+        if leg == "resample":
+            _resample_leg(a.clips, a.iters, a.seed, power_limit, dev)
             continue
         varlen, loop, pad = ways[leg]
         for fn in (varlen, pad, loop):  # warm-up: modules, workspace growth
