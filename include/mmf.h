@@ -170,9 +170,28 @@ int mmf_modspec_varlen(mmf_plan* plan, const float* mfcc_dev, int64_t n_clips, i
 
 /* RMS envelope: librosa.feature.rms(frame_length, hop_length, center,
  * pad_mode='constant') (script/calc.py:326-331, script/mfcc.py:247) ->
- * rms_dev [n_clips, T_rms] float32, T_rms = 1 + (n + 2*pad - frame_length)/hop. */
+ * rms_dev [n_clips, T_rms] float32, T_rms = 1 + (n + 2*pad - frame_length)/hop.
+ * Each frame is summed in one fixed order (lane l of a warp: fmaf over samples l, l + 32, ...; then an xor-shuffle
+ * tree 16, 8, 4, 2, 1; then sqrtf(s / frame_length)), so a row's bits do not depend on its batch. */
 int mmf_rms(mmf_plan* plan, const float* pcm_dev, int64_t n_clips, int64_t n_samples, int64_t clip_stride,
             int32_t frame_length, int32_t hop_length, int32_t center, float* rms_dev, void* stream);
+
+/* Host-only: output offsets of the RMS envelopes of a packed batch (no plan, no device).  Clip i is samples
+ * [offsets_host[i], offsets_host[i+1]) with geom_host[2i] = frame_length_i, geom_host[2i+1] = hop_i (in samples at the
+ * clip's own rate); pad_i = center ? frame_length_i / 2 : 0 and T_amp_i = 1 + (len_i + 2 pad_i - frame_length_i) /
+ * hop_i.  amp_off_host[n_clips+1] = prefix sums of T_amp_i.  The offsets are checked as mmf_features_host_varlen
+ * checks them; frame_length or hop < 1 fails with MMF_ERR_INVALID, a clip shorter than its frame without center with
+ * MMF_ERR_TOO_SHORT, the message naming the clip. */
+int mmf_amp_varlen_sizes(int64_t n_clips, const int64_t* offsets_host, const int32_t* geom_host, int32_t center,
+                         int64_t* amp_off_host);
+
+/* mmf_rms for packed clips of different lengths and frame geometries, in one launch: clip i of the packed float32
+ * x_dev[offsets_host[i] .. offsets_host[i+1]) with geom_host[2i .. 2i+1] goes to amp_dev[amp_off[i] .. amp_off[i+1])
+ * (mmf_amp_varlen_sizes).  Each block is bit-identical to mmf_rms on that clip alone.  The checks are those of
+ * mmf_amp_varlen_sizes, before anything is launched.  Asynchronous on `stream` (the descriptors are copied from
+ * pageable memory before it returns). */
+int mmf_rms_varlen(mmf_plan* plan, const float* x_dev, int64_t n_clips, const int64_t* offsets_host,
+                   const int32_t* geom_host, int32_t center, float* amp_dev, void* stream);
 
 /* Parameters of the post-MFCC part of get_MFCCS_change (script/mfcc.py:393-425). */
 typedef struct {
@@ -313,6 +332,35 @@ int mmf_resample_varlen(mmf_plan* plan, const float* x_dev, int64_t n_clips, con
                         const mmf_resample_clip* rs_host, const float* h_host, int64_t n_h, float* y_dev,
                         int64_t y_stride, void* stream);
 
+/* The RMS amplitude envelope in the host-buffer bundle (calculate_amplitude_envelope, script/calc.py:221-343, method
+ * 'RMS', outFilter None or 'iir').  out_n_sections = 0: the raw envelope only; otherwise out_sos holds the
+ * zero-phase output filter (designed at 1 / hopLen, as applyFilter designs it). */
+typedef struct {
+  int32_t center;
+  int32_t out_n_sections;
+  double out_sos[16 * 6];
+} mmf_amp_params;
+
+/* mmf_features_host_varlen_resampled plus each clip's RMS envelope at its native rate.
+ *  - rs_host and h_host may be NULL: every clip is then at the plan's rate, as in mmf_features_host_varlen(_pcm16).
+ *  - amp = NULL: exactly mmf_features_host_varlen_resampled (amp_host and amp_filt_host must then be NULL).
+ *  - Otherwise the envelope of clip i is taken from its native samples (float32, or int16 scaled by 1/32768) with
+ *    geom_host[2i] = frame_length_i, geom_host[2i+1] = hop_i and amp->center; amp_host (float32) and amp_filt_host
+ *    (float64, the envelope through amp->out_sos; needs out_n_sections > 0) receive it packed at amp_off
+ *    (mmf_amp_varlen_sizes).  Either may be NULL.  Each clip's blocks are bit-identical to mmf_rms, then
+ *    mmf_sosfiltfilt (x_is_f32 = 1) on that clip alone, whatever chunk it lands in.
+ *  - The MFCC side and its checks are unchanged.  The amplitude checks are those of mmf_amp_varlen_sizes; with a
+ *    filter, an envelope of at most padlen frames fails with MMF_ERR_TOO_SHORT naming the clip, before anything is
+ *    queued.
+ *  - Per chunk, the envelope is one launch reading the chunk's copied samples and, with a filter, one more for every
+ *    envelope the chunk-parallel filter takes; longer envelopes are filtered one by one. */
+int mmf_features_host_varlen_amp(mmf_plan* plan, const void* pcm_host, int32_t pcm16, int64_t n_clips,
+                                 const int64_t* offsets_host, const mmf_resample_clip* rs_host, const float* h_host,
+                                 int64_t n_h, const mmf_change_params* prm, const mmf_modspec_params* mod,
+                                 const mmf_amp_params* amp, const int32_t* geom_host, double* tot_host,
+                                 float* mfcc_host, float* delta_host, float* mag_host, float* band_host,
+                                 float* amp_host, double* amp_filt_host);
+
 /* Hilbert amplitude envelope |scipy.signal.hilbert(x)| of each row (script/calc.py:284-286, method 'Hilb'),
  * any length n <= 2^26 (an hour at 16 kHz): O(n log n) -- the length-n transforms scipy runs are evaluated as
  * Bluestein chirp transforms over a power-of-two FFT in float64; signals of at most 4096 samples use the
@@ -349,7 +397,8 @@ int mmf_mfcc_change_host(mmf_plan* plan, const float* pcm_host, int64_t n_clips,
                          int64_t clip_stride, const mmf_change_params* prm, double* tot_host, float* mfcc_host);
 
 /* sizeof() of the ABI structs as this library was compiled (0: mmf_config,
- * 1: mmf_change_params, 2: mmf_modspec_params, 3: mmf_resample_clip) so bindings can verify their layout. */
+ * 1: mmf_change_params, 2: mmf_modspec_params, 3: mmf_resample_clip, 4: mmf_amp_params) so bindings can verify their
+ * layout. */
 int mmf_abi_sizeof(int32_t which);
 
 /* Number of kernels this library has launched on the calling thread since the

@@ -26,6 +26,7 @@ from .api import (  # noqa: F401
     applyFilter,
     band_bins,
     calculate_amplitude_envelope,
+    calculate_amplitude_envelope_many,
     get_amplitude,
     get_MFCCS_change,
     get_MFCCS_change_batch,

@@ -113,6 +113,14 @@ class mmf_resample_clip(C.Structure):
     ]
 
 
+class mmf_amp_params(C.Structure):
+    _fields_ = [
+        ("center", C.c_int32),
+        ("out_n_sections", C.c_int32),
+        ("out_sos", C.c_double * 96),
+    ]
+
+
 OBJ_DIR = PKG_DIR / "build"
 
 
@@ -226,6 +234,13 @@ _SIGNATURES = {
          _vp, _vp, _vp, _vp, _vp],
     ),
     "mmf_resample_varlen": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _i64, _vp]),
+    "mmf_features_host_varlen_amp": (
+        C.c_int,
+        [_vp, _vp, _i32, _i64, _vp, _vp, _vp, _i64, C.POINTER(mmf_change_params), C.POINTER(mmf_modspec_params),
+         C.POINTER(mmf_amp_params), _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    ),
+    "mmf_amp_varlen_sizes": (C.c_int, [_i64, _vp, _vp, _i32, _vp]),
+    "mmf_rms_varlen": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _i32, _vp, _vp]),
     "mmf_pcm16_to_f32": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
     "mmf_hilbert_envelope": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _vp, _i64, _vp]),
     "mmf_find_peaks": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _i32, _i32, _vp, _vp, _vp]),

@@ -759,6 +759,64 @@ def calculate_amplitude_envelope(
 get_amplitude = calculate_amplitude_envelope
 
 
+def calculate_amplitude_envelope_many(
+    clips,
+    sr,
+    /,
+    *,
+    method="RMS",
+    winLen=0.1,
+    hopLen=0.01,
+    center=True,
+    outFilter=None,
+    outFiltType="low",
+    outFiltCutOff=[12],
+    outFiltLen=6,
+    outFiltPolyOrd=3,
+    device=None,
+):
+    """:func:`calculate_amplitude_envelope` (method ``'RMS'``) for a list of 1-D clips of any lengths: one packed
+    upload and one ``mmf_rms_varlen`` launch for all of them.  ``sr`` is one rate for every clip or one rate per clip;
+    each clip's frame geometry is ``int(winLen * sr_i)``, ``int(hopLen * sr_i)``.  The output filter, if any, runs per
+    clip as the single call runs it.  Returns one ``(amp, ampT)`` per clip, equal to
+    ``calculate_amplitude_envelope(clip, sr_i, ...)`` bit for bit; an error names the clip's index."""
+    if method != "RMS":
+        raise ValueError(f"calculate_amplitude_envelope_many takes method 'RMS' only, not {method!r}")
+    clips = [np.asarray(c) for c in clips]
+    if any(c.ndim != 1 for c in clips):
+        raise ValueError("calculate_amplitude_envelope_many takes 1-D clips")
+    if not clips:
+        return []
+    rates = [float(r) for r in (sr if np.ndim(sr) else [sr] * len(clips))]
+    if len(rates) != len(clips):
+        raise ValueError(f"sr has {len(rates)} rates for {len(clips)} clips")
+    di = _device_index(device)
+    plan = _any_plan(di)
+    offsets = np.zeros(len(clips) + 1, np.int64)
+    np.cumsum([c.shape[0] for c in clips], out=offsets[1:])
+    geom = [(int(winLen * r), int(hopLen * r)) for r in rates]
+    try:
+        packed = np.concatenate([c.astype(np.float32, copy=False) for c in clips])
+        amp, amp_off = plan.rms_varlen(packed, offsets, geom, bool(center))
+        out = []
+        host = amp.cpu().numpy() if outFilter is None else None
+        for i in range(len(clips)):
+            a0, a1 = int(amp_off[i]), int(amp_off[i + 1])
+            ampT = np.arange(a1 - a0) * hopLen  # script/calc.py:333-337
+            if outFilter is None:
+                out.append((host[a0:a1], ampT))
+                continue
+            try:
+                y = _apply_filter_dev(plan, amp[a0:a1], 1 / hopLen, filt=outFilter, filtType=outFiltType,
+                                      cutOff=outFiltCutOff, filtLen=outFiltLen, polyOrd=outFiltPolyOrd)
+            except ValueError as e:  # an envelope too short for the output filter: name the clip
+                raise ValueError(f"clip {i}: {e}") from None
+            out.append((y.cpu().numpy() if y is not None else None, ampT))
+    except MmfError as e:
+        _raise_from(e)
+    return out
+
+
 # ---------------------------------------------------------------------------
 # batch feature bundle (log-mel, MFCC, delta, MFCC change, modulation spectrum)
 # ---------------------------------------------------------------------------
@@ -806,7 +864,23 @@ class FeatureExtractor:
         preemph: float = 0.0,
         device=None,
         flags: int = 0,
+        amp_winLen: float = 0.1,
+        amp_hopLen: float = 0.01,
+        amp_center: bool = True,
+        amp_outFilter=None,
+        amp_outFiltType="low",
+        amp_outFiltCutOff=[12],
+        amp_outFiltLen=6,
     ):
+        # the envelope's output filter is validated before any device work, with applyFilter's exceptions
+        if amp_outFilter is None:
+            self.amp_sos = None
+        elif amp_outFilter == "iir":
+            self.amp_sos = _design_iir(1 / amp_hopLen, amp_outFiltCutOff, amp_outFiltLen, amp_outFiltType)
+        else:
+            raise ValueError(f"the feature bundle takes amp_outFilter None or 'iir', not {amp_outFilter!r} (use "
+                             "calculate_amplitude_envelope_many for 'fir' and 'sg')")
+        self.amp_winLen, self.amp_hopLen, self.amp_center = float(amp_winLen), float(amp_hopLen), bool(amp_center)
         self.sr, self.tStep, self.winLen = float(sr), float(tStep), float(winLen)
         self.plan = _change_setup(sr, tStep, winLen, n_mfcc, n_fft, fmin, sr / 2 if fmax is None else fmax, n_mels, preemph, device, flags)
         sos = _butter_sos(filtOrd, filtCutoff / ((1 / tStep) / 2), "low")
@@ -817,6 +891,15 @@ class FeatureExtractor:
     def modspec_geometry(self, T: int):
         Lw, Hw, nfft, _ = modspec_sizes(T, self.frame_rate, self.mod_win_s, self.mod_hop_s)
         return Lw, Hw, nfft, band_bins(nfft, self.frame_rate, self.bands_hz)
+
+    def _amp(self, want, n_clips, rates):
+        """The ``amp`` argument of :meth:`Plan.features_host_varlen` when ``want`` holds ``"amplitude"``: each clip's
+        frame geometry at its own rate (``rates``, else the extractor's), as calc.py:326-331 computes it."""
+        if "amplitude" not in want:
+            return None
+        rates = [self.sr] * n_clips if rates is None else [float(r) for r in rates]
+        geom = [(int(self.amp_winLen * r), int(self.amp_hopLen * r)) for r in rates]
+        return geom, self.amp_center, self.amp_sos
 
     def host_call(self, pcm_host, *, want=("totChange", "mfcc", "delta", "modspec", "band_energy"), out=None):
         """Host buffers in, host buffers out, through the single C-ABI bundle call."""
@@ -835,10 +918,17 @@ class FeatureExtractor:
         :meth:`Plan.features_host_varlen` with this extractor's modulation geometry; each clip's blocks equal
         :meth:`host_call` on that clip alone, bit for bit.  ``rates``: each clip's sample rate; clips are then
         resampled to the extractor's rate on the device as the WAV loader resamples them, and each clip's blocks
-        equal :meth:`host_call` on the loader's resampled clip."""
+        equal :meth:`host_call` on the loader's resampled clip.
+
+        ``"amplitude"`` in ``want`` adds each clip's RMS envelope with this extractor's ``amp_*`` settings, taken at
+        the clip's own rate (``rates``, else the extractor's) from its native samples (int16 scaled by 1/32768):
+        ``amplitude`` packed at ``amp_offsets``; clip ``i``'s block equals :func:`calculate_amplitude_envelope` on that
+        clip as float32, bit for bit."""
         mod = self.modspec_geometry(0) if ("modspec" in want or "band_energy" in want) else None
         try:
-            return self.plan.features_host_varlen(pcm_host, offsets, self.prm, mod, want=want, out=out, rates=rates)
+            amp = self._amp(want, len(offsets) - 1, rates)
+            return self.plan.features_host_varlen(pcm_host, offsets, self.prm, mod, want=want, out=out, rates=rates,
+                                                  amp=amp)
         except MmfError as e:
             _raise_from(e)
 
@@ -847,8 +937,10 @@ class FeatureExtractor:
         Concatenates them once and returns one dict per clip of zero-copy views into the packed arrays, shaped as
         :func:`mfcc_features_batch` returns one clip without its batch axis (``totChange [T]``, ``mfcc`` /
         ``delta [n_mfcc, T]``, ``modspec [n_mfcc, W, nfft/2+1]``, ``band_energy [W, n_bands]``), plus ``T``, the
-        frame times (at the extractor's rate when ``rates`` are given).  A corpus already held in one buffer should
-        call :meth:`host_varlen` with its offsets instead, which saves the concatenation."""
+        frame times (at the extractor's rate when ``rates`` are given).  With ``"amplitude"`` in ``want``, each dict
+        also holds ``amplitude`` and ``ampT``, what :func:`calculate_amplitude_envelope` returns for the clip.  A corpus
+        already held in one buffer should call :meth:`host_varlen` with its offsets instead, which saves the
+        concatenation."""
         clips = [np.asarray(c) for c in clips]
         if not clips:
             return []
@@ -875,6 +967,10 @@ class FeatureExtractor:
             if "band_energy" in res:
                 d["band_energy"] = res["band_energy"][n_bands * w0 : n_bands * w1].reshape(W, n_bands)
             d["T"] = _time_anchors(T, self.tStep, self.winLen)
+            if "amplitude" in res:
+                a0, a1 = int(res["amp_offsets"][i]), int(res["amp_offsets"][i + 1])
+                d["amplitude"] = res["amplitude"][a0:a1]
+                d["ampT"] = np.arange(a1 - a0) * self.amp_hopLen  # script/calc.py:333-337
             out.append(d)
         return out
 
@@ -884,7 +980,9 @@ class FeatureExtractor:
         when every file is 16-bit PCM, else as float32) to be resampled on the device to the extractor's rate.
         Returns one dict per file, as :meth:`host_many` does; each file's blocks equal :meth:`host_call` on
         ``_read_audio(path, sr)[channel]``, bit for bit (rows are resampled independently, so selecting the channel
-        first changes nothing).  A file that is not RIFF/WAVE raises ``ValueError`` naming its path."""
+        first changes nothing).  A file that is not RIFF/WAVE raises ``ValueError`` naming its path.  ``amplitude`` is
+        taken at the file's own rate on samples in [-1, 1]: for a 16-bit file, times 32768 it equals
+        :func:`calculate_amplitude_envelope` of the raw samples, as the GUI computes it (``main.py:843-849``)."""
         rates, clips = [], []
         for p in paths:
             file_sr, data = _parse_wav(p)

@@ -465,6 +465,7 @@ int mmf_abi_sizeof(int32_t which) {
     case 1: return (int)sizeof(mmf_change_params);
     case 2: return (int)sizeof(mmf_modspec_params);
     case 3: return (int)sizeof(mmf_resample_clip);
+    case 4: return (int)sizeof(mmf_amp_params);
     default: return -1;
   }
 }
@@ -1191,24 +1192,6 @@ int mmf_modspec_varlen(mmf_plan* plan, const float* mfcc_dev, int64_t n_clips, i
                             nfft, mag_dev, band_dev, (cudaStream_t)stream);
 }
 
-int mmf_rms(mmf_plan* plan, const float* pcm_dev, int64_t n_clips, int64_t n_samples, int64_t clip_stride,
-            int32_t frame_length, int32_t hop_length, int32_t center, float* rms_dev, void* stream) {
-  if (!plan || !pcm_dev || !rms_dev) return fail(MMF_ERR_INVALID, "NULL argument");
-  if (frame_length < 1 || hop_length < 1) return fail(MMF_ERR_INVALID, "frame_length and hop_length must be positive");
-  const int pad = center ? frame_length / 2 : 0;
-  const int64_t padded = n_samples + 2 * (int64_t)pad;
-  if (padded < frame_length) return fail(MMF_ERR_TOO_SHORT, "Input is too short for frame_length");
-  const int64_t T = 1 + (padded - frame_length) / hop_length;
-  MMF_CUDA(cudaSetDevice(plan->cfg.device));
-  for (int64_t c0 = 0; c0 < n_clips; c0 += 65535) {
-    const int64_t nc = std::min<int64_t>(65535, n_clips - c0);
-    cudaError_t e = rms_launch(pcm_dev + (size_t)c0 * clip_stride, nc, n_samples, clip_stride, frame_length,
-                               hop_length, pad, T, rms_dev + (size_t)c0 * T, (cudaStream_t)stream);
-    if (e != cudaSuccess) return cuda_fail(e, "rms_kernel launch");
-  }
-  return MMF_OK;
-}
-
 }  // extern "C"
 
 namespace mmf {
@@ -1558,7 +1541,7 @@ static int change_varlen_run(mmf_plan* plan, const ChangeVarlen& v, unsigned cha
       e = change_fused_launch(mfcc, nv, c.n_mfcc, first, rows, pitch, prm->diff_method, pa, po,
                               v.split_out ? 1 : prm->out_kind, v.split_out ? raw : tot_dev, v.fsmem, nullptr, st, &fvl);
     }
-    if (e == cudaSuccess && v.split_out) e = sosfiltfilt_par_varlen_launch(raw, nv, pitch, po, fvl, tot_dev, st);
+    if (e == cudaSuccess && v.split_out) e = sosfiltfilt_par_varlen_launch(raw, 0, nv, pitch, po, fvl, tot_dev, st);
     if (e != cudaSuccess) return cuda_fail(e, "change_fused_kernel (variable-length) launch");
   }
 
@@ -1837,6 +1820,56 @@ static int64_t resample_desc(int64_t c0, int64_t c1, const int64_t* offsets, int
   return items;
 }
 
+// RMS-envelope geometry of a packed batch (mmf_amp_varlen_sizes, calc.py:326-331), after the offsets passed
+// validate_offsets: amp_off[n_clips + 1], the prefix sums of each clip's frame count (no plan or device needed)
+static int amp_sizes(int64_t n_clips, const int64_t* offsets, const int32_t* geom, int center, int64_t* amp_off) {
+  if (!geom) return fail(MMF_ERR_INVALID, "geom_host is NULL");
+  amp_off[0] = 0;
+  for (int64_t i = 0; i < n_clips; ++i) {
+    const int fl = geom[2 * i], hop = geom[2 * i + 1];
+    const int64_t len = offsets[i + 1] - offsets[i];
+    char buf[160];
+    if (fl < 1 || hop < 1) {
+      std::snprintf(buf, sizeof(buf), "clip %lld: frame_length (%d) and hop (%d) must be >= 1", (long long)i, fl, hop);
+      return fail(MMF_ERR_INVALID, buf);
+    }
+    const int64_t padded = len + (center ? 2 * (int64_t)(fl / 2) : 0);
+    if (padded < fl) {
+      std::snprintf(buf, sizeof(buf), "clip %lld: Input is too short (n=%lld) for frame_length=%d", (long long)i,
+                    (long long)len, fl);
+      return fail(MMF_ERR_TOO_SHORT, buf);
+    }
+    amp_off[i + 1] = amp_off[i] + 1 + (padded - fl) / hop;
+  }
+  return MMF_OK;
+}
+
+// Device descriptors of clips [c0, c1) of a packed batch for rms_varlen_launch: RmsClip[nc], then first_item[nc + 1],
+// appended to `desc` (16-byte aligned parts).  Sources count from `base`, outputs from amp_off[c0].  Returns the number
+// of work items, or -1 past 2^31 - 1.
+static int64_t rms_desc(int64_t c0, int64_t c1, const int64_t* offsets, int64_t base, const int32_t* geom, int center,
+                        const int64_t* amp_off, std::vector<unsigned char>& desc, size_t& o_clips, size_t& o_first) {
+  const int64_t nc = c1 - c0;
+  o_clips = align_up(desc.size(), 16);
+  o_first = align_up(o_clips + (size_t)nc * sizeof(RmsClip), 16);
+  desc.resize(align_up(o_first + (size_t)(nc + 1) * 4, 16), 0);
+  RmsClip* cl = (RmsClip*)(desc.data() + o_clips);
+  unsigned* first = (unsigned*)(desc.data() + o_first);
+  int64_t items = 0;
+  for (int64_t k = 0; k < nc; ++k) {
+    const int64_t i = c0 + k;
+    const int fl = geom[2 * i], hop = geom[2 * i + 1];
+    const RmsClip r{(long)(offsets[i] - base), (long)(offsets[i + 1] - offsets[i]), (long)(amp_off[i] - amp_off[c0]),
+                    (long)(amp_off[i + 1] - amp_off[i]), fl, hop, center ? fl / 2 : 0, rms_frames_per_item(fl, hop)};
+    cl[k] = r;
+    first[k] = (unsigned)items;
+    items += (r.T + r.F - 1) / r.F;
+    if (items > 0x7fffffffLL) return -1;
+  }
+  first[nc] = (unsigned)items;
+  return items;
+}
+
 // frame_off / win_off of a packed batch (mmf_features_varlen_sizes); n_win_i = 0 without modulation windows
 static void packed_sizes(int n_fft, int hop, int win, int mod_hop, int64_t n_clips, const int64_t* offsets,
                          int64_t* frame_off, int64_t* win_off) {
@@ -1861,18 +1894,50 @@ struct HostChunk {
   size_t o_desc, o_cv_desc, o_mv_desc;  // desc, cv.desc and mv.desc in the descriptor region of the call
   size_t o_h2d, o_pcm, o_tot, o_mfcc, o_delta, o_mag, o_band, o_ptot, o_pmfcc, o_pdelta, o_pmag, o_pband,
       o_scratch, end;
+  // the amplitude envelope (when requested): its launch's work items and descriptors, and the output filter's: the
+  // envelopes on the chunk-parallel route (FusedVarlen parts in desc, amax = their widest tables) and the others
+  int64_t amp_items = 0, amp_np = 0;
+  std::vector<int64_t> amp_single;
+  SosPar amax;
+  size_t o_acl, o_afirst, o_fclips, o_fT, o_fpidx, o_foff, o_fpars;  // within desc
+  size_t o_amp, o_ampf;                                                // in the slot
 };
 
 // pcm_host: float32 samples, or (pcm16 != 0) int16 samples converted on the device.  resampled: clip i reaches the
-// plan's rate as rs[i] says, with taps from h[n_h]; otherwise every clip is at the plan's rate.
+// plan's rate as rs[i] says, with taps from h[n_h]; otherwise every clip is at the plan's rate.  amp: the RMS envelope
+// of each clip's native samples, frame geometry geom[2i], geom[2i + 1], to amp_host and / or, through the output
+// filter, amp_filt_host (NULL: none, and exactly the launches and copies of the call without it).
 static int features_host_varlen_impl(mmf_plan* plan, const void* pcm_host_v, int pcm16, int64_t n_clips,
                                      const int64_t* offsets, bool resampled, const mmf_resample_clip* rs,
                                      const float* h_taps, int64_t n_h, const mmf_change_params* prm,
                                      const mmf_modspec_params* mod, double* tot_host, float* mfcc_host,
-                                     float* delta_host, float* mag_host, float* band_host) {
+                                     float* delta_host, float* mag_host, float* band_host,
+                                     const mmf_amp_params* amp = nullptr, const int32_t* geom = nullptr,
+                                     float* amp_host = nullptr, double* amp_filt_host = nullptr) {
   int rc = validate_offsets(n_clips, offsets);
   if (rc) return rc;
   if (resampled && (rc = validate_resample(n_clips, offsets, rs, h_taps, n_h))) return rc;
+  if (!amp && (amp_host || amp_filt_host))
+    return fail(MMF_ERR_INVALID, "amplitude outputs requested without parameters");
+  const bool want_amp = amp && (amp_host || amp_filt_host);
+  std::vector<int64_t> A;  // envelope offsets (amp_sizes)
+  SosArgs so_amp;
+  if (want_amp) {
+    A.resize((size_t)n_clips + 1);
+    if ((rc = amp_sizes(n_clips, offsets, geom, amp->center, A.data()))) return rc;
+    if (amp_filt_host) {
+      if (amp->out_n_sections < 1) return fail(MMF_ERR_INVALID, "amp_filt_host needs out_n_sections >= 1");
+      if ((rc = fill_sos(amp->out_sos, amp->out_n_sections, &so_amp))) return rc;
+      for (int64_t i = 0; i < n_clips; ++i)
+        if (A[i + 1] - A[i] <= so_amp.padlen) {
+          char buf[192];
+          std::snprintf(buf, sizeof(buf),
+                        "clip %lld: The length of the input vector x must be greater than padlen, which is %d.",
+                        (long long)i, so_amp.padlen);
+          return fail(MMF_ERR_TOO_SHORT, buf);
+        }
+    }
+  }
   if (!plan || !pcm_host_v || !prm || !tot_host) return fail(MMF_ERR_INVALID, "NULL argument");
   if ((mag_host || band_host) && !mod) return fail(MMF_ERR_INVALID, "modulation outputs requested without parameters");
   const mmf_config& c = plan->cfg;
@@ -1954,6 +2019,55 @@ static int features_host_varlen_impl(mmf_plan* plan, const void* pcm_host_v, int
       ((int*)(h.desc.data() + h.o_cnt_w))[i] = (int)(Wo[c0 + i + 1] - Wo[c0 + i]);
       ((int64_t*)(h.desc.data() + h.o_off_w))[i] = Wo[c0 + i] - Wo[c0];
     }
+    if (want_amp) {
+      h.amp_items = rms_desc(c0, c1, offsets, offsets[c0], geom, amp->center, A.data(), h.desc, h.o_acl, h.o_afirst);
+      if (h.amp_items < 0) return fail(MMF_ERR_UNSUPPORTED, "a chunk of more than 2^31 - 1 envelope work items");
+    }
+    if (want_amp && amp_filt_host) {
+      // each envelope takes the route of its own mmf_sosfiltfilt call: the chunk-parallel kernel when
+      // sos_par_fill takes its length (all of them in one launch, each with the tables of its own chunk length), the
+      // single-row routes otherwise
+      std::vector<int> par_clips, Ti((size_t)nc), par_of_cl(kSosParMaxChunk + 1, -1);
+      std::vector<int2> pidx((size_t)nc, int2{0, 0});
+      std::vector<long> off((size_t)nc);
+      std::vector<SosPar> pars;
+      for (int64_t k = 0; k < nc; ++k) {
+        const int64_t Tk = A[c0 + k + 1] - A[c0 + k];
+        off[k] = (long)(A[c0 + k] - A[c0]);
+        Ti[k] = (int)std::min<int64_t>(Tk, 0x7fffffff);
+        SosPar sp;
+        if (!sos_par_fill(so_amp, (long)Tk, &sp)) {
+          h.amp_single.push_back(k);
+          continue;
+        }
+        int& idx = par_of_cl[sp.CL];
+        if (idx < 0) {
+          idx = (int)pars.size();
+          pars.push_back(sp);
+          if (idx == 0 || sp.CL > h.amax.CL) h.amax = sp;
+        }
+        pidx[k] = int2{idx, idx};
+        par_clips.push_back((int)k);
+      }
+      h.amp_np = (int64_t)par_clips.size();
+      size_t da = h.desc.size();
+      auto atake = [&](size_t bytes) {
+        const size_t o = da;
+        da += align_up(std::max<size_t>(bytes, 1), 16);
+        return o;
+      };
+      h.o_fclips = atake(par_clips.size() * 4);
+      h.o_fT = atake((size_t)nc * 4);
+      h.o_fpidx = atake((size_t)nc * 8);
+      h.o_foff = atake((size_t)nc * 8);
+      h.o_fpars = atake(pars.size() * sizeof(SosPar));
+      h.desc.resize(da, 0);
+      if (!par_clips.empty()) std::memcpy(h.desc.data() + h.o_fclips, par_clips.data(), par_clips.size() * 4);
+      std::memcpy(h.desc.data() + h.o_fT, Ti.data(), (size_t)nc * 4);
+      std::memcpy(h.desc.data() + h.o_fpidx, pidx.data(), (size_t)nc * 8);
+      std::memcpy(h.desc.data() + h.o_foff, off.data(), (size_t)nc * 8);
+      if (!pars.empty()) std::memcpy(h.desc.data() + h.o_fpars, pars.data(), pars.size() * sizeof(SosPar));
+    }
     // descriptors of every chunk go up together before the first chunk runs (a copy from pageable memory waits for
     // its stream: inside the loop it would hold back the next chunk's queueing)
     const bool mod_c = h.mv.W > 0;
@@ -1984,6 +2098,9 @@ static int features_host_varlen_impl(mmf_plan* plan, const void* pcm_host_v, int
     h.o_pmag = mod_c && mag_host ? take((size_t)nm * wins * nb * 4) : 0;
     h.o_pband = mod_c && nbe > 0 ? take(wins * nbe * 4) : 0;
     h.o_scratch = take(std::max(h.cv.bytes, mod_c ? h.mv.bytes : 0));
+    const size_t n_amp = want_amp ? (size_t)(A[c1] - A[c0]) : 0;
+    h.o_amp = want_amp ? take(n_amp * 4) : 0;
+    h.o_ampf = want_amp && amp_filt_host ? take(n_amp * 8) : 0;
     h.end = o;
     slot = std::max(slot, o);
     c0 = c1;
@@ -2023,6 +2140,28 @@ static int features_host_varlen_impl(mmf_plan* plan, const void* pcm_host_v, int
       const unsigned char* dd = d_desc + h.o_desc;
       MMF_CUDA(cudaMemcpyAsync(dev(h.o_h2d), (const unsigned char*)pcm_host_v + (size_t)offsets[h.c0] * isz,
                                (size_t)(offsets[h.c1] - offsets[h.c0]) * isz, cudaMemcpyHostToDevice, st));
+      // the envelope reads the native samples as they arrived, straight into its packed blocks
+      float* d_amp = want_amp ? (float*)dev(h.o_amp) : nullptr;
+      double* d_ampf = want_amp && amp_filt_host ? (double*)dev(h.o_ampf) : nullptr;
+      if (want_amp) {
+        cudaError_t ea = rms_varlen_launch(dev(h.o_h2d), pcm16, (const RmsClip*)(dd + h.o_acl),
+                                           (const unsigned*)(dd + h.o_afirst), (long)nc, (long)h.amp_items, d_amp, st);
+        if (ea != cudaSuccess) return cuda_fail(ea, "rms_varlen_kernel launch");
+      }
+      if (d_ampf) {
+        if (h.amp_np) {
+          const FusedVarlen fvl{(const int*)(dd + h.o_fclips), (const int*)(dd + h.o_fT),
+                                (const SosPar*)(dd + h.o_fpars), (const int2*)(dd + h.o_fpidx),
+                                (const long*)(dd + h.o_foff)};
+          cudaError_t ea = sosfiltfilt_par_varlen_launch(d_amp, 1, (long)h.amp_np, 0, h.amax, fvl, d_ampf, st);
+          if (ea != cudaSuccess) return cuda_fail(ea, "sosfiltfilt_par_kernel (envelopes) launch");
+        }
+        for (int64_t k : h.amp_single) {
+          const int64_t a0 = A[h.c0 + k] - A[h.c0], Tk = A[h.c0 + k + 1] - A[h.c0 + k];
+          cudaError_t ea = sosfiltfilt_any(d_amp + a0, 1, 1, (long)Tk, (long)Tk, 1, 0, so_amp, d_ampf + a0, (long)Tk, st);
+          if (ea != cudaSuccess) return cuda_fail(ea, "sosfiltfilt (envelope)");
+        }
+      }
       float* d_pcm = (float*)dev(h.o_pcm);
       cudaError_t e = resample_rows_launch(dev(h.o_h2d), pcm16, (const RsClip*)(dd + h.o_rs),
                                            (const unsigned*)(dd + h.o_first), (long)nc, (long)h.items,
@@ -2068,6 +2207,9 @@ static int features_host_varlen_impl(mmf_plan* plan, const void* pcm_host_v, int
       if (d_band && (rc2 = out(d_band, h.o_pband, 4, 1, nbe, W * nbe, cnt_w, off_w, band_host + (size_t)nbe * Wo[h.c0],
                                (size_t)nbe * wins * 4)))
         return rc2;
+      const size_t n_amp = want_amp ? (size_t)(A[h.c1] - A[h.c0]) : 0;
+      if (amp_host) MMF_CUDA(cudaMemcpyAsync(amp_host + A[h.c0], d_amp, n_amp * 4, cudaMemcpyDeviceToHost, st));
+      if (d_ampf) MMF_CUDA(cudaMemcpyAsync(amp_filt_host + A[h.c0], d_ampf, n_amp * 8, cudaMemcpyDeviceToHost, st));
     }
     return MMF_OK;
   };
@@ -2101,6 +2243,22 @@ static int resample_dev(mmf_plan* plan, const float* x_dev, const std::vector<Rs
                              (long)first.back(), (const float*)(d + o_h), y_dev, (long)y_stride, st);
   cudaFreeAsync(d, st);
   if (e != cudaSuccess) return cuda_fail(e, "resample_rows_kernel launch");
+  return MMF_OK;
+}
+
+// One ragged RMS launch on `st` over float32 x_dev from host descriptors (RmsClip at o_clips, first_item at o_first of
+// `desc`), which go up to stream-ordered scratch as resample_dev's do.
+static int rms_run(mmf_plan* plan, const float* x_dev, const std::vector<unsigned char>& desc, size_t o_clips,
+                   size_t o_first, int64_t n_clips, int64_t n_items, float* out_dev, cudaStream_t st) {
+  MMF_CUDA(cudaSetDevice(plan->cfg.device));
+  unsigned char* d = nullptr;
+  MMF_CUDA(cudaMallocAsync((void**)&d, desc.size(), st));
+  cudaError_t e = cudaMemcpyAsync(d, desc.data(), desc.size(), cudaMemcpyHostToDevice, st);
+  if (e == cudaSuccess)
+    e = rms_varlen_launch(x_dev, 0, (const RmsClip*)(d + o_clips), (const unsigned*)(d + o_first), (long)n_clips,
+                          (long)n_items, out_dev, st);
+  cudaFreeAsync(d, st);
+  if (e != cudaSuccess) return cuda_fail(e, "rms_varlen_kernel launch");
   return MMF_OK;
 }
 
@@ -2144,6 +2302,41 @@ int mmf_features_host_varlen_pcm16(mmf_plan* plan, const int16_t* pcm16_host, in
                                    float* delta_host, float* mag_host, float* band_host) {
   return mmf::features_host_varlen_impl(plan, pcm16_host, 1, n_clips, offsets_host, false, nullptr, nullptr, 0, prm, mod,
                                         tot_host, mfcc_host, delta_host, mag_host, band_host);
+}
+
+int mmf_features_host_varlen_amp(mmf_plan* plan, const void* pcm_host, int32_t pcm16, int64_t n_clips,
+                                 const int64_t* offsets_host, const mmf_resample_clip* rs_host, const float* h_host,
+                                 int64_t n_h, const mmf_change_params* prm, const mmf_modspec_params* mod,
+                                 const mmf_amp_params* amp, const int32_t* geom_host, double* tot_host,
+                                 float* mfcc_host, float* delta_host, float* mag_host, float* band_host,
+                                 float* amp_host, double* amp_filt_host) {
+  return mmf::features_host_varlen_impl(plan, pcm_host, pcm16 ? 1 : 0, n_clips, offsets_host, rs_host != nullptr,
+                                        rs_host, h_host, n_h, prm, mod, tot_host, mfcc_host, delta_host, mag_host,
+                                        band_host, amp, geom_host, amp_host, amp_filt_host);
+}
+
+int mmf_amp_varlen_sizes(int64_t n_clips, const int64_t* offsets_host, const int32_t* geom_host, int32_t center,
+                         int64_t* amp_off_host) {
+  using namespace mmf;
+  int rc = validate_offsets(n_clips, offsets_host);
+  if (rc) return rc;
+  if (!amp_off_host) return fail(MMF_ERR_INVALID, "amp_off_host is NULL");
+  return amp_sizes(n_clips, offsets_host, geom_host, center, amp_off_host);
+}
+
+int mmf_rms_varlen(mmf_plan* plan, const float* x_dev, int64_t n_clips, const int64_t* offsets_host,
+                   const int32_t* geom_host, int32_t center, float* amp_dev, void* stream) {
+  using namespace mmf;
+  int rc = validate_offsets(n_clips, offsets_host);
+  if (rc) return rc;
+  std::vector<int64_t> A((size_t)n_clips + 1);
+  if ((rc = amp_sizes(n_clips, offsets_host, geom_host, center, A.data()))) return rc;
+  if (!plan || !x_dev || !amp_dev) return fail(MMF_ERR_INVALID, "NULL argument");
+  std::vector<unsigned char> desc;
+  size_t o_clips, o_first;
+  const int64_t items = rms_desc(0, n_clips, offsets_host, 0, geom_host, center, A.data(), desc, o_clips, o_first);
+  if (items < 0) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 work items");
+  return rms_run(plan, x_dev, desc, o_clips, o_first, n_clips, items, amp_dev, (cudaStream_t)stream);
 }
 
 }  // extern "C"
@@ -2245,6 +2438,31 @@ int mmf_resample_varlen(mmf_plan* plan, const float* x_dev, int64_t n_clips, con
   const unsigned* f = (const unsigned*)(desc.data() + o_first);
   return resample_dev(plan, x_dev, std::vector<RsClip>(c, c + n_clips), std::vector<unsigned>(f, f + n_clips + 1),
                       h_host, n_taps, y_dev, y_stride, (cudaStream_t)stream);
+}
+
+// one descriptor per row of the ragged kernel (rows of equal length: the grid has no row limit)
+int mmf_rms(mmf_plan* plan, const float* pcm_dev, int64_t n_clips, int64_t n_samples, int64_t clip_stride,
+            int32_t frame_length, int32_t hop_length, int32_t center, float* rms_dev, void* stream) {
+  if (!plan || !pcm_dev || !rms_dev) return fail(MMF_ERR_INVALID, "NULL argument");
+  if (n_clips < 1) return fail(MMF_ERR_INVALID, "n_clips must be positive");
+  if (frame_length < 1 || hop_length < 1) return fail(MMF_ERR_INVALID, "frame_length and hop_length must be positive");
+  const int pad = center ? frame_length / 2 : 0;
+  const int64_t padded = n_samples + 2 * (int64_t)pad;
+  if (padded < frame_length) return fail(MMF_ERR_TOO_SHORT, "Input is too short for frame_length");
+  const int64_t T = 1 + (padded - frame_length) / hop_length;
+  const int F = rms_frames_per_item(frame_length, hop_length);
+  const int64_t per = (T + F - 1) / F;
+  if (per * n_clips > 0x7fffffffLL) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 work items");
+  const size_t o_first = align_up((size_t)n_clips * sizeof(RmsClip), 16);
+  std::vector<unsigned char> desc(o_first + ((size_t)n_clips + 1) * 4);
+  RmsClip* cl = (RmsClip*)desc.data();
+  unsigned* first = (unsigned*)(desc.data() + o_first);
+  for (int64_t r = 0; r < n_clips; ++r) {
+    cl[r] = RmsClip{(long)(r * clip_stride), (long)n_samples, (long)(r * T), (long)T, frame_length, hop_length, pad, F};
+    first[r] = (unsigned)(r * per);
+  }
+  first[n_clips] = (unsigned)(n_clips * per);
+  return rms_run(plan, pcm_dev, desc, 0, o_first, n_clips, n_clips * per, rms_dev, (cudaStream_t)stream);
 }
 
 int mmf_mfcc_change_host(mmf_plan* plan, const float* pcm_host, int64_t n_clips, int64_t n_samples,

@@ -102,8 +102,9 @@ constexpr int kParWarps = 4;
 constexpr int kFusedPerThread = 9;
 constexpr int kFusedMaxWarps = 12;  // 384 threads, <= 85 registers: two CTAs per SM
 
-// VL (variable-length batch): row r is clip vl.clips[r] at x + clip * x_row_stride with its own frame count and
-// cascade tables (vl.pidx[clip].y); a warp's buffer is `s_stride` doubles, the largest 32 * CL of the launch.
+// VL (variable-length batch): row r is clip vl.clips[r] at x + clip * x_row_stride (packed: at x + vl.off[clip], and
+// so is its output row in y) with its own frame count and cascade tables (vl.pidx[clip].y); a warp's buffer is
+// `s_stride` doubles, the largest 32 * CL of the launch.
 template <typename TIn, int NS, bool VL>
 __global__ void __launch_bounds__(kParWarps * 32)
     sosfiltfilt_par_kernel(const TIn* __restrict__ x, long rows, int T, long x_row_stride, int group_rows,
@@ -121,10 +122,12 @@ __global__ void __launch_bounds__(kParWarps * 32)
   const int S = 32 * a.CL, p = a.padlen, L = T + 2 * p;
   double* buf = sm_par + (size_t)warp * s_stride;
   const long g = row / group_rows, gi = row - g * group_rows;
-  warp_load_odd_ext<TIn>(x + g * group_stride + gi * x_row_stride, T, p, buf, S, lane);
+  const bool packed = VL && vl.off != nullptr;
+  const long xo = packed ? vl.off[row] : g * group_stride + gi * x_row_stride;
+  double* dst = y + (packed ? xo : row * y_row_stride);
+  warp_load_odd_ext<TIn>(x + xo, T, p, buf, S, lane);
   const SosRegs<NS> c(a);
   warp_sosfiltfilt<NS>(buf, L, a, c, lane);
-  double* dst = y + row * y_row_stride;
   for (int t = lane; t < T; t += 32) dst[t] = buf[p + t];
 }
 
@@ -141,27 +144,35 @@ static cudaError_t par_launch_ns(const TIn* x, long rows, long T, long xs, int g
   return cudaGetLastError();
 }
 
-template <int NS>
-static cudaError_t par_varlen_ns(const double* x, long rows, long pitch, const SosPar& amax, const FusedVarlen& vl,
+template <typename TIn, int NS>
+static cudaError_t par_varlen_ns(const TIn* x, long rows, long pitch, const SosPar& amax, const FusedVarlen& vl,
                                  double* y, cudaStream_t st) {
   const unsigned grid = (unsigned)((rows + kParWarps - 1) / kParWarps);
   const size_t smem = (size_t)kParWarps * 32 * amax.CL * sizeof(double);
-  auto kfn = sosfiltfilt_par_kernel<double, NS, true>;
+  auto kfn = sosfiltfilt_par_kernel<TIn, NS, true>;
   MMF_SMEM_ONCE(kfn, 200 * 1024);
   kfn<<<grid, kParWarps * 32, smem, st>>>(x, rows, (int)pitch, pitch, 1, pitch, amax, y, pitch, vl, 32 * amax.CL);
   count_launch();
   return cudaGetLastError();
 }
 
-cudaError_t sosfiltfilt_par_varlen_launch(const double* x, long rows, long pitch, const SosPar& amax,
-                                          const FusedVarlen& vl, double* y, cudaStream_t st) {
+template <typename TIn>
+static cudaError_t par_varlen_t(const TIn* x, long rows, long pitch, const SosPar& amax, const FusedVarlen& vl,
+                                double* y, cudaStream_t st) {
   switch (amax.ns) {
-    case 1: return par_varlen_ns<1>(x, rows, pitch, amax, vl, y, st);
-    case 2: return par_varlen_ns<2>(x, rows, pitch, amax, vl, y, st);
-    case 3: return par_varlen_ns<3>(x, rows, pitch, amax, vl, y, st);
-    case 4: return par_varlen_ns<4>(x, rows, pitch, amax, vl, y, st);
+    case 1: return par_varlen_ns<TIn, 1>(x, rows, pitch, amax, vl, y, st);
+    case 2: return par_varlen_ns<TIn, 2>(x, rows, pitch, amax, vl, y, st);
+    case 3: return par_varlen_ns<TIn, 3>(x, rows, pitch, amax, vl, y, st);
+    case 4: return par_varlen_ns<TIn, 4>(x, rows, pitch, amax, vl, y, st);
     default: return cudaErrorInvalidValue;
   }
+}
+
+// x_is_f32: float32 rows (the RMS envelope), odd-extended in float32 as the single-row call extends them
+cudaError_t sosfiltfilt_par_varlen_launch(const void* x, int x_is_f32, long rows, long pitch, const SosPar& amax,
+                                          const FusedVarlen& vl, double* y, cudaStream_t st) {
+  if (x_is_f32) return par_varlen_t<float>((const float*)x, rows, pitch, amax, vl, y, st);
+  return par_varlen_t<double>((const double*)x, rows, pitch, amax, vl, y, st);
 }
 
 template <typename TIn>

@@ -214,17 +214,19 @@ bool change_fused_lm_supported(const SosPar& a1, const SosPar* a2, int n_mfcc, i
                                long T, size_t* smem_out);
 // variable-length batch of the fused kernel and the batched output filter: launch item b is clip clips[b] with T[clip]
 // frames and the cascade tables pars[pidx[clip].x] (row filter) / pars[pidx[clip].y] (output filter); the launch's
-// T is the row pitch and its SosPar arguments are the ones with the largest chunk (they size shared memory)
+// T is the row pitch and its SosPar arguments are the ones with the largest chunk (they size shared memory).  off
+// (batched output filter only): packed rows, clip's input and output rows both at off[clip] (null: at clip * pitch)
 struct FusedVarlen {
   const int* clips;
   const int* T;
   const SosPar* pars;
   const int2* pidx;
+  const long* off = nullptr;
 };
 cudaError_t change_fused_launch(const float* mfcc, long n_clips, int n_mfcc, int first, int rows, long T, int method,
                                 const SosPar& a1, const SosPar& a2, int out_kind, double* tot, size_t smem,
                                 const FusedMfccArgs* lm, cudaStream_t st, const FusedVarlen* vl = nullptr);
-cudaError_t sosfiltfilt_par_varlen_launch(const double* x, long rows, long pitch, const SosPar& amax,
+cudaError_t sosfiltfilt_par_varlen_launch(const void* x, int x_is_f32, long rows, long pitch, const SosPar& amax,
                                           const FusedVarlen& vl, double* y, cudaStream_t st);
 cudaError_t varlen_tails_launch(long n_clips, const int* T, int pitch, double* tot, float* logmel, int n_mels,
                                 float* mfcc, float* delta, int n_mfcc, cudaStream_t st);
@@ -248,8 +250,26 @@ cudaError_t modspec_clip_launch(const float* mfcc, long n_clips, int n_coef, lon
                                 long wc, const float* hann, const float2* tw1, const float2* tw2, float* mag,
                                 float* band, const int* lo, const int* hi, int n_bands, cudaStream_t st,
                                 const ModVarlen* vl = nullptr);
-cudaError_t rms_launch(const float* pcm, long n_clips, long n, long stride, int frame_length, int hop, int pad,
-                       long T, float* out, cudaStream_t st);
+// One clip of a ragged RMS-envelope launch (device descriptor, built on the host): the len samples at x + src, frames
+// of frame_length samples every hop from -pad (samples outside [0, len) read as 0), T frames written from out + out.
+// A work item is F consecutive frames of one clip; its span (F - 1) * hop + frame_length is staged in shared memory
+// when it fits kRmsSpan floats, read from global memory otherwise.
+struct RmsClip {
+  long src, len, out, T;
+  int frame_length, hop, pad, F;
+};
+constexpr int kRmsWarps = 8;      // one frame per warp at a time
+constexpr int kRmsSpan = 12288;   // floats of a work item's staged span (48 KB)
+// frames per work item of a clip (see RmsClip)
+inline int rms_frames_per_item(int frame_length, int hop) {
+  if (frame_length > kRmsSpan) return kRmsWarps;
+  const int fit = (kRmsSpan - frame_length) / hop + 1, F = fit < 64 ? fit : 64;
+  return F >= kRmsWarps ? F - F % kRmsWarps : F;
+}
+// Clip c owns work items [first_item[c], first_item[c + 1]) (ceil(T / F) each).  x is float32 or (pcm16) int16 scaled
+// by 1/32768 as pcm16_to_f32_kernel scales it.
+cudaError_t rms_varlen_launch(const void* x, int pcm16, const RmsClip* clips, const unsigned* first_item, long n_clips,
+                              long n_items, float* out, cudaStream_t st);
 cudaError_t fill_i32_launch(int* p, long n, int v, cudaStream_t st);
 cudaError_t hilbert_envelope_launch(const float* x, long n_clips, long n, long stride, float* amp, long amp_stride,
                                     int sm_count, cudaStream_t st);

@@ -975,32 +975,73 @@ cudaError_t modspec_launch(const float* mfcc, long n_clips, int n_coef, long T, 
 }
 
 // ---------------------------------------------------------------------------
-// RMS envelope (librosa.feature.rms; script/calc.py:326-331): one warp per frame.
+// Ragged RMS envelope (librosa.feature.rms, pad_mode='constant'; script/calc.py:326-331) of packed clips.  Each frame
+// is one warp's sum: lane l accumulates fmaf(v, v, s) over i = l, l + 32, ... from 0, samples outside [0, len) read as
+// 0, then the xor-shuffle tree 16, 8, 4, 2, 1 and sqrtf(s / frame_length).  That order is the contract: every output's
+// bits are fixed by it, whatever chunk or batch the clip sits in (a running sum over the hop would be cheaper and
+// would change them).  A work item (one CTA) is F consecutive frames of one clip (RmsClip); its span of
+// (F - 1) * hop + frame_length samples is read from global memory once, int16 scaled on load as pcm16_to_f32_kernel
+// scales it, into shared memory, where the overlapping frames (10x at 0.1 s / 0.01 s) find it.  A clip whose frame
+// alone is over kRmsSpan reads its frames from global memory in the same order.
 // ---------------------------------------------------------------------------
-__global__ void rms_kernel(const float* __restrict__ pcm, long n, long stride, int frame_length, int hop, int pad,
-                           long T, float* __restrict__ out) {
-  const long w = ((long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  if (w >= T) return;
-  const long clip = blockIdx.y;
-  const float* x = pcm + (size_t)clip * stride;
-  const long start = w * hop - pad;
-  float s = 0.0f;
-  for (int i = lane; i < frame_length; i += 32) {
-    const long m = start + i;
-    const float v = (m >= 0 && m < n) ? x[m] : 0.0f;
-    s = fmaf(v, v, s);
+template <typename X>
+__global__ void __launch_bounds__(kRmsWarps * 32) rms_varlen_kernel(const X* __restrict__ x,
+                                                                     const RmsClip* __restrict__ clips,
+                                                                     const unsigned* __restrict__ first_item,
+                                                                     long n_clips, float* __restrict__ out) {
+  __shared__ float xs[kRmsSpan];
+  constexpr float kq = 1.0f / 32768.0f;
+  const unsigned item = blockIdx.x;
+  long clip = 0, hi_c = n_clips - 1;  // the clip owning this item: the last with first_item[clip] <= item
+  while (clip < hi_c) {
+    const long mid = (clip + hi_c + 1) >> 1;
+    if (first_item[mid] <= item) clip = mid;
+    else hi_c = mid - 1;
   }
+  const RmsClip c = clips[clip];
+  const X* xr = x + c.src;
+  auto ld = [&](long m) -> float {
+    if (m < 0 || m >= c.len) return 0.0f;
+    if constexpr (sizeof(X) == 2) return (float)xr[m] * kq;
+    else return xr[m];
+  };
+  const long f0 = (long)(item - first_item[clip]) * c.F;
+  const int nf = (int)min((long)c.F, c.T - f0);
+  const long start0 = f0 * c.hop - c.pad;
+  const bool staged = (long)(c.F - 1) * c.hop + c.frame_length <= kRmsSpan;  // the same for every item of the clip
+  if (staged) {
+    const int span = (nf - 1) * c.hop + c.frame_length;
+    for (int j = threadIdx.x; j < span; j += kRmsWarps * 32) xs[j] = ld(start0 + j);
+    __syncthreads();
+  }
+  const int lane = threadIdx.x & 31;
+  for (int f = threadIdx.x >> 5; f < nf; f += kRmsWarps) {
+    float s = 0.0f;
+    if (staged) {
+      const float* w = xs + f * c.hop;
+      for (int i = lane; i < c.frame_length; i += 32) {
+        const float v = w[i];
+        s = fmaf(v, v, s);
+      }
+    } else {
+      const long start = start0 + (long)f * c.hop;
+      for (int i = lane; i < c.frame_length; i += 32) {
+        const float v = ld(start + i);
+        s = fmaf(v, v, s);
+      }
+    }
 #pragma unroll
-  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-  if (lane == 0) out[(size_t)clip * T + w] = sqrtf(s / (float)frame_length);
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if (lane == 0) out[c.out + f0 + f] = sqrtf(s / (float)c.frame_length);
+  }
 }
 
-cudaError_t rms_launch(const float* pcm, long n_clips, long n, long stride, int frame_length, int hop, int pad, long T,
-                       float* out, cudaStream_t st) {
-  const int threads = 256;  // 8 frames per block
-  dim3 grid((unsigned)((T + 7) / 8), (unsigned)n_clips);
-  rms_kernel<<<grid, threads, 0, st>>>(pcm, n, stride, frame_length, hop, pad, T, out);
+cudaError_t rms_varlen_launch(const void* x, int pcm16, const RmsClip* clips, const unsigned* first_item, long n_clips,
+                              long n_items, float* out, cudaStream_t st) {
+  if (pcm16)
+    rms_varlen_kernel<<<(unsigned)n_items, kRmsWarps * 32, 0, st>>>((const int16_t*)x, clips, first_item, n_clips, out);
+  else
+    rms_varlen_kernel<<<(unsigned)n_items, kRmsWarps * 32, 0, st>>>((const float*)x, clips, first_item, n_clips, out);
   count_launch();
   return cudaGetLastError();
 }

@@ -9,7 +9,6 @@ memory and streams only; all arithmetic happens in ``libmmf_b200.so``).
 from __future__ import annotations
 
 import ctypes as C
-import functools
 import math
 from collections import OrderedDict
 from dataclasses import dataclass, replace
@@ -17,7 +16,7 @@ from dataclasses import dataclass, replace
 import numpy as np
 
 from . import _lib
-from ._lib import MmfError, check, mmf_change_params, mmf_config, mmf_modspec_params
+from ._lib import MmfError, check, mmf_amp_params, mmf_change_params, mmf_config, mmf_modspec_params
 
 
 @dataclass(frozen=True)
@@ -519,6 +518,30 @@ class Plan:
         )
         return out
 
+    def rms_varlen(self, x, offsets, geom, center: bool = True):
+        """:meth:`rms` for clips of different lengths and frame geometries packed back to back, in one launch.
+
+        ``x`` is a 1-D float32 device tensor (or host array); clip ``i`` is ``x[offsets[i]:offsets[i + 1]]`` with
+        ``geom[i] = (frame_length_i, hop_i)``.  Returns ``(amp, amp_offsets)``: the float32 envelopes packed clip after
+        clip, clip ``i``'s at ``amp[amp_offsets[i]:amp_offsets[i + 1]]``, each equal to :meth:`rms` on that clip alone,
+        bit for bit."""
+        torch = _torch()
+        x = x if isinstance(x, torch.Tensor) else torch.as_tensor(np.ascontiguousarray(x, dtype=np.float32))
+        x = x.to(device=self.device, dtype=torch.float32).contiguous()
+        if x.dim() != 1:
+            raise ValueError("rms_varlen takes a 1-D packed buffer")
+        offs, geom, amp_off = amp_sizes(offsets, geom, center)
+        if offs[-1] > x.shape[0]:
+            raise ValueError(f"offsets[{len(offs) - 1}] = {offs[-1]} is past the end of the {x.shape[0]}-sample buffer")
+        amp = torch.empty((int(amp_off[-1]),), device=self.device, dtype=torch.float32)
+        check(
+            _lib.lib().mmf_rms_varlen(
+                self._h, x.data_ptr(), len(offs) - 1, offs.ctypes.data, geom.ctypes.data, 1 if center else 0,
+                amp.data_ptr(), _stream_ptr(self.device),
+            )
+        )
+        return amp, amp_off
+
     def hilbert_envelope(self, x):
         """``np.abs(scipy.signal.hilbert(x))`` along the last axis, float32 on the device."""
         torch = _torch()
@@ -760,7 +783,7 @@ class Plan:
         return out
 
     def features_host_varlen(self, pcm_host: np.ndarray, offsets, prm: mmf_change_params, mod=None, *,
-                             want=("totChange",), out=None, rates=None):
+                             want=("totChange",), out=None, rates=None, amp=None):
         """:meth:`features_host` for clips of different lengths packed back to back in one host buffer.
 
         ``pcm_host`` is 1-D float32 or int16 (raw WAV samples, scaled by 1/32768 on the device); clip ``i`` is
@@ -774,7 +797,12 @@ class Plan:
         ``rates``: one source sample rate per clip.  Each clip then crosses PCIe at its own rate and is resampled on
         the device to the plan's rate with the loader's filter (:func:`resample_descriptors`), straight into the rows
         the ragged path reads; its blocks equal :meth:`features_host` on ``resample_poly(x, up, down, "hq")`` of that
-        clip alone (after ``pcm16_to_f32`` for int16), bit for bit, and ``frames`` count frames at the plan's rate."""
+        clip alone (after ``pcm16_to_f32`` for int16), bit for bit, and ``frames`` count frames at the plan's rate.
+
+        ``amp = (geom, center, out_sos or None)`` adds each clip's RMS envelope, taken from its native samples (int16
+        scaled by 1/32768) with ``geom[i] = (frame_length_i, hop_i)``: ``amplitude``, float32, or float64 through the
+        zero-phase ``out_sos`` when one is given, packed at ``amp_offsets`` (int64 ``[B + 1]``).  Clip ``i``'s block
+        equals :meth:`rms` (then :meth:`sosfiltfilt`) on that clip alone, bit for bit."""
         pcm_host = np.asarray(pcm_host)
         pcm16 = pcm_host.dtype == np.int16
         if not pcm16 and pcm_host.dtype != np.float32:
@@ -830,29 +858,41 @@ class Plan:
                 ptr[k] = None
         if ("modspec" in want or "band_energy" in want) and mp is None:
             raise ValueError("modspec / band_energy requested without modulation parameters")
-        if rates is not None:
-            fn = functools.partial(_lib.lib().mmf_features_host_varlen_resampled, self._h, pcm_host.ctypes.data,
-                                   1 if pcm16 else 0, B, offs.ctypes.data, rs.ctypes.data,
-                                   h.ctypes.data if len(h) else None, len(h))
-        else:
-            fn = functools.partial(_lib.lib().mmf_features_host_varlen_pcm16 if pcm16 else
-                                   _lib.lib().mmf_features_host_varlen, self._h, pcm_host.ctypes.data, B,
-                                   offs.ctypes.data)
-        check(
-            fn(
-                C.byref(prm),
-                C.byref(mp) if mp is not None else None,
-                ptr["totChange"],
-                ptr["mfcc"],
-                ptr["delta"],
-                ptr["modspec"],
-                ptr["band_energy"],
+        outs = (C.byref(prm), C.byref(mp) if mp is not None else None)
+        ptrs = (ptr["totChange"], ptr["mfcc"], ptr["delta"], ptr["modspec"], ptr["band_energy"])
+        if amp is not None:
+            geom, center, out_sos = amp
+            _, geom, amp_off = amp_sizes(offs, geom, center)
+            dt = np.float64 if out_sos is not None else np.float32
+            a = out.get("amplitude")
+            if a is None or a.shape != (int(amp_off[-1]),) or a.dtype != dt or not a.flags.c_contiguous:
+                a = np.empty(int(amp_off[-1]), dt)
+                out["amplitude"] = a
+            resampled = rates is not None
+            check(
+                _lib.lib().mmf_features_host_varlen_amp(
+                    self._h, pcm_host.ctypes.data, 1 if pcm16 else 0, B, offs.ctypes.data,
+                    rs.ctypes.data if resampled else None, h.ctypes.data if resampled and len(h) else None,
+                    len(h) if resampled else 0, *outs, C.byref(make_amp_params(center, out_sos)), geom.ctypes.data,
+                    *ptrs, a.ctypes.data if out_sos is None else None, a.ctypes.data if out_sos is not None else None,
+                )
             )
-        )
+        elif rates is not None:
+            check(
+                _lib.lib().mmf_features_host_varlen_resampled(
+                    self._h, pcm_host.ctypes.data, 1 if pcm16 else 0, B, offs.ctypes.data, rs.ctypes.data,
+                    h.ctypes.data if len(h) else None, len(h), *outs, *ptrs,
+                )
+            )
+        else:
+            fn = _lib.lib().mmf_features_host_varlen_pcm16 if pcm16 else _lib.lib().mmf_features_host_varlen
+            check(fn(self._h, pcm_host.ctypes.data, B, offs.ctypes.data, *outs, *ptrs))
         out["frames"] = np.diff(frame_off)
         out["windows"] = np.diff(win_off)
         out["frame_offsets"] = frame_off
         out["window_offsets"] = win_off
+        if amp is not None:
+            out["amp_offsets"] = amp_off
         return out
 
     def mfcc_change_host(self, pcm_host: np.ndarray, prm: mmf_change_params, *, want_mfcc: bool = False):
@@ -889,6 +929,36 @@ class Plan:
                 )
             )
         return (tot, mf) if want_mfcc else tot
+
+
+def amp_sizes(offsets, geom, center: bool):
+    """``(offsets, geom, amp_offsets)`` of a packed batch's RMS envelopes (``mmf_amp_varlen_sizes``, no device
+    needed): ``offsets`` as int64 ``[B + 1]``, ``geom`` as int32 ``[B, 2]`` rows ``(frame_length_i, hop_i)``, and the
+    prefix sums of ``T_amp_i = 1 + (len_i + 2 pad_i - frame_length_i) // hop_i``.  A bad clip raises
+    :class:`MmfError` naming it."""
+    offs = np.ascontiguousarray(np.asarray(offsets, dtype=np.int64).reshape(-1))
+    B = offs.shape[0] - 1
+    geom = np.ascontiguousarray(np.asarray(geom, dtype=np.int32).reshape(-1, 2))
+    if geom.shape[0] != B:
+        raise ValueError(f"geom has {geom.shape[0]} rows for {B} clips")
+    amp_off = np.zeros(B + 1, np.int64)
+    check(_lib.lib().mmf_amp_varlen_sizes(B, offs.ctypes.data, geom.ctypes.data, 1 if center else 0,
+                                          amp_off.ctypes.data))
+    return offs, geom, amp_off
+
+
+def make_amp_params(center: bool, out_sos=None) -> mmf_amp_params:
+    """Pack the envelope parameters of the host-buffer bundle: ``center`` and the optional zero-phase output filter."""
+    ap = mmf_amp_params()
+    ap.center = 1 if center else 0
+    if out_sos is not None:
+        out_sos = np.ascontiguousarray(out_sos, dtype=np.float64)
+        if out_sos.ndim != 2 or out_sos.shape[1] != 6 or out_sos.shape[0] > 16:
+            raise ValueError("out_sos must be [n_sections <= 16, 6]")
+        ap.out_n_sections = out_sos.shape[0]
+        for i, v in enumerate(out_sos.ravel()):
+            ap.out_sos[i] = v
+    return ap
 
 
 def _modspec_params(mod):
@@ -930,6 +1000,8 @@ def clear_plans() -> None:
 
 
 __all__ = [
+    "amp_sizes",
+    "make_amp_params",
     "design_resample_filter",
     "resample_descriptors",
     "resample_ratio",

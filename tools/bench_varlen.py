@@ -26,11 +26,17 @@ the tree's mmf_resample_poly launches, so the leg can time an older tree too) an
 mmf_resample_varlen launch over all of them; and one pinned copy of the packed int16 bytes, against which the
 call's own time shows whether resampling and features stay under the copy.
 
+The amplitude leg adds the RMS envelope (FeatureExtractor's amp_* defaults: 0.1 s window, 0.01 s hop, centred) to
+host_varlen(want=every output) on the resample leg's corpus (with rates=) and on the host leg's 16 kHz float32 corpus:
+the call without it, with the raw envelope and with the 'iir' output filter.  It also times the route without the
+bundle, calculate_amplitude_envelope per clip at its native rate, and with torch.profiler the envelope kernels over
+the same clips: one mmf_rms_varlen launch, and Plan.rms per clip (whatever kernel the tree's mmf_rms launches).
+
 Workload: 1024 clips at 16 kHz with the bench's frame geometry (win 400 / hop 160 / n_fft 512, 40 mel, 13 MFCC,
 gradient, Butterworth output filter), lengths uniform in [2 s, 20 s] from a fixed seed.  Prints, per leg, the median
 ms of each way and audio-seconds per second as one JSON line, with the GPU's name and power limit.
 
-    python tools/bench_varlen.py [--clips 1024] [--iters 10] [--loop-iters 3] [--legs change,features,host,resample]
+    python tools/bench_varlen.py [--clips 1024] [--iters 10] [--loop-iters 3] [--legs change,features,host,resample,amplitude]
 """
 import argparse
 import json
@@ -145,10 +151,8 @@ def _profiled_kernel_ms(fn, match):
     return sum(e.device_time_total for e in prof.key_averages() if match in e.key) / 1e3
 
 
-def _resample_leg(n_clips, iters, seed, power_limit, dev):
-    from modulation_mfcc_b200 import _lib
-
-    sr_in, sr = 44100, 16000
+def _int16_corpus(n_clips, seed, sr_in):
+    """The resample leg's corpus: int16 clips of 2-20 s at sr_in, packed in one pinned buffer."""
     rng = np.random.default_rng(seed)
     lengths = [int(n) for n in rng.integers(2 * sr_in, 20 * sr_in + 1, n_clips)]
     offsets = np.zeros(n_clips + 1, np.int64)
@@ -157,6 +161,14 @@ def _resample_leg(n_clips, iters, seed, power_limit, dev):
     for i in range(n_clips):
         x = mm.synth_clip(seed + i, lengths[i], sr_in)
         packed[offsets[i] : offsets[i + 1]] = np.clip(np.round(x * 32768.0), -32768, 32767).astype(np.int16)
+    return packed, offsets, lengths
+
+
+def _resample_leg(n_clips, iters, seed, power_limit, dev):
+    from modulation_mfcc_b200 import _lib
+
+    sr_in, sr = 44100, 16000
+    packed, offsets, lengths = _int16_corpus(n_clips, seed, sr_in)
     clips = [packed[offsets[i] : offsets[i + 1]] for i in range(n_clips)]
     audio_s = sum(lengths) / sr_in
     fx = mm.FeatureExtractor(sr, device=0)
@@ -199,6 +211,52 @@ def _resample_leg(n_clips, iters, seed, power_limit, dev):
         res["resample_then_host_many_ms"] = _median_host_ms(before, max(1, iters // 5))
         res["resample_then_host_many_audio_s_per_s"] = audio_s / (res["resample_then_host_many_ms"] / 1e3)
     print(json.dumps(res), flush=True)
+
+
+def _amplitude_leg(pcm, lengths16, n_clips, iters, seed, power_limit, dev):
+    """The RMS envelope inside the host-buffer bundle; see the module docstring."""
+    want = ("totChange", "mfcc", "delta", "modspec", "band_energy")
+    fxs = {"raw": mm.FeatureExtractor(16000, device=0), "iir": mm.FeatureExtractor(16000, device=0, amp_outFilter="iir")}
+    plan = fxs["raw"].plan
+    sr_in = 44100
+    packed44, offsets44, lengths44 = _int16_corpus(n_clips, seed, sr_in)
+    host16 = pcm.cpu().numpy()
+    offsets16 = np.zeros(len(lengths16) + 1, np.int64)
+    np.cumsum(lengths16, out=offsets16[1:])
+    packed16 = _pinned((int(offsets16[-1]),), np.float32)
+    for i, n in enumerate(lengths16):
+        packed16[offsets16[i] : offsets16[i + 1]] = host16[i, :n]
+    corpora = [("int16_44k_rates", packed44, offsets44, [sr_in] * n_clips, sr_in),
+               ("float32_16k", packed16, offsets16, None, 16000)]
+    for name, packed, offsets, rates, rate in corpora:
+        B = len(offsets) - 1
+        audio_s = float(offsets[-1] - offsets[0]) / rate
+        res = {"leg": "amplitude", "corpus": name, "gpu": torch.cuda.get_device_name(dev), "power_limit": power_limit,
+               "clips": B, "audio_s": audio_s, "h2d_bytes": packed.nbytes}
+        for k, (fx, w) in {"none": (fxs["raw"], want), "raw": (fxs["raw"], want + ("amplitude",)),
+                           "iir": (fxs["iir"], want + ("amplitude",))}.items():
+            out = {key: v for key, v in fx.host_varlen(packed, offsets, want=w, rates=rates).items()
+                   if key in w}
+            out = {key: _pinned(v.shape, v.dtype.type) for key, v in out.items()}
+            call = lambda fx=fx, w=w, out=out: fx.host_varlen(packed, offsets, want=w, out=out, rates=rates)  # noqa: E731
+            res[f"host_varlen_{k}_ms"] = _median_host_ms(call, iters)
+            res[f"host_varlen_{k}_audio_s_per_s"] = audio_s / (res[f"host_varlen_{k}_ms"] / 1e3)
+        # the route without the bundle: calculate_amplitude_envelope per clip at its native rate (float32 samples)
+        clips = [packed[offsets[i] : offsets[i + 1]] for i in range(B)]
+        clips = [c.astype(np.float32) / np.float32(32768.0) if c.dtype == np.int16 else c for c in clips]
+        loop = lambda: [mm.calculate_amplitude_envelope(c, rate) for c in clips]  # noqa: E731
+        loop()
+        res["per_clip_loop_ms"] = _median_host_ms(loop, max(1, iters // 5))
+        # kernel time over the same clips: one ragged launch, and mmf_rms per clip (whatever kernel the tree launches)
+        x_dev = torch.from_numpy(np.concatenate(clips)).to(dev)
+        offs0 = offsets - offsets[0]
+        fl, hop = int(0.1 * rate), int(0.01 * rate)
+        geom = [(fl, hop)] * B
+        rows = [x_dev[offs0[i] : offs0[i + 1]] for i in range(B)]
+        res["rms_varlen_kernel_ms"] = _profiled_kernel_ms(lambda: plan.rms_varlen(x_dev, offs0, geom, True), "rms")
+        res["rms_per_clip_kernel_ms"] = _profiled_kernel_ms(lambda: [plan.rms(r, fl, hop) for r in rows], "rms")
+        res["frames"] = int(mm.plan.amp_sizes(offs0, geom, True)[2][-1])
+        print(json.dumps(res), flush=True)
 
 
 def main():
@@ -250,6 +308,9 @@ def main():
             continue
         if leg == "resample":
             _resample_leg(a.clips, a.iters, a.seed, power_limit, dev)
+            continue
+        if leg == "amplitude":
+            _amplitude_leg(pcm, lengths, a.clips, a.iters, a.seed, power_limit, dev)
             continue
         varlen, loop, pad = ways[leg]
         for fn in (varlen, pad, loop):  # warm-up: modules, workspace growth
