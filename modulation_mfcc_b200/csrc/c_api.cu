@@ -25,10 +25,11 @@ static int fail(int code, const std::string& msg) {
 static int cuda_fail(cudaError_t e, const char* where) {
   return fail(MMF_ERR_CUDA, std::string(where) + ": " + cudaGetErrorString(e));
 }
-static int too_short(int padlen) {
-  char buf[128];
-  std::snprintf(buf, sizeof(buf), "The length of the input vector x must be greater than padlen, which is %d.", padlen);
-  return fail(MMF_ERR_TOO_SHORT, buf);
+// scipy's message; clip >= 0: a batch's, naming the clip
+static int too_short(int padlen, int64_t clip = -1) {
+  const std::string at = clip < 0 ? "" : "clip " + std::to_string(clip) + ": ";
+  return fail(MMF_ERR_TOO_SHORT, at + "The length of the input vector x must be greater than padlen, which is " +
+                                     std::to_string(padlen) + ".");
 }
 #define MMF_CUDA(call)                                   \
   do {                                                   \
@@ -100,6 +101,58 @@ static void* carve(unsigned char*& cur, size_t bytes) {
   cur += align_up(bytes, 256);
   return r;
 }
+
+// the same bump allocation over offsets: the start of `bytes` at `end`, which moves past them
+static size_t ws_take(size_t& end, size_t bytes) {
+  const size_t o = end;
+  end += align_up(bytes, 256);
+  return o;
+}
+
+// Descriptors built on the host for one upload: typed arrays appended back to back, each at a multiple of kDescAlign
+// bytes, which every descriptor type's alignment divides (8 at most: the doubles of SosPar, the longs of RsClip and
+// RmsClip).  A blob appended to another, or copied to device memory aligned to 16, keeps every part aligned.
+constexpr size_t kDescAlign = 16;
+struct DescBlob {
+  std::vector<unsigned char> bytes;
+  size_t size() const { return bytes.size(); }
+  // appends src[0, n) and returns its offset
+  template <typename T>
+  size_t put(const T* src, size_t n) {
+    static_assert(kDescAlign % alignof(T) == 0, "descriptor type aligned wider than kDescAlign");
+    const size_t o = align_up(bytes.size(), kDescAlign);
+    bytes.resize(o + n * sizeof(T), 0);
+    if (n) std::memcpy(bytes.data() + o, src, n * sizeof(T));
+    return o;
+  }
+  template <typename T>
+  size_t put(const std::vector<T>& v) { return put(v.data(), v.size()); }
+};
+
+// One ragged launch's descriptors: clips [n], first_item[n + 1]; items: their total (-1: past 2^31 - 1)
+struct RaggedParts {
+  size_t clips = 0, first = 0;
+  int64_t items = 0;
+};
+
+// Distinct chunk tables (SosPar) of a batch.  A row's tables depend on its cascade and on its length only through
+// the chunk length (sos_par_chunk), so rows of one chunk length share them.
+struct SosParSet {
+  std::vector<SosPar> pars;
+  // index in pars of the tables of cascade `which` (0 or 1), `a`, for rows of T samples; -1 when the kernel takes none
+  int index(int which, const SosArgs& a, long T) {
+    const int cl = sos_par_chunk(a, T);
+    if (cl < 0) return -1;
+    int& idx = of_chunk[which][cl];
+    SosPar sp;
+    if (idx < 0 && sos_par_fill(a, T, &sp)) {
+      idx = (int)pars.size();
+      pars.push_back(sp);
+    }
+    return idx;
+  }
+  std::vector<int> of_chunk[2] = {std::vector<int>(kSosParMaxChunk + 1, -1), std::vector<int>(kSosParMaxChunk + 1, -1)};
+};
 
 static int fill_sos(const double* sos, int n_sections, SosArgs* a) {
   if (n_sections < 1 || n_sections > 16) return fail(MMF_ERR_UNSUPPORTED, "n_sections must be in [1, 16]");
@@ -1035,8 +1088,8 @@ struct ModspecVarlen {
   std::vector<int64_t> single;                   // clips on the fast / generic kernel
   std::vector<ModItem> items;
   bool tails = false;
-  size_t o_items = 0, o_nwin = 0, desc_bytes = 0, o_single = 0, bytes = 0;  // workspace layout (bytes: all of it)
-  std::vector<unsigned char> desc;  // the descriptors (work items, window counts): desc_bytes at the workspace start
+  DescBlob desc;  // the descriptors, at the workspace start: work items and window counts
+  size_t o_items = 0, o_nwin = 0, o_single = 0, bytes = 0;  // workspace layout (bytes: all of it)
 };
 
 // W of a batch, checking every T[i] in [0, pitch] (no plan or device needed)
@@ -1091,19 +1144,15 @@ static int modspec_varlen_route(unsigned flags, const int64_t* T_host, int64_t n
       v.items[k++] = ModItem{(int)i, (int)w0, (int)std::min<long>(r.wc, v.n_win[i] - w0), v.n_win[i]};
     }
   }
-  // workspace: work items and window counts, then the single-clip region (input rows, magnitudes)
-  v.o_items = 0;
-  v.o_nwin = align_up(v.items.size() * sizeof(ModItem), 256);
-  v.desc_bytes = v.o_nwin + (size_t)n_clips * 4;
-  v.o_single = align_up(v.desc_bytes, 256);
+  // workspace: the descriptors, then the single-clip region (input rows, magnitudes)
+  v.o_items = v.desc.put(v.items);
+  v.o_nwin = v.desc.put(v.n_win);
+  v.o_single = align_up(v.desc.size(), 256);
   size_t single_bytes = 0;
   for (int64_t i : v.single)
     single_bytes = std::max(single_bytes, align_up((size_t)n_coef * T_host[i] * 4, 256) +
                                               (want_mag ? (size_t)n_coef * v.n_win[i] * v.nb * 4 : 0));
   v.bytes = v.o_single + single_bytes;
-  v.desc.assign(v.desc_bytes, 0);
-  if (!v.items.empty()) std::memcpy(v.desc.data() + v.o_items, v.items.data(), v.items.size() * sizeof(ModItem));
-  std::memcpy(v.desc.data() + v.o_nwin, v.n_win.data(), (size_t)n_clips * 4);
   return MMF_OK;
 }
 
@@ -1117,7 +1166,7 @@ static int modspec_varlen_run(mmf_plan* plan, const ModspecVarlen& v, unsigned c
   const int64_t n_clips = v.n_clips, W = v.W;
   const int nbe = v.nbe, nb = v.nb;
   if (!dd) {
-    MMF_CUDA(cudaMemcpyAsync(base, v.desc.data(), v.desc_bytes, cudaMemcpyHostToDevice, st));
+    MMF_CUDA(cudaMemcpyAsync(base, v.desc.bytes.data(), v.desc.size(), cudaMemcpyHostToDevice, st));
     dd = base;
   }
 
@@ -1341,13 +1390,12 @@ struct ChangeVarlen {
   std::vector<int2> pidx;
   std::vector<unsigned> first_unit;
   std::vector<int64_t> fallback;  // clips on the single-clip path
-  std::vector<SosPar> pars;       // distinct chunk tables of the call (they depend on the clip's length only)
+  SosParSet tables;               // row filter (cascade 0) and output filter (cascade 1)
   int i1 = -1, i2 = -1;           // the longest batched clip's tables: they size the launches' shared memory
   size_t fsmem = 0;
-  // workspace layout (bytes: all of it)
-  size_t o_len = 0, o_tall = 0, o_tk1 = 0, o_first = 0, o_clips = 0, o_pidx = 0, o_pars = 0, desc_bytes = 0;
-  size_t o_logmel = 0, o_clipmax = 0, o_mfcc = 0, o_raw = 0, o_single = 0, bytes = 0;
-  std::vector<unsigned char> desc;  // the descriptors: desc_bytes at the workspace start
+  DescBlob desc;  // the descriptors, at the workspace start
+  size_t o_len = 0, o_tall = 0, o_tk1 = 0, o_first = 0, o_clips = 0, o_pidx = 0, o_pars = 0;
+  size_t o_logmel = 0, o_clipmax = 0, o_mfcc = 0, o_raw = 0, o_single = 0, bytes = 0;  // workspace (bytes: all of it)
 };
 
 // Routing (host only).  The lengths are in [1, 2^31 - n_fft); `index_base` is added to the clip index that a
@@ -1375,13 +1423,7 @@ static int change_varlen_route(const mmf_plan* plan, int64_t n_clips, const int6
   for (int64_t i = 0; i < n_clips; ++i) {
     v.T_all[i] = (int)mmf_num_frames(n_samples_host[i], c.n_fft, c.hop_length);
     const int padlen = std::max(sa.padlen, out_iir ? so.padlen : 0);
-    if (v.T_all[i] <= padlen) {
-      char buf[192];
-      std::snprintf(buf, sizeof(buf),
-                    "clip %lld: The length of the input vector x must be greater than padlen, which is %d.",
-                    (long long)(index_base + i), v.T_all[i] <= sa.padlen ? sa.padlen : so.padlen);
-      return fail(MMF_ERR_TOO_SHORT, buf);
-    }
+    if (v.T_all[i] <= padlen) return too_short(v.T_all[i] <= sa.padlen ? sa.padlen : so.padlen, index_base + i);
   }
 
   // route A = MFCC folded into the fused kernel, B = FP32 MFCC kernel + fused kernel
@@ -1392,21 +1434,7 @@ static int change_varlen_route(const mmf_plan* plan, int64_t n_clips, const int6
                          plan->d_dct_tc == nullptr;
   const bool batched = !plan->generic && !(c.flags & MMF_FLAG_UNFUSED_CHANGE) && (route_a || mfcc_fp32) &&
                        sa.n_sections <= kParMaxSections && (!out_iir || so.n_sections == sa.n_sections);
-  std::vector<SosPar>& pars = v.pars;
-  std::vector<int> par_of_cl[2] = {std::vector<int>(kSosParMaxChunk + 1, -1), std::vector<int>(kSosParMaxChunk + 1, -1)};
-  auto par_index = [&](int which, const SosArgs& a, long T) -> int {
-    const long L = T + 2L * a.padlen;
-    if (L > 32L * kSosParMaxChunk) return -1;
-    const int cl = (int)((L + 31) / 32) | 1;  // sos_par_fill's chunk length
-    int& idx = par_of_cl[which][cl];
-    if (idx < 0) {
-      SosPar sp;
-      if (!sos_par_fill(a, T, &sp)) return -1;
-      idx = (int)pars.size();
-      pars.push_back(sp);
-    }
-    return idx;
-  };
+  const std::vector<SosPar>& pars = v.tables.pars;
   const int unit = plan->d_mel_tc ? 128 : plan->TF;  // K1 work unit: a 128-frame block or a TF-frame tile
   v.T_k1.assign((size_t)n_clips, 0);
   v.pidx.assign((size_t)n_clips, int2{0, 0});
@@ -1419,8 +1447,8 @@ static int change_varlen_route(const mmf_plan* plan, int64_t n_clips, const int6
     bool ok = batched;
     int a = -1, b = -1;
     if (ok) {
-      a = par_index(0, sa, T);
-      b = out_iir ? par_index(1, so, T) : a;
+      a = v.tables.index(0, sa, T);
+      b = out_iir ? v.tables.index(1, so, T) : a;
       ok = a >= 0 && b >= 0;
     }
     size_t sm = 0;
@@ -1450,24 +1478,18 @@ static int change_varlen_route(const mmf_plan* plan, int64_t n_clips, const int6
   // workspace: descriptors, then the batched intermediates, then the single-clip region
   const size_t n = (size_t)n_clips;
   const int pitch = v.pitch;
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    const size_t o = off;
-    off += align_up(bytes, 256);
-    return o;
-  };
-  v.o_len = take(n * 8);
-  v.o_tall = take(n * 4);
-  v.o_tk1 = take(n * 4);
-  v.o_first = take((n + 1) * 4);
-  v.o_clips = take(std::max<size_t>(1, v.clips.size()) * 4);
-  v.o_pidx = take(n * 8);
-  v.o_pars = take(std::max<size_t>(1, pars.size()) * sizeof(SosPar));
-  v.desc_bytes = off;
-  v.o_logmel = (nv && !want_logmel) ? take(n * c.n_mels * pitch * 4) : 0;
-  v.o_clipmax = take(n * 4);
-  v.o_mfcc = (nv && !route_a && !want_mfcc) ? take(n * c.n_mfcc * pitch * 4) : 0;
-  v.o_raw = v.split_out ? take(n * pitch * 8) : 0;
+  v.o_len = v.desc.put(v.len);
+  v.o_tall = v.desc.put(v.T_all);
+  v.o_tk1 = v.desc.put(v.T_k1);
+  v.o_first = v.desc.put(v.first_unit);
+  v.o_clips = v.desc.put(v.clips);
+  v.o_pidx = v.desc.put(v.pidx);
+  v.o_pars = v.desc.put(pars);
+  size_t off = align_up(v.desc.size(), 256);
+  v.o_logmel = (nv && !want_logmel) ? ws_take(off, n * c.n_mels * pitch * 4) : 0;
+  v.o_clipmax = ws_take(off, n * 4);
+  v.o_mfcc = (nv && !route_a && !want_mfcc) ? ws_take(off, n * c.n_mfcc * pitch * 4) : 0;
+  v.o_raw = v.split_out ? ws_take(off, n * pitch * 8) : 0;
   v.o_single = off;
   size_t single_bytes = 0;
   for (int64_t i : v.fallback) {
@@ -1479,14 +1501,6 @@ static int change_varlen_route(const mmf_plan* plan, int64_t n_clips, const int6
     single_bytes = std::max(single_bytes, b);
   }
   v.bytes = v.o_single + single_bytes;
-  v.desc.assign(v.desc_bytes, 0);
-  std::memcpy(v.desc.data() + v.o_len, v.len.data(), n * 8);
-  std::memcpy(v.desc.data() + v.o_tall, v.T_all.data(), n * 4);
-  std::memcpy(v.desc.data() + v.o_tk1, v.T_k1.data(), n * 4);
-  std::memcpy(v.desc.data() + v.o_first, v.first_unit.data(), (n + 1) * 4);
-  if (nv) std::memcpy(v.desc.data() + v.o_clips, v.clips.data(), v.clips.size() * 4);
-  std::memcpy(v.desc.data() + v.o_pidx, v.pidx.data(), n * 8);
-  if (!pars.empty()) std::memcpy(v.desc.data() + v.o_pars, pars.data(), pars.size() * sizeof(SosPar));
   return MMF_OK;
 }
 
@@ -1503,7 +1517,7 @@ static int change_varlen_run(mmf_plan* plan, const ChangeVarlen& v, unsigned cha
   const int64_t nv = (int64_t)v.clips.size();
   int rc;
   if (!dd) {
-    MMF_CUDA(cudaMemcpyAsync(base, v.desc.data(), v.desc_bytes, cudaMemcpyHostToDevice, st));
+    MMF_CUDA(cudaMemcpyAsync(base, v.desc.bytes.data(), v.desc.size(), cudaMemcpyHostToDevice, st));
     dd = base;
   }
   const int* d_tall = (const int*)(dd + v.o_tall);
@@ -1521,8 +1535,8 @@ static int change_varlen_run(mmf_plan* plan, const ChangeVarlen& v, unsigned cha
                           (const int2*)(dd + v.o_pidx)};
     const int clamp = logmel_dev ? 1 : 0;
     double* raw = v.split_out ? (double*)(base + v.o_raw) : nullptr;
-    const SosPar& pa = v.pars[v.i1];
-    const SosPar& po = v.pars[v.i2];
+    const SosPar& pa = v.tables.pars[v.i1];
+    const SosPar& po = v.tables.pars[v.i2];
     cudaError_t e;
     if (v.route_a) {
       const FusedMfccArgs lm{plan->d_dct, plan->nc_pad, logmel, clipmax, c.n_mels, c.top_db, mfcc_dev, delta_dev, clamp};
@@ -1611,6 +1625,29 @@ int mmf_mfcc_change_varlen(mmf_plan* plan, const float* pcm_dev, int64_t n_clips
 
 }  // extern "C"
 
+namespace mmf {
+
+// Chunk budget of the host-buffer calls, in bytes of float32 PCM on the device, from a sweep on B200 (bench e2e legs,
+// 1024 x 10 s clips): float32 host input 8 / 16 / 24 / 32 / 48 / 96 MB -> 0.68 / 0.81 / 0.82 / 0.82 / 0.81 / 0.80 M
+// audio-s/s (small chunks pay launch + copy set-up, large ones a longer unoverlapped head and tail); int16 host input
+// moves half the bytes per clip and keeps gaining up to 96 MB (0.94 / 1.16 / 1.25 / 1.34 / 1.37 / 1.44 M)
+constexpr size_t kHostChunkF32 = 32u << 20, kHostChunkI16 = 96u << 20;
+
+// Runs `body`, which queues work on both plan streams, then drains both streams whatever it returned: queued copies
+// target caller-owned host buffers.  The body's error comes first.
+template <typename Body>
+static int run_and_drain(mmf_plan* plan, Body&& body) {
+  const int rc = body();
+  const cudaError_t e0 = cudaStreamSynchronize(plan->streams[0]);
+  const cudaError_t e1 = cudaStreamSynchronize(plan->streams[1]);
+  if (rc) return rc;
+  if (e0 != cudaSuccess) return cuda_fail(e0, "host path, stream 0");
+  if (e1 != cudaSuccess) return cuda_fail(e1, "host path, stream 1");
+  return MMF_OK;
+}
+
+}  // namespace mmf
+
 // pcm_host: float32 samples, or (pcm16 != 0) int16 samples converted on the device
 static int features_host_impl(mmf_plan* plan, const void* pcm_host_v, int pcm16, int64_t n_clips, int64_t n_samples,
                               int64_t clip_stride, const mmf_change_params* prm, const mmf_modspec_params* mod,
@@ -1639,11 +1676,7 @@ static int features_host_impl(mmf_plan* plan, const void* pcm_host_v, int pcm16,
   const bool need_mfcc_dev = mfcc_host || want_mod;
   // chunk the batch so that H2D of chunk i+1 overlaps compute of chunk i (two streams, two slots)
   const size_t clip_bytes = (size_t)n_samples * 4;
-  // chunk size in bytes of float32 PCM on the device, from a sweep on B200 (bench e2e legs, 1024 x 10 s clips):
-  // float32 host input 8 / 16 / 24 / 32 / 48 / 96 MB -> 0.68 / 0.81 / 0.82 / 0.82 / 0.81 / 0.80 M audio-s/s (small
-  // chunks pay launch + copy set-up, large ones a longer unoverlapped head and tail); int16 host input moves half
-  // the bytes per clip and keeps gaining up to 96 MB (0.94 / 1.16 / 1.25 / 1.34 / 1.37 / 1.44 M)
-  const size_t chunk_bytes = pcm16 ? (96u << 20) : (32u << 20);
+  const size_t chunk_bytes = pcm16 ? kHostChunkI16 : kHostChunkF32;
   int64_t chunk = std::max<int64_t>(1, (int64_t)(chunk_bytes / clip_bytes));
   chunk = std::min<int64_t>(chunk, n_clips);
   const size_t pcm_slot = align_up((size_t)chunk * n_samples * 4, 256);
@@ -1661,28 +1694,20 @@ static int features_host_impl(mmf_plan* plan, const void* pcm_host_v, int pcm16,
   if (want_mod && n_win > 0 &&
       (rc = ensure_mod_tables(plan, mod->win, mod->nfft, mod->band_lo, mod->band_hi, band_host ? mod->n_bands : 0)))
     return rc;
-  // every exit below drains both streams: queued copies target caller-owned host buffers
-  auto body = [&]() -> int {
+  return run_and_drain(plan, [&]() -> int {
   int64_t done = 0;
   for (int i = 0; done < n_clips; ++i, done += chunk) {
     const int s = i & 1;
     const int64_t nc = std::min<int64_t>(chunk, n_clips - done);
     cudaStream_t st = plan->streams[s];
-    unsigned char* cur = (unsigned char*)plan->host_ws + (64 << 10) + (size_t)s * slot;
-    float* d_pcm = (float*)cur;
-    cur += pcm_slot;
-    int16_t* d_raw = pcm16 ? (int16_t*)cur : nullptr;
-    cur += raw_slot;
-    double* d_tot = (double*)cur;
-    cur += tot_slot;
-    float* d_mfcc = need_mfcc_dev ? (float*)cur : nullptr;
-    cur += mfcc_slot;
-    float* d_delta = delta_host ? (float*)cur : nullptr;
-    cur += delta_slot;
-    float* d_mag = mag_slot ? (float*)cur : nullptr;
-    cur += mag_slot;
-    float* d_band = band_slot ? (float*)cur : nullptr;
-    cur += band_slot;
+    unsigned char* cur = (unsigned char*)plan->host_ws + (64 << 10) + (size_t)s * slot;  // (unused: size 0)
+    float* d_pcm = (float*)carve(cur, pcm_slot);
+    int16_t* d_raw = (int16_t*)carve(cur, raw_slot);
+    double* d_tot = (double*)carve(cur, tot_slot);
+    float* d_mfcc = need_mfcc_dev ? (float*)carve(cur, mfcc_slot) : nullptr;
+    float* d_delta = delta_host ? (float*)carve(cur, delta_slot) : nullptr;
+    float* d_mag = mag_slot ? (float*)carve(cur, mag_slot) : nullptr;
+    float* d_band = band_slot ? (float*)carve(cur, band_slot) : nullptr;
     // stream order serialises reuse of slot s (chunk i-2 ran on the same stream)
     if (pcm16) {
       if (clip_stride == n_samples) {
@@ -1726,14 +1751,7 @@ static int features_host_impl(mmf_plan* plan, const void* pcm_host_v, int pcm16,
                                (size_t)nc * n_win * mod->n_bands * 4, cudaMemcpyDeviceToHost, st));
   }
   return MMF_OK;
-  };
-  rc = body();
-  const cudaError_t e0 = cudaStreamSynchronize(plan->streams[0]);
-  const cudaError_t e1 = cudaStreamSynchronize(plan->streams[1]);
-  if (rc) return rc;
-  if (e0 != cudaSuccess) return cuda_fail(e0, "host path, stream 0");
-  if (e1 != cudaSuccess) return cuda_fail(e1, "host path, stream 1");
-  return MMF_OK;
+  });
 }
 
 namespace mmf {
@@ -1757,9 +1775,10 @@ static int validate_offsets(int64_t n_clips, const int64_t* offsets) {
 }
 
 // Resampling descriptors of a packed batch (mmf_features_host_varlen_resampled, mmf_resample_varlen), after the
-// offsets passed validate_offsets; no plan or device needed.  Taps are checked only for the clips that read them.
+// offsets passed validate_offsets; no plan or device needed.  Taps are checked only for the clips that read them;
+// *n_taps (0 on entry) becomes n_h when some clip does.
 static int validate_resample(int64_t n_clips, const int64_t* offsets, const mmf_resample_clip* rs, const float* h,
-                             int64_t n_h) {
+                             int64_t n_h, int64_t* n_taps) {
   if (!rs) return fail(MMF_ERR_INVALID, "rs_host is NULL");
   for (int64_t i = 0; i < n_clips; ++i) {
     const mmf_resample_clip& r = rs[i];
@@ -1777,6 +1796,7 @@ static int validate_resample(int64_t n_clips, const int64_t* offsets, const mmf_
     if (r.n_out != (int64_t)((num + r.down - 1) / r.down))
       return bad(copy ? "a clip at the plan's rate needs n_out = its length" : "n_out must be ceil(len * up / down)");
     if (copy) continue;
+    *n_taps = n_h;
     if (r.len_h < 1 || r.len_h > (1 << 22)) return bad("len_h must be in [1, 2^22]");
     if (!h || r.tap0 < 0 || r.tap0 > n_h - r.len_h) return bad("taps [tap0, tap0 + len_h) must lie in the tap table");
     if (r.n_pre_remove < 0) return bad("n_pre_remove must be >= 0");
@@ -1784,40 +1804,28 @@ static int validate_resample(int64_t n_clips, const int64_t* offsets, const mmf_
   return MMF_OK;
 }
 
-// Device descriptors of clips [c0, c1) of a packed batch for resample_rows_launch: RsClip[nc], then first_item[nc + 1],
-// appended to `desc` (16-byte aligned parts).  Sources count from `base`; rs == NULL: every clip at the plan's rate.
-// Returns the number of work items, or -1 past 2^31 - 1.
-static int64_t resample_desc(int64_t c0, int64_t c1, const int64_t* offsets, int64_t base,
-                             const mmf_resample_clip* rs, std::vector<unsigned char>& desc, size_t& o_clips,
-                             size_t& o_first) {
+// Descriptors of clips [c0, c1) of a packed batch for resample_rows_launch, appended to `desc`.  Sources count from
+// `base`; rs == NULL: every clip at the plan's rate.
+static RaggedParts resample_desc(int64_t c0, int64_t c1, const int64_t* offsets, int64_t base,
+                                 const mmf_resample_clip* rs, DescBlob& desc) {
   const int64_t nc = c1 - c0;
-  o_clips = align_up(desc.size(), 16);
-  o_first = align_up(o_clips + (size_t)nc * sizeof(RsClip), 16);
-  desc.resize(align_up(o_first + (size_t)(nc + 1) * 4, 16), 0);
-  RsClip* cl = (RsClip*)(desc.data() + o_clips);
-  unsigned* first = (unsigned*)(desc.data() + o_first);
+  std::vector<RsClip> cl((size_t)nc);
+  std::vector<unsigned> first((size_t)nc + 1);
   int64_t items = 0;
   for (int64_t k = 0; k < nc; ++k) {
     const int64_t i = c0 + k, len = offsets[i + 1] - offsets[i];
-    RsClip r{};
-    r.src = (long)(offsets[i] - base);
-    r.n_in = (long)len;
-    r.copy = !rs || (rs[i].up == 1 && rs[i].down == 1);
-    r.n_out = (long)(r.copy ? len : rs[i].n_out);
-    if (!r.copy) {
-      r.up = rs[i].up;
-      r.down = rs[i].down;
-      r.len_h = rs[i].len_h;
-      r.n_pre_remove = (long)rs[i].n_pre_remove;
-      r.tap0 = (long)rs[i].tap0;
-    }
-    cl[k] = r;
+    const long src = (long)(offsets[i] - base);
+    if (!rs || (rs[i].up == 1 && rs[i].down == 1))
+      cl[k] = RsClip{src, (long)len, 0, (long)len, 0, 0, 0, 0, 1};
+    else
+      cl[k] = RsClip{src, (long)len, (long)rs[i].n_pre_remove, (long)rs[i].n_out, (long)rs[i].tap0, rs[i].up,
+                     rs[i].down, rs[i].len_h, 0};
     first[k] = (unsigned)items;
-    items += (r.n_out + kRsOut - 1) / kRsOut;
-    if (items > 0x7fffffffLL) return -1;
+    items += (cl[k].n_out + kRsOut - 1) / kRsOut;
+    if (items > 0x7fffffffLL) return RaggedParts{0, 0, -1};
   }
   first[nc] = (unsigned)items;
-  return items;
+  return RaggedParts{desc.put(cl), desc.put(first), items};
 }
 
 // RMS-envelope geometry of a packed batch (mmf_amp_varlen_sizes, calc.py:326-331), after the offsets passed
@@ -1844,30 +1852,120 @@ static int amp_sizes(int64_t n_clips, const int64_t* offsets, const int32_t* geo
   return MMF_OK;
 }
 
-// Device descriptors of clips [c0, c1) of a packed batch for rms_varlen_launch: RmsClip[nc], then first_item[nc + 1],
-// appended to `desc` (16-byte aligned parts).  Sources count from `base`, outputs from amp_off[c0].  Returns the number
-// of work items, or -1 past 2^31 - 1.
-static int64_t rms_desc(int64_t c0, int64_t c1, const int64_t* offsets, int64_t base, const int32_t* geom, int center,
-                        const int64_t* amp_off, std::vector<unsigned char>& desc, size_t& o_clips, size_t& o_first) {
+// Host half of a ragged RMS envelope (mmf_rms_varlen, the envelope of the host bundle): the descriptors of the
+// envelope launch and, with an output filter, each envelope's route -- that of its own mmf_sosfiltfilt call: the
+// chunk-parallel kernel when it takes the envelope's length (all of them in one launch, each with the tables of its
+// own chunk length), the single-row routes otherwise.
+struct EnvelopeVarlen {
+  int64_t n_clips = 0;
+  std::vector<int64_t> off;       // envelope k: frames [off[k], off[k + 1]) of the output
+  const SosArgs* filt = nullptr;  // the output filter (null: none)
+  SosParSet tables;
+  int amax = -1;                  // the widest tables: they size the batched filter's launch
+  std::vector<int> par;           // envelopes on the chunk-parallel route
+  std::vector<int64_t> single;    // the others
+  DescBlob desc;
+  RaggedParts rms;                                               // the envelope launch (RmsClip)
+  size_t o_par = 0, o_T = 0, o_pidx = 0, o_off = 0, o_pars = 0;  // the batched filter (FusedVarlen)
+};
+
+// Routing of clips [c0, c1) of a packed batch whose amp_sizes are amp_off (host only).  Sources count from `base`,
+// outputs from amp_off[c0].  Returns the number of envelope work items, -1 past 2^31 - 1.
+static int64_t envelope_route(int64_t c0, int64_t c1, const int64_t* offsets, int64_t base, const int32_t* geom,
+                              int center, const int64_t* amp_off, const SosArgs* filt, EnvelopeVarlen& v) {
   const int64_t nc = c1 - c0;
-  o_clips = align_up(desc.size(), 16);
-  o_first = align_up(o_clips + (size_t)nc * sizeof(RmsClip), 16);
-  desc.resize(align_up(o_first + (size_t)(nc + 1) * 4, 16), 0);
-  RmsClip* cl = (RmsClip*)(desc.data() + o_clips);
-  unsigned* first = (unsigned*)(desc.data() + o_first);
+  v.n_clips = nc;
+  v.filt = filt;
+  v.off.resize((size_t)nc + 1);
+  std::vector<RmsClip> cl((size_t)nc);
+  std::vector<unsigned> first((size_t)nc + 1);
   int64_t items = 0;
   for (int64_t k = 0; k < nc; ++k) {
     const int64_t i = c0 + k;
     const int fl = geom[2 * i], hop = geom[2 * i + 1];
-    const RmsClip r{(long)(offsets[i] - base), (long)(offsets[i + 1] - offsets[i]), (long)(amp_off[i] - amp_off[c0]),
+    v.off[k] = amp_off[i] - amp_off[c0];
+    cl[k] = RmsClip{(long)(offsets[i] - base), (long)(offsets[i + 1] - offsets[i]), (long)v.off[k],
                     (long)(amp_off[i + 1] - amp_off[i]), fl, hop, center ? fl / 2 : 0, rms_frames_per_item(fl, hop)};
-    cl[k] = r;
     first[k] = (unsigned)items;
-    items += (r.T + r.F - 1) / r.F;
+    items += (cl[k].T + cl[k].F - 1) / cl[k].F;
     if (items > 0x7fffffffLL) return -1;
   }
   first[nc] = (unsigned)items;
+  v.off[nc] = amp_off[c1] - amp_off[c0];
+  v.rms = RaggedParts{v.desc.put(cl), v.desc.put(first), items};
+  if (!filt) return items;
+  std::vector<int> T((size_t)nc);
+  std::vector<int2> pidx((size_t)nc, int2{0, 0});
+  for (int64_t k = 0; k < nc; ++k) {
+    const int64_t Tk = v.off[k + 1] - v.off[k];
+    T[k] = (int)std::min<int64_t>(Tk, 0x7fffffff);
+    const int idx = v.tables.index(0, *filt, (long)Tk);
+    if (idx < 0) {
+      v.single.push_back(k);
+      continue;
+    }
+    if (v.amax < 0 || v.tables.pars[idx].CL > v.tables.pars[v.amax].CL) v.amax = idx;
+    pidx[k] = int2{idx, idx};
+    v.par.push_back((int)k);
+  }
+  v.o_par = v.desc.put(v.par);
+  v.o_T = v.desc.put(T);
+  v.o_pidx = v.desc.put(pidx);
+  v.o_off = v.desc.put(v.off.data(), (size_t)nc);
+  v.o_pars = v.desc.put(v.tables.pars);
   return items;
+}
+
+// Device half: the envelope launch over x (float32, or int16 when pcm16) into amp and, with the output filter, the
+// batched filter launch and the single-row filters into amp_filt, all on `st`.  dd: v.desc on the device.
+static int envelope_run(const EnvelopeVarlen& v, const unsigned char* dd, const void* x, int pcm16, float* amp,
+                        double* amp_filt, cudaStream_t st) {
+  cudaError_t e = rms_varlen_launch(x, pcm16, (const RmsClip*)(dd + v.rms.clips), (const unsigned*)(dd + v.rms.first),
+                                    (long)v.n_clips, (long)v.rms.items, amp, st);
+  if (e != cudaSuccess) return cuda_fail(e, "rms_varlen_kernel launch");
+  if (amp_filt && !v.par.empty()) {
+    const FusedVarlen fvl{(const int*)(dd + v.o_par), (const int*)(dd + v.o_T), (const SosPar*)(dd + v.o_pars),
+                          (const int2*)(dd + v.o_pidx), (const long*)(dd + v.o_off)};
+    e = sosfiltfilt_par_varlen_launch(amp, 1, (long)v.par.size(), 0, v.tables.pars[v.amax], fvl, amp_filt, st);
+    if (e != cudaSuccess) return cuda_fail(e, "sosfiltfilt_par_kernel (envelopes) launch");
+  }
+  for (int64_t k : v.single) {
+    const int64_t a0 = v.off[k], Tk = v.off[k + 1] - v.off[k];
+    e = sosfiltfilt_any(amp + a0, 1, 1, (long)Tk, (long)Tk, 1, 0, *v.filt, amp_filt + a0, (long)Tk, st);
+    if (e != cudaSuccess) return cuda_fail(e, "sosfiltfilt (envelope)");
+  }
+  return MMF_OK;
+}
+
+// Uploads `desc` to stream-ordered scratch on `st` and runs launch(its device address) there; the scratch is freed in
+// stream order after it.  (A pageable source: the copy is staged, so the host blob may go when this returns.)
+template <typename Launch>
+static int run_uploaded(mmf_plan* plan, const DescBlob& desc, cudaStream_t st, Launch&& launch) {
+  MMF_CUDA(cudaSetDevice(plan->cfg.device));
+  unsigned char* d = nullptr;
+  MMF_CUDA(cudaMallocAsync((void**)&d, desc.size(), st));
+  const cudaError_t e = cudaMemcpyAsync(d, desc.bytes.data(), desc.size(), cudaMemcpyHostToDevice, st);
+  const int rc = e != cudaSuccess ? cuda_fail(e, "descriptor upload") : launch((const unsigned char*)d);
+  cudaFreeAsync(d, st);
+  return rc;
+}
+
+// One ragged RMS launch on `st` over float32 x from the host descriptors of v (no output filter)
+static int rms_run(mmf_plan* plan, const float* x, const EnvelopeVarlen& v, float* out, cudaStream_t st) {
+  return run_uploaded(plan, v.desc, st,
+                      [&](const unsigned char* d) { return envelope_run(v, d, x, 0, out, nullptr, st); });
+}
+
+// One ragged resampling launch on `st`: the descriptors at p of `desc`, which takes the taps h[n_h]
+static int resample_dev(mmf_plan* plan, const float* x_dev, DescBlob& desc, const RaggedParts& p, const float* h,
+                        int64_t n_h, int64_t n_clips, float* y_dev, int64_t y_stride, cudaStream_t st) {
+  const size_t o_h = desc.put(h, (size_t)n_h);
+  return run_uploaded(plan, desc, st, [&](const unsigned char* d) {
+    const cudaError_t e = resample_rows_launch(x_dev, 0, (const RsClip*)(d + p.clips), (const unsigned*)(d + p.first),
+                                               (long)n_clips, (long)p.items, (const float*)(d + o_h), y_dev,
+                                               (long)y_stride, st);
+    return e == cudaSuccess ? MMF_OK : cuda_fail(e, "resample_rows_kernel launch");
+  });
 }
 
 // frame_off / win_off of a packed batch (mmf_features_varlen_sizes); n_win_i = 0 without modulation windows
@@ -1881,385 +1979,288 @@ static void packed_sizes(int n_fft, int hop, int win, int mod_hop, int64_t n_cli
   }
 }
 
-// One chunk of a packed host-buffer batch: a run of consecutive clips, its routing, and where its buffers sit in its
-// slot of the host-path workspace (byte offsets from the slot's start).
-struct HostChunk {
-  int64_t c0, c1;  // clips [c0, c1)
-  int64_t stride;  // samples per staged row: the chunk's longest clip, rounded up to 16 bytes for the TMA
-  ChangeVarlen cv;
-  ModspecVarlen mv;  // routed when the chunk has modulation windows (mv.W > 0)
-  int64_t items;   // staging work items (resample_rows_launch)
-  std::vector<unsigned char> desc;  // staging and compaction descriptors
-  size_t o_rs, o_first, o_cnt_t, o_off_t, o_cnt_w, o_off_w;  // within desc
-  size_t o_desc, o_cv_desc, o_mv_desc;  // desc, cv.desc and mv.desc in the descriptor region of the call
-  size_t o_h2d, o_pcm, o_tot, o_mfcc, o_delta, o_mag, o_band, o_ptot, o_pmfcc, o_pdelta, o_pmag, o_pband,
-      o_scratch, end;
-  // the amplitude envelope (when requested): its launch's work items and descriptors, and the output filter's: the
-  // envelopes on the chunk-parallel route (FusedVarlen parts in desc, amax = their widest tables) and the others
-  int64_t amp_items = 0, amp_np = 0;
-  std::vector<int64_t> amp_single;
-  SosPar amax;
-  size_t o_acl, o_afirst, o_fclips, o_fT, o_fpidx, o_foff, o_fpars;  // within desc
-  size_t o_amp, o_ampf;                                                // in the slot
+// A packed host-buffer call: the arguments of the packed entry points in their order, then what the host-only checks
+// derive from them.  pcm: float32 samples, or (pcm16 != 0) int16 samples converted on the device.  resampled: clip i
+// reaches the plan's rate as rs[i] says, with taps from h_taps[n_h]; otherwise every clip is at the plan's rate.
+// amp_prm: the RMS envelope of each clip's native samples, frame geometry geom[2i], geom[2i + 1], to amp and / or,
+// through the output filter, amp_filt (NULL: none, and exactly the launches and copies of the call without it).
+struct PackedBatch {
+  const void* pcm;
+  int pcm16;
+  int64_t n_clips;
+  const int64_t* offsets;
+  const mmf_resample_clip* rs;
+  const float* h_taps;
+  int64_t n_h;
+  const mmf_change_params* prm;
+  const mmf_modspec_params* mod;
+  const mmf_amp_params* amp_prm;
+  const int32_t* geom;
+  double* tot;
+  float *mfcc, *delta, *mag, *band;
+  float* amp = nullptr;
+  double* amp_filt = nullptr;
+  bool resampled = false;
+  size_t isz = pcm16 ? 2 : 4;  // bytes per sample as they cross PCIe
+  // from the checks
+  int64_t n_taps = 0;  // taps that go up with the descriptors: none unless some clip reads them
+  bool want_mod = false, want_amp = false, need_mfcc_dev = false;
+  int nb = 0, nbe = 0;  // modulation bins per window; band outputs actually written
+  SosArgs amp_sos;      // the envelopes' output filter (amp_filt)
+  // len: samples at the plan's rate (what the ragged path sees); T: frames.  F, Wo, A [n_clips + 1]: packed offsets
+  // of frames, modulation windows and envelope frames
+  std::vector<int64_t> len, T, F, Wo, A;
 };
 
-// pcm_host: float32 samples, or (pcm16 != 0) int16 samples converted on the device.  resampled: clip i reaches the
-// plan's rate as rs[i] says, with taps from h[n_h]; otherwise every clip is at the plan's rate.  amp: the RMS envelope
-// of each clip's native samples, frame geometry geom[2i], geom[2i + 1], to amp_host and / or, through the output
-// filter, amp_filt_host (NULL: none, and exactly the launches and copies of the call without it).
-static int features_host_varlen_impl(mmf_plan* plan, const void* pcm_host_v, int pcm16, int64_t n_clips,
-                                     const int64_t* offsets, bool resampled, const mmf_resample_clip* rs,
-                                     const float* h_taps, int64_t n_h, const mmf_change_params* prm,
-                                     const mmf_modspec_params* mod, double* tot_host, float* mfcc_host,
-                                     float* delta_host, float* mag_host, float* band_host,
-                                     const mmf_amp_params* amp = nullptr, const int32_t* geom = nullptr,
-                                     float* amp_host = nullptr, double* amp_filt_host = nullptr) {
-  int rc = validate_offsets(n_clips, offsets);
+// Byte offsets of a chunk's buffers in its slot of the host-path workspace, in the order they are laid out
+struct HostSlot {
+  size_t h2d = 0, pcm = 0, tot = 0, mfcc = 0, delta = 0, mag = 0, band = 0;
+  size_t ptot = 0, pmfcc = 0, pdelta = 0, pmag = 0, pband = 0, scratch = 0, amp = 0, amp_filt = 0, end = 0;
+};
+
+// per-clip row lengths (int) and packed offsets (long) of a compaction, in the call's descriptors
+struct PackedRows {
+  size_t cnt = 0, off = 0;
+};
+
+// One chunk of a packed host-buffer batch: a run of consecutive clips, its routed stages and its slot
+struct HostChunk {
+  // clips [c0, c1); stride: samples per staged row, the chunk's longest clip rounded up to 16 bytes for the TMA
+  int64_t c0 = 0, c1 = 0, stride = 0;
+  RaggedParts stage;       // the staging launch (resample_rows_launch)
+  PackedRows frames, wins;  // compaction of the per-frame and the per-window outputs
+  ChangeVarlen cv;
+  ModspecVarlen mv;    // routed when the chunk has modulation windows (mv.W > 0)
+  EnvelopeVarlen env;  // routed when the envelope is requested
+  size_t o_cv = 0, o_mv = 0, o_env = 0;  // cv.desc, mv.desc and env.desc in the call's descriptors
+  HostSlot slot;
+};
+
+// Stage 1 (host only): the checks that precede routing, in the order the callers see them, and the packed sizes
+static int packed_check(const mmf_plan* plan, PackedBatch& b) {
+  const mmf_amp_params* amp = b.amp_prm;
+  int rc = validate_offsets(b.n_clips, b.offsets);
   if (rc) return rc;
-  if (resampled && (rc = validate_resample(n_clips, offsets, rs, h_taps, n_h))) return rc;
-  if (!amp && (amp_host || amp_filt_host))
-    return fail(MMF_ERR_INVALID, "amplitude outputs requested without parameters");
-  const bool want_amp = amp && (amp_host || amp_filt_host);
-  std::vector<int64_t> A;  // envelope offsets (amp_sizes)
-  SosArgs so_amp;
-  if (want_amp) {
-    A.resize((size_t)n_clips + 1);
-    if ((rc = amp_sizes(n_clips, offsets, geom, amp->center, A.data()))) return rc;
-    if (amp_filt_host) {
+  if (b.resampled && (rc = validate_resample(b.n_clips, b.offsets, b.rs, b.h_taps, b.n_h, &b.n_taps))) return rc;
+  if (!amp && (b.amp || b.amp_filt)) return fail(MMF_ERR_INVALID, "amplitude outputs requested without parameters");
+  const size_t n = (size_t)b.n_clips;
+  b.want_amp = amp && (b.amp || b.amp_filt);
+  if (b.want_amp) {
+    b.A.resize(n + 1);
+    if ((rc = amp_sizes(b.n_clips, b.offsets, b.geom, amp->center, b.A.data()))) return rc;
+    if (b.amp_filt) {
       if (amp->out_n_sections < 1) return fail(MMF_ERR_INVALID, "amp_filt_host needs out_n_sections >= 1");
-      if ((rc = fill_sos(amp->out_sos, amp->out_n_sections, &so_amp))) return rc;
-      for (int64_t i = 0; i < n_clips; ++i)
-        if (A[i + 1] - A[i] <= so_amp.padlen) {
-          char buf[192];
-          std::snprintf(buf, sizeof(buf),
-                        "clip %lld: The length of the input vector x must be greater than padlen, which is %d.",
-                        (long long)i, so_amp.padlen);
-          return fail(MMF_ERR_TOO_SHORT, buf);
-        }
+      if ((rc = fill_sos(amp->out_sos, amp->out_n_sections, &b.amp_sos))) return rc;
+      for (size_t i = 0; i < n; ++i)
+        if (b.A[i + 1] - b.A[i] <= b.amp_sos.padlen) return too_short(b.amp_sos.padlen, (int64_t)i);
     }
   }
-  if (!plan || !pcm_host_v || !prm || !tot_host) return fail(MMF_ERR_INVALID, "NULL argument");
-  if ((mag_host || band_host) && !mod) return fail(MMF_ERR_INVALID, "modulation outputs requested without parameters");
-  const mmf_config& c = plan->cfg;
-  const bool want_mod = mod && (mag_host || band_host) && mod->win > 0;
-  if (want_mod && (rc = validate_modspec(mod->win, mod->hop, mod->nfft, mod->n_bands, mod->band_lo, mod->band_hi,
-                                         band_host != nullptr)))
+  if (!plan || !b.pcm || !b.prm || !b.tot) return fail(MMF_ERR_INVALID, "NULL argument");
+  if ((b.mag || b.band) && !b.mod) return fail(MMF_ERR_INVALID, "modulation outputs requested without parameters");
+  const mmf_modspec_params* mod = b.mod;
+  b.want_mod = mod && (b.mag || b.band) && mod->win > 0;
+  if (b.want_mod && (rc = validate_modspec(mod->win, mod->hop, mod->nfft, mod->n_bands, mod->band_lo, mod->band_hi,
+                                           b.band != nullptr)))
     return rc;
-  const int nm = c.n_mfcc;
-  const int nb = want_mod ? mod->nfft / 2 + 1 : 0;
-  const int nbe = want_mod && band_host ? mod->n_bands : 0;  // band outputs actually written
-  const bool need_mfcc_dev = mfcc_host || want_mod;
-  const size_t n = (size_t)n_clips;
-  // len_in: samples as they cross PCIe; len: samples at the plan's rate (what the ragged path sees)
-  std::vector<int64_t> len_in(n), len(n), out_off(n + 1, 0), T(n), F(n + 1), Wo(n + 1);
+  b.nb = b.want_mod ? mod->nfft / 2 + 1 : 0;
+  b.nbe = b.want_mod && b.band ? mod->n_bands : 0;
+  b.need_mfcc_dev = b.mfcc || b.want_mod;
+  b.len = b.T = std::vector<int64_t>(n);
+  b.F = b.Wo = std::vector<int64_t>(n + 1);
+  std::vector<int64_t> out_off(n + 1, 0);
   for (size_t i = 0; i < n; ++i) {
-    len_in[i] = offsets[i + 1] - offsets[i];
-    len[i] = rs ? rs[i].n_out : len_in[i];
-    out_off[i + 1] = out_off[i] + len[i];
+    b.len[i] = b.rs ? b.rs[i].n_out : b.offsets[i + 1] - b.offsets[i];
+    out_off[i + 1] = out_off[i] + b.len[i];
   }
-  packed_sizes(c.n_fft, c.hop_length, want_mod ? mod->win : 0, want_mod ? mod->hop : 1, n_clips, out_off.data(),
-               F.data(), Wo.data());
-  for (size_t i = 0; i < n; ++i) T[i] = F[i + 1] - F[i];
-  // the tap table goes up with the descriptors when some clip reads it
-  int64_t n_taps = 0;
-  for (size_t i = 0; rs && i < n; ++i) n_taps = (rs[i].up == 1 && rs[i].down == 1) ? n_taps : n_h;
+  packed_sizes(plan->cfg.n_fft, plan->cfg.hop_length, b.want_mod ? mod->win : 0, b.want_mod ? mod->hop : 1, b.n_clips,
+               out_off.data(), b.F.data(), b.Wo.data());
+  for (size_t i = 0; i < n; ++i) b.T[i] = b.F[i + 1] - b.F[i];
+  return MMF_OK;
+}
 
-  // ---- chunks, planned and routed before anything is queued.  Budgets in bytes of float32 samples, those of
-  // features_host_impl (from its sweep): the samples of a chunk as they cross PCIe, and its staged rows at the plan's
-  // rate at twice that, so that one long clip among short ones cannot inflate the padded intermediates.  A clip over
-  // either budget is a chunk alone.
-  const int64_t budget = pcm16 ? (96 << 20) : (32 << 20);
-  const size_t isz = pcm16 ? 2 : 4;
-  std::vector<HostChunk> chunks;
-  // the descriptor region: the taps, then each chunk's descriptors
-  size_t slot = 0, desc_bytes = align_up((size_t)n_taps * 4, 256);
-  for (int64_t c0 = 0; c0 < n_clips;) {
-    int64_t c1 = c0 + 1, real = len_in[c0], n_max = len[c0];
+// A chunk's routing, with every check in stage order, and its staging and compaction descriptors, appended to the
+// call's
+static int route_chunk(const mmf_plan* plan, const PackedBatch& b, HostChunk& h, DescBlob& desc) {
+  const int64_t c0 = h.c0, c1 = h.c1, nc = c1 - c0;
+  int rc = change_varlen_route(plan, nc, b.len.data() + c0, b.prm, false, b.need_mfcc_dev, b.delta != nullptr, c0,
+                               h.cv);
+  if (rc) return rc;
+  int64_t W = 0;
+  for (int64_t i = c0; i < c1; ++i) W = std::max(W, b.Wo[i + 1] - b.Wo[i]);
+  if (W > 0x7fffffff) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 windows per clip");
+  if (b.want_mod && W > 0 &&
+      (rc = modspec_varlen_route((unsigned)plan->cfg.flags, b.T.data() + c0, nc, plan->cfg.n_mfcc, W, b.mod->win,
+                                 b.mod->hop, b.mod->nfft, b.nbe, b.mag != nullptr, h.mv)))
+    return rc;
+  h.stage = resample_desc(c0, c1, b.offsets, b.offsets[c0], b.rs, desc);
+  if (h.stage.items < 0) return fail(MMF_ERR_UNSUPPORTED, "a chunk of more than 2^31 - 1 staging work items");
+  auto packed_rows = [&](const std::vector<int64_t>& pre) {
+    std::vector<int> cnt((size_t)nc);
+    std::vector<int64_t> off((size_t)nc);
+    for (int64_t k = 0; k < nc; ++k) {
+      cnt[k] = (int)(pre[c0 + k + 1] - pre[c0 + k]);
+      off[k] = pre[c0 + k] - pre[c0];
+    }
+    return PackedRows{desc.put(cnt), desc.put(off)};
+  };
+  h.frames = packed_rows(b.F);
+  h.wins = packed_rows(b.Wo);
+  if (b.want_amp && envelope_route(c0, c1, b.offsets, b.offsets[c0], b.geom, b.amp_prm->center, b.A.data(),
+                                   b.amp_filt ? &b.amp_sos : nullptr, h.env) < 0)
+    return fail(MMF_ERR_UNSUPPORTED, "a chunk of more than 2^31 - 1 envelope work items");
+  return MMF_OK;
+}
+
+static HostSlot layout_slot(const PackedBatch& b, const HostChunk& h, int nm) {
+  const size_t nc = (size_t)(h.c1 - h.c0), pitch = (size_t)h.cv.pitch, W = (size_t)h.mv.W;
+  const size_t frames = (size_t)(b.F[h.c1] - b.F[h.c0]), wins = (size_t)(b.Wo[h.c1] - b.Wo[h.c0]);
+  const bool mod_c = h.mv.W > 0;
+  HostSlot s;
+  size_t& o = s.end;
+  s.h2d = ws_take(o, (size_t)(b.offsets[h.c1] - b.offsets[h.c0]) * b.isz);
+  s.pcm = ws_take(o, nc * h.stride * 4);
+  s.tot = ws_take(o, nc * pitch * 8);
+  s.mfcc = b.need_mfcc_dev ? ws_take(o, nc * nm * pitch * 4) : 0;
+  s.delta = b.delta ? ws_take(o, nc * nm * pitch * 4) : 0;
+  s.mag = mod_c && b.mag ? ws_take(o, nc * nm * W * b.nb * 4) : 0;
+  s.band = mod_c && b.nbe > 0 ? ws_take(o, nc * W * b.nbe * 4) : 0;
+  s.ptot = ws_take(o, frames * 8);
+  s.pmfcc = b.mfcc ? ws_take(o, nm * frames * 4) : 0;
+  s.pdelta = b.delta ? ws_take(o, nm * frames * 4) : 0;
+  s.pmag = mod_c && b.mag ? ws_take(o, nm * wins * b.nb * 4) : 0;
+  s.pband = mod_c && b.nbe > 0 ? ws_take(o, wins * b.nbe * 4) : 0;
+  s.scratch = ws_take(o, std::max(h.cv.bytes, mod_c ? h.mv.bytes : 0));
+  s.amp = b.want_amp ? ws_take(o, (size_t)(b.A[h.c1] - b.A[h.c0]) * 4) : 0;
+  s.amp_filt = b.amp_filt ? ws_take(o, (size_t)(b.A[h.c1] - b.A[h.c0]) * 8) : 0;
+  return s;
+}
+
+// Stage 2 (host only): the chunks, each routed, its descriptors appended to `desc` and its slot laid out; `slot`:
+// the largest.  Chunk policy: maximal runs of consecutive clips whose samples as they cross PCIe stay within the
+// chunk budget (bytes of float32 samples) and whose staged rows at the plan's rate stay within twice that, so that one
+// long clip among short ones cannot inflate the padded intermediates.  A clip over either budget is a chunk alone.
+static int plan_chunks(const mmf_plan* plan, const PackedBatch& b, std::vector<HostChunk>& chunks, DescBlob& desc,
+                       size_t& slot) {
+  const int64_t budget = (int64_t)(b.pcm16 ? kHostChunkI16 : kHostChunkF32);
+  for (int64_t c0 = 0; c0 < b.n_clips;) {
+    int64_t c1 = c0 + 1, n_max = b.len[c0];
     // (at most 65535 clips: the compaction's one CTA per row stays far inside the grid limit)
-    while (c1 < n_clips && c1 - c0 < 65535) {
-      const int64_t m = std::max(n_max, len[c1]);
-      if ((real + len_in[c1]) * 4 > budget || (c1 + 1 - c0) * ((m + 3) & ~3LL) * 4 > 2 * budget) break;
-      real += len_in[c1];
+    while (c1 < b.n_clips && c1 - c0 < 65535) {
+      const int64_t m = std::max(n_max, b.len[c1]);
+      if ((b.offsets[c1 + 1] - b.offsets[c0]) * 4 > budget || (c1 + 1 - c0) * ((m + 3) & ~3LL) * 4 > 2 * budget)
+        break;
       n_max = m;
       ++c1;
     }
-    chunks.emplace_back();
+    chunks.push_back({c0, c1, (n_max + 3) & ~3LL});
     HostChunk& h = chunks.back();
-    h.c0 = c0;
-    h.c1 = c1;
-    h.stride = (n_max + 3) & ~3LL;
-    const int64_t nc = c1 - c0;
-    if ((rc = change_varlen_route(plan, nc, len.data() + c0, prm, false, need_mfcc_dev, delta_host != nullptr, c0,
-                                  h.cv)))
-      return rc;
-    int64_t W = 0;
-    for (int64_t i = c0; i < c1; ++i) W = std::max(W, Wo[i + 1] - Wo[i]);
-    if (W > 0x7fffffff) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 windows per clip");
-    if (want_mod && W > 0 &&
-        (rc = modspec_varlen_route((unsigned)c.flags, T.data() + c0, nc, nm, W, mod->win, mod->hop, mod->nfft, nbe,
-                                   mag_host != nullptr, h.mv)))
-      return rc;
-    // descriptors: the staging launch's, then frames / windows and their packed offsets per clip
-    h.items = resample_desc(c0, c1, offsets, offsets[c0], rs, h.desc, h.o_rs, h.o_first);
-    if (h.items < 0) return fail(MMF_ERR_UNSUPPORTED, "a chunk of more than 2^31 - 1 staging work items");
-    size_t d = h.desc.size();
-    auto dtake = [&](size_t bytes) {
-      const size_t o = d;
-      d += align_up(bytes, 16);
-      return o;
-    };
-    h.o_cnt_t = dtake(nc * 4);
-    h.o_off_t = dtake(nc * 8);
-    h.o_cnt_w = dtake(nc * 4);
-    h.o_off_w = dtake(nc * 8);
-    h.desc.resize(d, 0);
-    for (int64_t i = 0; i < nc; ++i) {
-      ((int*)(h.desc.data() + h.o_cnt_t))[i] = (int)T[c0 + i];
-      ((int64_t*)(h.desc.data() + h.o_off_t))[i] = F[c0 + i] - F[c0];
-      ((int*)(h.desc.data() + h.o_cnt_w))[i] = (int)(Wo[c0 + i + 1] - Wo[c0 + i]);
-      ((int64_t*)(h.desc.data() + h.o_off_w))[i] = Wo[c0 + i] - Wo[c0];
-    }
-    if (want_amp) {
-      h.amp_items = rms_desc(c0, c1, offsets, offsets[c0], geom, amp->center, A.data(), h.desc, h.o_acl, h.o_afirst);
-      if (h.amp_items < 0) return fail(MMF_ERR_UNSUPPORTED, "a chunk of more than 2^31 - 1 envelope work items");
-    }
-    if (want_amp && amp_filt_host) {
-      // each envelope takes the route of its own mmf_sosfiltfilt call: the chunk-parallel kernel when
-      // sos_par_fill takes its length (all of them in one launch, each with the tables of its own chunk length), the
-      // single-row routes otherwise
-      std::vector<int> par_clips, Ti((size_t)nc), par_of_cl(kSosParMaxChunk + 1, -1);
-      std::vector<int2> pidx((size_t)nc, int2{0, 0});
-      std::vector<long> off((size_t)nc);
-      std::vector<SosPar> pars;
-      for (int64_t k = 0; k < nc; ++k) {
-        const int64_t Tk = A[c0 + k + 1] - A[c0 + k];
-        off[k] = (long)(A[c0 + k] - A[c0]);
-        Ti[k] = (int)std::min<int64_t>(Tk, 0x7fffffff);
-        SosPar sp;
-        if (!sos_par_fill(so_amp, (long)Tk, &sp)) {
-          h.amp_single.push_back(k);
-          continue;
-        }
-        int& idx = par_of_cl[sp.CL];
-        if (idx < 0) {
-          idx = (int)pars.size();
-          pars.push_back(sp);
-          if (idx == 0 || sp.CL > h.amax.CL) h.amax = sp;
-        }
-        pidx[k] = int2{idx, idx};
-        par_clips.push_back((int)k);
-      }
-      h.amp_np = (int64_t)par_clips.size();
-      size_t da = h.desc.size();
-      auto atake = [&](size_t bytes) {
-        const size_t o = da;
-        da += align_up(std::max<size_t>(bytes, 1), 16);
-        return o;
-      };
-      h.o_fclips = atake(par_clips.size() * 4);
-      h.o_fT = atake((size_t)nc * 4);
-      h.o_fpidx = atake((size_t)nc * 8);
-      h.o_foff = atake((size_t)nc * 8);
-      h.o_fpars = atake(pars.size() * sizeof(SosPar));
-      h.desc.resize(da, 0);
-      if (!par_clips.empty()) std::memcpy(h.desc.data() + h.o_fclips, par_clips.data(), par_clips.size() * 4);
-      std::memcpy(h.desc.data() + h.o_fT, Ti.data(), (size_t)nc * 4);
-      std::memcpy(h.desc.data() + h.o_fpidx, pidx.data(), (size_t)nc * 8);
-      std::memcpy(h.desc.data() + h.o_foff, off.data(), (size_t)nc * 8);
-      if (!pars.empty()) std::memcpy(h.desc.data() + h.o_fpars, pars.data(), pars.size() * sizeof(SosPar));
-    }
-    // descriptors of every chunk go up together before the first chunk runs (a copy from pageable memory waits for
-    // its stream: inside the loop it would hold back the next chunk's queueing)
-    const bool mod_c = h.mv.W > 0;
-    h.o_desc = desc_bytes;
-    desc_bytes += align_up(h.desc.size(), 256);
-    h.o_cv_desc = desc_bytes;
-    desc_bytes += align_up(h.cv.desc.size(), 256);
-    h.o_mv_desc = desc_bytes;
-    desc_bytes += mod_c ? align_up(h.mv.desc.size(), 256) : 0;
-    // the slot: PCM as it crossed PCIe, staged rows, padded outputs, packed outputs, ragged scratch
-    const size_t pitch = (size_t)h.cv.pitch, frames = (size_t)(F[c1] - F[c0]), wins = (size_t)(Wo[c1] - Wo[c0]);
-    size_t o = 0;
-    auto take = [&](size_t bytes) {
-      const size_t r = o;
-      o += align_up(bytes, 256);
-      return r;
-    };
-    h.o_h2d = take((size_t)real * isz);
-    h.o_pcm = take((size_t)nc * h.stride * 4);
-    h.o_tot = take((size_t)nc * pitch * 8);
-    h.o_mfcc = need_mfcc_dev ? take((size_t)nc * nm * pitch * 4) : 0;
-    h.o_delta = delta_host ? take((size_t)nc * nm * pitch * 4) : 0;
-    h.o_mag = mod_c && mag_host ? take((size_t)nc * nm * W * nb * 4) : 0;
-    h.o_band = mod_c && nbe > 0 ? take((size_t)nc * W * nbe * 4) : 0;
-    h.o_ptot = take(frames * 8);
-    h.o_pmfcc = mfcc_host ? take((size_t)nm * frames * 4) : 0;
-    h.o_pdelta = delta_host ? take((size_t)nm * frames * 4) : 0;
-    h.o_pmag = mod_c && mag_host ? take((size_t)nm * wins * nb * 4) : 0;
-    h.o_pband = mod_c && nbe > 0 ? take(wins * nbe * 4) : 0;
-    h.o_scratch = take(std::max(h.cv.bytes, mod_c ? h.mv.bytes : 0));
-    const size_t n_amp = want_amp ? (size_t)(A[c1] - A[c0]) : 0;
-    h.o_amp = want_amp ? take(n_amp * 4) : 0;
-    h.o_ampf = want_amp && amp_filt_host ? take(n_amp * 8) : 0;
-    h.end = o;
-    slot = std::max(slot, o);
+    if (const int rc = route_chunk(plan, b, h, desc)) return rc;
+    h.slot = layout_slot(b, h, plan->cfg.n_mfcc);
+    slot = std::max(slot, h.slot.end);
     c0 = c1;
   }
-
-  MMF_CUDA(cudaSetDevice(c.device));
+  // then every chunk's stage descriptors (mostly chunk tables), copied once into one allocation
+  size_t bytes = desc.size();
+  for (const HostChunk& h : chunks) bytes += 3 * kDescAlign + h.cv.desc.size() + h.mv.desc.size() + h.env.desc.size();
+  desc.bytes.reserve(bytes);
+  for (HostChunk& h : chunks) {
+    h.o_cv = desc.put(h.cv.desc.bytes);
+    h.o_mv = desc.put(h.mv.desc.bytes);
+    h.o_env = desc.put(h.env.desc.bytes);
+  }
   slot = align_up(slot, 256);
-  if ((rc = ensure_host_ws(plan, desc_bytes + 2 * slot))) return rc;
-  // the modulation tables are (re)built with a device-wide synchronisation: do it before any copy is queued
-  bool any_mod = false;
-  for (const HostChunk& h : chunks) any_mod |= h.mv.W > 0;
-  if (any_mod && (rc = ensure_mod_tables(plan, mod->win, mod->nfft, mod->band_lo, mod->band_hi, nbe))) return rc;
+  return MMF_OK;
+}
 
-  // every exit below drains both streams: queued copies target caller-owned host buffers
-  auto body = [&]() -> int {
-    unsigned char* d_desc = (unsigned char*)plan->host_ws;
-    {
-      std::vector<unsigned char> all(desc_bytes);
-      if (n_taps) std::memcpy(all.data(), h_taps, (size_t)n_taps * 4);
-      for (const HostChunk& h : chunks) {
-        std::memcpy(all.data() + h.o_desc, h.desc.data(), h.desc.size());
-        std::memcpy(all.data() + h.o_cv_desc, h.cv.desc.data(), h.cv.desc.size());
-        if (h.mv.W > 0) std::memcpy(all.data() + h.o_mv_desc, h.mv.desc.data(), h.mv.desc.size());
-      }
-      // (complete before either stream reads it)
-      MMF_CUDA(cudaMemcpyAsync(d_desc, all.data(), desc_bytes, cudaMemcpyHostToDevice, plan->streams[0]));
-      MMF_CUDA(cudaStreamSynchronize(plan->streams[0]));
-    }
-    for (size_t k = 0; k < chunks.size(); ++k) {
-      const HostChunk& h = chunks[k];
-      const int s = (int)(k & 1);
-      cudaStream_t st = plan->streams[s];
-      // stream order serialises reuse of slot s (chunk k-2 ran on the same stream)
-      unsigned char* base = (unsigned char*)plan->host_ws + desc_bytes + (size_t)s * slot;
-      const int64_t nc = h.c1 - h.c0;
-      auto dev = [&](size_t o) { return (void*)(base + o); };
-      const unsigned char* dd = d_desc + h.o_desc;
-      MMF_CUDA(cudaMemcpyAsync(dev(h.o_h2d), (const unsigned char*)pcm_host_v + (size_t)offsets[h.c0] * isz,
-                               (size_t)(offsets[h.c1] - offsets[h.c0]) * isz, cudaMemcpyHostToDevice, st));
-      // the envelope reads the native samples as they arrived, straight into its packed blocks
-      float* d_amp = want_amp ? (float*)dev(h.o_amp) : nullptr;
-      double* d_ampf = want_amp && amp_filt_host ? (double*)dev(h.o_ampf) : nullptr;
-      if (want_amp) {
-        cudaError_t ea = rms_varlen_launch(dev(h.o_h2d), pcm16, (const RmsClip*)(dd + h.o_acl),
-                                           (const unsigned*)(dd + h.o_afirst), (long)nc, (long)h.amp_items, d_amp, st);
-        if (ea != cudaSuccess) return cuda_fail(ea, "rms_varlen_kernel launch");
-      }
-      if (d_ampf) {
-        if (h.amp_np) {
-          const FusedVarlen fvl{(const int*)(dd + h.o_fclips), (const int*)(dd + h.o_fT),
-                                (const SosPar*)(dd + h.o_fpars), (const int2*)(dd + h.o_fpidx),
-                                (const long*)(dd + h.o_foff)};
-          cudaError_t ea = sosfiltfilt_par_varlen_launch(d_amp, 1, (long)h.amp_np, 0, h.amax, fvl, d_ampf, st);
-          if (ea != cudaSuccess) return cuda_fail(ea, "sosfiltfilt_par_kernel (envelopes) launch");
-        }
-        for (int64_t k : h.amp_single) {
-          const int64_t a0 = A[h.c0 + k] - A[h.c0], Tk = A[h.c0 + k + 1] - A[h.c0 + k];
-          cudaError_t ea = sosfiltfilt_any(d_amp + a0, 1, 1, (long)Tk, (long)Tk, 1, 0, so_amp, d_ampf + a0, (long)Tk, st);
-          if (ea != cudaSuccess) return cuda_fail(ea, "sosfiltfilt (envelope)");
-        }
-      }
-      float* d_pcm = (float*)dev(h.o_pcm);
-      cudaError_t e = resample_rows_launch(dev(h.o_h2d), pcm16, (const RsClip*)(dd + h.o_rs),
-                                           (const unsigned*)(dd + h.o_first), (long)nc, (long)h.items,
-                                           (const float*)d_desc, d_pcm, (long)h.stride, st);
-      if (e != cudaSuccess) return cuda_fail(e, "resample_rows_kernel launch");
-      double* d_tot = (double*)dev(h.o_tot);
-      float* d_mfcc = need_mfcc_dev ? (float*)dev(h.o_mfcc) : nullptr;
-      float* d_delta = delta_host ? (float*)dev(h.o_delta) : nullptr;
-      int rc2 = change_varlen_run(plan, h.cv, base + h.o_scratch, d_desc + h.o_cv_desc, d_pcm, h.stride, prm, d_tot,
-                                  nullptr, d_mfcc, d_delta, st);
-      if (rc2) return rc2;
-      const bool mod_c = h.mv.W > 0;
-      float* d_mag = mod_c && mag_host ? (float*)dev(h.o_mag) : nullptr;
-      float* d_band = mod_c && nbe > 0 ? (float*)dev(h.o_band) : nullptr;
-      if (mod_c && (rc2 = modspec_varlen_run(plan, h.mv, base + h.o_scratch, d_desc + h.o_mv_desc, d_mfcc, nm,
-                                             h.cv.pitch, mod->win, mod->hop, mod->nfft, d_mag, d_band, st)))
-        return rc2;
-      // padded rows -> packed blocks -> one copy back per output
-      const int* cnt_t = (const int*)(dd + h.o_cnt_t);
-      const long* off_t = (const long*)(dd + h.o_off_t);
-      const int* cnt_w = (const int*)(dd + h.o_cnt_w);
-      const long* off_w = (const long*)(dd + h.o_off_w);
-      const size_t frames = (size_t)(F[h.c1] - F[h.c0]), wins = (size_t)(Wo[h.c1] - Wo[h.c0]);
-      const long pitch = h.cv.pitch, W = (long)h.mv.W;
-      auto out = [&](const void* src, size_t o_dst, int eb, int rows, int unit, long pitch_el, const int* cnt,
-                     const long* off, void* host, size_t bytes) -> int {
-        if (!bytes) return MMF_OK;
-        cudaError_t ce = compact_rows_launch(src, dev(o_dst), eb, (long)nc, rows, unit, pitch_el, cnt, off, st);
-        if (ce != cudaSuccess) return cuda_fail(ce, "compact_rows_kernel launch");
-        MMF_CUDA(cudaMemcpyAsync(host, dev(o_dst), bytes, cudaMemcpyDeviceToHost, st));
-        return MMF_OK;
-      };
-      if ((rc2 = out(d_tot, h.o_ptot, 8, 1, 1, pitch, cnt_t, off_t, tot_host + F[h.c0], frames * 8))) return rc2;
-      if (mfcc_host && (rc2 = out(d_mfcc, h.o_pmfcc, 4, nm, 1, pitch, cnt_t, off_t, mfcc_host + (size_t)nm * F[h.c0],
-                                  (size_t)nm * frames * 4)))
-        return rc2;
-      if (delta_host && (rc2 = out(d_delta, h.o_pdelta, 4, nm, 1, pitch, cnt_t, off_t,
-                                   delta_host + (size_t)nm * F[h.c0], (size_t)nm * frames * 4)))
-        return rc2;
-      if (d_mag && (rc2 = out(d_mag, h.o_pmag, 4, nm, nb, W * nb, cnt_w, off_w,
-                              mag_host + (size_t)nm * nb * Wo[h.c0], (size_t)nm * nb * wins * 4)))
-        return rc2;
-      if (d_band && (rc2 = out(d_band, h.o_pband, 4, 1, nbe, W * nbe, cnt_w, off_w, band_host + (size_t)nbe * Wo[h.c0],
-                               (size_t)nbe * wins * 4)))
-        return rc2;
-      const size_t n_amp = want_amp ? (size_t)(A[h.c1] - A[h.c0]) : 0;
-      if (amp_host) MMF_CUDA(cudaMemcpyAsync(amp_host + A[h.c0], d_amp, n_amp * 4, cudaMemcpyDeviceToHost, st));
-      if (d_ampf) MMF_CUDA(cudaMemcpyAsync(amp_filt_host + A[h.c0], d_ampf, n_amp * 8, cudaMemcpyDeviceToHost, st));
-    }
+// Stage 3: one chunk's device sequence on `st`.  One H2D copy of its packed samples; the envelope, read from the
+// native samples as they arrived; the staging launch into rows at the plan's rate; the change and modulation stages;
+// then per output one compaction (padded rows -> packed blocks) and one D2H copy.  dd: the call's descriptors on the
+// device, taps: the tap table there; base: the chunk's slot.
+static int run_chunk(mmf_plan* plan, const PackedBatch& b, const HostChunk& h, const unsigned char* dd,
+                     const float* taps, unsigned char* base, cudaStream_t st) {
+  const int64_t nc = h.c1 - h.c0;
+  const int nm = plan->cfg.n_mfcc;
+  const HostSlot& s = h.slot;
+  auto dev = [&](size_t o) { return (void*)(base + o); };
+  MMF_CUDA(cudaMemcpyAsync(dev(s.h2d), (const unsigned char*)b.pcm + (size_t)b.offsets[h.c0] * b.isz,
+                           (size_t)(b.offsets[h.c1] - b.offsets[h.c0]) * b.isz, cudaMemcpyHostToDevice, st));
+  float* d_amp = b.want_amp ? (float*)dev(s.amp) : nullptr;
+  double* d_ampf = b.amp_filt ? (double*)dev(s.amp_filt) : nullptr;
+  int rc;
+  if (b.want_amp && (rc = envelope_run(h.env, dd + h.o_env, dev(s.h2d), b.pcm16, d_amp, d_ampf, st))) return rc;
+  float* d_pcm = (float*)dev(s.pcm);
+  cudaError_t e = resample_rows_launch(dev(s.h2d), b.pcm16, (const RsClip*)(dd + h.stage.clips),
+                                       (const unsigned*)(dd + h.stage.first), (long)nc, (long)h.stage.items, taps,
+                                       d_pcm, (long)h.stride, st);
+  if (e != cudaSuccess) return cuda_fail(e, "resample_rows_kernel launch");
+  double* d_tot = (double*)dev(s.tot);
+  float* d_mfcc = b.need_mfcc_dev ? (float*)dev(s.mfcc) : nullptr;
+  float* d_delta = b.delta ? (float*)dev(s.delta) : nullptr;
+  if ((rc = change_varlen_run(plan, h.cv, base + s.scratch, dd + h.o_cv, d_pcm, h.stride, b.prm, d_tot, nullptr,
+                              d_mfcc, d_delta, st)))
+    return rc;
+  const bool mod_c = h.mv.W > 0;
+  float* d_mag = mod_c && b.mag ? (float*)dev(s.mag) : nullptr;
+  float* d_band = mod_c && b.nbe > 0 ? (float*)dev(s.band) : nullptr;
+  if (mod_c && (rc = modspec_varlen_run(plan, h.mv, base + s.scratch, dd + h.o_mv, d_mfcc, nm, h.cv.pitch,
+                                        b.mod->win, b.mod->hop, b.mod->nfft, d_mag, d_band, st)))
+    return rc;
+  // one requested output (host != null): padded rows -> packed blocks in the slot -> one copy back
+  const long pitch = h.cv.pitch, W = (long)h.mv.W;
+  auto out = [&](const void* src, size_t o_dst, int eb, int rows, int unit, long pitch_el, bool per_win,
+                 void* host) -> int {
+    const int64_t* pre = per_win ? b.Wo.data() : b.F.data();
+    const size_t blk = (size_t)eb * rows * unit, n = (size_t)(pre[h.c1] - pre[h.c0]);
+    if (!host || !n) return MMF_OK;
+    const PackedRows& pr = per_win ? h.wins : h.frames;
+    cudaError_t ce = compact_rows_launch(src, dev(o_dst), eb, (long)nc, rows, unit, pitch_el,
+                                         (const int*)(dd + pr.cnt), (const long*)(dd + pr.off), st);
+    if (ce != cudaSuccess) return cuda_fail(ce, "compact_rows_kernel launch");
+    MMF_CUDA(cudaMemcpyAsync((char*)host + blk * pre[h.c0], dev(o_dst), blk * n, cudaMemcpyDeviceToHost, st));
     return MMF_OK;
   };
-  rc = body();
-  const cudaError_t e0 = cudaStreamSynchronize(plan->streams[0]);
-  const cudaError_t e1 = cudaStreamSynchronize(plan->streams[1]);
+  if ((rc = out(d_tot, s.ptot, 8, 1, 1, pitch, false, b.tot)) ||
+      (rc = out(d_mfcc, s.pmfcc, 4, nm, 1, pitch, false, b.mfcc)) ||
+      (rc = out(d_delta, s.pdelta, 4, nm, 1, pitch, false, b.delta)) ||
+      (rc = out(d_mag, s.pmag, 4, nm, b.nb, W * b.nb, true, d_mag ? b.mag : nullptr)) ||
+      (rc = out(d_band, s.pband, 4, 1, b.nbe, W * b.nbe, true, d_band ? b.band : nullptr)))
+    return rc;
+  const size_t n_amp = b.want_amp ? (size_t)(b.A[h.c1] - b.A[h.c0]) : 0;
+  if (b.amp) MMF_CUDA(cudaMemcpyAsync(b.amp + b.A[h.c0], d_amp, n_amp * 4, cudaMemcpyDeviceToHost, st));
+  if (d_ampf) MMF_CUDA(cudaMemcpyAsync(b.amp_filt + b.A[h.c0], d_ampf, n_amp * 8, cudaMemcpyDeviceToHost, st));
+  return MMF_OK;
+}
+
+// The packed host-buffer bundle: the host-only checks, the chunk plan, then each chunk's device sequence
+static int features_host_varlen_impl(mmf_plan* plan, PackedBatch b) {
+  int rc = packed_check(plan, b);
   if (rc) return rc;
-  if (e0 != cudaSuccess) return cuda_fail(e0, "host path, stream 0");
-  if (e1 != cudaSuccess) return cuda_fail(e1, "host path, stream 1");
-  return MMF_OK;
-}
-
-// One ragged resampling launch on `st` from host descriptors: descriptors, work-item offsets and taps h[n_h] go up in
-// one copy to stream-ordered scratch (pageable source: the copy is staged, so the host data may go when this returns).
-static int resample_dev(mmf_plan* plan, const float* x_dev, const std::vector<RsClip>& cl,
-                        const std::vector<unsigned>& first, const float* h, int64_t n_h, float* y_dev,
-                        int64_t y_stride, cudaStream_t st) {
-  const size_t o_first = align_up(cl.size() * sizeof(RsClip), 256);
-  const size_t o_h = align_up(o_first + first.size() * 4, 256);
-  const size_t bytes = o_h + (size_t)n_h * 4;
-  std::vector<unsigned char> up(bytes);
-  std::memcpy(up.data(), cl.data(), cl.size() * sizeof(RsClip));
-  std::memcpy(up.data() + o_first, first.data(), first.size() * 4);
-  if (n_h) std::memcpy(up.data() + o_h, h, (size_t)n_h * 4);
+  // every chunk is routed before anything is queued; the call's descriptors: the taps, then each chunk's
+  DescBlob desc;
+  const size_t o_taps = desc.put(b.h_taps, (size_t)b.n_taps);
+  std::vector<HostChunk> chunks;
+  size_t slot = 0;
+  if ((rc = plan_chunks(plan, b, chunks, desc, slot))) return rc;
   MMF_CUDA(cudaSetDevice(plan->cfg.device));
-  unsigned char* d = nullptr;
-  MMF_CUDA(cudaMallocAsync((void**)&d, bytes, st));
-  cudaError_t e = cudaMemcpyAsync(d, up.data(), bytes, cudaMemcpyHostToDevice, st);
-  if (e == cudaSuccess)
-    e = resample_rows_launch(x_dev, 0, (const RsClip*)d, (const unsigned*)(d + o_first), (long)cl.size(),
-                             (long)first.back(), (const float*)(d + o_h), y_dev, (long)y_stride, st);
-  cudaFreeAsync(d, st);
-  if (e != cudaSuccess) return cuda_fail(e, "resample_rows_kernel launch");
-  return MMF_OK;
-}
-
-// One ragged RMS launch on `st` over float32 x_dev from host descriptors (RmsClip at o_clips, first_item at o_first of
-// `desc`), which go up to stream-ordered scratch as resample_dev's do.
-static int rms_run(mmf_plan* plan, const float* x_dev, const std::vector<unsigned char>& desc, size_t o_clips,
-                   size_t o_first, int64_t n_clips, int64_t n_items, float* out_dev, cudaStream_t st) {
-  MMF_CUDA(cudaSetDevice(plan->cfg.device));
-  unsigned char* d = nullptr;
-  MMF_CUDA(cudaMallocAsync((void**)&d, desc.size(), st));
-  cudaError_t e = cudaMemcpyAsync(d, desc.data(), desc.size(), cudaMemcpyHostToDevice, st);
-  if (e == cudaSuccess)
-    e = rms_varlen_launch(x_dev, 0, (const RmsClip*)(d + o_clips), (const unsigned*)(d + o_first), (long)n_clips,
-                          (long)n_items, out_dev, st);
-  cudaFreeAsync(d, st);
-  if (e != cudaSuccess) return cuda_fail(e, "rms_varlen_kernel launch");
-  return MMF_OK;
+  const size_t o_slots = align_up(desc.size(), 256);
+  if ((rc = ensure_host_ws(plan, o_slots + 2 * slot))) return rc;
+  // the modulation tables are (re)built with a device-wide synchronisation: do it before any copy is queued
+  if (b.want_mod && b.Wo[b.n_clips] > 0 &&
+      (rc = ensure_mod_tables(plan, b.mod->win, b.mod->nfft, b.mod->band_lo, b.mod->band_hi, b.nbe)))
+    return rc;
+  return run_and_drain(plan, [&]() -> int {
+    // every chunk's descriptors go up in one copy, complete before either stream reads them: a copy from pageable
+    // memory waits for its stream, so inside the loop it would hold back the next chunk's queueing
+    unsigned char* d_desc = (unsigned char*)plan->host_ws;
+    MMF_CUDA(cudaMemcpyAsync(d_desc, desc.bytes.data(), desc.size(), cudaMemcpyHostToDevice, plan->streams[0]));
+    MMF_CUDA(cudaStreamSynchronize(plan->streams[0]));
+    // stream order serialises reuse of slot k & 1 (chunk k - 2 ran on the same stream)
+    for (size_t k = 0; k < chunks.size(); ++k)
+      if (const int rc2 = run_chunk(plan, b, chunks[k], d_desc, (const float*)(d_desc + o_taps),
+                                    d_desc + o_slots + (k & 1) * slot, plan->streams[k & 1]))
+        return rc2;
+    return MMF_OK;
+  });
 }
 
 }  // namespace mmf
@@ -2283,8 +2284,8 @@ int mmf_features_varlen_sizes(const mmf_config* cfg, const mmf_modspec_params* m
 int mmf_features_host_varlen(mmf_plan* plan, const float* pcm_host, int64_t n_clips, const int64_t* offsets_host,
                              const mmf_change_params* prm, const mmf_modspec_params* mod, double* tot_host,
                              float* mfcc_host, float* delta_host, float* mag_host, float* band_host) {
-  return mmf::features_host_varlen_impl(plan, pcm_host, 0, n_clips, offsets_host, false, nullptr, nullptr, 0, prm, mod,
-                                        tot_host, mfcc_host, delta_host, mag_host, band_host);
+  return mmf::features_host_varlen_impl(plan, {pcm_host, 0, n_clips, offsets_host, nullptr, nullptr, 0, prm, mod,
+                                               nullptr, nullptr, tot_host, mfcc_host, delta_host, mag_host, band_host});
 }
 
 int mmf_features_host_varlen_resampled(mmf_plan* plan, const void* pcm_host, int32_t pcm16, int64_t n_clips,
@@ -2292,16 +2293,17 @@ int mmf_features_host_varlen_resampled(mmf_plan* plan, const void* pcm_host, int
                                        const float* h_host, int64_t n_h, const mmf_change_params* prm,
                                        const mmf_modspec_params* mod, double* tot_host, float* mfcc_host,
                                        float* delta_host, float* mag_host, float* band_host) {
-  return mmf::features_host_varlen_impl(plan, pcm_host, pcm16 ? 1 : 0, n_clips, offsets_host, true, rs_host, h_host,
-                                        n_h, prm, mod, tot_host, mfcc_host, delta_host, mag_host, band_host);
+  return mmf::features_host_varlen_impl(plan, {pcm_host, pcm16 ? 1 : 0, n_clips, offsets_host, rs_host, h_host, n_h,
+                                               prm, mod, nullptr, nullptr, tot_host, mfcc_host, delta_host, mag_host,
+                                               band_host, nullptr, nullptr, true});
 }
 
 int mmf_features_host_varlen_pcm16(mmf_plan* plan, const int16_t* pcm16_host, int64_t n_clips,
                                    const int64_t* offsets_host, const mmf_change_params* prm,
                                    const mmf_modspec_params* mod, double* tot_host, float* mfcc_host,
                                    float* delta_host, float* mag_host, float* band_host) {
-  return mmf::features_host_varlen_impl(plan, pcm16_host, 1, n_clips, offsets_host, false, nullptr, nullptr, 0, prm, mod,
-                                        tot_host, mfcc_host, delta_host, mag_host, band_host);
+  return mmf::features_host_varlen_impl(plan, {pcm16_host, 1, n_clips, offsets_host, nullptr, nullptr, 0, prm, mod,
+                                               nullptr, nullptr, tot_host, mfcc_host, delta_host, mag_host, band_host});
 }
 
 int mmf_features_host_varlen_amp(mmf_plan* plan, const void* pcm_host, int32_t pcm16, int64_t n_clips,
@@ -2310,9 +2312,9 @@ int mmf_features_host_varlen_amp(mmf_plan* plan, const void* pcm_host, int32_t p
                                  const mmf_amp_params* amp, const int32_t* geom_host, double* tot_host,
                                  float* mfcc_host, float* delta_host, float* mag_host, float* band_host,
                                  float* amp_host, double* amp_filt_host) {
-  return mmf::features_host_varlen_impl(plan, pcm_host, pcm16 ? 1 : 0, n_clips, offsets_host, rs_host != nullptr,
-                                        rs_host, h_host, n_h, prm, mod, tot_host, mfcc_host, delta_host, mag_host,
-                                        band_host, amp, geom_host, amp_host, amp_filt_host);
+  return mmf::features_host_varlen_impl(plan, {pcm_host, pcm16 ? 1 : 0, n_clips, offsets_host, rs_host, h_host, n_h,
+                                               prm, mod, amp, geom_host, tot_host, mfcc_host, delta_host, mag_host,
+                                               band_host, amp_host, amp_filt_host, rs_host != nullptr});
 }
 
 int mmf_amp_varlen_sizes(int64_t n_clips, const int64_t* offsets_host, const int32_t* geom_host, int32_t center,
@@ -2332,11 +2334,10 @@ int mmf_rms_varlen(mmf_plan* plan, const float* x_dev, int64_t n_clips, const in
   std::vector<int64_t> A((size_t)n_clips + 1);
   if ((rc = amp_sizes(n_clips, offsets_host, geom_host, center, A.data()))) return rc;
   if (!plan || !x_dev || !amp_dev) return fail(MMF_ERR_INVALID, "NULL argument");
-  std::vector<unsigned char> desc;
-  size_t o_clips, o_first;
-  const int64_t items = rms_desc(0, n_clips, offsets_host, 0, geom_host, center, A.data(), desc, o_clips, o_first);
-  if (items < 0) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 work items");
-  return rms_run(plan, x_dev, desc, o_clips, o_first, n_clips, items, amp_dev, (cudaStream_t)stream);
+  EnvelopeVarlen v;
+  if (envelope_route(0, n_clips, offsets_host, 0, geom_host, center, A.data(), nullptr, v) < 0)
+    return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 work items");
+  return rms_run(plan, x_dev, v, amp_dev, (cudaStream_t)stream);
 }
 
 }  // extern "C"
@@ -2412,14 +2413,17 @@ int mmf_resample_poly(mmf_plan* plan, const float* x_dev, int64_t n_clips, int64
     first[r] = (unsigned)(r * per);
   }
   first[n_clips] = (unsigned)(n_clips * per);
-  return resample_dev(plan, x_dev, cl, first, h_host, len_h, y_dev, y_stride, (cudaStream_t)stream);
+  DescBlob desc;
+  const RaggedParts p{desc.put(cl), desc.put(first), n_clips * per};
+  return resample_dev(plan, x_dev, desc, p, h_host, len_h, n_clips, y_dev, y_stride, (cudaStream_t)stream);
 }
 
 int mmf_resample_varlen(mmf_plan* plan, const float* x_dev, int64_t n_clips, const int64_t* offsets_host,
                         const mmf_resample_clip* rs_host, const float* h_host, int64_t n_h, float* y_dev,
                         int64_t y_stride, void* stream) {
   int rc = validate_offsets(n_clips, offsets_host);
-  if (rc || (rc = validate_resample(n_clips, offsets_host, rs_host, h_host, n_h))) return rc;
+  int64_t n_taps = 0;
+  if (rc || (rc = validate_resample(n_clips, offsets_host, rs_host, h_host, n_h, &n_taps))) return rc;
   if (!plan || !x_dev || !y_dev) return fail(MMF_ERR_INVALID, "NULL argument");
   for (int64_t i = 0; i < n_clips; ++i)
     if (rs_host[i].n_out > y_stride) {
@@ -2428,16 +2432,10 @@ int mmf_resample_varlen(mmf_plan* plan, const float* x_dev, int64_t n_clips, con
                     (long long)rs_host[i].n_out, (long long)y_stride);
       return fail(MMF_ERR_INVALID, buf);
     }
-  int64_t n_taps = 0;
-  for (int64_t i = 0; i < n_clips; ++i) n_taps = (rs_host[i].up == 1 && rs_host[i].down == 1) ? n_taps : n_h;
-  std::vector<unsigned char> desc;
-  size_t o_rs, o_first;
-  const int64_t items = resample_desc(0, n_clips, offsets_host, 0, rs_host, desc, o_rs, o_first);
-  if (items < 0) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 work items");
-  const RsClip* c = (const RsClip*)(desc.data() + o_rs);
-  const unsigned* f = (const unsigned*)(desc.data() + o_first);
-  return resample_dev(plan, x_dev, std::vector<RsClip>(c, c + n_clips), std::vector<unsigned>(f, f + n_clips + 1),
-                      h_host, n_taps, y_dev, y_stride, (cudaStream_t)stream);
+  DescBlob desc;
+  const RaggedParts p = resample_desc(0, n_clips, offsets_host, 0, rs_host, desc);
+  if (p.items < 0) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 work items");
+  return resample_dev(plan, x_dev, desc, p, h_host, n_taps, n_clips, y_dev, y_stride, (cudaStream_t)stream);
 }
 
 // one descriptor per row of the ragged kernel (rows of equal length: the grid has no row limit)
@@ -2453,16 +2451,17 @@ int mmf_rms(mmf_plan* plan, const float* pcm_dev, int64_t n_clips, int64_t n_sam
   const int F = rms_frames_per_item(frame_length, hop_length);
   const int64_t per = (T + F - 1) / F;
   if (per * n_clips > 0x7fffffffLL) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 work items");
-  const size_t o_first = align_up((size_t)n_clips * sizeof(RmsClip), 16);
-  std::vector<unsigned char> desc(o_first + ((size_t)n_clips + 1) * 4);
-  RmsClip* cl = (RmsClip*)desc.data();
-  unsigned* first = (unsigned*)(desc.data() + o_first);
+  std::vector<RmsClip> cl((size_t)n_clips);
+  std::vector<unsigned> first((size_t)n_clips + 1);
   for (int64_t r = 0; r < n_clips; ++r) {
     cl[r] = RmsClip{(long)(r * clip_stride), (long)n_samples, (long)(r * T), (long)T, frame_length, hop_length, pad, F};
     first[r] = (unsigned)(r * per);
   }
   first[n_clips] = (unsigned)(n_clips * per);
-  return rms_run(plan, pcm_dev, desc, 0, o_first, n_clips, n_clips * per, rms_dev, (cudaStream_t)stream);
+  EnvelopeVarlen v;
+  v.n_clips = n_clips;
+  v.rms = RaggedParts{v.desc.put(cl), v.desc.put(first), n_clips * per};
+  return rms_run(plan, pcm_dev, v, rms_dev, (cudaStream_t)stream);
 }
 
 int mmf_mfcc_change_host(mmf_plan* plan, const float* pcm_host, int64_t n_clips, int64_t n_samples,

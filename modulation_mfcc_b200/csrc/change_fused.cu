@@ -87,12 +87,15 @@ static bool sos_par_cached(const SosArgs& src, int cl, SosPar* out) {
   return true;
 }
 
-bool sos_par_fill(const SosArgs& src, long T, SosPar* out) {
+int sos_par_chunk(const SosArgs& src, long T) {
   const long L = T + 2L * src.padlen;
-  if (L > 32L * kSosParMaxChunk) return false;
-  int cl = (int)((L + 31) / 32);
-  if ((cl & 1) == 0) ++cl;
-  return sos_par_cached(src, cl, out);
+  if (L > 32L * kSosParMaxChunk) return -1;
+  return (int)((L + 31) / 32) | 1;
+}
+
+bool sos_par_fill(const SosArgs& src, long T, SosPar* out) {
+  const int cl = sos_par_chunk(src, T);
+  return cl > 0 && sos_par_cached(src, cl, out);
 }
 
 // ---------------------------------------------------------------------------

@@ -188,6 +188,8 @@ cudaError_t sosfiltfilt_launch_grouped(const void* x, int x_is_f32, long rows, l
 // chunk-parallel zero-phase IIR and the fused per-clip change kernel (change_fused.cu)
 constexpr int kSosParMaxChunk = 191;  // rows up to 32*191 = 6112 extended samples stay in shared memory
 struct SosPar;
+// chunk length of the tables for rows of T samples (odd), or -1 when the row is too long for the kernel
+int sos_par_chunk(const SosArgs& src, long T);
 bool sos_par_fill(const SosArgs& src, long T, SosPar* out);
 cudaError_t sosfiltfilt_par_launch(const void* x, int x_is_f32, long rows, long T, long xs, int group_rows,
                                    long group_stride, const SosPar& a, double* y, long ys, cudaStream_t st);

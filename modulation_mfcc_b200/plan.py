@@ -753,16 +753,8 @@ class Plan:
             "modspec": ((B, nm, n_win, nb), np.float32),
             "band_energy": ((B, n_win, n_bands), np.float32),
         }
-        ptr = {}
-        for k, (shp, dt) in shapes.items():
-            if k in want or k == "totChange":
-                a = out.get(k)
-                if a is None or a.shape != shp or a.dtype != dt or not a.flags.c_contiguous:
-                    a = np.empty(shp, dt)
-                    out[k] = a
-                ptr[k] = a.ctypes.data
-            else:
-                ptr[k] = None
+        ptr = {k: _out_array(out, k, *sd).ctypes.data if k in want or k == "totChange" else None
+               for k, sd in shapes.items()}
         fn = _lib.lib().mmf_features_host_pcm16 if pcm16 else _lib.lib().mmf_features_host
         check(
             fn(
@@ -847,46 +839,31 @@ class Plan:
         }
         out = {} if out is None else out
         ptr = {}
-        for k, (shp, dt) in shapes.items():
-            if k in want or k == "totChange":
-                a = out.get(k)
-                if a is None or a.shape != shp or a.dtype != dt or not a.flags.c_contiguous:
-                    a = np.empty(shp, dt)
-                    out[k] = a
-                ptr[k] = a.ctypes.data if a.size else None  # (no modulation window in any clip: nothing to write)
-            else:
-                ptr[k] = None
+        for k, sd in shapes.items():
+            a = _out_array(out, k, *sd) if k in want or k == "totChange" else None
+            # (size 0: no modulation window in any clip, nothing to write)
+            ptr[k] = a.ctypes.data if a is not None and a.size else None
         if ("modspec" in want or "band_energy" in want) and mp is None:
             raise ValueError("modspec / band_energy requested without modulation parameters")
-        outs = (C.byref(prm), C.byref(mp) if mp is not None else None)
-        ptrs = (ptr["totChange"], ptr["mfcc"], ptr["delta"], ptr["modspec"], ptr["band_energy"])
+        # one entry point for every variant: rs = NULL means every clip at the plan's rate, amp = NULL no envelope
+        rs_p = h_p = None
+        n_h = 0
+        if rates is not None:
+            rs_p, h_p, n_h = rs.ctypes.data, h.ctypes.data if len(h) else None, len(h)
+        amp_p = geom_p = a_p = af_p = None
         if amp is not None:
             geom, center, out_sos = amp
             _, geom, amp_off = amp_sizes(offs, geom, center)
-            dt = np.float64 if out_sos is not None else np.float32
-            a = out.get("amplitude")
-            if a is None or a.shape != (int(amp_off[-1]),) or a.dtype != dt or not a.flags.c_contiguous:
-                a = np.empty(int(amp_off[-1]), dt)
-                out["amplitude"] = a
-            resampled = rates is not None
-            check(
-                _lib.lib().mmf_features_host_varlen_amp(
-                    self._h, pcm_host.ctypes.data, 1 if pcm16 else 0, B, offs.ctypes.data,
-                    rs.ctypes.data if resampled else None, h.ctypes.data if resampled and len(h) else None,
-                    len(h) if resampled else 0, *outs, C.byref(make_amp_params(center, out_sos)), geom.ctypes.data,
-                    *ptrs, a.ctypes.data if out_sos is None else None, a.ctypes.data if out_sos is not None else None,
-                )
+            a = _out_array(out, "amplitude", (int(amp_off[-1]),), np.float64 if out_sos is not None else np.float32)
+            amp_p, geom_p = C.byref(make_amp_params(center, out_sos)), geom.ctypes.data
+            a_p, af_p = (None, a.ctypes.data) if out_sos is not None else (a.ctypes.data, None)
+        check(
+            _lib.lib().mmf_features_host_varlen_amp(
+                self._h, pcm_host.ctypes.data, 1 if pcm16 else 0, B, offs.ctypes.data, rs_p, h_p, n_h,
+                C.byref(prm), C.byref(mp) if mp is not None else None, amp_p, geom_p,
+                ptr["totChange"], ptr["mfcc"], ptr["delta"], ptr["modspec"], ptr["band_energy"], a_p, af_p,
             )
-        elif rates is not None:
-            check(
-                _lib.lib().mmf_features_host_varlen_resampled(
-                    self._h, pcm_host.ctypes.data, 1 if pcm16 else 0, B, offs.ctypes.data, rs.ctypes.data,
-                    h.ctypes.data if len(h) else None, len(h), *outs, *ptrs,
-                )
-            )
-        else:
-            fn = _lib.lib().mmf_features_host_varlen_pcm16 if pcm16 else _lib.lib().mmf_features_host_varlen
-            check(fn(self._h, pcm_host.ctypes.data, B, offs.ctypes.data, *outs, *ptrs))
+        )
         out["frames"] = np.diff(frame_off)
         out["windows"] = np.diff(win_off)
         out["frame_offsets"] = frame_off
@@ -929,6 +906,15 @@ class Plan:
                 )
             )
         return (tot, mf) if want_mfcc else tot
+
+
+def _out_array(out: dict, key: str, shape, dtype) -> np.ndarray:
+    """``out[key]`` when it is a C-contiguous array of this shape and dtype, else a new one, stored there."""
+    a = out.get(key)
+    if a is None or a.shape != shape or a.dtype != dtype or not a.flags.c_contiguous:
+        a = np.empty(shape, dtype)
+        out[key] = a
+    return a
 
 
 def amp_sizes(offsets, geom, center: bool):
