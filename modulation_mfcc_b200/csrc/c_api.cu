@@ -920,6 +920,37 @@ static cudaError_t sosfiltfilt_any(const void* x, int x_is_f32, long rows, long 
   return sosfiltfilt_launch_grouped(x, x_is_f32, rows, T, xs, group_rows, group_stride, a, y, ys, st);
 }
 
+// The K3 (clamp + DCT-II (+ delta)) kernel: a decision of the plan alone.  Tensor-core DCT-II (mma.sync TF32 x3) on
+// request only: measured 185 us against 95 us for the FP32 kernel on the bench workload (DESIGN.md section 4).
+// MMF_FLAG_TC_DCT: tcgen05 GEMM over 128-frame tiles (mfcc_tc.cu), where the plan built its operand.
+enum MfccKernel { kMfccFp32, kMfccMma, kMfccTc };
+static MfccKernel mfcc_kernel(const mmf_plan* p) {
+  if ((p->cfg.flags & MMF_FLAG_MMA_DCT) && mfcc_mma_supported(p->cfg.n_mfcc, p->cfg.n_mels)) return kMfccMma;
+  return p->d_dct_tc ? kMfccTc : kMfccFp32;
+}
+
+// kernel k over n_clips clips of T frames, 65535 clips per launch; vT: each clip's own frame count (fp32 kernel only)
+static int mfcc_run(const mmf_plan* p, MfccKernel k, float* logmel, const int* clipmax, int64_t n_clips, int64_t T,
+                    float* mfcc, float* delta, int clamp_in_place, cudaStream_t st, const int* vT = nullptr) {
+  const mmf_config& c = p->cfg;
+  for (int64_t c0 = 0; c0 < n_clips; c0 += 65535) {
+    const int64_t nc = std::min<int64_t>(65535, n_clips - c0);
+    float *lm = logmel + (size_t)c0 * c.n_mels * T, *mf = mfcc + (size_t)c0 * c.n_mfcc * T;
+    float* dl = delta ? delta + (size_t)c0 * c.n_mfcc * T : nullptr;
+    const cudaError_t e =
+        k == kMfccMma ? mfcc_mma_launch(p->d_dct_bfrag, lm, clipmax + c0, nc, T, c.n_mels, c.n_mfcc, c.top_db, mf, dl,
+                                        clamp_in_place, st)
+        : k == kMfccTc ? mfcc_tc_launch(p->d_dct_tc, p->dct_tc_kp, lm, clipmax + c0, nc, T, c.n_mels, c.n_mfcc,
+                                        c.top_db, mf, dl, clamp_in_place, p->sm_count, st)
+                       : mfcc_launch(p->d_dct, p->nc_pad, lm, clipmax + c0, nc, T, c.n_mels, c.n_mfcc, c.top_db, mf,
+                                     dl, clamp_in_place, st, vT ? vT + c0 : nullptr);
+    if (e != cudaSuccess)
+      return cuda_fail(e, k == kMfccTc ? "mfcc_tc_kernel launch"
+                          : vT ? "mfcc_kernel (variable-length) launch" : "mfcc_kernel launch");
+  }
+  return MMF_OK;
+}
+
 }  // namespace mmf
 
 extern "C" {
@@ -954,29 +985,8 @@ int mmf_mfcc(mmf_plan* plan, float* logmel_dev, const int32_t* clipmax_dev, int6
   if (!plan || !logmel_dev || !clipmax_dev || !mfcc_dev) return fail(MMF_ERR_INVALID, "NULL argument");
   if (n_clips < 1 || T < 1) return fail(MMF_ERR_INVALID, "n_clips and T must be positive");
   MMF_CUDA(cudaSetDevice(plan->cfg.device));
-  for (int64_t c0 = 0; c0 < n_clips; c0 += 65535) {
-    const int64_t nc = std::min<int64_t>(65535, n_clips - c0);
-    float* lm = logmel_dev + (size_t)c0 * plan->cfg.n_mels * T;
-    float* mf = mfcc_dev + (size_t)c0 * plan->cfg.n_mfcc * T;
-    float* dl = delta_dev ? delta_dev + (size_t)c0 * plan->cfg.n_mfcc * T : nullptr;
-    // Tensor-core DCT-II (mma.sync TF32 x3) on request only: measured 185 us against 95 us for the
-    // FP32 kernel on the bench workload (DESIGN.md section 4)
-    const bool mma = (plan->cfg.flags & MMF_FLAG_MMA_DCT) && mfcc_mma_supported(plan->cfg.n_mfcc, plan->cfg.n_mels);
-    if (!mma && plan->d_dct_tc != nullptr) {
-      // MMF_FLAG_TC_DCT: tcgen05 GEMM over 128-frame tiles (mfcc_tc.cu)
-      cudaError_t et = mfcc_tc_launch(plan->d_dct_tc, plan->dct_tc_kp, lm, clipmax_dev + c0, nc, T, plan->cfg.n_mels,
-                                      plan->cfg.n_mfcc, plan->cfg.top_db, mf, dl, clamp_in_place, plan->sm_count,
-                                      (cudaStream_t)stream);
-      if (et == cudaSuccess) continue;
-      if (et != cudaErrorNotSupported) return cuda_fail(et, "mfcc_tc_kernel launch");
-    }
-    cudaError_t e = mma ? mfcc_mma_launch(plan->d_dct_bfrag, lm, clipmax_dev + c0, nc, T, plan->cfg.n_mels,
-                                          plan->cfg.n_mfcc, plan->cfg.top_db, mf, dl, clamp_in_place, (cudaStream_t)stream)
-                        : mfcc_launch(plan->d_dct, plan->nc_pad, lm, clipmax_dev + c0, nc, T, plan->cfg.n_mels,
-                                      plan->cfg.n_mfcc, plan->cfg.top_db, mf, dl, clamp_in_place, (cudaStream_t)stream);
-    if (e != cudaSuccess) return cuda_fail(e, "mfcc_kernel launch");
-  }
-  return MMF_OK;
+  return mfcc_run(plan, mfcc_kernel(plan), logmel_dev, clipmax_dev, n_clips, T, mfcc_dev, delta_dev, clamp_in_place,
+                  (cudaStream_t)stream);
 }
 
 int mmf_sosfiltfilt(mmf_plan* plan, const void* x_dev, int32_t x_is_f32, int64_t rows, int64_t T,
@@ -1256,6 +1266,43 @@ static size_t change_ws_bytes(const mmf_plan* p, int64_t n_clips, int64_t T, boo
   return b;
 }
 
+// Route of the stage after the log-mel: K3 folded into the fused kernel (FROM_LM), the K3 kernel then the fused kernel,
+// or the K3 kernel then separate filter and derivative + norm kernels.  smem: the fused kernel's shared memory.
+enum ChangePath { kChangeFolded, kChangeFused, kChangeUnfused };
+struct ChangeRoute { ChangePath path; MfccKernel k3; size_t smem; };
+
+// One kernel per clip from log-mel to the curve: clamp + DCT-II feed the float64 row buffers in shared memory directly;
+// MFCC / delta go to HBM only if the caller asked for them.  Measured on the bench workload: 1 % faster than the
+// separate MFCC kernel without a delta output, 1 % slower with one when the modulation spectrum follows (DESIGN.md
+// section 4) -- hence the default.  The fused kernel's DCT phase takes up to kFusedNC coefficients.
+static bool change_folds(const mmf_plan* p, bool want_delta) {
+  const unsigned f = (unsigned)p->cfg.flags;
+  return ((f & MMF_FLAG_FOLD_MFCC) || !want_delta) && !(f & (MMF_FLAG_SEPARATE_MFCC | MMF_FLAG_MMA_DCT)) &&
+         p->cfg.n_mfcc <= kFusedNC;
+}
+
+// Batches: the output filter of the curve runs as its own launch (one warp per clip, all clips at once) instead of on
+// ONE warp of the per-clip CTA while its other 11 wait (27 % of that kernel's stall samples, ncu round 2); the raw
+// curve makes an 8 KB round trip per clip.  Same routine on the same buffer contents: bit-identical.
+static bool change_split_out(bool out_iir, int64_t n_clips) { return out_iir && n_clips >= 32; }
+
+// The route of n_clips clips of T frames, for run_post and for each clip of a variable-length batch.  pa / po: the row
+// and (out_iir) output filter's chunk tables at T, null where the chunk-parallel kernel does not take the row.
+static ChangeRoute change_route(const mmf_plan* p, bool want_delta, int first, int rows, int64_t T, bool out_iir,
+                                const SosPar* pa, const SosPar* po, int64_t n_clips) {
+  const mmf_config& c = p->cfg;
+  ChangeRoute r{kChangeUnfused, mfcc_kernel(p), 0};
+  if ((c.flags & MMF_FLAG_UNFUSED_CHANGE) || !pa || (out_iir && !po)) return r;
+  const SosPar* a2 = out_iir ? po : nullptr;
+  const bool split = change_split_out(out_iir, n_clips);
+  if (change_folds(p, want_delta) && n_clips <= 0x7fffffff &&
+      change_fused_lm_supported(*pa, a2, split, c.n_mfcc, c.n_mels, first, rows, T, &r.smem))
+    r.path = kChangeFolded;
+  else if (change_fused_supported(*pa, a2, split, rows, T, &r.smem))
+    r.path = kChangeFused;
+  return r;
+}
+
 // log-mel -> clamp -> MFCC (+delta) -> zero-phase Butterworth per coefficient ->
 // derivative + norm -> output filter.  `cur` bumps through caller-provided workspace.
 static int run_post(mmf_plan* p, unsigned char*& cur, float* logmel, const int* clipmax, int64_t n_clips, int64_t T,
@@ -1268,47 +1315,33 @@ static int run_post(mmf_plan* p, unsigned char*& cur, float* logmel, const int* 
   SosArgs sa, so;
   int rc = fill_sos(prm->sos, prm->n_sections, &sa);
   if (rc) return rc;
-  if (prm->out_kind == 0 && (rc = fill_sos(prm->out_sos, prm->out_n_sections, &so))) return rc;
-  if (T <= sa.padlen) return too_short(sa.padlen);
-  if (prm->out_kind == 0 && T <= so.padlen) return too_short(so.padlen);
-  SosPar pa, po;
-  size_t fsmem = 0;
   const bool out_iir = prm->out_kind == 0;
-  const bool par_ok = !(c.flags & MMF_FLAG_UNFUSED_CHANGE) && sos_par_fill(sa, T, &pa) &&
-                      (!out_iir || sos_par_fill(so, T, &po));
-  // one kernel per clip from log-mel to the curve: clamp + DCT-II (K3) feed the float64 row buffers in
-  // shared memory directly; MFCC / delta go to HBM only if the caller asked for them.  Measured on the
-  // bench workload: 1 % faster than the separate MFCC kernel without a delta output, 1 % slower with
-  // one when the modulation spectrum follows (DESIGN.md section 4) -- hence the default.
-  // Batches: the output filter of the curve runs as its own launch (one warp per clip, all clips at once) instead of
-  // on ONE warp of the per-clip CTA while its other 11 wait (27 % of that kernel's stall samples, ncu round 2); the
-  // raw curve makes an 8 KB round trip per clip.  Same routine on the same buffer contents: bit-identical.
-  const bool split_out = out_iir && par_ok && n_clips >= 32;
-  const bool fold = (c.flags & MMF_FLAG_FOLD_MFCC) || delta_out == nullptr;
-  if (par_ok && fold && !(c.flags & (MMF_FLAG_SEPARATE_MFCC | MMF_FLAG_MMA_DCT)) && n_clips <= 0x7fffffff &&
-      change_fused_lm_supported(pa, out_iir ? &po : nullptr, c.n_mfcc, c.n_mels, first, rows, T, &fsmem)) {
+  if (out_iir && (rc = fill_sos(prm->out_sos, prm->out_n_sections, &so))) return rc;
+  if (T <= sa.padlen) return too_short(sa.padlen);
+  if (out_iir && T <= so.padlen) return too_short(so.padlen);
+  SosPar pa, po;
+  const bool has_pa = sos_par_fill(sa, T, &pa), has_po = out_iir && sos_par_fill(so, T, &po);
+  const ChangeRoute r = change_route(p, delta_out != nullptr, first, rows, T, out_iir, has_pa ? &pa : nullptr,
+                                     has_po ? &po : nullptr, n_clips);
+  float* mfcc = nullptr;
+  if (r.path != kChangeFolded) {
+    mfcc = mfcc_out ? mfcc_out : (float*)carve(cur, (size_t)n_clips * c.n_mfcc * T * 4);
+    if ((rc = mfcc_run(p, r.k3, logmel, clipmax, n_clips, T, mfcc, delta_out, clamp_in_place, st))) return rc;
+  }
+  if (r.path != kChangeUnfused) {
+    // fused per-clip kernel: row filters, derivative + norm and the output filter with the
+    // float64 rows resident in shared memory (script/mfcc.py:393-425)
+    const bool folded = r.path == kChangeFolded, split_out = change_split_out(out_iir, n_clips);
     const FusedMfccArgs lm{p->d_dct, p->nc_pad, logmel, clipmax, c.n_mels, c.top_db, mfcc_out, delta_out,
                            clamp_in_place};
     double* raw = split_out ? (double*)carve(cur, (size_t)n_clips * T * 8) : nullptr;
-    cudaError_t e = change_fused_launch(nullptr, n_clips, c.n_mfcc, first, rows, T, prm->diff_method, pa,
-                                        out_iir ? po : pa, split_out ? 1 : prm->out_kind, split_out ? raw : tot, fsmem,
-                                        &lm, st);
-    if (e == cudaSuccess && split_out) e = sosfiltfilt_par_launch(raw, 0, n_clips, T, T, 1, T, po, tot, T, st);
-    if (e == cudaSuccess) return MMF_OK;
-    if (e != cudaErrorNotSupported) return cuda_fail(e, "change_fused_kernel (from log-mel) launch");
-  }
-  float* mfcc = mfcc_out ? mfcc_out : (float*)carve(cur, (size_t)n_clips * c.n_mfcc * T * 4);
-  if ((rc = mmf_mfcc(p, logmel, clipmax, n_clips, T, mfcc, delta_out, clamp_in_place, st))) return rc;
-  // fused per-clip kernel: row filters, derivative + norm and the output filter with the
-  // float64 rows resident in shared memory (script/mfcc.py:393-425)
-  if (par_ok && change_fused_supported(pa, out_iir ? &po : nullptr, rows, T, &fsmem)) {
-    double* raw = split_out ? (double*)carve(cur, (size_t)n_clips * T * 8) : nullptr;
     cudaError_t e = change_fused_launch(mfcc, n_clips, c.n_mfcc, first, rows, T, prm->diff_method, pa,
-                                        out_iir ? po : pa, split_out ? 1 : prm->out_kind, split_out ? raw : tot, fsmem,
-                                        nullptr, st);
+                                        out_iir ? po : pa, split_out ? 1 : prm->out_kind, split_out ? raw : tot, r.smem,
+                                        folded ? &lm : nullptr, st);
     if (e == cudaSuccess && split_out) e = sosfiltfilt_par_launch(raw, 0, n_clips, T, T, 1, T, po, tot, T, st);
-    if (e == cudaSuccess) return MMF_OK;
-    if (e != cudaErrorNotSupported) return cuda_fail(e, "change_fused_kernel launch");
+    if (e != cudaSuccess)
+      return cuda_fail(e, folded ? "change_fused_kernel (from log-mel) launch" : "change_fused_kernel launch");
+    return MMF_OK;
   }
   double* filt = (double*)carve(cur, (size_t)n_clips * rows * T * 8);
   double* raw = (double*)carve(cur, (size_t)n_clips * T * 8);
@@ -1384,7 +1417,8 @@ struct ChangeVarlen {
   int64_t n_clips = 0;
   int pitch = 0;  // frames per output row: the longest clip's T
   int first = 0, rows = 0;
-  bool out_iir = false, route_a = false, split_out = false;
+  bool split_out = false;
+  ChangePath path = kChangeFolded;  // the batched clips' route: folded, or the FP32 K3 kernel and the fused kernel
   std::vector<int64_t> len;
   std::vector<int> T_all, T_k1, clips;
   std::vector<int2> pidx;
@@ -1416,7 +1450,7 @@ static int change_varlen_route(const mmf_plan* plan, int64_t n_clips, const int6
   SosArgs sa, so;
   int rc = fill_sos(prm->sos, prm->n_sections, &sa);
   if (rc) return rc;
-  const bool out_iir = v.out_iir = prm->out_kind == 0;
+  const bool out_iir = prm->out_kind == 0;
   if (out_iir && (rc = fill_sos(prm->out_sos, prm->out_n_sections, &so))) return rc;
   v.pitch = (int)mmf_num_frames(n_max, c.n_fft, c.hop_length);
   v.T_all.assign((size_t)n_clips, 0);
@@ -1426,14 +1460,9 @@ static int change_varlen_route(const mmf_plan* plan, int64_t n_clips, const int6
     if (v.T_all[i] <= padlen) return too_short(v.T_all[i] <= sa.padlen ? sa.padlen : so.padlen, index_base + i);
   }
 
-  // route A = MFCC folded into the fused kernel, B = FP32 MFCC kernel + fused kernel
-  const bool fold = (c.flags & MMF_FLAG_FOLD_MFCC) || !want_delta;
-  // (more than kFusedNC coefficients never fold: the solo call then takes route B, and so does the batch)
-  const bool route_a = v.route_a = fold && !(c.flags & (MMF_FLAG_SEPARATE_MFCC | MMF_FLAG_MMA_DCT)) && c.n_mfcc <= kFusedNC;
-  const bool mfcc_fp32 = !((c.flags & MMF_FLAG_MMA_DCT) && mfcc_mma_supported(c.n_mfcc, c.n_mels)) &&
-                         plan->d_dct_tc == nullptr;
-  const bool batched = !plan->generic && !(c.flags & MMF_FLAG_UNFUSED_CHANGE) && (route_a || mfcc_fp32) &&
-                       sa.n_sections <= kParMaxSections && (!out_iir || so.n_sections == sa.n_sections);
+  // Each clip is routed as its own single-clip call.  The batch takes the clips whose route is its path: folded when
+  // the call folds, else the FP32 K3 kernel (the one that takes per-clip frame counts) and the fused kernel.
+  const ChangePath path = v.path = change_folds(plan, want_delta) ? kChangeFolded : kChangeFused;
   const std::vector<SosPar>& pars = v.tables.pars;
   const int unit = plan->d_mel_tc ? 128 : plan->TF;  // K1 work unit: a 128-frame block or a TF-frame tile
   v.T_k1.assign((size_t)n_clips, 0);
@@ -1444,17 +1473,15 @@ static int change_varlen_route(const mmf_plan* plan, int64_t n_clips, const int6
   int t_big = 0;
   for (int64_t i = 0; i < n_clips; ++i) {
     const int T = v.T_all[i];
-    bool ok = batched;
     int a = -1, b = -1;
-    if (ok) {
+    ChangeRoute r{kChangeUnfused, kMfccFp32, 0};
+    if (!plan->generic) {  // K1's ragged walk does not take the generic n_fft path
       a = v.tables.index(0, sa, T);
       b = out_iir ? v.tables.index(1, so, T) : a;
-      ok = a >= 0 && b >= 0;
+      r = change_route(plan, want_delta, first, rows, T, out_iir, a >= 0 ? &pars[a] : nullptr,
+                       b >= 0 ? &pars[b] : nullptr, 1);
     }
-    size_t sm = 0;
-    if (ok)
-      ok = route_a ? change_fused_lm_supported(pars[a], out_iir ? &pars[b] : nullptr, c.n_mfcc, c.n_mels, first, rows, T, &sm)
-                   : change_fused_supported(pars[a], out_iir ? &pars[b] : nullptr, rows, T, &sm);
+    const bool ok = r.path == path && (path == kChangeFolded || r.k3 == kMfccFp32);
     const uint64_t units = v.first_unit[i] + (ok ? (uint64_t)(T + unit - 1) / unit : 0);
     if (units > 0x7fffffffULL) return fail(MMF_ERR_UNSUPPORTED, "variable-length batch of more than 2^31 K1 blocks");
     v.first_unit[i + 1] = (unsigned)units;
@@ -1467,13 +1494,14 @@ static int change_varlen_route(const mmf_plan* plan, int64_t n_clips, const int6
     v.clips.push_back((int)i);
     if (T > t_big) {
       t_big = T;
-      v.fsmem = sm;
+      v.fsmem = r.smem;
       v.i1 = a;
       v.i2 = b;
     }
   }
   const int64_t nv = (int64_t)v.clips.size();
-  v.split_out = out_iir && nv >= 32;  // the batched output filter, as run_post does for a batch
+  if (!nv) v.tables.pars.clear();  // every clip takes the single-clip path: no launch reads the tables
+  v.split_out = change_split_out(out_iir, nv);
 
   // workspace: descriptors, then the batched intermediates, then the single-clip region
   const size_t n = (size_t)n_clips;
@@ -1488,7 +1516,7 @@ static int change_varlen_route(const mmf_plan* plan, int64_t n_clips, const int6
   size_t off = align_up(v.desc.size(), 256);
   v.o_logmel = (nv && !want_logmel) ? ws_take(off, n * c.n_mels * pitch * 4) : 0;
   v.o_clipmax = ws_take(off, n * 4);
-  v.o_mfcc = (nv && !route_a && !want_mfcc) ? ws_take(off, n * c.n_mfcc * pitch * 4) : 0;
+  v.o_mfcc = (nv && path == kChangeFused && !want_mfcc) ? ws_take(off, n * c.n_mfcc * pitch * 4) : 0;
   v.o_raw = v.split_out ? ws_take(off, n * pitch * 8) : 0;
   v.o_single = off;
   size_t single_bytes = 0;
@@ -1537,24 +1565,17 @@ static int change_varlen_run(mmf_plan* plan, const ChangeVarlen& v, unsigned cha
     double* raw = v.split_out ? (double*)(base + v.o_raw) : nullptr;
     const SosPar& pa = v.tables.pars[v.i1];
     const SosPar& po = v.tables.pars[v.i2];
-    cudaError_t e;
-    if (v.route_a) {
-      const FusedMfccArgs lm{plan->d_dct, plan->nc_pad, logmel, clipmax, c.n_mels, c.top_db, mfcc_dev, delta_dev, clamp};
-      e = change_fused_launch(nullptr, nv, c.n_mfcc, first, rows, pitch, prm->diff_method, pa, po,
-                              v.split_out ? 1 : prm->out_kind, v.split_out ? raw : tot_dev, v.fsmem, &lm, st, &fvl);
-    } else {
-      float* mfcc = mfcc_dev ? mfcc_dev : (float*)(base + v.o_mfcc);
-      e = cudaSuccess;
-      for (int64_t c0 = 0; c0 < n_clips && e == cudaSuccess; c0 += 65535) {
-        const int64_t nc = std::min<int64_t>(65535, n_clips - c0);
-        e = mfcc_launch(plan->d_dct, plan->nc_pad, logmel + (size_t)c0 * c.n_mels * pitch, clipmax + c0, nc, pitch,
-                        c.n_mels, c.n_mfcc, c.top_db, mfcc + (size_t)c0 * c.n_mfcc * pitch,
-                        delta_dev ? delta_dev + (size_t)c0 * c.n_mfcc * pitch : nullptr, clamp, st, d_tk1 + c0);
-      }
-      if (e != cudaSuccess) return cuda_fail(e, "mfcc_kernel (variable-length) launch");
-      e = change_fused_launch(mfcc, nv, c.n_mfcc, first, rows, pitch, prm->diff_method, pa, po,
-                              v.split_out ? 1 : prm->out_kind, v.split_out ? raw : tot_dev, v.fsmem, nullptr, st, &fvl);
+    const bool folded = v.path == kChangeFolded;
+    const FusedMfccArgs lm{plan->d_dct, plan->nc_pad, logmel, clipmax, c.n_mels, c.top_db, mfcc_dev, delta_dev, clamp};
+    float* mfcc = nullptr;
+    if (!folded) {
+      mfcc = mfcc_dev ? mfcc_dev : (float*)(base + v.o_mfcc);
+      if ((rc = mfcc_run(plan, kMfccFp32, logmel, clipmax, n_clips, pitch, mfcc, delta_dev, clamp, st, d_tk1)))
+        return rc;
     }
+    cudaError_t e = change_fused_launch(mfcc, nv, c.n_mfcc, first, rows, pitch, prm->diff_method, pa, po,
+                                        v.split_out ? 1 : prm->out_kind, v.split_out ? raw : tot_dev, v.fsmem,
+                                        folded ? &lm : nullptr, st, &fvl);
     if (e == cudaSuccess && v.split_out) e = sosfiltfilt_par_varlen_launch(raw, 0, nv, pitch, po, fvl, tot_dev, st);
     if (e != cudaSuccess) return cuda_fail(e, "change_fused_kernel (variable-length) launch");
   }
@@ -1590,11 +1611,10 @@ static int change_varlen_run(mmf_plan* plan, const ChangeVarlen& v, unsigned cha
 extern "C" {
 
 // Variable-length batch.  Each clip takes the route its own mmf_mfcc_change call would take -- which is what makes
-// its outputs bit-identical to that call: K1 is a decision of the configuration alone, the post-MFCC route depends on
-// the clip's T (the chunk-parallel IIR needs T + 2 padlen <= 6112, the fused kernel T <= 3456 and its shared memory).
-// Clips on the default routes -- clamp + DCT-II folded into the fused kernel, or the FP32 MFCC kernel followed by it
-// -- run in one launch per stage for the whole batch, each with the chunk tables (SosPar) of its own length; any other
-// clip runs the single-clip path in workspace and is copied into its padded rows.
+// its outputs bit-identical to that call: K1 is a decision of the configuration alone, the post-MFCC route
+// (change_route) depends on the clip's T.  Clips on the batch's route run in one launch per stage for the whole batch,
+// each with the chunk tables (SosPar) of its own length; any other clip runs the single-clip path in workspace and is
+// copied into its padded rows.
 int mmf_mfcc_change_varlen(mmf_plan* plan, const float* pcm_dev, int64_t n_clips, const int64_t* n_samples_host,
                            int64_t clip_stride, const mmf_change_params* prm, double* tot_dev, float* logmel_dev,
                            float* mfcc_dev, float* delta_dev, void* stream) {

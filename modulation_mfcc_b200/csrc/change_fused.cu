@@ -561,8 +561,11 @@ static size_t fused_row_doubles(const SosPar& a1, const SosPar* a2, int rows) {
   return doubles;
 }
 
-bool change_fused_supported(const SosPar& a1, const SosPar* a2, int rows, long T, size_t* smem_out) {
+bool change_fused_supported(const SosPar& a1, const SosPar* a2, bool split_out, int rows, long T, size_t* smem_out) {
   if (rows < 1 || T < 1 || T > (long)kFusedMaxWarps * 32 * kFusedPerThread) return false;
+  // equal section counts (the reference's default: outFilter None reuses the row filter, 'iir' uses the same order)
+  // get an instantiation; a kernel that leaves the output filter to its own launch instantiates the row filter only
+  if (a2 && !split_out && a2->ns != a1.ns) return false;
   const size_t smem = fused_row_doubles(a1, a2, rows) * sizeof(double);
   if (smem > 220 * 1024) return false;
   if (smem_out) *smem_out = smem;
@@ -570,10 +573,10 @@ bool change_fused_supported(const SosPar& a1, const SosPar* a2, int rows, long T
 }
 
 // with the MFCC stage folded in: + the DCT table
-bool change_fused_lm_supported(const SosPar& a1, const SosPar* a2, int n_mfcc, int n_mels, int first, int rows,
-                               long T, size_t* smem_out) {
+bool change_fused_lm_supported(const SosPar& a1, const SosPar* a2, bool split_out, int n_mfcc, int n_mels, int first,
+                               int rows, long T, size_t* smem_out) {
   size_t base = 0;
-  if (n_mfcc > kFusedNC || !change_fused_supported(a1, a2, rows, T, &base)) return false;
+  if (n_mfcc > kFusedNC || !change_fused_supported(a1, a2, split_out, rows, T, &base)) return false;
   const size_t smem = base + (size_t)n_mels * kFusedNC * sizeof(float);
   if (smem > 220 * 1024) return false;
   if (smem_out) *smem_out = smem;
@@ -607,8 +610,7 @@ static cudaError_t fused_launch_cl(const float* mfcc, long n_clips, int n_mfcc, 
 cudaError_t change_fused_launch(const float* mfcc, long n_clips, int n_mfcc, int first, int rows, long T, int method,
                                 const SosPar& a1, const SosPar& a2, int out_kind, double* tot, size_t smem,
                                 const FusedMfccArgs* lm, cudaStream_t st, const FusedVarlen* vl) {
-  // equal section counts (the reference's default: outFilter None reuses the row filter, 'iir' uses
-  // the same order) get an instantiation; anything else goes through the unfused kernels
+  // one instantiation per equal section count (change_fused_supported)
   const int k = a1.ns * 10 + (out_kind == 0 ? a2.ns : a1.ns);
   switch (k) {
 #define MMF_FUSED_CASE(A, B)                                                                                          \

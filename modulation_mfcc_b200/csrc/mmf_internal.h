@@ -196,7 +196,9 @@ cudaError_t sosfiltfilt_par_launch(const void* x, int x_is_f32, long rows, long 
 bool sos_long_supported(const SosArgs& a, long rows, long T);
 cudaError_t sosfiltfilt_long_launch(const void* x, int x_is_f32, long rows, long T, long xs, int group_rows,
                                     long group_stride, const SosArgs& a, double* y, long ys, cudaStream_t st);
-bool change_fused_supported(const SosPar& a1, const SosPar* a2, int rows, long T, size_t* smem_out);
+// a2: the output filter's tables (null: none); they size shared memory either way.  split_out: the kernel writes the
+// raw curve and the output filter runs as its own launch
+bool change_fused_supported(const SosPar& a1, const SosPar* a2, bool split_out, int rows, long T, size_t* smem_out);
 // K3 folded into the fused kernel (lm != nullptr) takes up to kFusedNC coefficients
 constexpr int kFusedNC = 16;
 // K3 folded into the fused kernel (lm != nullptr): the clip's MFCC rows go from the DCT straight into
@@ -212,8 +214,8 @@ struct FusedMfccArgs {
   float* delta_out;
   int clamp_in_place;
 };
-bool change_fused_lm_supported(const SosPar& a1, const SosPar* a2, int n_mfcc, int n_mels, int first, int rows,
-                               long T, size_t* smem_out);
+bool change_fused_lm_supported(const SosPar& a1, const SosPar* a2, bool split_out, int n_mfcc, int n_mels, int first,
+                               int rows, long T, size_t* smem_out);
 // variable-length batch of the fused kernel and the batched output filter: launch item b is clip clips[b] with T[clip]
 // frames and the cascade tables pars[pidx[clip].x] (row filter) / pars[pidx[clip].y] (output filter); the launch's
 // T is the row pitch and its SosPar arguments are the ones with the largest chunk (they size shared memory).  off

@@ -6,6 +6,7 @@ element at a frame >= T_i is exactly 0, and nothing past a clip's length is ever
 """
 
 import ctypes as C
+import re
 
 import numpy as np
 import pytest
@@ -42,7 +43,9 @@ def _cfg(name, flags=0):
 
 def _params(tStep, out_filter, remove_first=1, diff_method=0):
     sos = scipy.signal.butter(6, 12 / ((1 / tStep) / 2), "low", output="sos")
-    out = {"none": sos, "iir": scipy.signal.butter(6, 10 / ((1 / tStep) / 2), "low", output="sos"), "raw": None}
+    butter = lambda n: scipy.signal.butter(n, 10 / ((1 / tStep) / 2), "low", output="sos")  # noqa: E731
+    # iir4: 2 output-filter sections against the row filter's 3
+    out = {"none": sos, "iir": butter(6), "iir4": butter(4), "raw": None}
     return mm.make_change_params(sos, remove_first=remove_first, diff_method=diff_method, out_sos=out[out_filter]), sos
 
 
@@ -103,7 +106,11 @@ def _check_against_solo(plan, clips, prm, want_delta, want_feats=True):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", list(CONFIGS))
-@pytest.mark.parametrize("flags", [0, _lib.MMF_FLAG_NO_TC_MEL, _lib.MMF_FLAG_NO_TMA, _lib.MMF_FLAG_FOLD_MFCC])
+@pytest.mark.parametrize(
+    "flags",
+    [0, _lib.MMF_FLAG_NO_TC_MEL, _lib.MMF_FLAG_NO_TMA, _lib.MMF_FLAG_FOLD_MFCC, _lib.MMF_FLAG_SEPARATE_MFCC,
+     _lib.MMF_FLAG_MMA_DCT, _lib.MMF_FLAG_TC_DCT, _lib.MMF_FLAG_UNFUSED_CHANGE],
+)
 @pytest.mark.parametrize("want_delta", [False, True])
 def test_varlen_matches_solo_calls(name, flags, want_delta, cuda_device):
     """Every clip of a 40-clip batch (so the batched output filter runs) equals its own single-clip call."""
@@ -119,7 +126,7 @@ def test_varlen_matches_solo_calls(name, flags, want_delta, cuda_device):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("out_filter", ["none", "iir", "raw"])
+@pytest.mark.parametrize("out_filter", ["none", "iir", "raw", "iir4"])  # iir4: the solo call runs unfused
 @pytest.mark.parametrize("remove_first", [0, 1])
 @pytest.mark.parametrize("diff_method", [0, 1])
 def test_varlen_change_parameters(out_filter, remove_first, diff_method, cuda_device):
@@ -211,6 +218,75 @@ def test_one_launch_per_stage(name, max_frames, want_delta, cuda_device):
         counts.append(_lib.lib().mmf_launch_count(1))
     assert counts[0] == counts[1], counts
     assert counts[0] <= 7, counts
+
+
+# change-stage kernels -> route tokens (K1 kernels and copies are ignored); names demangled or mangled
+_CHANGE_KERNELS = {"mfcc_pk_kernel": "pk", "mfcc_kernel": "fp32", "mfcc_mma_kernel": "mma", "mfcc_tc_kernel": "tc",
+                   "sosfiltfilt_par_kernel": "iir", "sosfiltfilt_kernel": "iir", "sos_long_kernel": "iir",
+                   "sos_long_carry_kernel": "iir", "delta_norm_kernel": "delta_norm"}
+
+
+def _change_route_ran(fn):
+    """Route tokens of the change-stage kernels ``fn`` launches, in launch order; a run of IIR kernels is one "iir"."""
+    torch = _torch()
+    from torch.profiler import ProfilerActivity, profile
+
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    out = []
+    for e in sorted(prof.events(), key=lambda e: e.time_range.start):
+        m = re.search(r"change_fused_kernel(?:<\d+, \d+, (true|false)|ILi\d+ELi\d+ELb([01]))", e.name)
+        tok = ("fused_lm" if m.group(1) == "true" or m.group(2) == "1" else "fused") if m else None
+        for name, t in _CHANGE_KERNELS.items():
+            if tok is None and re.search(r"(?<![a-z_])" + name + r"(?![a-z_0-9])", e.name):
+                tok = t
+        if tok and not (tok == "iir" and out and out[-1] == "iir"):
+            out.append(tok)
+    return out
+
+
+# frames -> the fused kernel forms that take them at cfg1_16k with 12 kept rows and 3-section filters: the folded form
+# needs the DCT table besides the float64 rows in shared memory, so it stops first; 3000 fits the chunk-parallel IIR but
+# no fused form; 7000 neither
+_ROUTE_T = {400: ("lm", "fused"), 2260: ("fused",), 3000: (), 7000: ()}
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize(
+    "flags",
+    [0, _lib.MMF_FLAG_FOLD_MFCC, _lib.MMF_FLAG_SEPARATE_MFCC, _lib.MMF_FLAG_MMA_DCT, _lib.MMF_FLAG_TC_DCT,
+     _lib.MMF_FLAG_UNFUSED_CHANGE],
+)
+@pytest.mark.parametrize("want_delta", [False, True])
+def test_change_route_table(flags, want_delta, cuda_device):
+    """The kernels the single-clip change stage runs, over T x output filter x batch size.  The variable-length batch
+    sends each clip down this route, so this table pins what it must match."""
+    cfg, tStep = _cfg("cfg1_16k", flags)
+    plan = mm.get_plan(cfg)
+    k3 = {_lib.MMF_FLAG_MMA_DCT: "mma", _lib.MMF_FLAG_TC_DCT: "tc"}.get(flags, "pk")
+    folds = (flags == _lib.MMF_FLAG_FOLD_MFCC or not want_delta) and flags not in (
+        _lib.MMF_FLAG_SEPARATE_MFCC, _lib.MMF_FLAG_MMA_DCT)
+    wrong = []
+    for T, fits in _ROUTE_T.items():
+        for out_filter in ("iir", "iir4", "raw"):
+            prm, _ = _params(tStep, out_filter)
+            for n_clips in (1, 32):
+                split = out_filter != "raw" and n_clips >= 32  # the output filter as its own launch
+                # one instantiation per equal section count: unequal ones fuse only when the filter runs apart
+                fused = flags != _lib.MMF_FLAG_UNFUSED_CHANGE and (out_filter != "iir4" or split)
+                if fused and folds and "lm" in fits:
+                    want = ["fused_lm"] + ["iir"] * split
+                elif fused and "fused" in fits:
+                    want = [k3, "fused"] + ["iir"] * split
+                else:
+                    want = [k3, "iir", "delta_norm"] + ["iir"] * (out_filter != "raw")
+                pcm = _torch().zeros((n_clips, (T - 1) * cfg.hop_length), device="cuda")
+                ran = _change_route_ran(lambda: plan.mfcc_change(pcm, prm, want_delta=want_delta))
+                if ran != want:
+                    wrong.append((T, out_filter, n_clips, want, ran))
+    assert not wrong, wrong
 
 
 @pytest.mark.gpu
