@@ -363,10 +363,53 @@ int mmf_features_host_varlen_amp(mmf_plan* plan, const void* pcm_host, int32_t p
 
 /* Hilbert amplitude envelope |scipy.signal.hilbert(x)| of each row (script/calc.py:284-286, method 'Hilb'),
  * any length n <= 2^26 (an hour at 16 kHz): O(n log n) -- the length-n transforms scipy runs are evaluated as
- * Bluestein chirp transforms over a power-of-two FFT in float64; signals of at most 4096 samples use the
- * equivalent direct circular convolution with the discrete Hilbert kernel. */
+ * Bluestein chirp transforms over a power-of-two FFT in float64, the rows as one batch of mmf_hilbert_varlen;
+ * signals of at most 4096 samples use the equivalent direct circular convolution with the discrete Hilbert
+ * kernel. */
 int mmf_hilbert_envelope(mmf_plan* plan, const float* x_dev, int64_t n_clips, int64_t n, int64_t x_stride,
                          float* amp_dev, int64_t amp_stride, void* stream);
+
+/* mmf_hilbert_envelope for packed clips of different lengths: clip i of the packed float32
+ * x_dev[offsets_host[i] .. offsets_host[i+1]) has its envelope at the same range of amp_dev, counted from
+ * offsets_host[0] (amp_dev holds offsets_host[n_clips] - offsets_host[0] floats).  Each block is bit-identical to
+ * mmf_hilbert_envelope on that clip alone.  Clips of more than 4096 samples run together in a fixed number of
+ * launches (the chirp tables once per distinct length, then five FFTs of two or three pass-group launches each),
+ * in sub-batches of bounded scratch; shorter ones one by one.  The offsets are checked as mmf_rms_varlen checks
+ * them; a clip over 2^26 samples fails with MMF_ERR_UNSUPPORTED naming the clip; every check runs before anything
+ * is queued.  Asynchronous on `stream`. */
+int mmf_hilbert_varlen(mmf_plan* plan, const float* x_dev, int64_t n_clips, const int64_t* offsets_host,
+                       float* amp_dev, void* stream);
+
+/* The envelope of the host-buffer bundle (calculate_amplitude_envelope, script/calc.py:221-343, outFilter None or
+ * 'iir'): method MMF_ENV_RMS (frame geometry per clip, center) or MMF_ENV_HILBERT (one output per sample; center
+ * and the geometry are not read).  out_n_sections and out_sos as in mmf_amp_params. */
+#define MMF_ENV_RMS 0
+#define MMF_ENV_HILBERT 1
+typedef struct {
+  int32_t method;
+  int32_t center;
+  int32_t out_n_sections;
+  double out_sos[16 * 6];
+} mmf_env_params;
+
+/* Host-only: output offsets of the envelopes of a packed batch.  RMS: mmf_amp_varlen_sizes with env->center.
+ * Hilbert: amp_off_host = prefix sums of the clip lengths (geom_host may be NULL); a clip over 2^26 samples fails
+ * with MMF_ERR_UNSUPPORTED naming the clip.  An unknown method fails with MMF_ERR_INVALID. */
+int mmf_env_varlen_sizes(int64_t n_clips, const int64_t* offsets_host, const mmf_env_params* env,
+                         const int32_t* geom_host, int64_t* amp_off_host);
+
+/* mmf_features_host_varlen_amp with the envelope method in env (mmf_features_host_varlen_amp is this call with
+ * method MMF_ENV_RMS).  The Hilbert envelope of each chunk is taken from its copied native samples (float32, or
+ * int16 scaled by 1/32768) on the chunk's stream: equal, bit for bit, to mmf_hilbert_envelope on the clip alone
+ * and, with a filter, then to mmf_sosfiltfilt (x_is_f32 = 1) on that envelope; these long rows are filtered one by
+ * one.  With a filter, an envelope of at most padlen samples fails with MMF_ERR_TOO_SHORT naming the clip, before
+ * anything is queued. */
+int mmf_features_host_varlen_env(mmf_plan* plan, const void* pcm_host, int32_t pcm16, int64_t n_clips,
+                                 const int64_t* offsets_host, const mmf_resample_clip* rs_host, const float* h_host,
+                                 int64_t n_h, const mmf_change_params* prm, const mmf_modspec_params* mod,
+                                 const mmf_env_params* env, const int32_t* geom_host, double* tot_host,
+                                 float* mfcc_host, float* delta_host, float* mag_host, float* band_host,
+                                 float* amp_host, double* amp_filt_host);
 
 /* Local extrema of each float64 row with scipy.signal.find_peaks' default semantics (strictly higher
  * than both neighbours; a flat top reports its middle sample; end samples never qualify) -- the
@@ -397,8 +440,8 @@ int mmf_mfcc_change_host(mmf_plan* plan, const float* pcm_host, int64_t n_clips,
                          int64_t clip_stride, const mmf_change_params* prm, double* tot_host, float* mfcc_host);
 
 /* sizeof() of the ABI structs as this library was compiled (0: mmf_config,
- * 1: mmf_change_params, 2: mmf_modspec_params, 3: mmf_resample_clip, 4: mmf_amp_params) so bindings can verify their
- * layout. */
+ * 1: mmf_change_params, 2: mmf_modspec_params, 3: mmf_resample_clip, 4: mmf_amp_params, 5: mmf_env_params) so
+ * bindings can verify their layout. */
 int mmf_abi_sizeof(int32_t which);
 
 /* Number of kernels this library has launched on the calling thread since the

@@ -121,6 +121,19 @@ class mmf_amp_params(C.Structure):
     ]
 
 
+MMF_ENV_RMS = 0
+MMF_ENV_HILBERT = 1
+
+
+class mmf_env_params(C.Structure):
+    _fields_ = [
+        ("method", C.c_int32),
+        ("center", C.c_int32),
+        ("out_n_sections", C.c_int32),
+        ("out_sos", C.c_double * 96),
+    ]
+
+
 OBJ_DIR = PKG_DIR / "build"
 
 
@@ -239,7 +252,14 @@ _SIGNATURES = {
         [_vp, _vp, _i32, _i64, _vp, _vp, _vp, _i64, C.POINTER(mmf_change_params), C.POINTER(mmf_modspec_params),
          C.POINTER(mmf_amp_params), _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     ),
+    "mmf_features_host_varlen_env": (
+        C.c_int,
+        [_vp, _vp, _i32, _i64, _vp, _vp, _vp, _i64, C.POINTER(mmf_change_params), C.POINTER(mmf_modspec_params),
+         C.POINTER(mmf_env_params), _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    ),
     "mmf_amp_varlen_sizes": (C.c_int, [_i64, _vp, _vp, _i32, _vp]),
+    "mmf_env_varlen_sizes": (C.c_int, [_i64, _vp, C.POINTER(mmf_env_params), _vp, _vp]),
+    "mmf_hilbert_varlen": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _vp]),
     "mmf_rms_varlen": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _i32, _vp, _vp]),
     "mmf_pcm16_to_f32": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
     "mmf_hilbert_envelope": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _vp, _i64, _vp]),

@@ -775,13 +775,14 @@ def calculate_amplitude_envelope_many(
     outFiltPolyOrd=3,
     device=None,
 ):
-    """:func:`calculate_amplitude_envelope` (method ``'RMS'``) for a list of 1-D clips of any lengths: one packed
-    upload and one ``mmf_rms_varlen`` launch for all of them.  ``sr`` is one rate for every clip or one rate per clip;
-    each clip's frame geometry is ``int(winLen * sr_i)``, ``int(hopLen * sr_i)``.  The output filter, if any, runs per
-    clip as the single call runs it.  Returns one ``(amp, ampT)`` per clip, equal to
-    ``calculate_amplitude_envelope(clip, sr_i, ...)`` bit for bit; an error names the clip's index."""
-    if method != "RMS":
-        raise ValueError(f"calculate_amplitude_envelope_many takes method 'RMS' only, not {method!r}")
+    """:func:`calculate_amplitude_envelope` (method ``'RMS'`` or ``'Hilb'``) for a list of 1-D clips of any lengths:
+    one packed upload and one ragged call for all of them (``mmf_rms_varlen`` or ``mmf_hilbert_varlen``).  ``sr`` is
+    one rate for every clip or one rate per clip; each clip's RMS frame geometry is ``int(winLen * sr_i)``,
+    ``int(hopLen * sr_i)``.  The output filter, if any, runs per clip as the single call runs it.  Returns one
+    ``(amp, ampT)`` per clip, equal to ``calculate_amplitude_envelope(clip, sr_i, ...)`` bit for bit; an error names
+    the clip's index."""
+    if method not in ("RMS", "Hilb"):
+        raise ValueError(f"calculate_amplitude_envelope_many takes method 'RMS' or 'Hilb', not {method!r}")
     clips = [np.asarray(c) for c in clips]
     if any(c.ndim != 1 for c in clips):
         raise ValueError("calculate_amplitude_envelope_many takes 1-D clips")
@@ -797,7 +798,10 @@ def calculate_amplitude_envelope_many(
     geom = [(int(winLen * r), int(hopLen * r)) for r in rates]
     try:
         packed = np.concatenate([c.astype(np.float32, copy=False) for c in clips])
-        amp, amp_off = plan.rms_varlen(packed, offsets, geom, bool(center))
+        if method == "RMS":
+            amp, amp_off = plan.rms_varlen(packed, offsets, geom, bool(center))
+        else:
+            amp, amp_off = plan.hilbert_varlen(packed, offsets)
         out = []
         host = amp.cpu().numpy() if outFilter is None else None
         for i in range(len(clips)):
@@ -871,7 +875,11 @@ class FeatureExtractor:
         amp_outFiltType="low",
         amp_outFiltCutOff=[12],
         amp_outFiltLen=6,
+        amp_method: str = "RMS",
     ):
+        if amp_method not in ("RMS", "Hilb"):
+            raise ValueError(f"the feature bundle takes amp_method 'RMS' or 'Hilb', not {amp_method!r}")
+        self.amp_method = amp_method
         # the envelope's output filter is validated before any device work, with applyFilter's exceptions
         if amp_outFilter is None:
             self.amp_sos = None
@@ -920,15 +928,15 @@ class FeatureExtractor:
         resampled to the extractor's rate on the device as the WAV loader resamples them, and each clip's blocks
         equal :meth:`host_call` on the loader's resampled clip.
 
-        ``"amplitude"`` in ``want`` adds each clip's RMS envelope with this extractor's ``amp_*`` settings, taken at
-        the clip's own rate (``rates``, else the extractor's) from its native samples (int16 scaled by 1/32768):
-        ``amplitude`` packed at ``amp_offsets``; clip ``i``'s block equals :func:`calculate_amplitude_envelope` on that
-        clip as float32, bit for bit."""
+        ``"amplitude"`` in ``want`` adds each clip's envelope with this extractor's ``amp_*`` settings (``amp_method``
+        'RMS' or 'Hilb'), taken at the clip's own rate (``rates``, else the extractor's) from its native samples (int16
+        scaled by 1/32768): ``amplitude`` packed at ``amp_offsets``; clip ``i``'s block equals
+        :func:`calculate_amplitude_envelope` on that clip as float32, bit for bit."""
         mod = self.modspec_geometry(0) if ("modspec" in want or "band_energy" in want) else None
         try:
             amp = self._amp(want, len(offsets) - 1, rates)
             return self.plan.features_host_varlen(pcm_host, offsets, self.prm, mod, want=want, out=out, rates=rates,
-                                                  amp=amp)
+                                                  amp=amp, amp_method=self.amp_method)
         except MmfError as e:
             _raise_from(e)
 

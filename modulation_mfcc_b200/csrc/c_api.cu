@@ -519,6 +519,7 @@ int mmf_abi_sizeof(int32_t which) {
     case 2: return (int)sizeof(mmf_modspec_params);
     case 3: return (int)sizeof(mmf_resample_clip);
     case 4: return (int)sizeof(mmf_amp_params);
+    case 5: return (int)sizeof(mmf_env_params);
     default: return -1;
   }
 }
@@ -1652,6 +1653,11 @@ namespace mmf {
 // audio-s/s (small chunks pay launch + copy set-up, large ones a longer unoverlapped head and tail); int16 host input
 // moves half the bytes per clip and keeps gaining up to 96 MB (0.94 / 1.16 / 1.25 / 1.34 / 1.37 / 1.44 M)
 constexpr size_t kHostChunkF32 = 32u << 20, kHostChunkI16 = 96u << 20;
+// Scratch of one sub-batch of a ragged Hilbert envelope (two M-point float64 work buffers per clip, the chirp and the
+// transformed chirp filter per distinct length, the twiddles): a batch over it runs as several sub-batches of the
+// same few launches, a clip over it alone.  At 2 GB a sub-batch holds about 120 clips of 10 s at 16 kHz (M = 2^19),
+// some 15 000 CTAs per pass-group launch.
+constexpr size_t kHilbertScratch = 2ull << 30;
 
 // Runs `body`, which queues work on both plan streams, then drains both streams whatever it returned: queued copies
 // target caller-owned host buffers.  The body's error comes first.
@@ -1872,11 +1878,181 @@ static int amp_sizes(int64_t n_clips, const int64_t* offsets, const int32_t* geo
   return MMF_OK;
 }
 
+// Envelope geometry of a packed batch (mmf_env_varlen_sizes) after the offsets passed validate_offsets: RMS as
+// amp_sizes; Hilbert one output per sample, at most 2^26 samples per clip
+static int env_sizes(int64_t n_clips, const int64_t* offsets, const mmf_env_params* env, const int32_t* geom,
+                     int64_t* amp_off) {
+  char buf[160];
+  if (env->method == MMF_ENV_RMS) return amp_sizes(n_clips, offsets, geom, env->center, amp_off);
+  if (env->method != MMF_ENV_HILBERT) {
+    std::snprintf(buf, sizeof(buf), "unknown envelope method %d (MMF_ENV_RMS 0, MMF_ENV_HILBERT 1)", env->method);
+    return fail(MMF_ERR_INVALID, buf);
+  }
+  amp_off[0] = 0;
+  for (int64_t i = 0; i < n_clips; ++i) {
+    const int64_t len = offsets[i + 1] - offsets[i];
+    if (len > (1LL << 26)) {
+      std::snprintf(buf, sizeof(buf), "clip %lld: %lld samples; the Hilbert envelope takes at most 2^26",
+                    (long long)i, (long long)len);
+      return fail(MMF_ERR_UNSUPPORTED, buf);
+    }
+    amp_off[i + 1] = amp_off[i] + len;
+  }
+  return MMF_OK;
+}
+
+// The Hilbert route of a batch: clips of at most kHilDirectMax samples one by one through the direct convolution
+// (direct: n, src, out of each), the others in sub-batches of one hilbert_varlen_launch each
+struct HilSub {
+  size_t o_tab = 0, o_clip = 0, o_tab_first = 0, o_clip_first = 0, o_chirp_first = 0;  // in the route's DescBlob
+  HilBatch b{};        // counts, groups and twiddle offset; the pointers are set at run time
+  size_t scratch = 0;  // bytes of the sub-batch's scratch
+};
+struct HilbertVarlen {
+  std::vector<HilSub> subs;
+  std::vector<HilRow> direct;
+};
+
+static int hil_log2(long n) {
+  int m = 0;
+  while ((1L << m) < 2 * n - 1) ++m;
+  return m;
+}
+
+// one sub-batch of the clips `rows` (n, src, out set): the tables of each distinct n, shared by its clips, the work
+// buffers and the twiddles of the largest M in one scratch allocation (double2 offsets, 256-byte aligned regions);
+// rows ordered three-group rows first
+static void hilbert_sub(std::vector<HilRow> rows, HilbertVarlen& h, DescBlob& desc) {
+  auto region = [](long& end, long elems) {
+    const long o = end;
+    end += (elems + 15) & ~15L;
+    return o;
+  };
+  int mw = 0;
+  for (const HilRow& r : rows) mw = std::max(mw, hil_log2(r.n));
+  long end = 0;
+  const long w = region(end, 1L << (mw - 1));
+  std::vector<HilRow> tab;
+  for (size_t k = 0; k < rows.size(); ++k) {
+    HilRow& r = rows[k];
+    r.m = hil_log2(r.n);
+    r.G = hilbert_groups(r.m, r.L);
+    r.inv_env = 1.0 / ((double)(1L << r.m) * (double)r.n);
+    int t = -1;
+    for (size_t q = 0; q < tab.size() && t < 0; ++q)
+      if (tab[q].n == r.n) t = (int)q;
+    if (t < 0) {
+      t = (int)tab.size();
+      HilRow tr = r;
+      tr.c = region(end, r.n);
+      tr.bf = tr.buf0 = region(end, 1L << r.m);
+      tab.push_back(tr);
+    }
+    r.c = tab[t].c;
+    r.bf = tab[t].bf;
+    r.buf0 = region(end, 1L << r.m);
+    r.buf1 = region(end, 1L << r.m);
+    if (tab[t].buf1 == 0) tab[t].buf1 = r.buf0;  // the chirp filter's other buffer: its first clip's (offset 0 is w)
+  }
+  HilSub sb;
+  HilBatch& b = sb.b;
+  b.w = w;
+  b.mw = mw;
+  b.G = 2;
+  auto order = [&](std::vector<HilRow>& v, long& n3, long& items, long& items3, size_t& o_rows, size_t& o_first) {
+    std::stable_partition(v.begin(), v.end(), [](const HilRow& r) { return r.G == 3; });
+    std::vector<unsigned> first(v.size() + 1, 0);
+    n3 = 0;
+    for (size_t k = 0; k < v.size(); ++k) {
+      first[k + 1] = first[k] + (unsigned)hilbert_items(v[k].m);
+      if (v[k].G == 3) n3 = (long)k + 1, b.G = 3;
+    }
+    items = first[v.size()];
+    items3 = first[n3];
+    o_rows = desc.put(v);
+    o_first = desc.put(first);
+  };
+  b.n_tab = (long)tab.size();
+  b.n_clip = (long)rows.size();
+  order(tab, b.n_tab3, b.tab_items, b.tab_items3, sb.o_tab, sb.o_tab_first);
+  order(rows, b.n_clip3, b.clip_items, b.clip_items3, sb.o_clip, sb.o_clip_first);
+  std::vector<unsigned> chirp(tab.size() + 1, 0);
+  for (size_t q = 0; q < tab.size(); ++q) chirp[q + 1] = chirp[q] + (unsigned)((tab[q].n + 255) / 256);
+  b.chirp_items = chirp[tab.size()];
+  sb.o_chirp_first = desc.put(chirp);
+  sb.scratch = (size_t)end * 16;
+  h.subs.push_back(sb);
+}
+
+// clips k < n.size(): n[k] samples at x + src[k], envelope at amp + out[k].  Sub-batches: maximal runs of the FFT
+// clips whose scratch stays within kHilbertScratch
+static void hilbert_route(const std::vector<long>& src, const std::vector<long>& n, const std::vector<long>& out,
+                          HilbertVarlen& h, DescBlob& desc) {
+  std::vector<HilRow> cur;
+  std::vector<long> lens;
+  size_t bytes = 0;
+  int mw = 0;
+  for (size_t k = 0; k < n.size(); ++k) {
+    HilRow r{};
+    r.n = n[k];
+    r.src = src[k];
+    r.out = out[k];
+    if (n[k] <= kHilDirectMax) {
+      h.direct.push_back(r);
+      continue;
+    }
+    const int m = hil_log2(n[k]);
+    const size_t M16 = ((size_t)16 << m) + 256, tables = M16 + (size_t)n[k] * 16 + 256;
+    bool seen = std::find(lens.begin(), lens.end(), n[k]) != lens.end();
+    if (!cur.empty() && bytes + 2 * M16 + (seen ? 0 : tables) + ((size_t)8 << std::max(mw, m)) > kHilbertScratch) {
+      hilbert_sub(std::move(cur), h, desc);
+      cur.clear();
+      lens.clear();
+      bytes = 0;
+      mw = 0;
+      seen = false;
+    }
+    cur.push_back(r);
+    if (!seen) lens.push_back(n[k]);
+    bytes += 2 * M16 + (seen ? 0 : tables);
+    mw = std::max(mw, m);
+  }
+  if (!cur.empty()) hilbert_sub(std::move(cur), h, desc);
+}
+
+// Device half: every sub-batch in stream-ordered scratch, then the direct clips, on `st`.  dd: the descriptors there
+static int hilbert_run(const HilbertVarlen& h, const unsigned char* dd, const void* x, int pcm16, float* amp,
+                       int sm_count, cudaStream_t st) {
+  for (const HilSub& sb : h.subs) {
+    HilBatch b = sb.b;
+    b.tab = (const HilRow*)(dd + sb.o_tab);
+    b.clip = (const HilRow*)(dd + sb.o_clip);
+    b.tab_first = (const unsigned*)(dd + sb.o_tab_first);
+    b.clip_first = (const unsigned*)(dd + sb.o_clip_first);
+    b.chirp_first = (const unsigned*)(dd + sb.o_chirp_first);
+    b.x = x;
+    b.pcm16 = pcm16;
+    b.amp = amp;
+    MMF_CUDA(cudaMallocAsync((void**)&b.s, sb.scratch, st));
+    const cudaError_t e = hilbert_varlen_launch(b, st);
+    cudaFreeAsync(b.s, st);
+    if (e != cudaSuccess) return cuda_fail(e, "hilbert_group_kernel launch");
+  }
+  for (const HilRow& r : h.direct) {
+    const void* xr = pcm16 ? (const void*)((const int16_t*)x + r.src) : (const void*)((const float*)x + r.src);
+    const cudaError_t e = hilbert_envelope_launch(xr, pcm16, 1, r.n, r.n, amp + r.out, r.n, sm_count, st);
+    if (e != cudaSuccess) return cuda_fail(e, "hilbert_conv_kernel launch");
+  }
+  return MMF_OK;
+}
+
 // Host half of a ragged RMS envelope (mmf_rms_varlen, the envelope of the host bundle): the descriptors of the
 // envelope launch and, with an output filter, each envelope's route -- that of its own mmf_sosfiltfilt call: the
 // chunk-parallel kernel when it takes the envelope's length (all of them in one launch, each with the tables of its
 // own chunk length), the single-row routes otherwise.
 struct EnvelopeVarlen {
+  int method = MMF_ENV_RMS;
+  HilbertVarlen hil;              // the Hilbert envelope's launches (method MMF_ENV_HILBERT)
   int64_t n_clips = 0;
   std::vector<int64_t> off;       // envelope k: frames [off[k], off[k + 1]) of the output
   const SosArgs* filt = nullptr;  // the output filter (null: none)
@@ -1891,6 +2067,7 @@ struct EnvelopeVarlen {
 
 // Routing of clips [c0, c1) of a packed batch whose amp_sizes are amp_off (host only).  Sources count from `base`,
 // outputs from amp_off[c0].  Returns the number of envelope work items, -1 past 2^31 - 1.
+static void filter_route(EnvelopeVarlen& v);
 static int64_t envelope_route(int64_t c0, int64_t c1, const int64_t* offsets, int64_t base, const int32_t* geom,
                               int center, const int64_t* amp_off, const SosArgs* filt, EnvelopeVarlen& v) {
   const int64_t nc = c1 - c0;
@@ -1913,7 +2090,34 @@ static int64_t envelope_route(int64_t c0, int64_t c1, const int64_t* offsets, in
   first[nc] = (unsigned)items;
   v.off[nc] = amp_off[c1] - amp_off[c0];
   v.rms = RaggedParts{v.desc.put(cl), v.desc.put(first), items};
-  if (!filt) return items;
+  filter_route(v);
+  return items;
+}
+
+// Hilbert routing of clips [c0, c1) (host only): sources count from `base`, outputs from amp_off[c0]
+static void hilbert_env_route(int64_t c0, int64_t c1, const int64_t* offsets, int64_t base, const int64_t* amp_off,
+                              const SosArgs* filt, EnvelopeVarlen& v) {
+  const int64_t nc = c1 - c0;
+  v.method = MMF_ENV_HILBERT;
+  v.n_clips = nc;
+  v.filt = filt;
+  v.off.resize((size_t)nc + 1);
+  std::vector<long> src((size_t)nc), n((size_t)nc), out((size_t)nc);
+  for (int64_t k = 0; k <= nc; ++k) v.off[k] = amp_off[c0 + k] - amp_off[c0];
+  for (int64_t k = 0; k < nc; ++k) {
+    src[k] = (long)(offsets[c0 + k] - base);
+    n[k] = (long)(offsets[c0 + k + 1] - offsets[c0 + k]);
+    out[k] = (long)v.off[k];
+  }
+  hilbert_route(src, n, out, v.hil, v.desc);
+  filter_route(v);
+}
+
+// With an output filter, each envelope's route: that of its own mmf_sosfiltfilt call (see EnvelopeVarlen)
+static void filter_route(EnvelopeVarlen& v) {
+  if (!v.filt) return;
+  const int64_t nc = v.n_clips;
+  const SosArgs* filt = v.filt;
   std::vector<int> T((size_t)nc);
   std::vector<int2> pidx((size_t)nc, int2{0, 0});
   for (int64_t k = 0; k < nc; ++k) {
@@ -1933,16 +2137,20 @@ static int64_t envelope_route(int64_t c0, int64_t c1, const int64_t* offsets, in
   v.o_pidx = v.desc.put(pidx);
   v.o_off = v.desc.put(v.off.data(), (size_t)nc);
   v.o_pars = v.desc.put(v.tables.pars);
-  return items;
 }
 
 // Device half: the envelope launch over x (float32, or int16 when pcm16) into amp and, with the output filter, the
 // batched filter launch and the single-row filters into amp_filt, all on `st`.  dd: v.desc on the device.
 static int envelope_run(const EnvelopeVarlen& v, const unsigned char* dd, const void* x, int pcm16, float* amp,
-                        double* amp_filt, cudaStream_t st) {
-  cudaError_t e = rms_varlen_launch(x, pcm16, (const RmsClip*)(dd + v.rms.clips), (const unsigned*)(dd + v.rms.first),
-                                    (long)v.n_clips, (long)v.rms.items, amp, st);
-  if (e != cudaSuccess) return cuda_fail(e, "rms_varlen_kernel launch");
+                        double* amp_filt, int sm_count, cudaStream_t st) {
+  cudaError_t e;
+  if (v.method == MMF_ENV_HILBERT) {
+    if (const int rc = hilbert_run(v.hil, dd, x, pcm16, amp, sm_count, st)) return rc;
+  } else {
+    e = rms_varlen_launch(x, pcm16, (const RmsClip*)(dd + v.rms.clips), (const unsigned*)(dd + v.rms.first),
+                          (long)v.n_clips, (long)v.rms.items, amp, st);
+    if (e != cudaSuccess) return cuda_fail(e, "rms_varlen_kernel launch");
+  }
   if (amp_filt && !v.par.empty()) {
     const FusedVarlen fvl{(const int*)(dd + v.o_par), (const int*)(dd + v.o_T), (const SosPar*)(dd + v.o_pars),
                           (const int2*)(dd + v.o_pidx), (const long*)(dd + v.o_off)};
@@ -1962,6 +2170,7 @@ static int envelope_run(const EnvelopeVarlen& v, const unsigned char* dd, const 
 template <typename Launch>
 static int run_uploaded(mmf_plan* plan, const DescBlob& desc, cudaStream_t st, Launch&& launch) {
   MMF_CUDA(cudaSetDevice(plan->cfg.device));
+  if (!desc.size()) return launch(nullptr);
   unsigned char* d = nullptr;
   MMF_CUDA(cudaMallocAsync((void**)&d, desc.size(), st));
   const cudaError_t e = cudaMemcpyAsync(d, desc.bytes.data(), desc.size(), cudaMemcpyHostToDevice, st);
@@ -1970,10 +2179,11 @@ static int run_uploaded(mmf_plan* plan, const DescBlob& desc, cudaStream_t st, L
   return rc;
 }
 
-// One ragged RMS launch on `st` over float32 x from the host descriptors of v (no output filter)
+// One ragged envelope (RMS or Hilbert) on `st` over float32 x from the host descriptors of v (no output filter)
 static int rms_run(mmf_plan* plan, const float* x, const EnvelopeVarlen& v, float* out, cudaStream_t st) {
-  return run_uploaded(plan, v.desc, st,
-                      [&](const unsigned char* d) { return envelope_run(v, d, x, 0, out, nullptr, st); });
+  return run_uploaded(plan, v.desc, st, [&](const unsigned char* d) {
+    return envelope_run(v, d, x, 0, out, nullptr, plan->sm_count, st);
+  });
 }
 
 // One ragged resampling launch on `st`: the descriptors at p of `desc`, which takes the taps h[n_h]
@@ -2002,7 +2212,8 @@ static void packed_sizes(int n_fft, int hop, int win, int mod_hop, int64_t n_cli
 // A packed host-buffer call: the arguments of the packed entry points in their order, then what the host-only checks
 // derive from them.  pcm: float32 samples, or (pcm16 != 0) int16 samples converted on the device.  resampled: clip i
 // reaches the plan's rate as rs[i] says, with taps from h_taps[n_h]; otherwise every clip is at the plan's rate.
-// amp_prm: the RMS envelope of each clip's native samples, frame geometry geom[2i], geom[2i + 1], to amp and / or,
+// env_prm: the envelope of each clip's native samples (RMS: frame geometry geom[2i], geom[2i + 1]; Hilbert: one
+// output per sample), to amp and / or,
 // through the output filter, amp_filt (NULL: none, and exactly the launches and copies of the call without it).
 struct PackedBatch {
   const void* pcm;
@@ -2014,7 +2225,7 @@ struct PackedBatch {
   int64_t n_h;
   const mmf_change_params* prm;
   const mmf_modspec_params* mod;
-  const mmf_amp_params* amp_prm;
+  const mmf_env_params* env_prm;
   const int32_t* geom;
   double* tot;
   float *mfcc, *delta, *mag, *band;
@@ -2058,7 +2269,7 @@ struct HostChunk {
 
 // Stage 1 (host only): the checks that precede routing, in the order the callers see them, and the packed sizes
 static int packed_check(const mmf_plan* plan, PackedBatch& b) {
-  const mmf_amp_params* amp = b.amp_prm;
+  const mmf_env_params* amp = b.env_prm;
   int rc = validate_offsets(b.n_clips, b.offsets);
   if (rc) return rc;
   if (b.resampled && (rc = validate_resample(b.n_clips, b.offsets, b.rs, b.h_taps, b.n_h, &b.n_taps))) return rc;
@@ -2067,7 +2278,7 @@ static int packed_check(const mmf_plan* plan, PackedBatch& b) {
   b.want_amp = amp && (b.amp || b.amp_filt);
   if (b.want_amp) {
     b.A.resize(n + 1);
-    if ((rc = amp_sizes(b.n_clips, b.offsets, b.geom, amp->center, b.A.data()))) return rc;
+    if ((rc = env_sizes(b.n_clips, b.offsets, amp, b.geom, b.A.data()))) return rc;
     if (b.amp_filt) {
       if (amp->out_n_sections < 1) return fail(MMF_ERR_INVALID, "amp_filt_host needs out_n_sections >= 1");
       if ((rc = fill_sos(amp->out_sos, amp->out_n_sections, &b.amp_sos))) return rc;
@@ -2125,8 +2336,11 @@ static int route_chunk(const mmf_plan* plan, const PackedBatch& b, HostChunk& h,
   };
   h.frames = packed_rows(b.F);
   h.wins = packed_rows(b.Wo);
-  if (b.want_amp && envelope_route(c0, c1, b.offsets, b.offsets[c0], b.geom, b.amp_prm->center, b.A.data(),
-                                   b.amp_filt ? &b.amp_sos : nullptr, h.env) < 0)
+  const SosArgs* filt = b.amp_filt ? &b.amp_sos : nullptr;
+  if (b.want_amp && b.env_prm->method == MMF_ENV_HILBERT)
+    hilbert_env_route(c0, c1, b.offsets, b.offsets[c0], b.A.data(), filt, h.env);
+  else if (b.want_amp && envelope_route(c0, c1, b.offsets, b.offsets[c0], b.geom, b.env_prm->center, b.A.data(), filt,
+                                        h.env) < 0)
     return fail(MMF_ERR_UNSUPPORTED, "a chunk of more than 2^31 - 1 envelope work items");
   return MMF_OK;
 }
@@ -2207,7 +2421,9 @@ static int run_chunk(mmf_plan* plan, const PackedBatch& b, const HostChunk& h, c
   float* d_amp = b.want_amp ? (float*)dev(s.amp) : nullptr;
   double* d_ampf = b.amp_filt ? (double*)dev(s.amp_filt) : nullptr;
   int rc;
-  if (b.want_amp && (rc = envelope_run(h.env, dd + h.o_env, dev(s.h2d), b.pcm16, d_amp, d_ampf, st))) return rc;
+  if (b.want_amp &&
+      (rc = envelope_run(h.env, dd + h.o_env, dev(s.h2d), b.pcm16, d_amp, d_ampf, plan->sm_count, st)))
+    return rc;
   float* d_pcm = (float*)dev(s.pcm);
   cudaError_t e = resample_rows_launch(dev(s.h2d), b.pcm16, (const RsClip*)(dd + h.stage.clips),
                                        (const unsigned*)(dd + h.stage.first), (long)nc, (long)h.stage.items, taps,
@@ -2326,15 +2542,57 @@ int mmf_features_host_varlen_pcm16(mmf_plan* plan, const int16_t* pcm16_host, in
                                                nullptr, nullptr, tot_host, mfcc_host, delta_host, mag_host, band_host});
 }
 
+int mmf_features_host_varlen_env(mmf_plan* plan, const void* pcm_host, int32_t pcm16, int64_t n_clips,
+                                 const int64_t* offsets_host, const mmf_resample_clip* rs_host, const float* h_host,
+                                 int64_t n_h, const mmf_change_params* prm, const mmf_modspec_params* mod,
+                                 const mmf_env_params* env, const int32_t* geom_host, double* tot_host,
+                                 float* mfcc_host, float* delta_host, float* mag_host, float* band_host,
+                                 float* amp_host, double* amp_filt_host) {
+  return mmf::features_host_varlen_impl(plan, {pcm_host, pcm16 ? 1 : 0, n_clips, offsets_host, rs_host, h_host, n_h,
+                                               prm, mod, env, geom_host, tot_host, mfcc_host, delta_host, mag_host,
+                                               band_host, amp_host, amp_filt_host, rs_host != nullptr});
+}
+
 int mmf_features_host_varlen_amp(mmf_plan* plan, const void* pcm_host, int32_t pcm16, int64_t n_clips,
                                  const int64_t* offsets_host, const mmf_resample_clip* rs_host, const float* h_host,
                                  int64_t n_h, const mmf_change_params* prm, const mmf_modspec_params* mod,
                                  const mmf_amp_params* amp, const int32_t* geom_host, double* tot_host,
                                  float* mfcc_host, float* delta_host, float* mag_host, float* band_host,
                                  float* amp_host, double* amp_filt_host) {
-  return mmf::features_host_varlen_impl(plan, {pcm_host, pcm16 ? 1 : 0, n_clips, offsets_host, rs_host, h_host, n_h,
-                                               prm, mod, amp, geom_host, tot_host, mfcc_host, delta_host, mag_host,
-                                               band_host, amp_host, amp_filt_host, rs_host != nullptr});
+  mmf_env_params env{};
+  if (amp) {
+    env.method = MMF_ENV_RMS;
+    env.center = amp->center;
+    env.out_n_sections = amp->out_n_sections;
+    std::memcpy(env.out_sos, amp->out_sos, sizeof(env.out_sos));
+  }
+  return mmf_features_host_varlen_env(plan, pcm_host, pcm16, n_clips, offsets_host, rs_host, h_host, n_h, prm, mod,
+                                      amp ? &env : nullptr, geom_host, tot_host, mfcc_host, delta_host, mag_host,
+                                      band_host, amp_host, amp_filt_host);
+}
+
+int mmf_env_varlen_sizes(int64_t n_clips, const int64_t* offsets_host, const mmf_env_params* env,
+                         const int32_t* geom_host, int64_t* amp_off_host) {
+  using namespace mmf;
+  int rc = validate_offsets(n_clips, offsets_host);
+  if (rc) return rc;
+  if (!env || !amp_off_host) return fail(MMF_ERR_INVALID, "env and amp_off_host must not be NULL");
+  return env_sizes(n_clips, offsets_host, env, geom_host, amp_off_host);
+}
+
+int mmf_hilbert_varlen(mmf_plan* plan, const float* x_dev, int64_t n_clips, const int64_t* offsets_host,
+                       float* amp_dev, void* stream) {
+  using namespace mmf;
+  int rc = validate_offsets(n_clips, offsets_host);
+  if (rc) return rc;
+  mmf_env_params env{};
+  env.method = MMF_ENV_HILBERT;
+  std::vector<int64_t> A((size_t)n_clips + 1);
+  if ((rc = env_sizes(n_clips, offsets_host, &env, nullptr, A.data()))) return rc;
+  if (!plan || !x_dev || !amp_dev) return fail(MMF_ERR_INVALID, "NULL argument");
+  EnvelopeVarlen v;
+  hilbert_env_route(0, n_clips, offsets_host, 0, A.data(), nullptr, v);
+  return rms_run(plan, x_dev, v, amp_dev, (cudaStream_t)stream);
 }
 
 int mmf_amp_varlen_sizes(int64_t n_clips, const int64_t* offsets_host, const int32_t* geom_host, int32_t center,
@@ -2384,14 +2642,22 @@ int mmf_hilbert_envelope(mmf_plan* plan, const float* x_dev, int64_t n_clips, in
   if (!plan || !x_dev || !amp_dev) return fail(MMF_ERR_INVALID, "NULL argument");
   if (n_clips < 1 || n < 1 || n > (1L << 26)) return fail(MMF_ERR_UNSUPPORTED, "need 1 <= n <= 2^26 samples");
   MMF_CUDA(cudaSetDevice(plan->cfg.device));
-  cudaError_t e;
-  if (n > 4096 && hilbert_fft_supported(n)) {
-    // O(n log n): Bluestein chirp transform over a power-of-two Stockham FFT, float64 (hilbert_fft.cu)
-    e = hilbert_fft_launch(x_dev, n_clips, n, x_stride, amp_dev, amp_stride, (cudaStream_t)stream);
-  } else {
-    // short signals: the equivalent circular convolution with the discrete Hilbert kernel, evaluated directly
-    e = hilbert_envelope_launch(x_dev, n_clips, n, x_stride, amp_dev, amp_stride, plan->sm_count, (cudaStream_t)stream);
+  if (n > kHilDirectMax) {
+    // O(n log n): the rows as one ragged batch of Bluestein transforms (hilbert_fft.cu)
+    EnvelopeVarlen v;
+    v.method = MMF_ENV_HILBERT;
+    v.n_clips = n_clips;
+    std::vector<long> src((size_t)n_clips), len((size_t)n_clips, (long)n), out((size_t)n_clips);
+    for (int64_t i = 0; i < n_clips; ++i) {
+      src[i] = (long)(i * x_stride);
+      out[i] = (long)(i * amp_stride);
+    }
+    hilbert_route(src, len, out, v.hil, v.desc);
+    return rms_run(plan, x_dev, v, amp_dev, (cudaStream_t)stream);
   }
+  // short signals: the equivalent circular convolution with the discrete Hilbert kernel, evaluated directly
+  const cudaError_t e = hilbert_envelope_launch(x_dev, 0, n_clips, n, x_stride, amp_dev, amp_stride, plan->sm_count,
+                                                (cudaStream_t)stream);
   if (e != cudaSuccess) return cuda_fail(e, "hilbert kernels launch");
   return MMF_OK;
 }

@@ -275,11 +275,51 @@ inline int rms_frames_per_item(int frame_length, int hop) {
 cudaError_t rms_varlen_launch(const void* x, int pcm16, const RmsClip* clips, const unsigned* first_item, long n_clips,
                               long n_items, float* out, cudaStream_t st);
 cudaError_t fill_i32_launch(int* p, long n, int v, cudaStream_t st);
-cudaError_t hilbert_envelope_launch(const float* x, long n_clips, long n, long stride, float* amp, long amp_stride,
-                                    int sm_count, cudaStream_t st);
-bool hilbert_fft_supported(long n);
-cudaError_t hilbert_fft_launch(const float* x, long n_clips, long n, long stride, float* amp, long amp_stride,
-                               cudaStream_t st);
+// direct circular convolution (clips of at most kHilDirectMax samples); x float32 or (pcm16) int16 scaled by 1/32768
+constexpr long kHilDirectMax = 4096;
+cudaError_t hilbert_envelope_launch(const void* x, int pcm16, long n_clips, long n, long stride, float* amp,
+                                    long amp_stride, int sm_count, cudaStream_t st);
+// ---- batched Bluestein Hilbert envelope (hilbert_fft.cu).  One transform of a launch (device descriptor, built on
+// the host): the clip's n samples at x + src, its envelope at amp + out; M = 2^m >= 2n - 1 in G pass groups of L[g]
+// bits (hilbert_groups).  Scratch regions are double2 offsets from the sub-batch's scratch base: the chirp c[n], the
+// transformed chirp filter bf[M] (shared by the clips of one n) and two work buffers.  A row of the chirp filter's
+// transform writes buf0 = bf and uses buf1 as its other buffer.
+struct HilRow {
+  long n, src, out;
+  long buf0, buf1, c, bf;
+  double inv_env;  // 1 / (M n)
+  int m, G, L[3];
+};
+// one launch: transform T (0: the chirp filters', 1-4: the clips'), pass group g over rows[n_rows], row r owning
+// CTAs [first[r], first[r + 1]); w: the twiddle table of the batch's largest M = 2^mw
+struct HilPass {
+  const HilRow* rows;
+  const unsigned* first;
+  long n_rows;
+  int T, g;
+  const void* x;
+  int pcm16;
+  double2* s;
+  const double2* w;
+  int mw;
+  float* amp;
+};
+// one sub-batch: tab = one row per distinct n (chirp_first: the chirp launch's CTAs of each), clip = one row per clip,
+// each ordered three-group rows first (n_*3 of them, owning the first *_items3 CTAs); w: offset of the twiddles
+struct HilBatch {
+  const HilRow *tab, *clip;
+  const unsigned *tab_first, *clip_first, *chirp_first;
+  long n_tab, n_tab3, n_clip, n_clip3, tab_items, tab_items3, clip_items, clip_items3, chirp_items;
+  const void* x;
+  int pcm16;
+  float* amp;
+  double2* s;
+  long w;
+  int mw, G;
+};
+int hilbert_groups(int m, int L[3]);  // pass groups of a transform of length 2^m, and their bits
+long hilbert_items(int m);            // CTAs of one row in every group launch
+cudaError_t hilbert_varlen_launch(const HilBatch& b, cudaStream_t st);
 cudaError_t find_peaks_launch(const double* x, long rows, long T, long stride, int minima, int max_peaks, int* idx,
                               int* count, cudaStream_t st);
 cudaError_t pcm16_to_f32_launch(const int16_t* x, long n, float* y, cudaStream_t st);

@@ -1264,8 +1264,16 @@ constexpr int kHilTN = kHilThreads * kHilR;     // outputs per block
 constexpr int kHilTK = 512;                     // taps per shared-memory chunk
 
 // partial[ks][n] = sum over k in the ks-th slice of g[k] * x[(n - k) mod N]
+// x: float32, or int16 scaled as pcm16_to_f32_kernel scales it
+template <typename X>
+__device__ __forceinline__ float hil_x(const X* x, long j) {
+  if constexpr (sizeof(X) == 2) return (float)x[j] * (1.0f / 32768.0f);
+  else return x[j];
+}
+
+template <typename X>
 __global__ void __launch_bounds__(kHilThreads)
-    hilbert_conv_kernel(const float* __restrict__ x, const float* __restrict__ g, long n, int ksplit,
+    hilbert_conv_kernel(const X* __restrict__ x, const float* __restrict__ g, long n, int ksplit,
                         double* __restrict__ partial) {
   __shared__ __align__(16) float sg[kHilTK];
   __shared__ __align__(16) float sx[kHilTN + kHilTK];
@@ -1284,7 +1292,7 @@ __global__ void __launch_bounds__(kHilThreads)
     for (int i = tid; i < kHilTN + kHilTK; i += kHilThreads) {
       long j = (n0 - k0 - (kHilTK - 1) + i) % n;
       if (j < 0) j += n;
-      sx[i] = x[j];
+      sx[i] = hil_x(x, j);
     }
     __syncthreads();
     float a32[kHilR];
@@ -1320,18 +1328,31 @@ __global__ void __launch_bounds__(kHilThreads)
   }
 }
 
-__global__ void hilbert_finish_kernel(const float* __restrict__ x, const double* __restrict__ partial, long n, int ksplit,
+template <typename X>
+__global__ void hilbert_finish_kernel(const X* __restrict__ x, const double* __restrict__ partial, long n, int ksplit,
                                       float* __restrict__ amp) {
   const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   double y = 0.0;
   for (int ks = 0; ks < ksplit; ++ks) y += partial[(size_t)ks * n + i];
-  const double xv = (double)x[i];
+  const double xv = (double)hil_x(x, i);
   amp[i] = (float)sqrt(xv * xv + y * y);
 }
 
-cudaError_t hilbert_envelope_launch(const float* x, long n_clips, long n, long stride, float* amp, long amp_stride,
-                                    int sm_count, cudaStream_t st) {
+template <typename X>
+static void hilbert_direct(const X* x, const float* g, long n_clips, long n, long stride, int n_blocks, int ksplit,
+                           double* partial, float* amp, long amp_stride, cudaStream_t st) {
+  for (long c = 0; c < n_clips; ++c) {
+    hilbert_conv_kernel<<<dim3((unsigned)n_blocks, (unsigned)ksplit), kHilThreads, 0, st>>>(x + c * stride, g, n, ksplit,
+                                                                                          partial);
+    hilbert_finish_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x + c * stride, partial, n, ksplit,
+                                                                       amp + c * amp_stride);
+    count_launch(2);
+  }
+}
+
+cudaError_t hilbert_envelope_launch(const void* x, int pcm16, long n_clips, long n, long stride, float* amp,
+                                    long amp_stride, int sm_count, cudaStream_t st) {
   float* g = nullptr;
   double* partial = nullptr;
   const int n_blocks = (int)((n + kHilTN - 1) / kHilTN);
@@ -1346,13 +1367,10 @@ cudaError_t hilbert_envelope_launch(const float* x, long n_clips, long n, long s
   }
   hilbert_kernel_table<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, g);
   count_launch();
-  for (long c = 0; c < n_clips; ++c) {
-    hilbert_conv_kernel<<<dim3((unsigned)n_blocks, (unsigned)ksplit), kHilThreads, 0, st>>>(x + c * stride, g, n, ksplit,
-                                                                                          partial);
-    hilbert_finish_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x + c * stride, partial, n, ksplit,
-                                                                       amp + c * amp_stride);
-    count_launch(2);
-  }
+  if (pcm16)
+    hilbert_direct((const int16_t*)x, g, n_clips, n, stride, n_blocks, ksplit, partial, amp, amp_stride, st);
+  else
+    hilbert_direct((const float*)x, g, n_clips, n, stride, n_blocks, ksplit, partial, amp, amp_stride, st);
   e = cudaGetLastError();
   cudaFreeAsync(g, st);
   cudaFreeAsync(partial, st);

@@ -16,7 +16,7 @@ from dataclasses import dataclass, replace
 import numpy as np
 
 from . import _lib
-from ._lib import MmfError, check, mmf_amp_params, mmf_change_params, mmf_config, mmf_modspec_params
+from ._lib import MmfError, check, mmf_amp_params, mmf_change_params, mmf_config, mmf_env_params, mmf_modspec_params
 
 
 @dataclass(frozen=True)
@@ -542,6 +542,30 @@ class Plan:
         )
         return amp, amp_off
 
+    def hilbert_varlen(self, x, offsets):
+        """:meth:`hilbert_envelope` for clips of different lengths packed back to back (``mmf_hilbert_varlen``).
+
+        ``x`` is a 1-D float32 device tensor (or host array); clip ``i`` is ``x[offsets[i]:offsets[i + 1]]``.  Returns
+        ``(amp, amp_offsets)``: the float32 envelopes packed clip after clip, clip ``i``'s at
+        ``amp[amp_offsets[i]:amp_offsets[i + 1]]`` (``amp_offsets = offsets - offsets[0]``), each equal to
+        :meth:`hilbert_envelope` on that clip alone, bit for bit."""
+        torch = _torch()
+        x = x if isinstance(x, torch.Tensor) else torch.as_tensor(np.ascontiguousarray(x, dtype=np.float32))
+        x = x.to(device=self.device, dtype=torch.float32).contiguous()
+        if x.dim() != 1:
+            raise ValueError("hilbert_varlen takes a 1-D packed buffer")
+        offs = np.ascontiguousarray(np.asarray(offsets, dtype=np.int64).reshape(-1))
+        amp_off = env_sizes(offs, make_env_params("Hilb"))
+        if offs[-1] > x.shape[0]:
+            raise ValueError(f"offsets[{len(offs) - 1}] = {offs[-1]} is past the end of the {x.shape[0]}-sample buffer")
+        amp = torch.empty((int(amp_off[-1]),), device=self.device, dtype=torch.float32)
+        check(
+            _lib.lib().mmf_hilbert_varlen(
+                self._h, x.data_ptr(), len(offs) - 1, offs.ctypes.data, amp.data_ptr(), _stream_ptr(self.device)
+            )
+        )
+        return amp, amp_off
+
     def hilbert_envelope(self, x):
         """``np.abs(scipy.signal.hilbert(x))`` along the last axis, float32 on the device."""
         torch = _torch()
@@ -775,7 +799,7 @@ class Plan:
         return out
 
     def features_host_varlen(self, pcm_host: np.ndarray, offsets, prm: mmf_change_params, mod=None, *,
-                             want=("totChange",), out=None, rates=None, amp=None):
+                             want=("totChange",), out=None, rates=None, amp=None, amp_method="RMS"):
         """:meth:`features_host` for clips of different lengths packed back to back in one host buffer.
 
         ``pcm_host`` is 1-D float32 or int16 (raw WAV samples, scaled by 1/32768 on the device); clip ``i`` is
@@ -794,7 +818,9 @@ class Plan:
         ``amp = (geom, center, out_sos or None)`` adds each clip's RMS envelope, taken from its native samples (int16
         scaled by 1/32768) with ``geom[i] = (frame_length_i, hop_i)``: ``amplitude``, float32, or float64 through the
         zero-phase ``out_sos`` when one is given, packed at ``amp_offsets`` (int64 ``[B + 1]``).  Clip ``i``'s block
-        equals :meth:`rms` (then :meth:`sosfiltfilt`) on that clip alone, bit for bit."""
+        equals :meth:`rms` (then :meth:`sosfiltfilt`) on that clip alone, bit for bit.  ``amp_method="Hilb"``: the
+        Hilbert envelope instead, one value per native sample (``geom`` and ``center`` are not read), equal to
+        :meth:`hilbert_envelope` (then :meth:`sosfiltfilt`) on that clip alone, bit for bit."""
         pcm_host = np.asarray(pcm_host)
         pcm16 = pcm_host.dtype == np.int16
         if not pcm16 and pcm_host.dtype != np.float32:
@@ -853,12 +879,17 @@ class Plan:
         amp_p = geom_p = a_p = af_p = None
         if amp is not None:
             geom, center, out_sos = amp
-            _, geom, amp_off = amp_sizes(offs, geom, center)
+            env = make_env_params(amp_method, center, out_sos)
+            if amp_method == "RMS":
+                _, geom, amp_off = amp_sizes(offs, geom, center)
+                geom_p = geom.ctypes.data
+            else:
+                amp_off = env_sizes(offs, env)
             a = _out_array(out, "amplitude", (int(amp_off[-1]),), np.float64 if out_sos is not None else np.float32)
-            amp_p, geom_p = C.byref(make_amp_params(center, out_sos)), geom.ctypes.data
+            amp_p = C.byref(env)
             a_p, af_p = (None, a.ctypes.data) if out_sos is not None else (a.ctypes.data, None)
         check(
-            _lib.lib().mmf_features_host_varlen_amp(
+            _lib.lib().mmf_features_host_varlen_env(
                 self._h, pcm_host.ctypes.data, 1 if pcm16 else 0, B, offs.ctypes.data, rs_p, h_p, n_h,
                 C.byref(prm), C.byref(mp) if mp is not None else None, amp_p, geom_p,
                 ptr["totChange"], ptr["mfcc"], ptr["delta"], ptr["modspec"], ptr["band_energy"], a_p, af_p,
@@ -945,6 +976,31 @@ def make_amp_params(center: bool, out_sos=None) -> mmf_amp_params:
         for i, v in enumerate(out_sos.ravel()):
             ap.out_sos[i] = v
     return ap
+
+
+AMP_METHODS = {"RMS": _lib.MMF_ENV_RMS, "Hilb": _lib.MMF_ENV_HILBERT}
+
+
+def make_env_params(method: str = "RMS", center: bool = True, out_sos=None) -> mmf_env_params:
+    """:func:`make_amp_params` with the envelope method: ``'RMS'`` or ``'Hilb'``."""
+    if method not in AMP_METHODS:
+        raise ValueError(f"amplitude method must be 'RMS' or 'Hilb', not {method!r}")
+    ap = make_amp_params(center, out_sos)
+    ep = mmf_env_params()
+    ep.method, ep.center, ep.out_n_sections = AMP_METHODS[method], ap.center, ap.out_n_sections
+    ep.out_sos[:] = list(ap.out_sos)
+    return ep
+
+
+def env_sizes(offsets, env: mmf_env_params, geom=None):
+    """``amp_offsets`` of a packed batch's envelopes (``mmf_env_varlen_sizes``, no device needed); ``geom`` (RMS only)
+    as in :func:`amp_sizes`.  A bad clip raises :class:`MmfError` naming it."""
+    offs = np.ascontiguousarray(np.asarray(offsets, dtype=np.int64).reshape(-1))
+    g = None if geom is None else np.ascontiguousarray(np.asarray(geom, dtype=np.int32).reshape(-1, 2))
+    amp_off = np.zeros(offs.shape[0], np.int64)
+    check(_lib.lib().mmf_env_varlen_sizes(offs.shape[0] - 1, offs.ctypes.data, C.byref(env),
+                                          g.ctypes.data if g is not None else None, amp_off.ctypes.data))
+    return amp_off
 
 
 def _modspec_params(mod):

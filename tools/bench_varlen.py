@@ -32,11 +32,17 @@ the call without it, with the raw envelope and with the 'iir' output filter.  It
 bundle, calculate_amplitude_envelope per clip at its native rate, and with torch.profiler the envelope kernels over
 the same clips: one mmf_rms_varlen launch, and Plan.rms per clip (whatever kernel the tree's mmf_rms launches).
 
+The hilbert leg times the Hilbert envelope ('Hilb') of the 16 kHz float32 corpus on the device: one
+mmf_hilbert_varlen call over the packed clips against Plan.hilbert_envelope per clip (whatever kernels the tree's
+mmf_hilbert_envelope launches, so the leg can time an older tree too), as CUDA-event wall time and as kernel time from
+torch.profiler.  Where the tree has it, it then times host_varlen(want=every output) on the resample leg's int16
+44.1 kHz corpus (with rates=) without the envelope and with amp_method='Hilb', raw and with the 'iir' output filter.
+
 Workload: 1024 clips at 16 kHz with the bench's frame geometry (win 400 / hop 160 / n_fft 512, 40 mel, 13 MFCC,
 gradient, Butterworth output filter), lengths uniform in [2 s, 20 s] from a fixed seed.  Prints, per leg, the median
 ms of each way and audio-seconds per second as one JSON line, with the GPU's name and power limit.
 
-    python tools/bench_varlen.py [--clips 1024] [--iters 10] [--loop-iters 3] [--legs change,features,host,resample,amplitude]
+    python tools/bench_varlen.py [--clips 1024] [--iters 10] [--loop-iters 3] [--legs change,features,host,resample,amplitude,hilbert]
 """
 import argparse
 import json
@@ -259,6 +265,52 @@ def _amplitude_leg(pcm, lengths16, n_clips, iters, seed, power_limit, dev):
         print(json.dumps(res), flush=True)
 
 
+def _hilbert_leg(pcm, lengths16, n_clips, iters, seed, power_limit, dev):
+    """The Hilbert envelope; see the module docstring."""
+    plan = mm.FeatureExtractor(16000, device=0).plan
+    B = len(lengths16)
+    offsets = np.zeros(B + 1, np.int64)
+    np.cumsum(lengths16, out=offsets[1:])
+    x_dev = torch.cat([pcm[i, :n] for i, n in enumerate(lengths16)]).contiguous()
+    rows = [x_dev[offsets[i] : offsets[i + 1]] for i in range(B)]
+    res = {"leg": "hilbert", "corpus": "float32_16k", "gpu": torch.cuda.get_device_name(dev),
+           "power_limit": power_limit, "clips": B, "audio_s": float(offsets[-1]) / 16000}
+    loop = lambda: [plan.hilbert_envelope(r) for r in rows]  # noqa: E731
+    loop()
+    res["per_clip_ms"] = _median_ms(loop, max(1, iters // 5))
+    res["per_clip_kernel_ms"] = _profiled_kernel_ms(loop, "")
+    if hasattr(plan, "hilbert_varlen"):
+        call = lambda: plan.hilbert_varlen(x_dev, offsets)  # noqa: E731
+        call()
+        res["varlen_ms"] = _median_ms(call, iters)
+        res["varlen_kernel_ms"] = _profiled_kernel_ms(call, "")
+        from modulation_mfcc_b200 import _lib
+
+        _lib.lib().mmf_launch_count(1)
+        call()
+        res["varlen_launches"] = _lib.lib().mmf_launch_count(1)
+    print(json.dumps(res), flush=True)
+    if not hasattr(plan, "hilbert_varlen"):
+        return
+    # the bundle with and without the envelope: int16 clips at 44.1 kHz resampled to the plan's 16 kHz
+    want = ("totChange", "mfcc", "delta", "modspec", "band_energy")
+    sr_in = 44100
+    packed, offs44, _ = _int16_corpus(n_clips, seed, sr_in)
+    rates = [sr_in] * n_clips
+    res = {"leg": "hilbert_bundle", "corpus": "int16_44k_rates", "gpu": torch.cuda.get_device_name(dev),
+           "power_limit": power_limit, "clips": n_clips, "audio_s": float(offs44[-1]) / sr_in}
+    for k, fx, w in (("none", mm.FeatureExtractor(16000, device=0), want),
+                     ("hilb_raw", mm.FeatureExtractor(16000, device=0, amp_method="Hilb"), want + ("amplitude",)),
+                     ("hilb_iir", mm.FeatureExtractor(16000, device=0, amp_method="Hilb", amp_outFilter="iir"),
+                      want + ("amplitude",))):
+        out = {key: v for key, v in fx.host_varlen(packed, offs44, want=w, rates=rates).items() if key in w}
+        out = {key: _pinned(v.shape, v.dtype.type) for key, v in out.items()}
+        call = lambda fx=fx, w=w, out=out: fx.host_varlen(packed, offs44, want=w, out=out, rates=rates)  # noqa: E731
+        res[f"host_varlen_{k}_ms"] = _median_host_ms(call, iters)
+        res[f"host_varlen_{k}_audio_s_per_s"] = res["audio_s"] / (res[f"host_varlen_{k}_ms"] / 1e3)
+    print(json.dumps(res), flush=True)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--clips", type=int, default=1024)
@@ -311,6 +363,9 @@ def main():
             continue
         if leg == "amplitude":
             _amplitude_leg(pcm, lengths, a.clips, a.iters, a.seed, power_limit, dev)
+            continue
+        if leg == "hilbert":
+            _hilbert_leg(pcm, lengths, a.clips, a.iters, a.seed, power_limit, dev)
             continue
         varlen, loop, pad = ways[leg]
         for fn in (varlen, pad, loop):  # warm-up: modules, workspace growth
