@@ -411,6 +411,54 @@ int mmf_features_host_varlen_env(mmf_plan* plan, const void* pcm_host, int32_t p
                                  float* mfcc_host, float* delta_host, float* mag_host, float* band_host,
                                  float* amp_host, double* amp_filt_host);
 
+/* The 'fir' and 'sg' output filters of applyFilter (script/mfcc.py:113-131), as coefficients designed on the host.
+ * MMF_FILT_FIR: scipy.signal.filtfilt(taps, 1, x), n_taps in [1, 4096].  MMF_FILT_SG: a banded stencil with dense
+ * edge rows, as mmf_stencil takes it (savgol_filter(mode='interp'), np.gradient, findiff).  All pointers are host
+ * pointers; the fields the kind does not use are ignored. */
+#define MMF_FILT_FIR 0
+#define MMF_FILT_SG 1
+typedef struct mmf_out_filter {
+  int32_t kind;          /* MMF_FILT_FIR or MMF_FILT_SG */
+  int32_t n_taps;        /* FIR */
+  const double* taps;    /* FIR: b[n_taps] */
+  int32_t half;          /* SG: y[t] = sum_o coef[o + half] * x[t + o] in the interior */
+  const double* coef;    /* SG: [2 * half + 1] */
+  int32_t n_edge;        /* SG: the first / last n_edge outputs are edge_l / edge_r ... */
+  int32_t n_edge_in;     /* ... [n_edge, n_edge_in] applied to the first / last n_edge_in inputs; n_edge >= half */
+  const double* edge_l;
+  const double* edge_r;
+} mmf_out_filter;
+
+/* Host-only: the checks of mmf_filter_varlen for n_rows rows of T_host[i] samples, without a plan or a device.
+ * FIR: T_i <= 3 * n_taps fails with MMF_ERR_TOO_SHORT and filtfilt's padlen message; SG: T_i < n_edge_in or
+ * T_i < 2 * n_edge fails with MMF_ERR_TOO_SHORT.  Both name the row ("clip i: ").  A bad kind, tap count or edge
+ * shape fails with MMF_ERR_INVALID or MMF_ERR_UNSUPPORTED. */
+int mmf_filter_varlen_check(const mmf_out_filter* filt, int64_t n_rows, const int64_t* T_host);
+
+/* The output filter filt over n_rows rows of any lengths, in a fixed number of launches (FIR: 2, SG: 1) whatever the
+ * row count: row i is the T_host[i] samples at x_dev + x_off_host[i] (float64, or x_is_f32 float32), its T_host[i]
+ * float64 outputs go to y_dev + y_off_host[i] (offsets in elements).  A padded [B, T_max] batch and a packed one
+ * are the same call.  Each row's output equals, bit for bit, mmf_fir_filtfilt / mmf_stencil on that row alone.
+ * Every check (mmf_filter_varlen_check) runs before anything is queued; the descriptors and coefficients are copied
+ * before the call returns, which is asynchronous on `stream`.  FIR scratch comes from the stream-ordered pool. */
+int mmf_filter_varlen(mmf_plan* plan, const mmf_out_filter* filt, const void* x_dev, int32_t x_is_f32, int64_t n_rows,
+                      const int64_t* x_off_host, const int64_t* T_host, double* y_dev, const int64_t* y_off_host,
+                      void* stream);
+
+/* mmf_features_host_varlen_env with an output filter on the MFCC-change curve.  change_out NULL: exactly
+ * mmf_features_host_varlen_env.  Otherwise prm->out_kind must be 1 (the raw curve; else MMF_ERR_INVALID): each
+ * chunk's raw curves are filtered by change_out (mmf_filter_varlen over the chunk's padded rows) and tot_host
+ * receives the filtered curves, each equal to mmf_filter_varlen on that clip's raw curve alone.  A clip too short
+ * for the change stage's Butterworth filter reports that first; otherwise a curve too short for change_out fails
+ * as mmf_filter_varlen_check fails, naming the clip, before anything is queued. */
+int mmf_features_host_varlen_out(mmf_plan* plan, const void* pcm_host, int32_t pcm16, int64_t n_clips,
+                                 const int64_t* offsets_host, const mmf_resample_clip* rs_host, const float* h_host,
+                                 int64_t n_h, const mmf_change_params* prm, const mmf_modspec_params* mod,
+                                 const mmf_env_params* env, const int32_t* geom_host,
+                                 const mmf_out_filter* change_out, double* tot_host, float* mfcc_host,
+                                 float* delta_host, float* mag_host, float* band_host, float* amp_host,
+                                 double* amp_filt_host);
+
 /* Local extrema of each float64 row with scipy.signal.find_peaks' default semantics (strictly higher
  * than both neighbours; a flat top reports its middle sample; end samples never qualify) -- the
  * landmark step the GUI runs on the curve (script/main.py:1566, :1601; script/calc.py:669, :681).
@@ -440,7 +488,8 @@ int mmf_mfcc_change_host(mmf_plan* plan, const float* pcm_host, int64_t n_clips,
                          int64_t clip_stride, const mmf_change_params* prm, double* tot_host, float* mfcc_host);
 
 /* sizeof() of the ABI structs as this library was compiled (0: mmf_config,
- * 1: mmf_change_params, 2: mmf_modspec_params, 3: mmf_resample_clip, 4: mmf_amp_params, 5: mmf_env_params) so
+ * 1: mmf_change_params, 2: mmf_modspec_params, 3: mmf_resample_clip, 4: mmf_amp_params, 5: mmf_env_params,
+ * 6: mmf_out_filter) so
  * bindings can verify their layout. */
 int mmf_abi_sizeof(int32_t which);
 

@@ -8,8 +8,10 @@ anywhere, computing requires a Blackwell GPU.
 from ._lib import MmfError, build, exported_symbols, lib  # noqa: F401
 from .plan import (  # noqa: F401
     MfccConfig,
+    OutFilter,
     Plan,
     clear_plans,
+    fir_filter,
     frame_sizes,
     get_plan,
     host_tables,
@@ -18,6 +20,7 @@ from .plan import (  # noqa: F401
     resample_descriptors,
     resample_ratio,
     sos_zi,
+    stencil_filter,
 )
 from .api import (  # noqa: F401
     MODULATION_BANDS_HZ,

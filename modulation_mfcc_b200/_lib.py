@@ -134,6 +134,24 @@ class mmf_env_params(C.Structure):
     ]
 
 
+MMF_FILT_FIR = 0
+MMF_FILT_SG = 1
+
+
+class mmf_out_filter(C.Structure):
+    _fields_ = [
+        ("kind", C.c_int32),
+        ("n_taps", C.c_int32),
+        ("taps", C.c_void_p),
+        ("half", C.c_int32),
+        ("coef", C.c_void_p),
+        ("n_edge", C.c_int32),
+        ("n_edge_in", C.c_int32),
+        ("edge_l", C.c_void_p),
+        ("edge_r", C.c_void_p),
+    ]
+
+
 OBJ_DIR = PKG_DIR / "build"
 
 
@@ -257,6 +275,13 @@ _SIGNATURES = {
         [_vp, _vp, _i32, _i64, _vp, _vp, _vp, _i64, C.POINTER(mmf_change_params), C.POINTER(mmf_modspec_params),
          C.POINTER(mmf_env_params), _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     ),
+    "mmf_features_host_varlen_out": (
+        C.c_int,
+        [_vp, _vp, _i32, _i64, _vp, _vp, _vp, _i64, C.POINTER(mmf_change_params), C.POINTER(mmf_modspec_params),
+         C.POINTER(mmf_env_params), _vp, C.POINTER(mmf_out_filter), _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    ),
+    "mmf_filter_varlen_check": (C.c_int, [C.POINTER(mmf_out_filter), _i64, _vp]),
+    "mmf_filter_varlen": (C.c_int, [_vp, C.POINTER(mmf_out_filter), _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp]),
     "mmf_amp_varlen_sizes": (C.c_int, [_i64, _vp, _vp, _i32, _vp]),
     "mmf_env_varlen_sizes": (C.c_int, [_i64, _vp, C.POINTER(mmf_env_params), _vp, _vp]),
     "mmf_hilbert_varlen": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _vp]),

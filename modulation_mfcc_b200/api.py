@@ -28,7 +28,7 @@ import scipy.signal
 
 from . import _lib
 from ._lib import MmfError
-from .plan import MfccConfig, Plan, frame_sizes, get_plan, make_change_params, resample_ratio
+from .plan import MfccConfig, Plan, fir_filter, frame_sizes, get_plan, make_change_params, resample_ratio, stencil_filter
 
 MODULATION_BANDS_HZ = ((0.5, 2.0), (2.0, 4.0), (4.0, 8.0), (8.0, 16.0), (16.0, 32.0))
 
@@ -195,9 +195,10 @@ def _findiff_stencil(deriv: int, acc: int):
 # ---------------------------------------------------------------------------
 
 
-def _apply_filter_dev(plan: Plan, x_dev, sr, *, filt, cutOff, filtLen, filtType, polyOrd, coeffs=None):
-    """Validation (same order and messages as script/mfcc.py:82-96) + GPU filtering
-    of a float64 device tensor along its last axis."""
+def _design_filter(sr, *, filt, cutOff, filtLen, filtType, polyOrd, coeffs=None, n=None):
+    """applyFilter's validation (same order and messages as script/mfcc.py:82-96) and filter design:
+    ``("iir", sos)``, ``("fir", taps)``, ``("sg", (coef, edge_l, edge_r))``, or None for a name the reference does
+    not know.  ``n``: the length of the row the 'sg' window is checked against (None: no check)."""
     if (filt is None) | (cutOff is None) | (cutOff is None):
         if cutOff is None:
             raise Exception("Cannot apply filter without specifying a cut Off freq. (CutOff is None).")
@@ -220,44 +221,78 @@ def _apply_filter_dev(plan: Plan, x_dev, sr, *, filt, cutOff, filtLen, filtType,
     ok = ((len(cutOff) == 1) and ((filtType == "lowpass") | (filtType == "highpass"))) | (
         (len(cutOff) == 2) and (filtType == "bandpass")
     )
-    y = None
+    if filt == "iir":
+        if coeffs is None:
+            w = cutOff / (sr / 2)
+            if ok:
+                return "iir", _butter_sos(filtLen, w, filtType)
+            raise Exception(
+                "only one or two cut off frequencies allowed. If two freqs are provided, filtType must be bandpass"
+            )
+        # reference quirk (script/mfcc.py:100-111): `sos` is never bound when coeffs is given
+        raise NameError("name 'sos' is not defined")
+    if filt == "fir":
+        if coeffs is None:
+            w = cutOff / (sr / 2)
+            if ok:
+                return "fir", scipy.signal.firwin(filtLen, w, window=("kaiser", 7.4), pass_zero=filtType)
+            raise Exception(
+                "only one or two cut off frequencies allowed. If two freqs are provided, filtType must be bandpass"
+            )
+        raise NameError("name 'bFil' is not defined")
+    if filt == "sg":
+        if len(cutOff) == 1:
+            if n is not None and n < filtLen:
+                raise ValueError("If mode is 'interp', window_length must be less than or equal to the size of x.")
+            return "sg", _savgol_stencil(int(filtLen), int(polyOrd), 0)
+        raise Exception("sg (savitsky Golay) filters can only be lowpass (one cutOff freq allowed)")
+    return None
+
+
+def _apply_filter_dev(plan: Plan, x_dev, sr, *, filt, cutOff, filtLen, filtType, polyOrd, coeffs=None):
+    """Validation (same order and messages as script/mfcc.py:82-96) + GPU filtering
+    of a float64 device tensor along its last axis."""
+    d = _design_filter(sr, filt=filt, cutOff=cutOff, filtLen=filtLen, filtType=filtType, polyOrd=polyOrd,
+                       coeffs=coeffs, n=x_dev.shape[-1])
+    if d is None:
+        return None
+    kind, des = d
     try:
-        if filt == "iir":
-            if coeffs is None:
-                w = cutOff / (sr / 2)
-                if ok:
-                    sos = _butter_sos(filtLen, w, filtType)
-                else:
-                    raise Exception(
-                        "only one or two cut off frequencies allowed. If two freqs are provided, filtType must be bandpass"
-                    )
-            else:
-                # reference quirk (script/mfcc.py:100-111): `sos` is never bound when coeffs is given
-                raise NameError("name 'sos' is not defined")
-            y = plan.sosfiltfilt(x_dev, sos)
-        if filt == "fir":
-            if coeffs is None:
-                w = cutOff / (sr / 2)
-                if ok:
-                    bFil = scipy.signal.firwin(filtLen, w, window=("kaiser", 7.4), pass_zero=filtType)
-                else:
-                    raise Exception(
-                        "only one or two cut off frequencies allowed. If two freqs are provided, filtType must be bandpass"
-                    )
-            else:
-                raise NameError("name 'bFil' is not defined")
-            y = plan.fir_filtfilt(x_dev, bFil)
-        if filt == "sg":
-            if len(cutOff) == 1:
-                if x_dev.shape[-1] < filtLen:
-                    raise ValueError("If mode is 'interp', window_length must be less than or equal to the size of x.")
-                coef, el, er = _savgol_stencil(int(filtLen), int(polyOrd), 0)
-                y = plan.stencil(x_dev, coef, el, er)
-            else:
-                raise Exception("sg (savitsky Golay) filters can only be lowpass (one cutOff freq allowed)")
+        if kind == "iir":
+            return plan.sosfiltfilt(x_dev, des)
+        if kind == "fir":
+            return plan.fir_filtfilt(x_dev, des)
+        return plan.stencil(x_dev, *des)
     except MmfError as e:
         _raise_from(e)
-    return y
+
+
+def _out_filter(sr, lengths=None, **post):
+    """applyFilter's 'fir' or 'sg' filter (``post``: its keywords) as a :class:`~.plan.OutFilter`, or None for a name
+    the reference does not know.  ``lengths``: the rows it will filter, checked as the per-row calls check them, the
+    first error naming its row; a ValueError of the design then names row 0, where a per-row loop would have met it."""
+    try:
+        d = _design_filter(sr, n=None if lengths is None else int(lengths[0]), **post)
+    except ValueError as e:
+        if lengths is None:
+            raise
+        raise ValueError(f"clip 0: {e}") from None
+    if d is None:
+        return None
+    kind, des = d
+    if kind == "iir":
+        raise ValueError("an 'iir' output filter runs through sosfiltfilt, not the ragged 'fir' / 'sg' filters")
+    f = fir_filter(des) if kind == "fir" else stencil_filter(*des)
+    if lengths is not None:
+        for i, n in enumerate(lengths):
+            if kind == "sg" and n < post["filtLen"]:
+                raise ValueError(f"clip {i}: If mode is 'interp', window_length must be less than or equal to the size "
+                                 "of x.")
+        try:
+            f.check(lengths)
+        except MmfError as e:
+            _raise_from(e)
+    return f
 
 
 def applyFilter(x, sr, /, *, filt="iir", cutOff=[None], filtLen=6, filtType="low", polyOrd=3, coeffs=None, device=None):
@@ -517,14 +552,13 @@ def get_MFCCS_change_many(
         )
         frames = res.pop("frames")
         tots = [res["totChange"][i, : frames[i]] for i in range(len(clips))]
-        if post is not None:
-            filtered = []
-            for i, t in enumerate(tots):
-                try:
-                    filtered.append(_apply_filter_dev(plan, t, 1 / tStep, **post))
-                except ValueError as e:  # a curve too short for the output filter: name the clip
-                    raise ValueError(f"clip {i}: {e}") from None
-            tots = filtered
+        if post is not None:  # one ragged launch for every curve; a curve too short for it names its clip
+            filt = _out_filter(1 / tStep, frames, **post)
+            if filt is None:  # unknown filter name: the reference returns None from applyFilter
+                tots = [None] * len(clips)
+            else:
+                y = plan.filter_varlen(res["totChange"], frames, filt)
+                tots = [y[i, : frames[i]] for i in range(len(clips))]
     except MmfError as e:
         _raise_from(e)
     out = []
@@ -803,16 +837,22 @@ def calculate_amplitude_envelope_many(
         else:
             amp, amp_off = plan.hilbert_varlen(packed, offsets)
         out = []
-        host = amp.cpu().numpy() if outFilter is None else None
+        post = dict(filt=outFilter, filtType=outFiltType, cutOff=outFiltCutOff, filtLen=outFiltLen,
+                    polyOrd=outFiltPolyOrd)
+        host = None
+        if outFilter is None:
+            host = amp.cpu().numpy()
+        elif outFilter in ("fir", "sg"):  # one ragged launch for every envelope; one too short for it names its clip
+            filt = _out_filter(1 / hopLen, np.diff(amp_off), **post)
+            host = plan.filter_varlen(amp, amp_off, filt).cpu().numpy()
         for i in range(len(clips)):
             a0, a1 = int(amp_off[i]), int(amp_off[i + 1])
             ampT = np.arange(a1 - a0) * hopLen  # script/calc.py:333-337
-            if outFilter is None:
+            if host is not None:
                 out.append((host[a0:a1], ampT))
                 continue
             try:
-                y = _apply_filter_dev(plan, amp[a0:a1], 1 / hopLen, filt=outFilter, filtType=outFiltType,
-                                      cutOff=outFiltCutOff, filtLen=outFiltLen, polyOrd=outFiltPolyOrd)
+                y = _apply_filter_dev(plan, amp[a0:a1], 1 / hopLen, **post)
             except ValueError as e:  # an envelope too short for the output filter: name the clip
                 raise ValueError(f"clip {i}: {e}") from None
             out.append((y.cpu().numpy() if y is not None else None, ampT))
@@ -876,7 +916,18 @@ class FeatureExtractor:
         amp_outFiltCutOff=[12],
         amp_outFiltLen=6,
         amp_method: str = "RMS",
+        diffMethod="grad",
+        outFilter=None,
+        outFiltType="low",
+        outFiltCutOff=[12],
+        outFiltLen=6,
+        outFiltPolyOrd=3,
     ):
+        """``diffMethod`` and ``outFilter`` / ``outFilt*`` set the MFCC-change curve as get_MFCCS_change sets it
+        (script/mfcc.py:405-425): None (the default) is Goldstein's low-pass with the change filter's own design,
+        'iir' a Butterworth of its own, 'fir' and 'sg' the zero-phase FIR and the Savitzky-Golay filter of
+        applyFilter.  They are validated here, before any device work, with applyFilter's exceptions; a filter name
+        applyFilter does not know raises ValueError."""
         if amp_method not in ("RMS", "Hilb"):
             raise ValueError(f"the feature bundle takes amp_method 'RMS' or 'Hilb', not {amp_method!r}")
         self.amp_method = amp_method
@@ -890,9 +941,21 @@ class FeatureExtractor:
                              "calculate_amplitude_envelope_many for 'fir' and 'sg')")
         self.amp_winLen, self.amp_hopLen, self.amp_center = float(amp_winLen), float(amp_hopLen), bool(amp_center)
         self.sr, self.tStep, self.winLen = float(sr), float(tStep), float(winLen)
-        self.plan = _change_setup(sr, tStep, winLen, n_mfcc, n_fft, fmin, sr / 2 if fmax is None else fmax, n_mels, preemph, device, flags)
-        sos = _butter_sos(filtOrd, filtCutoff / ((1 / tStep) / 2), "low")
-        self.prm = make_change_params(sos, remove_first=removeFirst, diff_method=0, out_sos=sos)
+        # the curve's output filter, validated before the plan exists.  'fir' / 'sg': the raw curve, then this filter;
+        # None and 'iir' run in the change stage
+        self.change_out = None
+        if outFilter == "iir":
+            _design_iir(1 / tStep, outFiltCutOff, outFiltLen, outFiltType)
+        elif outFilter is not None:
+            self.change_out = _out_filter(1 / tStep, filt=outFilter, cutOff=outFiltCutOff, filtLen=outFiltLen,
+                                          filtType=outFiltType, polyOrd=outFiltPolyOrd)
+            if self.change_out is None:
+                raise ValueError(f"outFilter must be None, 'iir', 'fir' or 'sg', not {outFilter!r}")
+        self.plan, self.prm, _ = _change_request(
+            sr, tStep, winLen, n_mfcc, n_fft, fmin, sr / 2 if fmax is None else fmax, removeFirst, filtCutoff, filtOrd,
+            diffMethod, outFilter, outFiltType, outFiltCutOff, outFiltLen, outFiltPolyOrd, n_mels, preemph, device,
+            flags,
+        )
         self.mod_win_s, self.mod_hop_s, self.bands_hz = mod_win_s, mod_hop_s, bands_hz
         self.frame_rate = 1.0 / tStep
 
@@ -915,9 +978,31 @@ class FeatureExtractor:
         T = self.plan.num_frames(pcm_host.shape[-1])
         mod = self.modspec_geometry(T) if ("modspec" in want or "band_energy" in want) else None
         try:
+            if self.change_out is not None:
+                return self._host_call_packed(pcm_host, T, mod, want, out)
             return self.plan.features_host(pcm_host, self.prm, mod, want=want, out=out)
         except MmfError as e:
             _raise_from(e)
+
+    def _host_call_packed(self, pcm_host, T, mod, want, out):
+        """:meth:`host_call` through the packed bundle, which runs the 'fir' / 'sg' curve filter: with clips of equal
+        length the packed blocks are the padded arrays, flattened."""
+        pcm = pcm_host if pcm_host.ndim == 2 else pcm_host[None, :]
+        B, N = pcm.shape
+        res = self.plan.features_host_varlen(np.ascontiguousarray(pcm).reshape(-1), np.arange(B + 1, dtype=np.int64) * N,
+                                             self.prm, mod, want=want, change_out=self.change_out)
+        nm, W = self.plan.cfg.n_mfcc, int(res["windows"][0])
+        nb, n_bands = (mod[2] // 2 + 1, len(mod[3])) if mod is not None else (0, 0)
+        shapes = {"totChange": (B, T), "mfcc": (B, nm, T), "delta": (B, nm, T), "modspec": (B, nm, W, nb),
+                  "band_energy": (B, W, n_bands)}
+        out = {} if out is None else out
+        for k, shape in shapes.items():
+            if k in res and (k in want or k == "totChange"):
+                a = out.get(k)
+                if a is None or a.shape != shape or a.dtype != res[k].dtype or not a.flags.c_contiguous:
+                    a = out[k] = np.empty(shape, res[k].dtype)
+                a[...] = res[k].reshape(shape)
+        return out
 
     def host_varlen(self, pcm_host, offsets, *, want=("totChange", "mfcc", "delta", "modspec", "band_energy"),
                     out=None, rates=None):
@@ -936,7 +1021,7 @@ class FeatureExtractor:
         try:
             amp = self._amp(want, len(offsets) - 1, rates)
             return self.plan.features_host_varlen(pcm_host, offsets, self.prm, mod, want=want, out=out, rates=rates,
-                                                  amp=amp, amp_method=self.amp_method)
+                                                  amp=amp, amp_method=self.amp_method, change_out=self.change_out)
         except MmfError as e:
             _raise_from(e)
 
@@ -1003,6 +1088,9 @@ class FeatureExtractor:
 
     def __call__(self, pcm, *, want_logmel: bool = True, want_modspec: bool = True):
         res = self.plan.mfcc_change(pcm, self.prm, want_logmel=want_logmel, want_mfcc=True, want_delta=True)
+        if self.change_out is not None:
+            tot = res["totChange"]
+            res["totChange"] = self.plan.filter_varlen(tot, [tot.shape[-1]] * tot.shape[0], self.change_out)
         if want_modspec:
             T = res["mfcc"].shape[-1]
             Lw, Hw, nfft, _ = modspec_sizes(T, self.frame_rate, self.mod_win_s, self.mod_hop_s)
@@ -1019,6 +1107,8 @@ class FeatureExtractor:
         res = self.plan.mfcc_change_varlen(pcm, lengths, self.prm, want_logmel=want_logmel, want_mfcc=True,
                                            want_delta=True)
         frames = res["frames"]
+        if self.change_out is not None:
+            res["totChange"] = self.plan.filter_varlen(res["totChange"], frames, self.change_out)
         # the modulation geometry does not depend on T, only each clip's window count does
         Lw, Hw, nfft, _ = modspec_sizes(0, self.frame_rate, self.mod_win_s, self.mod_hop_s)
         if want_modspec:

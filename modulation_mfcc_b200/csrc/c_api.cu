@@ -520,6 +520,7 @@ int mmf_abi_sizeof(int32_t which) {
     case 3: return (int)sizeof(mmf_resample_clip);
     case 4: return (int)sizeof(mmf_amp_params);
     case 5: return (int)sizeof(mmf_env_params);
+    case 6: return (int)sizeof(mmf_out_filter);
     default: return -1;
   }
 }
@@ -1018,56 +1019,6 @@ int mmf_delta_norm(mmf_plan* plan, const double* x_dev, int64_t n_clips, int32_t
                                       tot_dev + (size_t)c0 * T, (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(e, "delta_norm_kernel launch");
   }
-  return MMF_OK;
-}
-
-// small host arrays are staged through the plan workspace tail (first 64 KB reserved)
-static int stage_consts(mmf_plan* plan, const void* host, size_t bytes, size_t offset, void** dev, cudaStream_t st) {
-  int rc = ensure_ws(plan, std::max<size_t>(plan->ws_bytes, 1 << 20));
-  if (rc) return rc;
-  if (offset + bytes > (64 << 10)) return fail(MMF_ERR_UNSUPPORTED, "coefficient arrays larger than 64 KB");
-  *dev = (unsigned char*)plan->ws + offset;
-  MMF_CUDA(cudaMemcpyAsync(*dev, host, bytes, cudaMemcpyHostToDevice, st));
-  return MMF_OK;
-}
-
-int mmf_fir_filtfilt(mmf_plan* plan, const double* x_dev, int64_t rows, int64_t T, const double* b_host,
-                     int32_t n_taps, double* y_dev, double* work_dev, void* stream) {
-  if (!plan || !x_dev || !b_host || !y_dev || !work_dev) return fail(MMF_ERR_INVALID, "NULL argument");
-  if (n_taps < 1 || n_taps > 4096) return fail(MMF_ERR_UNSUPPORTED, "n_taps must be in [1, 4096]");
-  if (rows < 1 || rows > 65535) return fail(MMF_ERR_UNSUPPORTED, "rows must be in [1, 65535]");
-  if (T <= 3 * n_taps) return too_short(3 * n_taps);
-  MMF_CUDA(cudaSetDevice(plan->cfg.device));
-  void* b_dev = nullptr;
-  int rc = stage_consts(plan, b_host, (size_t)n_taps * 8, 0, &b_dev, (cudaStream_t)stream);
-  if (rc) return rc;
-  cudaError_t e = fir_filtfilt_launch(x_dev, rows, T, (const double*)b_dev, n_taps, y_dev, work_dev,
-                                      (cudaStream_t)stream);
-  if (e != cudaSuccess) return cuda_fail(e, "fir kernels launch");
-  return MMF_OK;
-}
-
-int mmf_stencil(mmf_plan* plan, const double* x_dev, int64_t rows, int64_t T, const double* coef_host, int32_t half,
-                const double* edge_l_host, const double* edge_r_host, int32_t n_edge, int32_t n_edge_in,
-                double* y_dev, void* stream) {
-  if (!plan || !x_dev || !coef_host || !y_dev) return fail(MMF_ERR_INVALID, "NULL argument");
-  if (half < 0 || n_edge < half || n_edge_in < 0) return fail(MMF_ERR_INVALID, "need n_edge >= half >= 0");
-  if (n_edge > 0 && (!edge_l_host || !edge_r_host)) return fail(MMF_ERR_INVALID, "edge matrices are NULL");
-  if (T < n_edge_in || T < 2 * n_edge) return fail(MMF_ERR_TOO_SHORT, "input shorter than the stencil's edge window");
-  if (rows < 1 || rows > 65535) return fail(MMF_ERR_UNSUPPORTED, "rows must be in [1, 65535]");
-  MMF_CUDA(cudaSetDevice(plan->cfg.device));
-  cudaStream_t st = (cudaStream_t)stream;
-  const size_t cb = (size_t)(2 * half + 1) * 8, eb = (size_t)n_edge * n_edge_in * 8;
-  void *c_dev = nullptr, *l_dev = nullptr, *r_dev = nullptr;
-  int rc = stage_consts(plan, coef_host, cb, 0, &c_dev, st);
-  if (rc) return rc;
-  if (eb) {
-    if ((rc = stage_consts(plan, edge_l_host, eb, align_up(cb, 256), &l_dev, st))) return rc;
-    if ((rc = stage_consts(plan, edge_r_host, eb, align_up(cb, 256) + align_up(eb, 256), &r_dev, st))) return rc;
-  }
-  cudaError_t e = stencil_launch(x_dev, rows, T, (const double*)c_dev, half, (const double*)l_dev,
-                                 (const double*)r_dev, n_edge, n_edge_in, y_dev, st);
-  if (e != cudaSuccess) return cuda_fail(e, "stencil_kernel launch");
   return MMF_OK;
 }
 
@@ -2179,6 +2130,108 @@ static int run_uploaded(mmf_plan* plan, const DescBlob& desc, cudaStream_t st, L
   return rc;
 }
 
+// ---- the 'fir' / 'sg' output filters over ragged rows (fir_varlen_launch, stencil_varlen_launch) ----
+
+// The checks of a filter's kind and coefficients, which do not depend on the rows
+static int filter_shape_check(const mmf_out_filter* f) {
+  if (!f) return fail(MMF_ERR_INVALID, "output filter is NULL");
+  if (f->kind == MMF_FILT_FIR) {
+    if (f->n_taps < 1 || f->n_taps > 4096) return fail(MMF_ERR_UNSUPPORTED, "n_taps must be in [1, 4096]");
+    if (!f->taps) return fail(MMF_ERR_INVALID, "taps is NULL");
+    return MMF_OK;
+  }
+  if (f->kind != MMF_FILT_SG) return fail(MMF_ERR_INVALID, "unknown output filter kind " + std::to_string(f->kind));
+  if (!f->coef) return fail(MMF_ERR_INVALID, "coef is NULL");
+  if (f->half < 0 || f->n_edge < f->half || f->n_edge_in < 0) return fail(MMF_ERR_INVALID, "need n_edge >= half >= 0");
+  if (f->n_edge > 0 && (!f->edge_l || !f->edge_r)) return fail(MMF_ERR_INVALID, "edge matrices are NULL");
+  return MMF_OK;
+}
+
+// A row of T samples too short for f: the single calls' error, naming the row when clip >= 0
+static int filter_row_check(const mmf_out_filter* f, int64_t T, int64_t clip) {
+  if (f->kind == MMF_FILT_FIR) return T <= 3 * (int64_t)f->n_taps ? too_short(3 * f->n_taps, clip) : MMF_OK;
+  if (T < f->n_edge_in || T < 2 * (int64_t)f->n_edge)
+    return fail(MMF_ERR_TOO_SHORT, (clip < 0 ? "" : "clip " + std::to_string(clip) + ": ") +
+                                       "input shorter than the stencil's edge window");
+  return MMF_OK;
+}
+
+// A ragged output-filter launch, host half: the rows, their work lists and the coefficients, in desc.  The FIR's
+// forward-pass scratch is packed row after row (work: its size in doubles).
+struct FilterVarlen {
+  int64_t n_rows = 0, work = 0;
+  RaggedParts a, b;  // SG: a; FIR: a the forward pass, b the backward pass (the same rows)
+  size_t taps = 0, coef = 0, el = 0, er = 0;
+  DescBlob desc;
+};
+
+// rows i < n: T[i] samples at x_off[i], outputs at y_off[i]; the rows passed filter_row_check
+static int filter_route(const mmf_out_filter* f, int64_t n, const int64_t* x_off, const int64_t* T,
+                        const int64_t* y_off, FilterVarlen& v) {
+  const bool fir = f->kind == MMF_FILT_FIR;
+  const int64_t ext = fir ? 6 * (int64_t)f->n_taps : 0;
+  std::vector<FiltRow> rows((size_t)n);
+  std::vector<unsigned> fa((size_t)n + 1), fb((size_t)n + 1);
+  int64_t ia = 0, ib = 0, w = 0;
+  for (int64_t i = 0; i < n; ++i) {
+    rows[i] = FiltRow{(long)x_off[i], (long)T[i], (long)y_off[i], (long)w};
+    fa[i] = (unsigned)ia;
+    fb[i] = (unsigned)ib;
+    ia += (T[i] + ext + kFiltOut - 1) / kFiltOut;
+    ib += (T[i] + kFiltOut - 1) / kFiltOut;
+    w += T[i] + ext;
+    if (ia > 0x7fffffffLL) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 work items");
+  }
+  fa[n] = (unsigned)ia;
+  fb[n] = (unsigned)ib;
+  v.n_rows = n;
+  v.a = RaggedParts{v.desc.put(rows), v.desc.put(fa), ia};
+  if (fir) {
+    v.b = RaggedParts{v.a.clips, v.desc.put(fb), ib};
+    v.taps = v.desc.put(f->taps, (size_t)f->n_taps);
+    v.work = w;
+  } else {
+    v.coef = v.desc.put(f->coef, (size_t)(2 * f->half + 1));
+    const size_t ne = (size_t)f->n_edge * f->n_edge_in;
+    if (ne) {
+      v.el = v.desc.put(f->edge_l, ne);
+      v.er = v.desc.put(f->edge_r, ne);
+    }
+  }
+  return MMF_OK;
+}
+
+// The device half on `st`: d, v.desc on the device; work: v.work doubles (FIR)
+static int filter_run(const mmf_out_filter* f, const FilterVarlen& v, const unsigned char* d, const void* x,
+                      int x_is_f32, double* y, double* work, cudaStream_t st) {
+  const FiltRow* rows = (const FiltRow*)(d + v.a.clips);
+  if (f->kind == MMF_FILT_FIR) {
+    const cudaError_t e = fir_varlen_launch(x, x_is_f32, rows, (long)v.n_rows, (const unsigned*)(d + v.a.first),
+                                            (long)v.a.items, (const unsigned*)(d + v.b.first), (long)v.b.items,
+                                            (const double*)(d + v.taps), f->n_taps, work, y, st);
+    return e == cudaSuccess ? MMF_OK : cuda_fail(e, "fir kernels launch");
+  }
+  const bool edges = (size_t)f->n_edge * f->n_edge_in > 0;
+  const cudaError_t e = stencil_varlen_launch(x, x_is_f32, rows, (long)v.n_rows, (const unsigned*)(d + v.a.first),
+                                              (long)v.a.items, (const double*)(d + v.coef), f->half,
+                                              edges ? (const double*)(d + v.el) : nullptr,
+                                              edges ? (const double*)(d + v.er) : nullptr, f->n_edge, f->n_edge_in,
+                                              y, st);
+  return e == cudaSuccess ? MMF_OK : cuda_fail(e, "stencil_varlen_kernel launch");
+}
+
+// One ragged filter launch on `st` with descriptors uploaded; work: caller's FIR scratch, else the stream-ordered pool
+static int filter_uploaded(mmf_plan* plan, const mmf_out_filter* f, const FilterVarlen& v, const void* x,
+                           int x_is_f32, double* y, double* work, cudaStream_t st) {
+  return run_uploaded(plan, v.desc, st, [&](const unsigned char* d) {
+    double* pool = nullptr;
+    if (!work && v.work) MMF_CUDA(cudaMallocAsync((void**)&pool, (size_t)v.work * sizeof(double), st));
+    const int rc = filter_run(f, v, d, x, x_is_f32, y, work ? work : pool, st);
+    if (pool) cudaFreeAsync(pool, st);
+    return rc;
+  });
+}
+
 // One ragged envelope (RMS or Hilbert) on `st` over float32 x from the host descriptors of v (no output filter)
 static int rms_run(mmf_plan* plan, const float* x, const EnvelopeVarlen& v, float* out, cudaStream_t st) {
   return run_uploaded(plan, v.desc, st, [&](const unsigned char* d) {
@@ -2232,6 +2285,7 @@ struct PackedBatch {
   float* amp = nullptr;
   double* amp_filt = nullptr;
   bool resampled = false;
+  const mmf_out_filter* change_out = nullptr;  // the MFCC-change curve's 'fir' / 'sg' filter (NULL: none)
   size_t isz = pcm16 ? 2 : 4;  // bytes per sample as they cross PCIe
   // from the checks
   int64_t n_taps = 0;  // taps that go up with the descriptors: none unless some clip reads them
@@ -2246,7 +2300,8 @@ struct PackedBatch {
 // Byte offsets of a chunk's buffers in its slot of the host-path workspace, in the order they are laid out
 struct HostSlot {
   size_t h2d = 0, pcm = 0, tot = 0, mfcc = 0, delta = 0, mag = 0, band = 0;
-  size_t ptot = 0, pmfcc = 0, pdelta = 0, pmag = 0, pband = 0, scratch = 0, amp = 0, amp_filt = 0, end = 0;
+  size_t ptot = 0, pmfcc = 0, pdelta = 0, pmag = 0, pband = 0, scratch = 0, amp = 0, amp_filt = 0, ctot = 0,
+         cwork = 0, end = 0;
 };
 
 // per-clip row lengths (int) and packed offsets (long) of a compaction, in the call's descriptors
@@ -2263,7 +2318,8 @@ struct HostChunk {
   ChangeVarlen cv;
   ModspecVarlen mv;    // routed when the chunk has modulation windows (mv.W > 0)
   EnvelopeVarlen env;  // routed when the envelope is requested
-  size_t o_cv = 0, o_mv = 0, o_env = 0;  // cv.desc, mv.desc and env.desc in the call's descriptors
+  FilterVarlen fv;     // the change curve's output filter, over the padded [nc, pitch] rows (change_out only)
+  size_t o_cv = 0, o_mv = 0, o_env = 0, o_fv = 0;  // cv.desc, mv.desc, env.desc and fv.desc in the call's descriptors
   HostSlot slot;
 };
 
@@ -2285,6 +2341,11 @@ static int packed_check(const mmf_plan* plan, PackedBatch& b) {
       for (size_t i = 0; i < n; ++i)
         if (b.A[i + 1] - b.A[i] <= b.amp_sos.padlen) return too_short(b.amp_sos.padlen, (int64_t)i);
     }
+  }
+  if (b.change_out) {
+    if ((rc = filter_shape_check(b.change_out))) return rc;
+    if (b.prm && b.prm->out_kind != 1)
+      return fail(MMF_ERR_INVALID, "change_out needs prm->out_kind == 1 (the raw curve)");
   }
   if (!plan || !b.pcm || !b.prm || !b.tot) return fail(MMF_ERR_INVALID, "NULL argument");
   if ((b.mag || b.band) && !b.mod) return fail(MMF_ERR_INVALID, "modulation outputs requested without parameters");
@@ -2336,6 +2397,11 @@ static int route_chunk(const mmf_plan* plan, const PackedBatch& b, HostChunk& h,
   };
   h.frames = packed_rows(b.F);
   h.wins = packed_rows(b.Wo);
+  if (b.change_out) {
+    std::vector<int64_t> off((size_t)nc);
+    for (int64_t k = 0; k < nc; ++k) off[k] = k * h.cv.pitch;
+    if ((rc = filter_route(b.change_out, nc, off.data(), b.T.data() + c0, off.data(), h.fv))) return rc;
+  }
   const SosArgs* filt = b.amp_filt ? &b.amp_sos : nullptr;
   if (b.want_amp && b.env_prm->method == MMF_ENV_HILBERT)
     hilbert_env_route(c0, c1, b.offsets, b.offsets[c0], b.A.data(), filt, h.env);
@@ -2366,6 +2432,8 @@ static HostSlot layout_slot(const PackedBatch& b, const HostChunk& h, int nm) {
   s.scratch = ws_take(o, std::max(h.cv.bytes, mod_c ? h.mv.bytes : 0));
   s.amp = b.want_amp ? ws_take(o, (size_t)(b.A[h.c1] - b.A[h.c0]) * 4) : 0;
   s.amp_filt = b.amp_filt ? ws_take(o, (size_t)(b.A[h.c1] - b.A[h.c0]) * 8) : 0;
+  s.ctot = b.change_out ? ws_take(o, nc * pitch * 8) : 0;
+  s.cwork = b.change_out ? ws_take(o, (size_t)h.fv.work * 8) : 0;
   return s;
 }
 
@@ -2395,12 +2463,14 @@ static int plan_chunks(const mmf_plan* plan, const PackedBatch& b, std::vector<H
   }
   // then every chunk's stage descriptors (mostly chunk tables), copied once into one allocation
   size_t bytes = desc.size();
-  for (const HostChunk& h : chunks) bytes += 3 * kDescAlign + h.cv.desc.size() + h.mv.desc.size() + h.env.desc.size();
+  for (const HostChunk& h : chunks)
+    bytes += 4 * kDescAlign + h.cv.desc.size() + h.mv.desc.size() + h.env.desc.size() + h.fv.desc.size();
   desc.bytes.reserve(bytes);
   for (HostChunk& h : chunks) {
     h.o_cv = desc.put(h.cv.desc.bytes);
     h.o_mv = desc.put(h.mv.desc.bytes);
     h.o_env = desc.put(h.env.desc.bytes);
+    h.o_fv = desc.put(h.fv.desc.bytes);
   }
   slot = align_up(slot, 256);
   return MMF_OK;
@@ -2435,6 +2505,11 @@ static int run_chunk(mmf_plan* plan, const PackedBatch& b, const HostChunk& h, c
   if ((rc = change_varlen_run(plan, h.cv, base + s.scratch, dd + h.o_cv, d_pcm, h.stride, b.prm, d_tot, nullptr,
                               d_mfcc, d_delta, st)))
     return rc;
+  if (b.change_out) {  // the raw curves -> their own rows, which the compaction then reads
+    double* d_ctot = (double*)dev(s.ctot);
+    if ((rc = filter_run(b.change_out, h.fv, dd + h.o_fv, d_tot, 0, d_ctot, (double*)dev(s.cwork), st))) return rc;
+    d_tot = d_ctot;
+  }
   const bool mod_c = h.mv.W > 0;
   float* d_mag = mod_c && b.mag ? (float*)dev(s.mag) : nullptr;
   float* d_band = mod_c && b.nbe > 0 ? (float*)dev(s.band) : nullptr;
@@ -2477,6 +2552,9 @@ static int features_host_varlen_impl(mmf_plan* plan, PackedBatch b) {
   std::vector<HostChunk> chunks;
   size_t slot = 0;
   if ((rc = plan_chunks(plan, b, chunks, desc, slot))) return rc;
+  // the change curves' output filter: checked after every clip passed the change stage's own length checks
+  for (int64_t i = 0; b.change_out && i < b.n_clips; ++i)
+    if ((rc = filter_row_check(b.change_out, b.T[i], i))) return rc;
   MMF_CUDA(cudaSetDevice(plan->cfg.device));
   const size_t o_slots = align_up(desc.size(), 256);
   if ((rc = ensure_host_ws(plan, o_slots + 2 * slot))) return rc;
@@ -2542,15 +2620,27 @@ int mmf_features_host_varlen_pcm16(mmf_plan* plan, const int16_t* pcm16_host, in
                                                nullptr, nullptr, tot_host, mfcc_host, delta_host, mag_host, band_host});
 }
 
+int mmf_features_host_varlen_out(mmf_plan* plan, const void* pcm_host, int32_t pcm16, int64_t n_clips,
+                                 const int64_t* offsets_host, const mmf_resample_clip* rs_host, const float* h_host,
+                                 int64_t n_h, const mmf_change_params* prm, const mmf_modspec_params* mod,
+                                 const mmf_env_params* env, const int32_t* geom_host,
+                                 const mmf_out_filter* change_out, double* tot_host, float* mfcc_host,
+                                 float* delta_host, float* mag_host, float* band_host, float* amp_host,
+                                 double* amp_filt_host) {
+  return mmf::features_host_varlen_impl(plan, {pcm_host, pcm16 ? 1 : 0, n_clips, offsets_host, rs_host, h_host, n_h,
+                                               prm, mod, env, geom_host, tot_host, mfcc_host, delta_host, mag_host,
+                                               band_host, amp_host, amp_filt_host, rs_host != nullptr, change_out});
+}
+
 int mmf_features_host_varlen_env(mmf_plan* plan, const void* pcm_host, int32_t pcm16, int64_t n_clips,
                                  const int64_t* offsets_host, const mmf_resample_clip* rs_host, const float* h_host,
                                  int64_t n_h, const mmf_change_params* prm, const mmf_modspec_params* mod,
                                  const mmf_env_params* env, const int32_t* geom_host, double* tot_host,
                                  float* mfcc_host, float* delta_host, float* mag_host, float* band_host,
                                  float* amp_host, double* amp_filt_host) {
-  return mmf::features_host_varlen_impl(plan, {pcm_host, pcm16 ? 1 : 0, n_clips, offsets_host, rs_host, h_host, n_h,
-                                               prm, mod, env, geom_host, tot_host, mfcc_host, delta_host, mag_host,
-                                               band_host, amp_host, amp_filt_host, rs_host != nullptr});
+  return mmf_features_host_varlen_out(plan, pcm_host, pcm16, n_clips, offsets_host, rs_host, h_host, n_h, prm, mod,
+                                      env, geom_host, nullptr, tot_host, mfcc_host, delta_host, mag_host, band_host,
+                                      amp_host, amp_filt_host);
 }
 
 int mmf_features_host_varlen_amp(mmf_plan* plan, const void* pcm_host, int32_t pcm16, int64_t n_clips,
@@ -2722,6 +2812,74 @@ int mmf_resample_varlen(mmf_plan* plan, const float* x_dev, int64_t n_clips, con
   const RaggedParts p = resample_desc(0, n_clips, offsets_host, 0, rs_host, desc);
   if (p.items < 0) return fail(MMF_ERR_UNSUPPORTED, "more than 2^31 - 1 work items");
   return resample_dev(plan, x_dev, desc, p, h_host, n_taps, n_clips, y_dev, y_stride, (cudaStream_t)stream);
+}
+
+// the single-row-type calls: one descriptor per row of the ragged kernels (the 65 535-row limit is theirs)
+int mmf_fir_filtfilt(mmf_plan* plan, const double* x_dev, int64_t rows, int64_t T, const double* b_host,
+                     int32_t n_taps, double* y_dev, double* work_dev, void* stream) {
+  if (!plan || !x_dev || !b_host || !y_dev || !work_dev) return fail(MMF_ERR_INVALID, "NULL argument");
+  if (n_taps < 1 || n_taps > 4096) return fail(MMF_ERR_UNSUPPORTED, "n_taps must be in [1, 4096]");
+  if (rows < 1 || rows > 65535) return fail(MMF_ERR_UNSUPPORTED, "rows must be in [1, 65535]");
+  if (T <= 3 * n_taps) return too_short(3 * n_taps);
+  mmf_out_filter f{};
+  f.kind = MMF_FILT_FIR;
+  f.n_taps = n_taps;
+  f.taps = b_host;
+  std::vector<int64_t> off((size_t)rows), len((size_t)rows, T);
+  for (int64_t r = 0; r < rows; ++r) off[r] = r * T;
+  FilterVarlen v;
+  int rc = filter_route(&f, rows, off.data(), len.data(), off.data(), v);
+  if (rc) return rc;
+  // work_dev [rows, T + 6 * n_taps] is the forward pass's scratch, packed as filter_route packs it
+  return filter_uploaded(plan, &f, v, x_dev, 0, y_dev, work_dev, (cudaStream_t)stream);
+}
+
+int mmf_stencil(mmf_plan* plan, const double* x_dev, int64_t rows, int64_t T, const double* coef_host, int32_t half,
+                const double* edge_l_host, const double* edge_r_host, int32_t n_edge, int32_t n_edge_in,
+                double* y_dev, void* stream) {
+  if (!plan || !x_dev || !coef_host || !y_dev) return fail(MMF_ERR_INVALID, "NULL argument");
+  if (half < 0 || n_edge < half || n_edge_in < 0) return fail(MMF_ERR_INVALID, "need n_edge >= half >= 0");
+  if (n_edge > 0 && (!edge_l_host || !edge_r_host)) return fail(MMF_ERR_INVALID, "edge matrices are NULL");
+  if (T < n_edge_in || T < 2 * n_edge) return fail(MMF_ERR_TOO_SHORT, "input shorter than the stencil's edge window");
+  if (rows < 1 || rows > 65535) return fail(MMF_ERR_UNSUPPORTED, "rows must be in [1, 65535]");
+  if (T < 1) return fail(MMF_ERR_INVALID, "T must be positive");
+  mmf_out_filter f{};
+  f.kind = MMF_FILT_SG;
+  f.half = half;
+  f.coef = coef_host;
+  f.n_edge = n_edge;
+  f.n_edge_in = n_edge_in;
+  f.edge_l = edge_l_host;
+  f.edge_r = edge_r_host;
+  std::vector<int64_t> off((size_t)rows), len((size_t)rows, T);
+  for (int64_t r = 0; r < rows; ++r) off[r] = r * T;
+  FilterVarlen v;
+  int rc = filter_route(&f, rows, off.data(), len.data(), off.data(), v);
+  if (rc) return rc;
+  return filter_uploaded(plan, &f, v, x_dev, 0, y_dev, nullptr, (cudaStream_t)stream);
+}
+
+int mmf_filter_varlen_check(const mmf_out_filter* filt, int64_t n_rows, const int64_t* T_host) {
+  int rc = filter_shape_check(filt);
+  if (rc) return rc;
+  if (n_rows < 1) return fail(MMF_ERR_INVALID, "n_rows must be positive");
+  if (!T_host) return fail(MMF_ERR_INVALID, "T_host is NULL");
+  for (int64_t i = 0; i < n_rows; ++i) {
+    if (T_host[i] < 1) return fail(MMF_ERR_INVALID, "clip " + std::to_string(i) + ": T must be positive");
+    if ((rc = filter_row_check(filt, T_host[i], i))) return rc;
+  }
+  return MMF_OK;
+}
+
+int mmf_filter_varlen(mmf_plan* plan, const mmf_out_filter* filt, const void* x_dev, int32_t x_is_f32, int64_t n_rows,
+                      const int64_t* x_off_host, const int64_t* T_host, double* y_dev, const int64_t* y_off_host,
+                      void* stream) {
+  int rc = mmf_filter_varlen_check(filt, n_rows, T_host);
+  if (rc) return rc;
+  if (!plan || !x_dev || !y_dev || !x_off_host || !y_off_host) return fail(MMF_ERR_INVALID, "NULL argument");
+  FilterVarlen v;
+  if ((rc = filter_route(filt, n_rows, x_off_host, T_host, y_off_host, v))) return rc;
+  return filter_uploaded(plan, filt, v, x_dev, x_is_f32 ? 1 : 0, y_dev, nullptr, (cudaStream_t)stream);
 }
 
 // one descriptor per row of the ragged kernel (rows of equal length: the grid has no row limit)

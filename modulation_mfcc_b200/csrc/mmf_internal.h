@@ -236,10 +236,24 @@ cudaError_t varlen_tails_launch(long n_clips, const int* T, int pitch, double* t
                                 float* mfcc, float* delta, int n_mfcc, cudaStream_t st);
 cudaError_t delta_norm_launch(const double* x, long n_clips, int rows, long T, int method, double* tot,
                               cudaStream_t st);
-cudaError_t fir_filtfilt_launch(const double* x, long rows, long T, const double* b_dev, int n_taps, double* y,
-                                double* work, cudaStream_t st);
-cudaError_t stencil_launch(const double* x, long rows, long T, const double* coef_dev, int half, const double* el_dev,
-                           const double* er_dev, int n_edge, int n_edge_in, double* y, cudaStream_t st);
+// One row of a ragged output-filter launch (device descriptor, built on the host): T samples at x + x (float64, or
+// float32 widened on load), T outputs written at y + y; the FIR's forward pass writes its T + 6 * n_taps samples at
+// work + w.  A work item is kFiltOut consecutive outputs of one row; row r owns items [first[r], first[r + 1]).
+struct FiltRow {
+  long x, T, y, w;
+};
+constexpr int kFiltOut = 256;
+// scipy.signal.filtfilt(b, 1, x) of each row: the forward pass over the odd-extended row into work (work list
+// first_fwd, ceil((T + 6 * n_taps) / kFiltOut) items per row), then the backward pass into y (first_bwd, ceil(T /
+// kFiltOut) items per row).  Two launches.
+cudaError_t fir_varlen_launch(const void* x, int x_is_f32, const FiltRow* rows, long n_rows, const unsigned* first_fwd,
+                              long n_fwd, const unsigned* first_bwd, long n_bwd, const double* b, int n_taps,
+                              double* work, double* y, cudaStream_t st);
+// Banded stencil with dense edge rows (coef[2 * half + 1]; edge_l, edge_r [n_edge, n_edge_in]) of each row.  One launch.
+cudaError_t stencil_varlen_launch(const void* x, int x_is_f32, const FiltRow* rows, long n_rows,
+                                  const unsigned* first_item, long n_items, const double* coef, int half,
+                                  const double* el, const double* er, int n_edge, int n_edge_in, double* y,
+                                  cudaStream_t st);
 cudaError_t modspec_launch(const float* mfcc, long n_clips, int n_coef, long T, int win, int hop, int nfft, float* mag,
                            float* band, const int* band_lo_dev, const int* band_hi_dev, int n_bands, cudaStream_t st);
 cudaError_t modspec_tails_launch(long n_clips, const int* n_win, long W, float* mag, int n_coef, int nb, float* band,

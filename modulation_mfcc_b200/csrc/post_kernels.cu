@@ -774,83 +774,128 @@ cudaError_t delta_norm_launch(const double* x, long n_clips, int rows, long T, i
 }
 
 // ---------------------------------------------------------------------------
-// scipy.signal.filtfilt(b, 1, x): zero-phase FIR.  With a == 1 the lfilter
-// initial state zi*x[0] is "the past was constantly x[0]", so each pass is a
-// plain convolution over the odd-extended signal with a constant extension
-// beyond its first sample -- no recurrence, one thread per output.
+// The 'fir' and 'sg' output filters (applyFilter, script/mfcc.py:113-131), ragged: one launch covers rows of any
+// lengths, each a FiltRow, driven by a flat work list (a work item is kFiltOut consecutive outputs of one row, one per
+// thread; row r owns items [first_item[r], first_item[r + 1]) and each CTA finds its row by binary search).  Rows are
+// float64 or float32; float32 is widened on load, which is exact, so a row's outputs do not depend on its input type.
+// Every output is one fma chain in a fixed order, the same whatever batch, layout or item the row lands in.
 // ---------------------------------------------------------------------------
-__device__ __forceinline__ double odd_ext_at(const double* xr, long T, int p, long i) {
-  if (i < p) return 2.0 * xr[0] - xr[p - i];
-  if (i < p + T) return xr[i - p];
-  return 2.0 * xr[T - 1] - xr[T - 2 - (i - p - T)];
+__device__ __forceinline__ long filt_row_of(const unsigned* __restrict__ first_item, long n_rows, unsigned item) {
+  long r = 0, hi = n_rows - 1;  // the last row with first_item[r] <= item
+  while (r < hi) {
+    const long mid = (r + hi + 1) >> 1;
+    if (first_item[mid] <= item) r = mid;
+    else hi = mid - 1;
+  }
+  return r;
 }
 
-__global__ void fir_fwd_kernel(const double* __restrict__ x, long T, int p, const double* __restrict__ b, int n_taps,
-                               double* __restrict__ work) {
-  const long L = T + 2L * p;
-  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+// scipy.signal.filtfilt(b, 1, x): zero-phase FIR.  With a == 1 the lfilter initial state zi*x[0] is "the past was
+// constantly x[0]", so each pass is a plain convolution over the odd-extended signal (p = 3 * n_taps samples at each
+// end) with a constant extension before its first sample: no recurrence, one thread per output.  The forward pass
+// writes the T + 2p extended outputs of a row to scratch (FiltRow::w), the backward pass reads them from the end.
+template <typename X>
+__device__ __forceinline__ double odd_ext_at(const X* xr, long T, int p, long i) {
+  if (i < p) return 2.0 * (double)xr[0] - (double)xr[p - i];
+  if (i < p + T) return (double)xr[i - p];
+  return 2.0 * (double)xr[T - 1] - (double)xr[T - 2 - (i - p - T)];
+}
+
+template <typename X>
+__global__ void __launch_bounds__(kFiltOut) fir_fwd_varlen_kernel(const X* __restrict__ x,
+                                                                  const FiltRow* __restrict__ rows,
+                                                                  const unsigned* __restrict__ first_item,
+                                                                  long n_rows, const double* __restrict__ b,
+                                                                  int n_taps, double* __restrict__ work) {
+  const long r = filt_row_of(first_item, n_rows, blockIdx.x);
+  const FiltRow c = rows[r];
+  const int p = 3 * n_taps;
+  const long L = c.T + 2L * p;
+  const long i = (long)(blockIdx.x - first_item[r]) * kFiltOut + threadIdx.x;
   if (i >= L) return;
-  const double* xr = x + (size_t)blockIdx.y * T;
+  const X* xr = x + c.x;
   double acc = 0.0;
   for (int j = n_taps - 1; j >= 0; --j) {
     const long m = i - j;
-    acc = fma(b[j], odd_ext_at(xr, T, p, m < 0 ? 0 : m), acc);
+    acc = fma(b[j], odd_ext_at(xr, c.T, p, m < 0 ? 0 : m), acc);
   }
-  work[(size_t)blockIdx.y * L + i] = acc;
+  work[c.w + i] = acc;
 }
 
-__global__ void fir_bwd_kernel(const double* __restrict__ work, long T, int p, const double* __restrict__ b,
-                               int n_taps, double* __restrict__ y) {
-  const long L = T + 2L * p;
-  const long n = (long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (n >= T) return;
-  const double* w = work + (size_t)blockIdx.y * L;
+__global__ void __launch_bounds__(kFiltOut) fir_bwd_varlen_kernel(const double* __restrict__ work,
+                                                                  const FiltRow* __restrict__ rows,
+                                                                  const unsigned* __restrict__ first_item,
+                                                                  long n_rows, const double* __restrict__ b,
+                                                                  int n_taps, double* __restrict__ y) {
+  const long r = filt_row_of(first_item, n_rows, blockIdx.x);
+  const FiltRow c = rows[r];
+  const int p = 3 * n_taps;
+  const long L = c.T + 2L * p;
+  const long n = (long)(blockIdx.x - first_item[r]) * kFiltOut + threadIdx.x;
+  if (n >= c.T) return;
+  const double* w = work + c.w;
   const long i = n + p;
   double acc = 0.0;
   for (int j = n_taps - 1; j >= 0; --j) {
     const long m = i + j;
     acc = fma(b[j], w[m >= L ? L - 1 : m], acc);
   }
-  y[(size_t)blockIdx.y * T + n] = acc;
+  y[c.y + n] = acc;
 }
 
-cudaError_t fir_filtfilt_launch(const double* x, long rows, long T, const double* b_dev, int n_taps, double* y,
-                                double* work, cudaStream_t st) {
-  const int p = 3 * n_taps;
-  const long L = T + 2L * p;
-  dim3 g1((unsigned)((L + 255) / 256), (unsigned)rows), g2((unsigned)((T + 255) / 256), (unsigned)rows);
-  fir_fwd_kernel<<<g1, 256, 0, st>>>(x, T, p, b_dev, n_taps, work);
-  fir_bwd_kernel<<<g2, 256, 0, st>>>(work, T, p, b_dev, n_taps, y);
+cudaError_t fir_varlen_launch(const void* x, int x_is_f32, const FiltRow* rows, long n_rows, const unsigned* first_fwd,
+                              long n_fwd, const unsigned* first_bwd, long n_bwd, const double* b, int n_taps,
+                              double* work, double* y, cudaStream_t st) {
+  if (x_is_f32)
+    fir_fwd_varlen_kernel<<<(unsigned)n_fwd, kFiltOut, 0, st>>>((const float*)x, rows, first_fwd, n_rows, b, n_taps,
+                                                                 work);
+  else
+    fir_fwd_varlen_kernel<<<(unsigned)n_fwd, kFiltOut, 0, st>>>((const double*)x, rows, first_fwd, n_rows, b, n_taps,
+                                                                 work);
+  fir_bwd_varlen_kernel<<<(unsigned)n_bwd, kFiltOut, 0, st>>>(work, rows, first_bwd, n_rows, b, n_taps, y);
   count_launch(2);
   return cudaGetLastError();
 }
 
-// ---------------------------------------------------------------------------
-// Banded stencil with dense boundary rows (np.gradient / savgol 'interp' /
-// findiff; script/calc.py:635-645, script/mfcc.py:130).
-// ---------------------------------------------------------------------------
-__global__ void stencil_kernel(const double* __restrict__ x, long T, const double* __restrict__ coef, int half,
-                               const double* __restrict__ el, const double* __restrict__ er, int n_edge,
-                               int n_edge_in, double* __restrict__ y) {
-  const long t = (long)blockIdx.x * blockDim.x + threadIdx.x;
+// Banded stencil with dense boundary rows (np.gradient / savgol 'interp' / findiff; script/calc.py:635-645,
+// script/mfcc.py:130): the first and last n_edge outputs are edge_l / edge_r applied to the first / last n_edge_in
+// inputs, the others coef applied to inputs t - half .. t + half.
+template <typename X>
+__global__ void __launch_bounds__(kFiltOut) stencil_varlen_kernel(const X* __restrict__ x,
+                                                                  const FiltRow* __restrict__ rows,
+                                                                  const unsigned* __restrict__ first_item,
+                                                                  long n_rows, const double* __restrict__ coef,
+                                                                  int half, const double* __restrict__ el,
+                                                                  const double* __restrict__ er, int n_edge,
+                                                                  int n_edge_in, double* __restrict__ y) {
+  const long r = filt_row_of(first_item, n_rows, blockIdx.x);
+  const FiltRow c = rows[r];
+  const long T = c.T;
+  const long t = (long)(blockIdx.x - first_item[r]) * kFiltOut + threadIdx.x;
   if (t >= T) return;
-  const double* xr = x + (size_t)blockIdx.y * T;
+  const X* xr = x + c.x;
   double acc = 0.0;
   if (t < n_edge) {
-    for (int i = 0; i < n_edge_in; ++i) acc = fma(el[t * n_edge_in + i], xr[i], acc);
+    for (int i = 0; i < n_edge_in; ++i) acc = fma(el[t * n_edge_in + i], (double)xr[i], acc);
   } else if (t >= T - n_edge) {
     const long q = t - (T - n_edge);
-    for (int i = 0; i < n_edge_in; ++i) acc = fma(er[q * n_edge_in + i], xr[T - n_edge_in + i], acc);
+    for (int i = 0; i < n_edge_in; ++i) acc = fma(er[q * n_edge_in + i], (double)xr[T - n_edge_in + i], acc);
   } else {
-    for (int o = -half; o <= half; ++o) acc = fma(coef[o + half], xr[t + o], acc);
+    for (int o = -half; o <= half; ++o) acc = fma(coef[o + half], (double)xr[t + o], acc);
   }
-  y[(size_t)blockIdx.y * T + t] = acc;
+  y[c.y + t] = acc;
 }
 
-cudaError_t stencil_launch(const double* x, long rows, long T, const double* coef_dev, int half, const double* el_dev,
-                           const double* er_dev, int n_edge, int n_edge_in, double* y, cudaStream_t st) {
-  dim3 grid((unsigned)((T + 255) / 256), (unsigned)rows);
-  stencil_kernel<<<grid, 256, 0, st>>>(x, T, coef_dev, half, el_dev, er_dev, n_edge, n_edge_in, y);
+cudaError_t stencil_varlen_launch(const void* x, int x_is_f32, const FiltRow* rows, long n_rows,
+                                  const unsigned* first_item, long n_items, const double* coef, int half,
+                                  const double* el, const double* er, int n_edge, int n_edge_in, double* y,
+                                  cudaStream_t st) {
+  if (x_is_f32)
+    stencil_varlen_kernel<<<(unsigned)n_items, kFiltOut, 0, st>>>((const float*)x, rows, first_item, n_rows, coef,
+                                                                   half, el, er, n_edge, n_edge_in, y);
+  else
+    stencil_varlen_kernel<<<(unsigned)n_items, kFiltOut, 0, st>>>((const double*)x, rows, first_item, n_rows, coef,
+                                                                   half, el, er, n_edge, n_edge_in, y);
   count_launch();
   return cudaGetLastError();
 }

@@ -16,7 +16,16 @@ from dataclasses import dataclass, replace
 import numpy as np
 
 from . import _lib
-from ._lib import MmfError, check, mmf_amp_params, mmf_change_params, mmf_config, mmf_env_params, mmf_modspec_params
+from ._lib import (
+    MmfError,
+    check,
+    mmf_amp_params,
+    mmf_change_params,
+    mmf_config,
+    mmf_env_params,
+    mmf_modspec_params,
+    mmf_out_filter,
+)
 
 
 @dataclass(frozen=True)
@@ -403,6 +412,41 @@ class Plan:
                 n_edge_in,
                 y.data_ptr(),
                 _stream_ptr(self.device),
+            )
+        )
+        return y
+
+    def filter_varlen(self, x, offsets_or_lengths, filt: "OutFilter"):
+        """The output filter ``filt`` (:func:`fir_filter` / :func:`stencil_filter`) over rows of any lengths, in a
+        fixed number of launches (``mmf_filter_varlen``).  ``x`` is a float64 or float32 device tensor: 1-D packed,
+        row ``i`` being ``x[offsets[i]:offsets[i + 1]]`` (``offsets_or_lengths`` holds ``B + 1`` offsets), or 2-D
+        ``[B, T_max]`` padded, row ``i`` being ``x[i, :lengths[i]]`` (``B`` lengths).  Returns float64 in the same
+        layout (the padding is 0); each row equals :meth:`fir_filtfilt` / :meth:`stencil` on that row
+        alone, bit for bit."""
+        torch = _torch()
+        if x.dtype not in (torch.float32, torch.float64):
+            x = x.to(torch.float64)
+        x = x.contiguous()
+        v = np.ascontiguousarray(np.asarray(offsets_or_lengths, dtype=np.int64).reshape(-1))
+        if x.dim() == 1:
+            if v.shape[0] < 2:
+                raise ValueError("offsets needs at least two entries")
+            x_off, T = np.ascontiguousarray(v[:-1]), np.ascontiguousarray(np.diff(v))
+            if v[-1] > x.shape[0] or v[0] < 0 or np.any(T < 0):
+                raise ValueError("offsets must be non-decreasing and within the buffer")
+        elif x.dim() == 2:
+            if v.shape[0] != x.shape[0]:
+                raise ValueError(f"{v.shape[0]} lengths for {x.shape[0]} rows")
+            if np.any(v > x.shape[1]):
+                raise ValueError(f"a length exceeds the row length {x.shape[1]}")
+            x_off, T = np.arange(x.shape[0], dtype=np.int64) * x.shape[1], v
+        else:
+            raise ValueError("filter_varlen takes a 1-D packed or a 2-D padded tensor")
+        y = torch.zeros(x.shape, device=self.device, dtype=torch.float64)
+        check(
+            _lib.lib().mmf_filter_varlen(
+                self._h, C.byref(filt.c), x.data_ptr(), 1 if x.dtype == torch.float32 else 0, T.shape[0],
+                x_off.ctypes.data, T.ctypes.data, y.data_ptr(), x_off.ctypes.data, _stream_ptr(self.device),
             )
         )
         return y
@@ -799,7 +843,8 @@ class Plan:
         return out
 
     def features_host_varlen(self, pcm_host: np.ndarray, offsets, prm: mmf_change_params, mod=None, *,
-                             want=("totChange",), out=None, rates=None, amp=None, amp_method="RMS"):
+                             want=("totChange",), out=None, rates=None, amp=None, amp_method="RMS",
+                             change_out=None):
         """:meth:`features_host` for clips of different lengths packed back to back in one host buffer.
 
         ``pcm_host`` is 1-D float32 or int16 (raw WAV samples, scaled by 1/32768 on the device); clip ``i`` is
@@ -820,7 +865,10 @@ class Plan:
         zero-phase ``out_sos`` when one is given, packed at ``amp_offsets`` (int64 ``[B + 1]``).  Clip ``i``'s block
         equals :meth:`rms` (then :meth:`sosfiltfilt`) on that clip alone, bit for bit.  ``amp_method="Hilb"``: the
         Hilbert envelope instead, one value per native sample (``geom`` and ``center`` are not read), equal to
-        :meth:`hilbert_envelope` (then :meth:`sosfiltfilt`) on that clip alone, bit for bit."""
+        :meth:`hilbert_envelope` (then :meth:`sosfiltfilt`) on that clip alone, bit for bit.
+
+        ``change_out``: an :class:`OutFilter` run over each raw change curve (``prm`` must ask for the raw curve,
+        ``out_sos=None``); clip ``i``'s ``totChange`` then equals :meth:`filter_varlen` on its raw curve alone."""
         pcm_host = np.asarray(pcm_host)
         pcm16 = pcm_host.dtype == np.int16
         if not pcm16 and pcm_host.dtype != np.float32:
@@ -889,9 +937,10 @@ class Plan:
             amp_p = C.byref(env)
             a_p, af_p = (None, a.ctypes.data) if out_sos is not None else (a.ctypes.data, None)
         check(
-            _lib.lib().mmf_features_host_varlen_env(
+            _lib.lib().mmf_features_host_varlen_out(
                 self._h, pcm_host.ctypes.data, 1 if pcm16 else 0, B, offs.ctypes.data, rs_p, h_p, n_h,
                 C.byref(prm), C.byref(mp) if mp is not None else None, amp_p, geom_p,
+                C.byref(change_out.c) if change_out is not None else None,
                 ptr["totChange"], ptr["mfcc"], ptr["delta"], ptr["modspec"], ptr["band_energy"], a_p, af_p,
             )
         )
@@ -979,6 +1028,44 @@ def make_amp_params(center: bool, out_sos=None) -> mmf_amp_params:
 
 
 AMP_METHODS = {"RMS": _lib.MMF_ENV_RMS, "Hilb": _lib.MMF_ENV_HILBERT}
+
+
+class OutFilter:
+    """A 'fir' or 'sg' output filter as the library takes it (``mmf_out_filter``), holding its host coefficients.
+    Build one with :func:`fir_filter` or :func:`stencil_filter`."""
+
+    def __init__(self, kind: int, arrays):
+        self.kind, self.arrays = kind, arrays  # the arrays stay alive as long as the struct that points at them
+        self.c = mmf_out_filter()
+        self.c.kind = kind
+
+    def check(self, lengths) -> None:
+        """The library's checks for rows of ``lengths`` samples, without a device (``mmf_filter_varlen_check``)."""
+        T = np.ascontiguousarray(np.asarray(lengths, dtype=np.int64).reshape(-1))
+        check(_lib.lib().mmf_filter_varlen_check(C.byref(self.c), T.shape[0], T.ctypes.data))
+
+
+def fir_filter(b) -> OutFilter:
+    """scipy.signal.filtfilt(b, 1, x) (applyFilter's 'fir', script/mfcc.py:126)."""
+    b = np.ascontiguousarray(b, dtype=np.float64).reshape(-1)
+    f = OutFilter(_lib.MMF_FILT_FIR, (b,))
+    f.c.n_taps, f.c.taps = b.shape[0], b.ctypes.data
+    return f
+
+
+def stencil_filter(coef, edge_l, edge_r) -> OutFilter:
+    """A banded stencil with dense edge rows, as :meth:`Plan.stencil` takes it (applyFilter's 'sg', np.gradient,
+    findiff)."""
+    coef = np.ascontiguousarray(coef, dtype=np.float64).reshape(-1)
+    edge_l = np.ascontiguousarray(edge_l, dtype=np.float64)
+    edge_r = np.ascontiguousarray(edge_r, dtype=np.float64)
+    f = OutFilter(_lib.MMF_FILT_SG, (coef, edge_l, edge_r))
+    n_edge, n_edge_in = edge_l.shape if edge_l.size else (0, 0)
+    f.c.half, f.c.coef = (coef.shape[0] - 1) // 2, coef.ctypes.data
+    f.c.n_edge, f.c.n_edge_in = n_edge, n_edge_in
+    f.c.edge_l = edge_l.ctypes.data if n_edge else None
+    f.c.edge_r = edge_r.ctypes.data if n_edge else None
+    return f
 
 
 def make_env_params(method: str = "RMS", center: bool = True, out_sos=None) -> mmf_env_params:

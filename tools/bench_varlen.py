@@ -38,11 +38,19 @@ mmf_hilbert_envelope launches, so the leg can time an older tree too), as CUDA-e
 torch.profiler.  Where the tree has it, it then times host_varlen(want=every output) on the resample leg's int16
 44.1 kHz corpus (with rates=) without the envelope and with amp_method='Hilb', raw and with the 'iir' output filter.
 
+The outfilter leg times the 'fir' (21 taps, 10 Hz) and 'sg' (11 points, order 3) output filters on the 100 Hz curves
+and envelopes of the 16 kHz float32 corpus: get_MFCCS_change_many at the bench's frame geometry and
+calculate_amplitude_envelope_many (RMS), each also without an output filter, so that the difference is the filter's
+cost (a per-clip loop in a tree without mmf_filter_varlen, one ragged call with it).  Where FeatureExtractor takes
+outFilter, it then times host_varlen(want=every output) on the resample leg's int16 44.1 kHz corpus (with rates=)
+with outFilter None, 'iir' (12 Hz, order 6), 'fir' and 'sg'.
+
 Workload: 1024 clips at 16 kHz with the bench's frame geometry (win 400 / hop 160 / n_fft 512, 40 mel, 13 MFCC,
 gradient, Butterworth output filter), lengths uniform in [2 s, 20 s] from a fixed seed.  Prints, per leg, the median
 ms of each way and audio-seconds per second as one JSON line, with the GPU's name and power limit.
 
-    python tools/bench_varlen.py [--clips 1024] [--iters 10] [--loop-iters 3] [--legs change,features,host,resample,amplitude,hilbert]
+    python tools/bench_varlen.py [--clips 1024] [--iters 10] [--loop-iters 3]
+                                 [--legs change,features,host,resample,amplitude,hilbert,outfilter]
 """
 import argparse
 import json
@@ -311,6 +319,48 @@ def _hilbert_leg(pcm, lengths16, n_clips, iters, seed, power_limit, dev):
     print(json.dumps(res), flush=True)
 
 
+OUT_FILTERS = {
+    "fir": dict(outFilter="fir", outFiltCutOff=[10], outFiltLen=21),
+    "sg": dict(outFilter="sg", outFiltCutOff=[12], outFiltLen=11, outFiltPolyOrd=3),
+}
+
+
+def _outfilter_leg(pcm, lengths, n_clips, iters, seed, power_limit, dev):
+    """The 'fir' and 'sg' output filters; see the module docstring."""
+    sr = 16000
+    host = pcm.cpu().numpy()
+    clips = [host[i, :n] for i, n in enumerate(lengths)]
+    res = {"leg": "outfilter", "corpus": "float32_16k", "gpu": torch.cuda.get_device_name(dev),
+           "power_limit": power_limit, "clips": len(clips), "audio_s": sum(lengths) / sr}
+    geom = dict(tStep=0.01, winLen=0.025, n_fft=512, n_mels=40, n_mfcc=13, minFreq=0.0, maxFreq=8000.0, device=0)
+    for k, kw in (("none", dict(outFilter=None)), *OUT_FILTERS.items()):
+        change = lambda kw=kw: mm.get_MFCCS_change_many(clips, sr, **geom, **kw)  # noqa: E731
+        env = lambda kw=kw: mm.calculate_amplitude_envelope_many(clips, sr, device=0, **kw)  # noqa: E731
+        for name, fn in (("change_many", change), ("envelope_many", env)):
+            fn()
+            res[f"{name}_{k}_ms"] = _median_host_ms(fn, iters)
+    print(json.dumps(res), flush=True)
+    try:
+        mm.FeatureExtractor(16000, device=0, **OUT_FILTERS["fir"])
+    except TypeError:  # a tree whose FeatureExtractor takes no output filter
+        return
+    want = ("totChange", "mfcc", "delta", "modspec", "band_energy")
+    sr_in = 44100
+    packed, offs44, _ = _int16_corpus(n_clips, seed, sr_in)
+    rates = [sr_in] * n_clips
+    res = {"leg": "outfilter_bundle", "corpus": "int16_44k_rates", "gpu": torch.cuda.get_device_name(dev),
+           "power_limit": power_limit, "clips": n_clips, "audio_s": float(offs44[-1]) / sr_in}
+    settings = {"none": {}, "iir": dict(outFilter="iir", outFiltCutOff=[12], outFiltLen=6), **OUT_FILTERS}
+    for k, kw in settings.items():
+        fx = mm.FeatureExtractor(16000, device=0, **kw)
+        out = {key: _pinned(v.shape, v.dtype.type) for key, v in fx.host_varlen(packed, offs44, want=want,
+                                                                               rates=rates).items() if key in want}
+        call = lambda fx=fx, out=out: fx.host_varlen(packed, offs44, want=want, out=out, rates=rates)  # noqa: E731
+        res[f"host_varlen_{k}_ms"] = _median_host_ms(call, iters)
+        res[f"host_varlen_{k}_audio_s_per_s"] = res["audio_s"] / (res[f"host_varlen_{k}_ms"] / 1e3)
+    print(json.dumps(res), flush=True)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--clips", type=int, default=1024)
@@ -366,6 +416,9 @@ def main():
             continue
         if leg == "hilbert":
             _hilbert_leg(pcm, lengths, a.clips, a.iters, a.seed, power_limit, dev)
+            continue
+        if leg == "outfilter":
+            _outfilter_leg(pcm, lengths, a.clips, a.iters, a.seed, power_limit, dev)
             continue
         varlen, loop, pad = ways[leg]
         for fn in (varlen, pad, loop):  # warm-up: modules, workspace growth
